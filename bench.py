@@ -3,7 +3,7 @@
 per-control-step plan latency).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg4|cfg3|cfg1]
-                    [--scaling strong|weak] [--no-extra] [--no-cpu-baseline]
+                    [--scaling strong|weak] [--no-extra] [--no-cpu-baseline] [--dump-outputs DIR]
 
 One "step" = one MPPI control step (``MPPIDelay.command``): K x H Neural Laplace rollout-steps.
 
@@ -27,6 +27,10 @@ sample index.
 * ``extra``    - (N = 1) the other BASELINE configs in the same run: config 1 and 3 plans (latency, fill factor), the
                  config 2 Fourier-ILT microbenchmark (GB/s against the measured HBM peak, S = 33 / 65 / 129) and config 5
                  (32 closed-loop instances per GPU, instance-batched).
+
+``--dump-outputs DIR`` writes, after the headline's timed steps (``value``, then ``e2e``), what the last of them left the
+caller (``dump_outputs``) as ``DIR/<name>.npy``.  The inputs depend on the arguments only, so two builds run with the
+same arguments can be compared array by array.
 """
 from __future__ import annotations
 
@@ -60,6 +64,7 @@ HOISTED_FLOP = {"oderl-pendulum": 307712, "oderl-cartpole": 325632, "oderl-acrob
 ENCODER_FLOP = 2 * 10 * 192 * 64  # ten 64x192 products per window: the hoisted GRU work (+ a 2x64 output layer)
 METRIC, UNIT = "mppi_rollout_steps_per_sec", "rollout-steps/s"
 N_SM = 148
+DUMP_SAMPLES = 4096  # per-sample trajectories kept by --dump-outputs: all of config 4's would be 130 MB
 
 
 def load_peaks():
@@ -328,6 +333,27 @@ def time_plan(ctx, env, K, H, group, steps, warmup, S=None, math=None):
     _, ms_e2e, _ = ctx.timed(e2e_step, steps, warmup)
     return {"ms_dev": ms_dev, "ms_e2e": ms_e2e, "launches": launches, "inp": inp, "model": model, "planner": planner,
             "state_dev": state_dev, "buf_dev": buf_dev}
+
+
+def dump_outputs(out_dir, planner):
+    """What the planner's last control step left its caller, as float32 ``out_dir/<name>.npy``: the action, the updated plan
+    ``U``, every sample's ``cost_total`` and ``omega``, and ``states``, ``perturbed_action`` and ``noise`` of DUMP_SAMPLES
+    samples drawn with a fixed seed.  Sharded plans: this rank's samples."""
+    import numpy as np
+    import torch
+
+    from neurallaplacecontrol_b200 import _lib
+
+    torch.cuda.synchronize()
+    Kl = planner.K_local
+    rows = np.sort(np.random.default_rng(0).choice(Kl, size=min(DUMP_SAMPLES, Kl), replace=False))
+    rows = torch.from_numpy(rows).to(planner.d)
+    out = {"action": planner._buf(_lib.BUF_ACTION, (planner.nu,)), "U": planner.U, "cost_total": planner.cost_total,
+           "omega": planner.omega, "states": planner.states[rows], "perturbed_action": planner.perturbed_action[rows],
+           "noise": planner.noise[rows]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def kernels_alone(ctx, r, env, H, steps):
@@ -609,6 +635,8 @@ def run_gpu(args, env, K, H, desc):
         sampler.start()
     head = time_plan(ctx, env, K_head, H, ctx.group, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, head["planner"])  # before kernels_alone reuses the planner's buffers
     ms_enc, ms_roll = kernels_alone(ctx, head, env, H, args.steps)
     split = in_step_split(ctx, head, args.steps)
     other = None
@@ -688,7 +716,12 @@ def main():
     ap.add_argument("--idle", type=float, default=1.0, help="seconds of idle before every timed region (equal power state for every number of the line)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the config 1/2/3/5 extras (N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the headline's last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl b200)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     env, K, H, desc = WORKLOADS[args.workload]

@@ -44,6 +44,14 @@ def test_reference_arm_prints_one_contract_line():
     assert d["value"] > 0 and d["config"]["workload"].startswith("oderl Pendulum")
 
 
+def test_rejects_zero_steps_and_dump_outputs_of_the_cpu_arm(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "out")]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120,
+                             cwd=ROOT)
+        assert out.returncode == 2 and out.stdout == "", (extra, out.stderr[-2000:])
+    assert not (tmp_path / "out").exists()
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "1"],
