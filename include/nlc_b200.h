@@ -119,6 +119,25 @@ int nlc_model_forward(nlc_model_t m, const float* obs_dev, const float* act_dev,
 int nlc_model_forward_ts(nlc_model_t m, const float* obs_dev, const float* act_dev, const float* ts_dev,
                          int K, int B, float* out_dev, float* scratch_dev /* [K][132] floats */, int math_mode, void* stream);
 
+/* Gradients of NeuralLaplaceModel.forward with per-sample prediction times (train_utils.py:388-407 loss.backward()).
+ * obs_dev, act_dev, ts_dev, K, B as in nlc_model_forward_ts; grad_out_dev [K][nx] is dLoss/d(out).
+ * grad_params_dev: nlc_model_grad_floats(desc) floats, OVERWRITTEN, the 16 parameters in named_parameters() order, each
+ * in its state_dict layout, at these float offsets (Hg = hidden/2, G3 = 3 Hg, gin = nu (+1 with encode_obs_time),
+ * in0 = 2S+nx+2, N3 = 2 nx S):
+ *   gru.weight_ih_l0 [G3][gin] at 0,             gru.weight_hh_l0 [G3][Hg] after it, gru.bias_ih_l0 [G3], gru.bias_hh_l0 [G3],
+ *   gru.weight_ih_l1 [G3][Hg], gru.weight_hh_l1 [G3][Hg], gru.bias_ih_l1 [G3], gru.bias_hh_l1 [G3],
+ *   linear_out.weight [2][Hg], linear_out.bias [2],
+ *   linear_tanh_stack.0.weight [hidden][in0], .0.bias [hidden], .2.weight [hidden][hidden], .2.bias [hidden],
+ *   .4.weight [N3][hidden], .4.bias [N3]      (each tensor directly after the previous one, no padding).
+ * grad_obs_dev [K][nx] and grad_act_dev [K][B][gin] (every stored input channel) may be NULL.
+ * workspace_dev: nlc_model_backward_workspace_bytes(m, K, B) bytes, 16-byte aligned.
+ * fp32 CUDA cores whatever math mode the forward used; deterministic (bit-identical results for identical inputs). */
+int64_t nlc_model_grad_floats(const nlc_model_desc* desc); /* host only: works without a GPU; < 0 on an invalid desc */
+int64_t nlc_model_backward_workspace_bytes(nlc_model_t m, int K, int B);
+int nlc_model_backward_ts(nlc_model_t m, const float* obs_dev, const float* act_dev, const float* ts_dev, int K, int B,
+                          const float* grad_out_dev, float* grad_params_dev, float* grad_obs_dev, float* grad_act_dev,
+                          void* workspace_dev, void* stream);
+
 /* ReverseGRUEncoder.forward (w_nl.py:25-29) over every window of a K x L action history:
  * hist_dev [K][L][gru_in] env units, windows [t, t+B) for t in [0, T), L = B-1+T.
  * p_dev [K][T][2].                                                                                 */

@@ -391,8 +391,11 @@ extern "C" int nlc_model_forward(nlc_model_t m, const float* obs_dev, const floa
 // ---------------------------------------------------------------------------------------------------------------------
 namespace nlc {
 
+// row_sph (optional, [K][2S]): the sphere coordinates [theta_s | phi_s] themselves - the first-layer input columns the
+// backward (model_grad.cu) multiplies into dW1
 __global__ void __launch_bounds__(128) forward_ts_prep_kernel(ModelDev m, int kH, int S, int Lp, int norm_time, float dt, const float* __restrict__ ts,
-                                                              int K, float* __restrict__ row_b1, float* __restrict__ row_tn) {
+                                                              int K, float* __restrict__ row_b1, float* __restrict__ row_tn,
+                                                              float* __restrict__ row_sph) {
   __shared__ float th[kMaxS], ph[kMaxS];
   const int k = blockIdx.x, n = threadIdx.x;
   float tn = ts[k];
@@ -404,6 +407,7 @@ __global__ void __launch_bounds__(128) forward_ts_prep_kernel(ModelDev m, int kH
     th[j] = atan2f(im, gamma);
     // phi = asin((r^2-1)/(r^2+1)) = 2 atan(r) - pi/2 (the asin form cancels for large r)
     ph[j] = 2.0f * atanf(sqrtf(fmaf(gamma, gamma, im * im))) - 1.57079632679489662f;
+    if (row_sph) { row_sph[(size_t)k * 2 * S + j] = th[j]; row_sph[(size_t)k * 2 * S + S + j] = ph[j]; }
   }
   __syncthreads();
   float acc = m.b1_raw[n];
@@ -411,6 +415,13 @@ __global__ void __launch_bounds__(128) forward_ts_prep_kernel(ModelDev m, int kH
   for (int j = 0; j < S; ++j) acc = fmaf(m.w1_full_t[(size_t)(S + j) * kH + n], ph[j], acc);
   row_b1[(size_t)k * kH + n] = acc;
   if (n == 0) row_tn[k] = tn;
+}
+
+int launch_forward_ts_prep(nlc_model_s* m, const float* ts, int K, float* row_b1, float* row_tn, float* row_sph, cudaStream_t s) {
+  forward_ts_prep_kernel<<<K, m->Hm, 0, s>>>(m->d, m->Hm, m->S, m->nx + 2, m->normalize && m->normalize_time, (float)m->dt, ts, K, row_b1,
+                                             row_tn, row_sph);
+  NLC_LAUNCH_OK("forward_ts_prep_kernel");
+  return NLC_OK;
 }
 
 }  // namespace nlc
@@ -429,8 +440,8 @@ extern "C" int nlc_model_forward_ts(nlc_model_t m, const float* obs_dev, const f
   const int mm = math_mode == NLC_MATH_TC_FP16 ? NLC_MATH_TC_SPLIT3 : math_mode;
   int rc = encode_history_impl(m, act_dev, m->gin, K, 1, B, p_action, mm, s);
   if (rc != NLC_OK) return rc;
-  forward_ts_prep_kernel<<<K, m->Hm, 0, s>>>(m->d, m->Hm, m->S, m->nx + 2, m->normalize && m->normalize_time, (float)m->dt, ts_dev, K, row_b1, row_tn);
-  NLC_LAUNCH_OK("forward_ts_prep_kernel");
+  rc = launch_forward_ts_prep(m, ts_dev, K, row_b1, row_tn, nullptr, s);
+  if (rc != NLC_OK) return rc;
   nlc_rollout_opts o;
   o.env = m->nx == 3 ? NLC_ENV_PENDULUM : (m->nx == 5 ? NLC_ENV_CARTPOLE : NLC_ENV_ACROBOT);
   o.state_constraint = 0; o.goal_x = 0.0f; o.dynamics = NLC_DYN_NEURAL_LAPLACE; o.delay = 0; o.dt = (float)m->dt;

@@ -13,6 +13,7 @@ import ctypes as C
 import numpy as np
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 
@@ -166,18 +167,36 @@ class NeuralLaplaceModel(nn.Module):
     # ---- forward -------------------------------------------------------------------------------------------------
     def forward(self, in_batch_obs, in_batch_action, ts_pred):
         """Predicted state difference, ``w_nl.py:117-145``.  ``in_batch_obs`` (K,nx), ``in_batch_action`` (K,B,nu)
-        or (K,nu), ``ts_pred`` (K,1) seconds.  CUDA tensors in, tensor of the input dtype out."""
+        or (K,nu), ``ts_pred`` (K,1) seconds.  CUDA tensors in, tensor of the input dtype out.
+
+        In grad mode, when a parameter or an input requires grad, the output carries a ``grad_fn`` like the reference
+        module's: its backward runs ``nlc_model_backward_ts`` (fp32 CUDA cores).  The forward values are the same either way."""
+        if torch.is_grad_enabled():
+            if torch.is_tensor(ts_pred) and ts_pred.requires_grad:
+                raise NotImplementedError("NeuralLaplaceModel: gradients with respect to ts_pred are not provided")
+            params = list(self.parameters())
+            if in_batch_obs.requires_grad or in_batch_action.requires_grad or any(p.requires_grad for p in params):
+                out = _ForwardWithGrad.apply(self, in_batch_obs, in_batch_action, ts_pred, *params)
+                return torch.squeeze(out.to(in_batch_obs.dtype))
+        out, _ = self._forward_kernels(in_batch_obs, in_batch_action, ts_pred)
+        return torch.squeeze(out.to(in_batch_obs.dtype))
+
+    def _inputs(self, in_batch_obs, in_batch_action, ts_pred):
         dev = self._device()
-        out_dtype = in_batch_obs.dtype
-        obs = in_batch_obs.to(device=dev, dtype=torch.float32).contiguous()
-        act = in_batch_action.to(device=dev, dtype=torch.float32)
+        obs = in_batch_obs.detach().to(device=dev, dtype=torch.float32).contiguous()
+        act = in_batch_action.detach().to(device=dev, dtype=torch.float32)
         if act.dim() == 2:
             act = act.unsqueeze(1)
         act = act.contiguous()
-        K, B = act.shape[0], act.shape[1]
-        ts = torch.as_tensor(ts_pred).to(device=dev, dtype=torch.float64).reshape(-1)
-        if ts.numel() not in (1, K):
+        ts = torch.as_tensor(ts_pred).detach().to(device=dev, dtype=torch.float64).reshape(-1)
+        if ts.numel() not in (1, act.shape[0]):
             raise ValueError("ts_pred must hold one time per sample")
+        return dev, obs, act, ts
+
+    def _forward_kernels(self, in_batch_obs, in_batch_action, ts_pred):
+        """(K, nx) fp32 output of the forward kernels and the prepared inputs (device, obs, act, ts)."""
+        dev, obs, act, ts = self._inputs(in_batch_obs, in_batch_action, ts_pred)
+        K, B = act.shape[0], act.shape[1]
         lib = _lib.load()
         out = torch.empty((K, self.output_dim), dtype=torch.float32, device=dev)
         t0 = float(ts[0])
@@ -196,4 +215,57 @@ class NeuralLaplaceModel(nn.Module):
                                                     scratch.data_ptr(), _lib.MATH_MODES[self.math_mode], _lib.current_stream_ptr()),
                            "nlc_model_forward_ts")
                 self.last_p_action = scratch.view(-1)[:2 * K].view(K, 2)
-        return torch.squeeze(out.to(out_dtype))
+        return out, (dev, obs, act, ts)
+
+    def _backward_kernels(self, prepared, grad_out, need_obs, need_act):
+        """fp32 gradients from ``nlc_model_backward_ts``: (flat parameter gradients in named_parameters() order, each in
+        its state_dict layout; d obs (K, nx) or None; d act (K, B, gin) or None)."""
+        dev, obs, act, ts = prepared
+        K, B = act.shape[0], act.shape[1]
+        lib = _lib.load()
+        ts32 = ts.expand(K).to(torch.float32).contiguous()  # one uniform time becomes a per-sample time
+        g = grad_out.detach().to(device=dev, dtype=torch.float32).reshape(K, self.output_dim).contiguous()
+        with torch.cuda.device(dev):
+            h = self.handle()
+            n = sum(p.numel() for p in self.parameters())
+            grad_params = torch.empty(n, dtype=torch.float32, device=dev)
+            g_obs = torch.empty_like(obs) if need_obs else None
+            g_act = torch.empty_like(act) if need_act else None
+            ws = torch.empty(int(lib.nlc_model_backward_workspace_bytes(h, K, B)), dtype=torch.uint8, device=dev)
+            _lib.check(lib.nlc_model_backward_ts(h, obs.data_ptr(), act.data_ptr(), ts32.data_ptr(), K, B, g.data_ptr(),
+                                                 grad_params.data_ptr(), _lib.ptr(g_obs), _lib.ptr(g_act), ws.data_ptr(),
+                                                 _lib.current_stream_ptr()), "nlc_model_backward_ts")
+        return grad_params, g_obs, g_act
+
+
+class _ForwardWithGrad(torch.autograd.Function):
+    """``NeuralLaplaceModel.forward`` as one autograd node: inputs ``(model, obs, act, ts, *parameters)``; the forward
+    launches exactly the kernels of the no-grad path, the backward ``nlc_model_backward_ts``."""
+
+    @staticmethod
+    def forward(ctx, model, obs, act, ts, *params):
+        out, prepared = model._forward_kernels(obs, act, ts)
+        ctx.model, ctx.prepared = model, prepared
+        ctx.obs_meta = (obs.shape, obs.dtype, obs.device)
+        ctx.act_meta = (act.shape, act.dtype, act.device)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        model = ctx.model
+        need = ctx.needs_input_grad
+        grad_params, g_obs, g_act = model._backward_kernels(ctx.prepared, grad_out, need[1], need[2])
+        out = [None, None, None, None]
+        if g_obs is not None:
+            shape, dtype, device = ctx.obs_meta
+            out[1] = g_obs.reshape(shape).to(device=device, dtype=dtype)
+        if g_act is not None:
+            shape, dtype, device = ctx.act_meta
+            out[2] = g_act.reshape(shape).to(device=device, dtype=dtype)
+        off = 0
+        for p, needs in zip(model.parameters(), need[4:]):
+            n = p.numel()
+            out.append(grad_params[off:off + n].view(p.shape).to(device=p.device, dtype=p.dtype) if needs else None)
+            off += n
+        return tuple(out)
