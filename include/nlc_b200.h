@@ -266,12 +266,20 @@ int nlc_planner_step(nlc_planner_t p, void* stream);
  * synchronises the stream.                                                                           */
 int nlc_planner_step_profile(nlc_planner_t p, float* ms_out, void* stream);
 
-/* Plans within half a wave of 128-sample tiles run their history encoder BESIDE the rollout kernel (the sequential rollout
- * leaves most SMs idle): *overlapped = 1 if this planner does.  *status = 1 if, in the last control step, the rollout gave
+/* Plans whose sequential rollout leaves SMs idle run their history encoder, wholly or in part, BESIDE the rollout kernel:
+ * up to 140 tiles of 128 samples, and ping-pong rollouts of one or two passes per CTA on at most 140 SMs (up to 560 tiles;
+ * config 4 on one GPU).  *overlapped = 1 if this planner does.  *status = 1 if, in the last control step, the rollout gave
  * up polling for the encoder's output (~1 s: the two kernels were not co-resident - a serialising tool, a shared GPU;
  * NLC_NO_OVERLAP=1 in the environment keeps the plain sequence); the step's results are then invalid.  Synchronises
  * the device.                                                                                       */
 int nlc_planner_overlap_status(nlc_planner_t p, int* overlapped, int* status);
+
+/* Host-side arithmetic of that schedule for K samples, horizon T and a tensor-core model of state size nx with S Fourier
+ * terms (no device is touched): out8 = {encoder beside the rollout, ping-pong rollout form, SMs of the rollout, rollout
+ * passes per CTA, first sample of the last pass (the samples before it are encoded before the fork), step-major encoder
+ * tiles of the last pass's samples encoded before the fork, those tiles in all, horizon steps encoded beside the rollout}.
+ * The math mode is the fp32-class tensor-core mode, with the NLC_NO_OVERLAP / NLC_OVERLAP_FACTOR overrides applied. */
+int nlc_debug_overlap_plan(int K, int T, int nx, int S, long long* out8);
 
 /* K sharded over the GPUs of ONE node (SURVEY 8e): exchange of the per-shard (beta, eta, W) triples on the device, without
  * a collective library.  Every shard owns a mailbox in its HBM; nlc_planner_exchange_export returns its CUDA IPC handle

@@ -96,6 +96,7 @@ SIGNATURES = {
     "nlc_planner_step": (C.c_int, [C.c_void_p, C.c_void_p]),
     "nlc_planner_step_profile": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.c_void_p]),
     "nlc_planner_overlap_status": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "nlc_debug_overlap_plan": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_longlong)]),
     "nlc_planner_exchange_export": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
     "nlc_planner_exchange_connect": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "nlc_planner_exchange_status": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),

@@ -143,6 +143,9 @@ constexpr int kE2Count = kE2Bout + 8;
 // the encoder runs on the other SMs for the rollout's duration.
 inline int pp_overlap_iters(int n_tiles) { return (n_tiles + 295) / 296; }
 inline int pp_overlap_grid(int n_tiles) { const int it = pp_overlap_iters(n_tiles); return (n_tiles + 2 * it - 1) / (2 * it); }
+// Pass q of CTA c rolls out samples [(q * grid + c) * 256, + 256): the passes before the last cover the first
+// (iters - 1) * grid * 256 samples, and the kernel's pass count ceil(K / (grid * 256)) equals pp_overlap_iters.
+inline int pp_overlap_k1(int n_tiles) { return (pp_overlap_iters(n_tiles) - 1) * pp_overlap_grid(n_tiles) * 256; }
 
 struct ModelHost {  // fp64 copies kept for re-folding at another prediction time
   double* w0 = nullptr;  // [Hm][2S+nx+2]

@@ -221,7 +221,8 @@ int launch_encode_fp32(nlc_model_s* m, const float* hist, int hist_ch, int K, in
 }
 
 int launch_encode_tc2(nlc_model_s* m, const float* hist, int hist_ch, int K, int T, int B, float* p, int split3, cudaStream_t stream,
-                      unsigned int* ready = nullptr, int max_ctas = 0, long long tile_begin = 0, long long tile_end = 0);
+                      unsigned int* ready = nullptr, int max_ctas = 0, long long tile_begin = 0, long long tile_end = -1,
+                      int k_sub = 0, bool with_head = false);
 
 // hist_ch: channels stored per history entry (model gin for nlc_model_forward, whose caller supplies the time channel
 // like the reference's forward; action_dim on the planner path, where encode_obs_time's channel is synthesised)
@@ -253,11 +254,14 @@ bool encoder_is_tensor_core(nlc_model_t m, int B, int math_mode) {
   return math_mode != NLC_MATH_FP32 && !(B < 2 || B * m->gin > 8 || m->gin > 2) && m->Hg == kHg;
 }
 
-// The planner's overlapped form: step-major tile order, ready[t] counts finished warps of step t (4 per tile), at most
-// max_ctas CTAs so that the rollout kernel keeps its SMs.
+// The planner's overlapped form: step-major tile order over the samples from k_sub on, ready[t] counts finished warps of step t
+// (4 per tile), tiles [tile_begin, tile_end) of that order (tile_end < 0: to the end), at most max_ctas CTAs so that the
+// rollout kernel keeps its SMs.  with_head: the same launch first encodes samples [0, k_sub) in the plain order.
 int encode_history_overlapped(nlc_model_t m, const float* hist_dev, int K, int T, int B, float* p_dev, int math_mode,
-                              unsigned int* ready, int max_ctas, long long tile_begin, long long tile_end, cudaStream_t s) {
-  return launch_encode_tc2(m, hist_dev, m->nu, K, T, B, p_dev, math_mode == NLC_MATH_TC_SPLIT3, s, ready, max_ctas, tile_begin, tile_end);
+                              unsigned int* ready, int max_ctas, long long tile_begin, long long tile_end, int k_sub, bool with_head,
+                              cudaStream_t s) {
+  return launch_encode_tc2(m, hist_dev, m->nu, K, T, B, p_dev, math_mode == NLC_MATH_TC_SPLIT3, s, ready, max_ctas, tile_begin, tile_end,
+                           k_sub, with_head);
 }
 
 }  // namespace nlc

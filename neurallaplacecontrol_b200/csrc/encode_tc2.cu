@@ -62,6 +62,11 @@ struct Args {
   int tiles_per_t;
   unsigned int* ready;
   long long tile_begin;  // first tile of this launch (step-major order only: the planner may split the encoder in two launches)
+  // plans of two rollout passes: the step-major order covers only the samples from k_off on (the pass that runs beside the
+  // encoder), and the first head_tiles tiles of the launch encode samples [0, k_off) in the plain order, without readiness
+  // counters.  Step-major tile j of the sub-plan is tile head_tiles + j of the launch.
+  int head_tiles;
+  int k_off;
   long long* trace;  // measurement only: clock64 timeline of CTA 0, [step][warp][8 events]
   ModelDev m;
 };
@@ -325,9 +330,10 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
 
   // hist offset of this thread's window in a tile (one integer division per tile, not per cell)
   auto window_base = [&](long long tile_) -> size_t {
-    if (a.tiles_per_t > 0) {  // step-major: one step t per tile, 128 consecutive samples
-      const int t = (int)((unsigned)tile_ / (unsigned)a.tiles_per_t);
-      int k = ((int)tile_ - t * a.tiles_per_t) * kRows + row;
+    if (a.tiles_per_t > 0 && (int)tile_ >= a.head_tiles) {  // step-major: one step t per tile, 128 consecutive samples
+      const int ts = (int)tile_ - a.head_tiles;
+      const int t = (int)((unsigned)ts / (unsigned)a.tiles_per_t);
+      int k = a.k_off + (ts - t * a.tiles_per_t) * kRows + row;
       if (k >= a.K) k = a.K - 1;
       return ((size_t)k * a.L + t) * a.hist_ch;
     }
@@ -511,9 +517,10 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
           const float2 p1 = *reinterpret_cast<const float2*>(&s.pout[1][row * 2]);
           const float2 p2 = *reinterpret_cast<const float2*>(&s.pout[2][row * 2]);
           const float2 pv = make_float2(((o0 + p0.x) + p1.x) + p2.x + cst[kC2Bout], ((o1 + p0.y) + p1.y) + p2.y + cst[kC2Bout + 1]);
-          if (a.tiles_per_t > 0) {
-            const int t = (int)((unsigned)tile / (unsigned)a.tiles_per_t);
-            const int k = ((int)tile - t * a.tiles_per_t) * kRows + row;
+          if (a.tiles_per_t > 0 && (int)tile >= a.head_tiles) {
+            const int ts = (int)tile - a.head_tiles;
+            const int t = (int)((unsigned)ts / (unsigned)a.tiles_per_t);
+            const int k = a.k_off + (ts - t * a.tiles_per_t) * kRows + row;
             if (k < a.K) *reinterpret_cast<float2*>(a.p_out + ((size_t)k * a.T + t) * 2) = pv;
             // publish: the warp's 32 outputs are ordered before lane 0's device-scope fence and counter bump
             __syncwarp();
@@ -543,17 +550,21 @@ static long long* g_enc_trace = nullptr;
 void set_encoder_trace(long long* p) { g_enc_trace = p; }
 
 int launch_encode_tc2(nlc_model_s* m, const float* hist, int hist_ch, int K, int T, int B, float* p, int split3, cudaStream_t stream,
-                      unsigned int* ready, int max_ctas, long long tile_begin, long long tile_end) {
+                      unsigned int* ready, int max_ctas, long long tile_begin, long long tile_end, int k_sub, bool with_head) {
   using namespace enc2;
   NLC_REQUIRE(B * m->gin <= 8, NLC_ERR_SHAPE, "tcgen05 encoder: window_length * input_width = %d exceeds 8", B * m->gin);
   NLC_REQUIRE(B >= 2, NLC_ERR_SHAPE, "tcgen05 encoder: window_length must be >= 2");
   NLC_REQUIRE(m->gin == 1 || m->gin == 2, NLC_ERR_SHAPE, "tcgen05 encoder: GRU input width %d has no instantiation", m->gin);
+  NLC_REQUIRE(!ready || (k_sub >= 0 && k_sub < K && ((long long)k_sub * T) % kRows == 0 && (!with_head || tile_begin == 0)), NLC_ERR_ARG,
+              "tcgen05 encoder: bad step-major sub-plan (first sample %d of %d)", k_sub, K);
   Args a;
   a.hist = hist; a.p_out = p; a.K = K; a.T = T; a.B = B; a.L = B - 1 + T; a.hist_ch = hist_ch;
   a.rows = (long long)K * T;
-  a.tiles_per_t = ready ? (K + kRows - 1) / kRows : 0;
+  a.tiles_per_t = ready ? (K - k_sub + kRows - 1) / kRows : 0;
   a.ready = ready;
   a.tile_begin = 0;
+  a.k_off = ready ? k_sub : 0;
+  a.head_tiles = ready && with_head ? (int)((long long)k_sub * T / kRows) : 0;
   a.m = m->d;
   a.trace = g_enc_trace;
   const int smem = (int)sizeof(Smem) + 128;
@@ -578,9 +589,11 @@ int launch_encode_tc2(nlc_model_s* m, const float* hist, int hist_ch, int K, int
   NLC_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   long long n_tiles = ready ? (long long)a.tiles_per_t * T : (a.rows + kRows - 1) / kRows;
   if (ready) {
-    // step-major: every tile is walked (rows beyond K are masked at the output); [tile_begin, tile_end) of them in this launch
-    if (tile_end > 0 && tile_end < n_tiles) n_tiles = tile_end;
-    a.tile_begin = tile_begin > 0 ? tile_begin : 0;
+    // step-major: every tile is walked (rows beyond K are masked at the output); [tile_begin, tile_end) of them in this launch,
+    // after the head if there is one
+    if (tile_end >= 0 && tile_end < n_tiles) n_tiles = tile_end;
+    n_tiles += a.head_tiles;
+    a.tile_begin = with_head ? 0 : (tile_begin > 0 ? tile_begin : 0);
     a.rows = n_tiles * kRows;
     if (a.tile_begin >= n_tiles) return NLC_OK;
   }

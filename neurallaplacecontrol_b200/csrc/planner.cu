@@ -64,7 +64,8 @@ int launch_combine_exchange(float* mailbox, int G, int stride, int T, int nu, fl
                             float* stats, unsigned long long* step_ctr, unsigned int* status, const StepTail& tl, cudaStream_t s);
 bool encoder_is_tensor_core(nlc_model_t m, int B, int math_mode);
 int encode_history_overlapped(nlc_model_t m, const float* hist_dev, int K, int T, int B, float* p_dev, int math_mode,
-                              unsigned int* ready, int max_ctas, long long tile_begin, long long tile_end, cudaStream_t s);
+                              unsigned int* ready, int max_ctas, long long tile_begin, long long tile_end, int k_sub, bool with_head,
+                              cudaStream_t s);
 bool rollout_can_overlap(const nlc_model_s* m, int K, int T, int math_mode);
 bool rollout_overlap_is_ping_pong(const nlc_model_s* m, int K);
 int launch_rollout_overlapped(nlc_model_s* m, const nlc_rollout_opts* o, const float* state, int sps, const float* p, const float* hist,
@@ -324,31 +325,65 @@ extern "C" int nlc_planner_buffer(nlc_planner_t p, int which, void** dev_ptr, in
 
 // stages 1-3 + the shard-local half of stage 4; `ev` (optional, 4 events) receives the stage boundaries:
 // ev[0] start | perturb | ev[1] | encoder | ev[2] | rollout + cost | ev[3] | (softmax follows)
-// Schedule of the overlapped step (see planner_rollout_impl): the rollout's form and SM count, and how many of the encoder's
-// step-major tiles run on all SMs before the fork.
-struct OverlapSchedule { bool pp; int roll_sms; long long split; };
+// Schedule of the overlapped step (see planner_rollout_impl): the rollout's form, SM count and passes; the samples [0, k1) of
+// the passes before the last, encoded in full before the fork; and how many of the encoder's step-major tiles of the last
+// pass's samples [k1, K) (sub_tiles per step) run on all SMs before the fork.
+struct OverlapSchedule { bool pp; int roll_sms, passes, k1, sub_tiles, beside_steps; long long split; };
 static OverlapSchedule overlap_schedule(const nlc_model_s* m, int K, int T) {
   const int n_tiles = (K + 127) / 128;
   OverlapSchedule s;
   s.pp = rollout_overlap_is_ping_pong(m, K);
   s.roll_sms = s.pp ? pp_overlap_grid(n_tiles) : n_tiles;
+  s.passes = s.pp ? pp_overlap_iters(n_tiles) : 1;
+  s.k1 = s.pp ? pp_overlap_k1(n_tiles) : 0;
+  s.sub_tiles = (K - s.k1 + 127) / 128;
   static const double factor = [] { const char* e = getenv("NLC_OVERLAP_FACTOR"); return e && e[0] ? atof(e) : 0.9; }();  // measurements
-  const double beside_tiles = factor * (148 - s.roll_sms) * (T * (s.pp ? 13.3 * pp_overlap_iters(n_tiles) : 9.5)) / 12.6;
-  long long beside_steps = (long long)(beside_tiles / n_tiles);
-  if (beside_steps > T) beside_steps = T;
-  // (also below half a wave of tiles: 64 tiles, T = 50 - the first 6 steps on all SMs, then 84 SMs beside the rollout:
-  // 0.554 -> 0.538 ms per step against everything beside the rollout)
-  if (beside_steps < 1) beside_steps = 1;
-  s.split = (long long)(T - beside_steps) * n_tiles;
+  const int enc_sms = 148 - s.roll_sms;
+  const long long total = (long long)T * s.sub_tiles;
+  if (s.passes == 1) {
+    const double beside_tiles = factor * enc_sms * (T * (s.pp ? 13.3 : 9.5)) / 12.6;
+    long long beside_steps = (long long)(beside_tiles / n_tiles);
+    if (beside_steps > T) beside_steps = T;
+    // (also below half a wave of tiles: 64 tiles, T = 50 - the first 6 steps on all SMs, then 84 SMs beside the rollout:
+    // 0.554 -> 0.538 ms per step against everything beside the rollout)
+    if (beside_steps < 1) beside_steps = 1;
+    s.split = (T - beside_steps) * n_tiles;
+  } else {
+    // Only the last pass waits for the encoder.  It needs the windows of step t when it begins step t - 1,
+    //   deadline(t) = ((passes - 1) T + t - 1) * 13.3 us after the fork.
+    // The encoder beside it walks the last m step-major tiles on enc_sms SMs at 12.6 us per tile; it has completed step t
+    // once the m - (T - 1 - t) sub_tiles beside tiles up to the end of step t are done:
+    //   (m - (T - 1 - t) sub_tiles) 12.6 / enc_sms <= factor * deadline(t)   for every step t,
+    // which holds trivially for the steps encoded before the fork.  m is the largest count that satisfies all of them; it
+    // need not end on a step boundary (config 4: the last 7.3 of 50 steps of the last pass's samples).
+    double m = (double)total;
+    for (int t = 0; t < T; ++t) {
+      const double bound = (double)(T - 1 - t) * s.sub_tiles + factor * 13.3 * ((s.passes - 1) * (double)T + t - 1) * enc_sms / 12.6;
+      if (bound < m) m = bound;
+    }
+    s.split = total - (m > 0.0 ? (long long)m : 0);
+  }
+  s.beside_steps = (int)((total - s.split) / s.sub_tiles);
   return s;
 }
-// host-side arithmetic only (tests/test_abi_cpu.py): out = {ping-pong form, SMs of the rollout, tiles before the fork, tiles in all}
+// host-side arithmetic only (tests/test_abi_cpu.py): out = {ping-pong form, SMs of the rollout, step-major tiles before the
+// fork, step-major tiles in all}
 extern "C" int nlc_debug_overlap_schedule(int K, int T, int nx, int S, long long* out4) {
   NLC_REQUIRE(out4 && K >= 1 && T >= 1, NLC_ERR_ARG, "nlc_debug_overlap_schedule: bad argument");
   nlc_model_s m{};
   m.nx = nx; m.S = S; m.Hm = 128;
   const OverlapSchedule s = overlap_schedule(&m, K, T);
-  out4[0] = s.pp ? 1 : 0; out4[1] = s.roll_sms; out4[2] = s.split; out4[3] = (long long)T * ((K + 127) / 128);
+  out4[0] = s.pp ? 1 : 0; out4[1] = s.roll_sms; out4[2] = s.split; out4[3] = (long long)T * s.sub_tiles;
+  return NLC_OK;
+}
+extern "C" int nlc_debug_overlap_plan(int K, int T, int nx, int S, long long* out8) {
+  NLC_REQUIRE(out8 && K >= 1 && T >= 1, NLC_ERR_ARG, "nlc_debug_overlap_plan: bad argument");
+  nlc_model_s m{};
+  m.nx = nx; m.S = S; m.Hm = 128;
+  const bool ov = rollout_can_overlap(&m, K, T, NLC_MATH_TC_SPLIT3);
+  const OverlapSchedule s = overlap_schedule(&m, K, T);
+  out8[0] = ov ? 1 : 0; out8[1] = s.pp ? 1 : 0; out8[2] = s.roll_sms; out8[3] = s.passes; out8[4] = s.k1;
+  out8[5] = s.split; out8[6] = (long long)T * s.sub_tiles; out8[7] = s.beside_steps;
   return NLC_OK;
 }
 
@@ -372,26 +407,30 @@ static int planner_rollout_impl(nlc_planner_t p, const float* state_dev, int sta
     // encoder || rollout: fork after stage 1, the encoder on this stream with all SMs but the rollout's, the rollout (one
     // 128-sample tile per CTA) on the side stream, join before stage 4.  The encoder is launched FIRST in host order: a
     // tool that serialises kernels then runs it to completion before the rollout starts polling.
-    const int n_tiles = (mp.K + 127) / 128;
     // (the readiness counters were zeroed by the previous step's combine kernel)
-    // The rollout takes n_tiles SMs (one tile per CTA, ~9.5 us per step) or, from 89 tiles, n_tiles / 2 (ping-pong form, ~13.3 us
-    // per step): the encoder has the other SMs for the rollout's duration.  What those cannot encode in that time (12.6 us per
+    // The rollout takes n_tiles SMs (one tile per CTA, ~9.5 us per step) or, from 89 tiles, n_tiles / 2 per pass (ping-pong form,
+    // ~13.3 us per step): the encoder has the other SMs for the rollout's duration.  What those cannot encode in that time (12.6 us per
     // tile and SM: measured at config 4 / its shards; a wrong estimate only makes the rollout poll a little longer) is encoded
     // on all SMs BEFORE the fork - the windows of the first steps, the encoder walking its tiles in step-major order.
+    // A ping-pong rollout of two passes per CTA (config 4 on one GPU: 512 tiles on 128 SMs) needs the windows of its first
+    // pass's samples [0, k1) from its first step on: those are encoded in full before the fork, in the same launch as the
+    // first steps of the last pass's samples [k1, K), the sub-plan whose step-major readiness the last pass polls ~T steps
+    // after the fork.
     const OverlapSchedule sch = overlap_schedule(p->model, mp.K, mp.T);
     const int roll_sms = sch.roll_sms;
-    const long long split = sch.split;  // first tile of the part that runs beside the rollout
-    if (split > 0) {
-      rc = encode_history_overlapped(p->model, p->hist, mp.K, mp.T, mp.B, p->p, p->d.math_mode, p->ready, 148, 0, split, s);
+    const long long split = sch.split;  // first step-major tile (of the sub-plan) of the part that runs beside the rollout
+    if (split > 0 || sch.k1 > 0) {
+      rc = encode_history_overlapped(p->model, p->hist, mp.K, mp.T, mp.B, p->p, p->d.math_mode, p->ready, 148, 0, split, sch.k1, true, s);
       if (rc != NLC_OK) return rc;
     }
     NLC_CUDA_OK(cudaEventRecord(p->ev_fork, s));
     NLC_CUDA_OK(cudaStreamWaitEvent(p->side_stream, p->ev_fork, 0));
-    rc = encode_history_overlapped(p->model, p->hist, mp.K, mp.T, mp.B, p->p, p->d.math_mode, p->ready, 148 - roll_sms, split, 0, s);
+    rc = encode_history_overlapped(p->model, p->hist, mp.K, mp.T, mp.B, p->p, p->d.math_mode, p->ready, 148 - roll_sms, split, -1, sch.k1,
+                                   false, s);
     if (rc != NLC_OK) return rc;
     if (ev) NLC_CUDA_OK(cudaEventRecord(ev[2], s));  // profile: end of the encoder's own span
     rc = launch_rollout_overlapped(p->model, &p->d.rollout, state_dev, state_per_sample, p->p, p->hist, p->pert_cost, mp.K, mp.T, mp.B,
-                                   mp.nu, p->cost_total, p->states, p->d.math_mode, p->ready, 4u * (unsigned)n_tiles, p->ready + mp.T,
+                                   mp.nu, p->cost_total, p->states, p->d.math_mode, p->ready, 4u * (unsigned)sch.sub_tiles, p->ready + mp.T,
                                    p->side_stream);
     if (rc != NLC_OK) return rc;
     if (ev) NLC_CUDA_OK(cudaEventRecord(ev[5], p->side_stream));  // profile: end of the rollout's span (it starts at ev[1])

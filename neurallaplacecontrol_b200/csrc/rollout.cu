@@ -284,14 +284,14 @@ bool rollout_can_overlap(const nlc_model_s* m, int K, int T, int math_mode) {
   static const bool off = [] { const char* e = getenv("NLC_NO_OVERLAP"); return e && e[0] == '1'; }();
   const char* f = getenv("NLC_ROLLOUT_TILES");  // a forced kernel form (parity tests) keeps the plain sequence
   // up to 74 tiles the encoder keeps at least half the SMs for the whole step; beyond, the planner runs the first part of the
-  // encoder alone and the rest beside the rollout (planner.cu) - worth it while the rollout leaves the encoder >= 8 SMs
+  // encoder alone and the rest beside the rollout (planner.cu) - worth it while the rollout leaves the encoder >= 8 SMs.
+  // Ping-pong plans of two passes per CTA (up to 560 tiles; config 4 on one GPU: 512 tiles = 128 CTAs x 2 passes, 20 SMs to
+  // spare) encode the first pass's samples before the fork and only the last steps of the last pass's samples beside the
+  // rollout: the last pass starts ~T steps after the fork, which leaves the encoder time for those steps.
   const int n_tiles = (K + 127) / 128;
   const bool pp_form = 2 * m->nx * m->S <= 256;  // shapes with a ping-pong instantiation (rollout_tc2.cu launch_one)
   return !off && !(f && f[0]) && math_mode != NLC_MATH_FP32 && rollout_has_tensor_core_form(m) && T >= 2 &&
-         (pp_form ? (n_tiles <= 140 || (pp_overlap_iters(n_tiles) == 1 && pp_overlap_grid(n_tiles) <= 140)) : n_tiles <= 140);
-  // (Plans of two or more passes per CTA - config 4 on one GPU: 512 tiles = 128 CTAs x 2 passes, 20 SMs to spare - were
-  // measured SLOWER overlapped, 3.85 against 3.58 ms: the first pass needs every step's windows within its own 0.66 ms, so
-  // only one step's worth can be encoded beside it, and the step-major tail starves the rollout.)
+         (pp_form ? (n_tiles <= 140 || (pp_overlap_iters(n_tiles) <= 2 && pp_overlap_grid(n_tiles) <= 140)) : n_tiles <= 140);
 }
 // The overlapped rollout's form: one tile per CTA on n_tiles SMs (9.5 us per step), or - from 89 tiles - the ping-pong form on
 // n_tiles / 2 SMs (13.3 us per step of a tile pair), which leaves the encoder 148 - n_tiles / 2 SMs for the whole rollout.

@@ -879,8 +879,9 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
 //              units; of every 32-column unit of the group-uniform (theta, phi) order, columns 8 cg .. 8 cg + 7).  The state of a sample is replicated in its four
 //              threads; partial ILT sums are exchanged through shared memory among the four warps of a row quarter.
 //   L3         first half = the first four units (128 columns), second half the rest (<= 128): A 128 + D 128 columns per tile.
-//   rows       a CTA owns one contiguous row range and walks it 256 rows (two tiles) per pass; a tile without rows in a pass
-//              keeps its hand-offs (the MMA warp's product sequence is fixed) but skips every epilogue.
+//   rows       a CTA owns one contiguous row range and walks it 256 rows (two tiles) per pass (the overlapped step: one
+//              256-row block per pass, pass-major over the grid); a tile without rows in a pass keeps its hand-offs (the MMA
+//              warp's product sequence is fixed) but skips every epilogue.
 template <int NX>
 struct SmemTailPP {
   alignas(8) uint64_t bar_w;
@@ -949,8 +950,12 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
   // samples of this CTA: one contiguous range, a multiple of 32 rows long (except at the end of the plan), walked 256 rows
   // (two tiles) per pass.  A last pass of at most 128 rows has ONE live tile: the other tile's phases are skipped and the pass
   // costs a one-tile chain instead of a full ping-pong pass (config 5's 352-tile groups: 0.80 -> 0.69 ms per rollout).
+  // Overlapped step (a.ready): pass-major instead - pass q of CTA c covers samples [(q * grid + c) * 256, + 256), so that every
+  // pass but the last reads windows the planner encoded before this launch, and only the last pass (samples from
+  // (passes - 1) * grid * 256 on, the encoder's step-major sub-plan) polls the readiness counters.
   const int per_cta = ((a.K + (int)gridDim.x - 1) / (int)gridDim.x + 31) / 32 * 32;
-  const int n_iter = (per_cta + 2 * kRows - 1) / (2 * kRows);
+  const int pass_rows = 2 * kRows * (int)gridDim.x;
+  const int n_iter = a.ready ? (a.K + pass_rows - 1) / pass_rows : (per_cta + 2 * kRows - 1) / (2 * kRows);
   const long long cta_b = (long long)blockIdx.x * per_cta;
   const int cta_begin = (int)(cta_b < a.K ? cta_b : a.K);
   const int cta_end = (cta_begin + per_cta < a.K) ? cta_begin + per_cta : a.K;
@@ -1018,24 +1023,32 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
   };
 
   for (int it = 0; it < n_iter; ++it) {
+    // rows [pass_begin, pass_end) of this pass; `poll`: the encoder may still be writing their windows
+    int pass_begin = cta_begin + 2 * it * kRows, pass_end = cta_end;
+    if (a.ready) {
+      pass_begin = min((it * (int)gridDim.x + (int)blockIdx.x) * (2 * kRows), a.K);
+      pass_end = pass_begin + 2 * kRows < a.K ? pass_begin + 2 * kRows : a.K;
+    }
+    const bool poll = a.ready && it + 1 == n_iter;
     // per-tile state: sample index, liveness bits (bit x), state and cost accumulator of both tiles
     int kk0, kk1, amask = 0, lmask = 0;
     float st0[NX], st1[NX], cost0 = 0.0f, cost1 = 0.0f;
 #pragma unroll
     for (int x = 0; x < 2; ++x) {
-      const int tile0 = cta_begin + (2 * it + x) * kRows;
-      int nr = cta_end - tile0;
+      const int tile0 = pass_begin + x * kRows;
+      int nr = pass_end - tile0;
       nr = nr < 0 ? 0 : (nr > kRows ? kRows : nr);
       if (32 * q < nr) amask |= 1 << x;     // warp-uniform: this warp has at least one live sample of tile x
       if (row < nr) lmask |= 1 << x;
-      const int k = row < nr ? tile0 + row : cta_end - 1;
+      const int k = row < nr ? tile0 + row : pass_end - 1;
       const float* sp = a.state0 + (size_t)(a.state_per_sample ? k / a.state_per_sample : 0) * NX;
 #pragma unroll
       for (int c = 0; c < NX; ++c) { if (x == 0) st0[c] = sp[c]; else st1[c] = sp[c]; }
       if (x == 0) kk0 = k; else kk1 = k;
       if (cg == 2) {
-        // (overlapped step: p is being written by the encoder beside this kernel - wait for step 0's windows, read through L2)
-        if (a.ready) wait_windows_ready(a, 0, lane);
+        // (last pass of the overlapped step: p is being written by the encoder beside this kernel - wait for step 0's windows,
+        // read through L2)
+        if (poll) wait_windows_ready(a, 0, lane);
         *reinterpret_cast<float2*>(&s.stage_p[x][row][0]) = __ldcg(reinterpret_cast<const float2*>(a.p + ((size_t)k * a.T) * 2));
       }
     }
@@ -1137,19 +1150,18 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
       // the running cost (column group 3) - start their way now as cp.async copies into per-sample shared-memory slots:
       // no registers held across the step (held in registers they were spilled right after the load, and the spill
       // store stalled the warp on the load at the top of every step)
-      // Overlapped step (a.ready: the encoder runs beside this kernel and publishes its windows step by step): the 128-byte line
-      // of p(k, t+1) also holds later steps that are not written yet, so it must not pass through L1 - ld.global.cg into two
-      // registers per tile once step t+1 is published, stored into the landing slot before the exchange barrier below.
+      // Last pass of the overlapped step (`poll`: the encoder runs beside this kernel and publishes its windows step by step):
+      // the 128-byte line of p(k, t+1) also holds later steps that are not written yet, so it must not pass through L1 -
+      // ld.global.cg into two registers per tile once step t+1 is published, stored into the landing slot before the exchange
+      // barrier below.  The poll and the load are issued behind the E1 hand-offs, where these warps wait for the M2 products
+      // anyway: at the top of the step their two dependent L2 round trips delayed E1 of every step.  Earlier passes read
+      // windows encoded before the launch; a pass is a 256-sample block, so none of their lines of p (2048 T bytes per block)
+      // holds a window of the polled pass.
       float2 pn0 = make_float2(0.f, 0.f), pn1 = make_float2(0.f, 0.f);
-      if (a.ready && cg == 2 && t + 1 < a.T) {
-        wait_windows_ready(a, t + 1, lane);
-        pn0 = __ldcg(reinterpret_cast<const float2*>(a.p + ((size_t)kk0 * a.T + t + 1) * 2));
-        pn1 = __ldcg(reinterpret_cast<const float2*>(a.p + ((size_t)kk1 * a.T + t + 1) * 2));
-      }
 #pragma unroll 1
       for (int x = 0; x < 2; ++x) {
         const int kx = x ? kk1 : kk0;
-        if (!a.ready && cg == 2 && t + 1 < a.T)
+        if (!poll && cg == 2 && t + 1 < a.T)
           asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(&s.stage_p[x][row][0])), "l"(a.p + ((size_t)kx * a.T + t + 1) * 2) : "memory");
         if (cg == 3 && ((lmask >> x) & 1) && a.cost_total) {
           const float* up = a.hist + ((size_t)kx * a.L + t + a.B - 1) * a.nu;
@@ -1162,6 +1174,11 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
 #pragma unroll 1
       for (int x = 0; x < 2; ++x) { wait_mma(x); mark(0 + x); hidden(x, false); handoff(x); }   // E1 -> M2
       ++nphase;
+      if (poll && cg == 2 && t + 1 < a.T) {
+        wait_windows_ready(a, t + 1, lane);
+        pn0 = __ldcg(reinterpret_cast<const float2*>(a.p + ((size_t)kk0 * a.T + t + 1) * 2));
+        pn1 = __ldcg(reinterpret_cast<const float2*>(a.p + ((size_t)kk1 * a.T + t + 1) * 2));
+      }
       mark(12);
 #pragma unroll 1
       for (int x = 0; x < 2; ++x) { wait_mma(x); mark(2 + x); hidden(x, true); handoff(x); }    // E2 -> M3a
@@ -1194,7 +1211,7 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
         ++nphase;
       }
       mark(15);
-      if (a.ready && cg == 2 && t + 1 < a.T) {
+      if (poll && cg == 2 && t + 1 < a.T) {
         *reinterpret_cast<float2*>(&s.stage_p[0][row][0]) = pn0;
         *reinterpret_cast<float2*>(&s.stage_p[1][row][0]) = pn1;
       }
