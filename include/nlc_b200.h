@@ -138,6 +138,30 @@ int nlc_model_backward_ts(nlc_model_t m, const float* obs_dev, const float* act_
                           const float* grad_out_dev, float* grad_params_dev, float* grad_obs_dev, float* grad_act_dev,
                           void* workspace_dev, void* stream);
 
+/* NeuralLaplaceModel.forward with several prediction times per sample: ts_pred (K, n_t) as the reference passes it to
+ * laplace_reconstruct (w_nl.py:137-144), which evaluates every (sample, time) pair (torchlaplace laplace_reconstruct,
+ * restated in oracle/ilt.py:83-107).  ts_dev [K][n_t] seconds, any order, per sample; out_dev [K][n_t][nx];
+ * p_action_dev [K][2] optional (the encoder output).  The K windows are encoded once; the MLP + ILT then runs over the
+ * K n_t rows on the kernels of nlc_model_forward_ts, so out[k][j] equals nlc_model_forward_ts at ts[k][j] bit for bit
+ * (math_mode likewise).  K n_t >= 2^31 is NLC_ERR_SHAPE.
+ * workspace_dev: nlc_model_forward_multi_workspace_bytes(m, K, n_t, B) bytes, 16-byte aligned:
+ * 4 (2 K + C (hidden_units + nx + 3)) bytes plus alignment, C = min(K n_t, 65536) rows per chunk.            */
+int64_t nlc_model_forward_multi_workspace_bytes(nlc_model_t m, int K, int n_t, int B);
+int nlc_model_forward_multi(nlc_model_t m, const float* obs_dev, const float* act_dev, const float* ts_dev, int K, int n_t,
+                            int B, float* out_dev, float* p_action_dev, void* workspace_dev, int math_mode, void* stream);
+
+/* Gradients of nlc_model_forward_multi (loss.backward() through w_nl.py:117-145 with ts_pred (K, n_t)).
+ * grad_out_dev [K][n_t][nx]; grad_params_dev, grad_obs_dev, grad_act_dev as in nlc_model_backward_ts.  An MLP/ILT
+ * stage over the K n_t rows, a fixed-order sum over j of each sample's gradient of [obs_n | p_action], then one
+ * encoder stage (BPTT) over the K samples; fp32 CUDA cores, deterministic.  K n_t >= 2^31 is NLC_ERR_SHAPE.
+ * workspace_dev: nlc_model_backward_multi_workspace_bytes(m, K, n_t, B) bytes, 16-byte aligned: 4 K (nx + 4) bytes,
+ * 4 C (hidden_units + 2 S + nx + 3) bytes for C = min(K n_t, 65536) rows per chunk, and the per-CTA partials and
+ * scratch of at most 148 CTAs, plus alignment.                                                                   */
+int64_t nlc_model_backward_multi_workspace_bytes(nlc_model_t m, int K, int n_t, int B);
+int nlc_model_backward_multi(nlc_model_t m, const float* obs_dev, const float* act_dev, const float* ts_dev, int K, int n_t,
+                             int B, const float* grad_out_dev, float* grad_params_dev, float* grad_obs_dev, float* grad_act_dev,
+                             void* workspace_dev, void* stream);
+
 /* ReverseGRUEncoder.forward (w_nl.py:25-29) over every window of a K x L action history:
  * hist_dev [K][L][gru_in] env units, windows [t, t+B) for t in [0, T), L = B-1+T.
  * p_dev [K][T][2].                                                                                 */

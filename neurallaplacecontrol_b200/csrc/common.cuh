@@ -71,6 +71,9 @@ struct StepTail {
 
 constexpr int kMaxNx = 8;
 constexpr int kMaxNu = 4;   // GRU input width limit (nu, or nu+1 with encode_obs_time)
+// Rows per chunk of nlc_model_forward_multi / nlc_model_backward_multi: the per-row buffers of one chunk (row_b1 is hidden_units
+// floats a row) stay at 36 MB at hidden 128, inside the 126 MB L2, and are bounded whatever K n_t is.
+constexpr int kMultiChunkRows = 65536;
 constexpr int kMaxS = 136;  // s-terms supported by the fused rollout (planner uses 17 or 33)
 
 // Device-resident, packed model.  Everything the kernels read is fp32.

@@ -392,12 +392,21 @@ extern "C" int nlc_model_forward(nlc_model_t m, const float* obs_dev, const floa
 namespace nlc {
 
 // row_sph (optional, [K][2S]): the sphere coordinates [theta_s | phi_s] themselves - the first-layer input columns the
-// backward (model_grad.cu) multiplies into dW1
+// backward (model_grad.cu) multiplies into dW1.
+// row_obs (optional, [K][nx]) and row_p ([K][2]): row k's copy of obs and p of sample (r0 + k) / n_t, for rows that are
+// (sample, time) pairs (nlc_model_forward_multi)
 __global__ void __launch_bounds__(128) forward_ts_prep_kernel(ModelDev m, int kH, int S, int Lp, int norm_time, float dt, const float* __restrict__ ts,
                                                               int K, float* __restrict__ row_b1, float* __restrict__ row_tn,
-                                                              float* __restrict__ row_sph) {
+                                                              float* __restrict__ row_sph, const float* __restrict__ obs,
+                                                              const float* __restrict__ p, long long r0, int n_t,
+                                                              float* __restrict__ row_obs, float* __restrict__ row_p) {
   __shared__ float th[kMaxS], ph[kMaxS];
   const int k = blockIdx.x, n = threadIdx.x;
+  if (row_obs && n < Lp) {
+    const size_t src = (size_t)((r0 + k) / n_t);
+    if (n < Lp - 2) row_obs[(size_t)k * (Lp - 2) + n] = obs[src * (Lp - 2) + n];
+    else row_p[(size_t)k * 2 + n - (Lp - 2)] = p[src * 2 + n - (Lp - 2)];
+  }
   float tn = ts[k];
   if (norm_time) tn = tn / (dt * 8.0f);  // w_nl.py:123
   const float T = 2.0f * (tn + 1.0e-6f);
@@ -417,11 +426,53 @@ __global__ void __launch_bounds__(128) forward_ts_prep_kernel(ModelDev m, int kH
   if (n == 0) row_tn[k] = tn;
 }
 
-int launch_forward_ts_prep(nlc_model_s* m, const float* ts, int K, float* row_b1, float* row_tn, float* row_sph, cudaStream_t s) {
+static int launch_prep(nlc_model_s* m, const float* ts, int K, float* row_b1, float* row_tn, float* row_sph, const float* obs,
+                       const float* p, long long r0, int n_t, float* row_obs, float* row_p, cudaStream_t s) {
   forward_ts_prep_kernel<<<K, m->Hm, 0, s>>>(m->d, m->Hm, m->S, m->nx + 2, m->normalize && m->normalize_time, (float)m->dt, ts, K, row_b1,
-                                             row_tn, row_sph);
+                                             row_tn, row_sph, obs, p, r0, n_t, row_obs, row_p);
   NLC_LAUNCH_OK("forward_ts_prep_kernel");
   return NLC_OK;
+}
+
+int launch_forward_ts_prep(nlc_model_s* m, const float* ts, int K, float* row_b1, float* row_tn, float* row_sph, cudaStream_t s) {
+  return launch_prep(m, ts, K, row_b1, row_tn, row_sph, nullptr, nullptr, 0, 1, nullptr, nullptr, s);
+}
+
+// The MLP + Fourier ILT of K rows with per-row obs [K][nx], encoder output p [K][2] and prepared row_b1 / row_tn; mm is
+// NLC_MATH_FP32 or NLC_MATH_TC_SPLIT3.
+static int forward_rows(nlc_model_s* m, const float* obs, const float* p, const float* act, const float* row_b1, const float* row_tn,
+                        int K, int B, float* out, int mm, cudaStream_t s) {
+  nlc_rollout_opts o;
+  o.env = m->nx == 3 ? NLC_ENV_PENDULUM : (m->nx == 5 ? NLC_ENV_CARTPOLE : NLC_ENV_ACROBOT);
+  o.state_constraint = 0; o.goal_x = 0.0f; o.dynamics = NLC_DYN_NEURAL_LAPLACE; o.delay = 0; o.dt = (float)m->dt;
+  if (mm == NLC_MATH_TC_SPLIT3 && rollout_has_tensor_core_form(m)) {
+    // representation MLP on the tensor cores: per-sample first-layer bias added in the first epilogue, per-sample Fourier phases
+    // and weights in the last (rollout_tc2.cu, kPerRow)
+    int rc = launch_rollout_tc2(m, &o, obs, 1, p, act, nullptr, K, 1, B, m->gin, nullptr, nullptr, out, 1, 1, s, nullptr, 0, nullptr,
+                                row_b1, row_tn);
+    if (rc != NLC_ERR_UNSUPPORTED) return rc;
+  }
+  if (mm != NLC_MATH_FP32 && K >= 4096)
+    warn_once(kWarnForwardTsFfma, "nlc_model_forward_ts: nx = %d, S = %d has no tcgen05 instantiation; %d samples run on the fp32 kernel",
+              m->nx, m->S, K);
+  return launch_rollout_fp32(m, &o, obs, 1, p, act, nullptr, K, 1, B, m->gin, nullptr, nullptr, out, s, row_b1, row_tn);
+}
+
+// workspace (floats): p [K][2] | row_b1 [C][H] | row_tn [C] | row_obs [C][nx] | row_p [C][2], C = min(K n_t, kMultiChunkRows)
+struct MultiFwdWs { size_t p, b1, tn, obs, rp, total; int C; };
+static size_t up64f(size_t n) { return (n + 63) / 64 * 64; }
+static MultiFwdWs multi_fwd_ws(const nlc_model_s* m, int K, int n_t) {
+  MultiFwdWs w;
+  const long long rows = (long long)K * n_t;
+  w.C = rows < kMultiChunkRows ? (int)rows : kMultiChunkRows;
+  size_t o = 0;
+  w.p = o; o += up64f((size_t)K * 2);
+  w.b1 = o; o += up64f((size_t)w.C * m->Hm);
+  w.tn = o; o += up64f(w.C);
+  w.obs = o; o += up64f((size_t)w.C * m->nx);
+  w.rp = o; o += up64f((size_t)w.C * 2);
+  w.total = o;
+  return w;
 }
 
 }  // namespace nlc
@@ -442,19 +493,41 @@ extern "C" int nlc_model_forward_ts(nlc_model_t m, const float* obs_dev, const f
   if (rc != NLC_OK) return rc;
   rc = launch_forward_ts_prep(m, ts_dev, K, row_b1, row_tn, nullptr, s);
   if (rc != NLC_OK) return rc;
-  nlc_rollout_opts o;
-  o.env = m->nx == 3 ? NLC_ENV_PENDULUM : (m->nx == 5 ? NLC_ENV_CARTPOLE : NLC_ENV_ACROBOT);
-  o.state_constraint = 0; o.goal_x = 0.0f; o.dynamics = NLC_DYN_NEURAL_LAPLACE; o.delay = 0; o.dt = (float)m->dt;
-  if (mm == NLC_MATH_TC_SPLIT3 && rollout_has_tensor_core_form(m)) {
-    // representation MLP on the tensor cores: per-sample first-layer bias added in the first epilogue, per-sample Fourier phases
-    // and weights in the last (rollout_tc2.cu, kPerRow)
-    rc = launch_rollout_tc2(m, &o, obs_dev, 1, p_action, act_dev, nullptr, K, 1, B, m->gin, nullptr, nullptr, out_dev, 1, 1, s, nullptr,
-                            0, nullptr, row_b1, row_tn);
-    if (rc != NLC_ERR_UNSUPPORTED) return rc;
+  return forward_rows(m, obs_dev, p_action, act_dev, row_b1, row_tn, K, B, out_dev, mm, s);
+}
+
+// NeuralLaplaceModel.forward with ts_pred (K, n_t): the K windows are encoded once; the MLP + ILT then runs over the K n_t rows
+// (sample k, time j) = row k n_t + j, chunk by chunk, on the kernels of nlc_model_forward_ts - each row is evaluated exactly as
+// nlc_model_forward_ts evaluates a sample at that time.
+extern "C" int64_t nlc_model_forward_multi_workspace_bytes(nlc_model_t m, int K, int n_t, int B) {
+  if (!m || K < 1 || n_t < 1 || B < 1) return NLC_ERR_ARG;
+  if ((long long)K * n_t >= (1LL << 31)) return NLC_ERR_SHAPE;
+  return (int64_t)(multi_fwd_ws(m, K, n_t).total * sizeof(float));
+}
+
+extern "C" int nlc_model_forward_multi(nlc_model_t m, const float* obs_dev, const float* act_dev, const float* ts_dev, int K, int n_t,
+                                       int B, float* out_dev, float* p_action_dev, void* workspace_dev, int math_mode, void* stream) {
+  NLC_REQUIRE(m && obs_dev && act_dev && ts_dev && out_dev && workspace_dev, NLC_ERR_ARG, "nlc_model_forward_multi: null pointer");
+  NLC_REQUIRE(K >= 1 && n_t >= 1 && B >= 1, NLC_ERR_ARG, "nlc_model_forward_multi: K, n_t and B must be positive");
+  NLC_REQUIRE((long long)K * n_t < (1LL << 31), NLC_ERR_SHAPE, "nlc_model_forward_multi: K n_t = %lld rows, 2^31 or more",
+              (long long)K * n_t);
+  NLC_REQUIRE(((uintptr_t)workspace_dev & 15) == 0, NLC_ERR_ARG, "nlc_model_forward_multi: workspace must be 16-byte aligned");
+  NLC_REQUIRE(math_mode == NLC_MATH_FP32 || math_mode == NLC_MATH_TC_SPLIT3 || math_mode == NLC_MATH_TC_FP16, NLC_ERR_ARG,
+              "unknown math_mode %d", math_mode);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const MultiFwdWs w = multi_fwd_ws(m, K, n_t);
+  float* ws = static_cast<float*>(workspace_dev);
+  float* p = p_action_dev ? p_action_dev : ws + w.p;
+  const int mm = math_mode == NLC_MATH_TC_FP16 ? NLC_MATH_TC_SPLIT3 : math_mode;  // as nlc_model_forward_ts
+  int rc = encode_history_impl(m, act_dev, m->gin, K, 1, B, p, mm, s);
+  if (rc != NLC_OK) return rc;
+  const long long n_rows = (long long)K * n_t;
+  for (long long r0 = 0; r0 < n_rows; r0 += w.C) {
+    const int rows = (int)(n_rows - r0 < w.C ? n_rows - r0 : w.C);
+    rc = launch_prep(m, ts_dev + r0, rows, ws + w.b1, ws + w.tn, nullptr, obs_dev, p, r0, n_t, ws + w.obs, ws + w.rp, s);
+    if (rc != NLC_OK) return rc;
+    rc = forward_rows(m, ws + w.obs, ws + w.rp, act_dev, ws + w.b1, ws + w.tn, rows, B, out_dev + r0 * m->nx, mm, s);
+    if (rc != NLC_OK) return rc;
   }
-  if (mm != NLC_MATH_FP32 && K >= 4096)
-    warn_once(kWarnForwardTsFfma, "nlc_model_forward_ts: nx = %d, S = %d has no tcgen05 instantiation; %d samples run on the fp32 kernel",
-              m->nx, m->S, K);
-  return launch_rollout_fp32(m, &o, obs_dev, 1, p_action, act_dev, nullptr, K, 1, B, m->gin, nullptr, nullptr, out_dev, s, row_b1,
-                             row_tn);
+  return NLC_OK;
 }

@@ -169,8 +169,11 @@ class NeuralLaplaceModel(nn.Module):
         """Predicted state difference, ``w_nl.py:117-145``.  ``in_batch_obs`` (K,nx), ``in_batch_action`` (K,B,nu)
         or (K,nu), ``ts_pred`` (K,1) seconds.  CUDA tensors in, tensor of the input dtype out.
 
+        ``ts_pred`` (K, n_t) with n_t >= 2 predicts at every (sample, time) pair, as the reference's ``laplace_reconstruct``
+        does: ``torch.squeeze`` of a (K, n_t, nx) result, each sample's history encoded once (``nlc_model_forward_multi``).
+
         In grad mode, when a parameter or an input requires grad, the output carries a ``grad_fn`` like the reference
-        module's: its backward runs ``nlc_model_backward_ts`` (fp32 CUDA cores).  The forward values are the same either way."""
+        module's: its backward runs ``nlc_model_backward_ts`` (``nlc_model_backward_multi`` for (K, n_t) times; fp32 CUDA cores).  The forward values are the same either way."""
         if torch.is_grad_enabled():
             if torch.is_tensor(ts_pred) and ts_pred.requires_grad:
                 raise NotImplementedError("NeuralLaplaceModel: gradients with respect to ts_pred are not provided")
@@ -188,16 +191,35 @@ class NeuralLaplaceModel(nn.Module):
         if act.dim() == 2:
             act = act.unsqueeze(1)
         act = act.contiguous()
-        ts = torch.as_tensor(ts_pred).detach().to(device=dev, dtype=torch.float64).reshape(-1)
+        ts = torch.as_tensor(ts_pred).detach().to(device=dev, dtype=torch.float64)
+        if ts.dim() == 2 and ts.shape[1] >= 2:  # several times per sample: (K, n_t), a 2-D tensor of its own
+            if ts.shape[0] != act.shape[0]:
+                raise ValueError(f"ts_pred of shape {tuple(ts.shape)} needs one row of times per sample ({act.shape[0]})")
+            return dev, obs, act, ts.contiguous()
+        ts = ts.reshape(-1)
         if ts.numel() not in (1, act.shape[0]):
             raise ValueError("ts_pred must hold one time per sample")
         return dev, obs, act, ts
 
     def _forward_kernels(self, in_batch_obs, in_batch_action, ts_pred):
-        """(K, nx) fp32 output of the forward kernels and the prepared inputs (device, obs, act, ts)."""
+        """(K, nx) or, for (K, n_t) times, (K, n_t, nx) fp32 output of the forward kernels and the prepared inputs
+        (device, obs, act, ts)."""
         dev, obs, act, ts = self._inputs(in_batch_obs, in_batch_action, ts_pred)
         K, B = act.shape[0], act.shape[1]
         lib = _lib.load()
+        if ts.dim() == 2:
+            n_t = ts.shape[1]
+            out = torch.empty((K, n_t, self.output_dim), dtype=torch.float32, device=dev)
+            p_action = torch.empty((K, 2), dtype=torch.float32, device=dev)
+            ts32 = ts.to(torch.float32).contiguous()
+            with torch.cuda.device(dev):
+                h = self.handle()
+                ws = torch.empty(int(lib.nlc_model_forward_multi_workspace_bytes(h, K, n_t, B)), dtype=torch.uint8, device=dev)
+                _lib.check(lib.nlc_model_forward_multi(h, obs.data_ptr(), act.data_ptr(), ts32.data_ptr(), K, n_t, B, out.data_ptr(),
+                                                       p_action.data_ptr(), ws.data_ptr(), _lib.MATH_MODES[self.math_mode],
+                                                       _lib.current_stream_ptr()), "nlc_model_forward_multi")
+            self.last_p_action = p_action
+            return out, (dev, obs, act, ts)
         out = torch.empty((K, self.output_dim), dtype=torch.float32, device=dev)
         t0 = float(ts[0])
         with torch.cuda.device(dev):
@@ -218,29 +240,39 @@ class NeuralLaplaceModel(nn.Module):
         return out, (dev, obs, act, ts)
 
     def _backward_kernels(self, prepared, grad_out, need_obs, need_act):
-        """fp32 gradients from ``nlc_model_backward_ts``: (flat parameter gradients in named_parameters() order, each in
-        its state_dict layout; d obs (K, nx) or None; d act (K, B, gin) or None)."""
+        """fp32 gradients from ``nlc_model_backward_ts`` (``nlc_model_backward_multi`` for (K, n_t) times): (flat parameter
+        gradients in named_parameters() order, each in its state_dict layout; d obs (K, nx) or None; d act (K, B, gin) or None)."""
         dev, obs, act, ts = prepared
         K, B = act.shape[0], act.shape[1]
         lib = _lib.load()
-        ts32 = ts.expand(K).to(torch.float32).contiguous()  # one uniform time becomes a per-sample time
-        g = grad_out.detach().to(device=dev, dtype=torch.float32).reshape(K, self.output_dim).contiguous()
+        multi = ts.dim() == 2
+        ts32 = (ts if multi else ts.expand(K)).to(torch.float32).contiguous()  # one uniform time becomes a per-sample time
+        g = grad_out.detach().to(device=dev, dtype=torch.float32)
+        g = (g.reshape(K, ts.shape[1], self.output_dim) if multi else g.reshape(K, self.output_dim)).contiguous()
         with torch.cuda.device(dev):
             h = self.handle()
             n = sum(p.numel() for p in self.parameters())
             grad_params = torch.empty(n, dtype=torch.float32, device=dev)
             g_obs = torch.empty_like(obs) if need_obs else None
             g_act = torch.empty_like(act) if need_act else None
-            ws = torch.empty(int(lib.nlc_model_backward_workspace_bytes(h, K, B)), dtype=torch.uint8, device=dev)
-            _lib.check(lib.nlc_model_backward_ts(h, obs.data_ptr(), act.data_ptr(), ts32.data_ptr(), K, B, g.data_ptr(),
-                                                 grad_params.data_ptr(), _lib.ptr(g_obs), _lib.ptr(g_act), ws.data_ptr(),
-                                                 _lib.current_stream_ptr()), "nlc_model_backward_ts")
+            if multi:
+                n_t = ts.shape[1]
+                ws = torch.empty(int(lib.nlc_model_backward_multi_workspace_bytes(h, K, n_t, B)), dtype=torch.uint8, device=dev)
+                _lib.check(lib.nlc_model_backward_multi(h, obs.data_ptr(), act.data_ptr(), ts32.data_ptr(), K, n_t, B, g.data_ptr(),
+                                                        grad_params.data_ptr(), _lib.ptr(g_obs), _lib.ptr(g_act), ws.data_ptr(),
+                                                        _lib.current_stream_ptr()), "nlc_model_backward_multi")
+            else:
+                ws = torch.empty(int(lib.nlc_model_backward_workspace_bytes(h, K, B)), dtype=torch.uint8, device=dev)
+                _lib.check(lib.nlc_model_backward_ts(h, obs.data_ptr(), act.data_ptr(), ts32.data_ptr(), K, B, g.data_ptr(),
+                                                     grad_params.data_ptr(), _lib.ptr(g_obs), _lib.ptr(g_act), ws.data_ptr(),
+                                                     _lib.current_stream_ptr()), "nlc_model_backward_ts")
         return grad_params, g_obs, g_act
 
 
 class _ForwardWithGrad(torch.autograd.Function):
     """``NeuralLaplaceModel.forward`` as one autograd node: inputs ``(model, obs, act, ts, *parameters)``; the forward
-    launches exactly the kernels of the no-grad path, the backward ``nlc_model_backward_ts``."""
+    launches exactly the kernels of the no-grad path, the backward ``nlc_model_backward_ts`` (``nlc_model_backward_multi``
+    for (K, n_t) times, whose output and ``grad_out`` are (K, n_t, nx))."""
 
     @staticmethod
     def forward(ctx, model, obs, act, ts, *params):
