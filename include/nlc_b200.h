@@ -12,7 +12,8 @@
  * entry point returns NLC_ERR_ARCH.
  *
  * Arithmetic: fp32 on the device (the reference runs fp64 on the CPU, mppi_with_model.py:65,101);
- * host-side constant folding is done in fp64 and rounded once.
+ * host-side constant folding is done in fp64 and rounded once.  The model's fp64 entry points
+ * (nlc_model_forward_f64 / nlc_model_backward_f64) compute in fp64 throughout.
  */
 #ifndef NLC_B200_H
 #define NLC_B200_H
@@ -161,6 +162,37 @@ int64_t nlc_model_backward_multi_workspace_bytes(nlc_model_t m, int K, int n_t, 
 int nlc_model_backward_multi(nlc_model_t m, const float* obs_dev, const float* act_dev, const float* ts_dev, int K, int n_t,
                              int B, const float* grad_out_dev, float* grad_params_dev, float* grad_obs_dev, float* grad_act_dev,
                              void* workspace_dev, void* stream);
+
+/* NeuralLaplaceModel.forward (w_nl.py:117-145) and its gradients (train_utils.py:388-407 loss.backward()) in fp64 throughout,
+ * the precision the reference trains in (train_utils.py:267 .double()).  Every prediction-time form goes through n_t:
+ * ts_dev [K][n_t] seconds (n_t = 1: one time per sample; a uniform time is passed per sample), out_dev [K][n_t][nx],
+ * p_action_dev [K][2] optional (the encoder output), grad_out_dev [K][n_t][nx]; obs_dev [K][nx], act_dev [K][B][gru_in] and
+ * grad_obs_dev / grad_act_dev (either may be NULL) as in nlc_model_backward_ts, all fp64.
+ * params_dev: the 16 parameters, fp64 on the device, nlc_model_grad_floats(desc) entries in the layout of grad_params_dev
+ * (named_parameters() order, each tensor in its state_dict layout, no padding).  The kernels read the weights from it on
+ * every call, never from the handle's fp32 arena: the handle gives only shapes, flags, dt and the normalisation constants
+ * (kept in fp64), so it stays valid across optimizer steps.  Non-finite parameters are not checked; they propagate.
+ * grad_params_dev: the same layout, fp64, OVERWRITTEN.
+ * The forward encodes the K windows once (tiles of 32 samples), then runs the MLP + ILT over the K n_t rows; the backward is
+ * the two-stage form of nlc_model_backward_multi for every n_t.  Deterministic: the grid, the tile-to-CTA assignment and
+ * every summation order depend on the shapes only.  K n_t >= 2^31 is NLC_ERR_SHAPE; a null required pointer or a
+ * workspace that is not 16-byte aligned is NLC_ERR_ARG; B in [1, 8].
+ * workspace_dev: nlc_model_{forward,backward}_f64_workspace_bytes(m, K, n_t, B) bytes, 16-byte aligned, bounded whatever
+ * n_t is (rows are walked in chunks of C = min(K n_t, 65536)).  With Hg = hidden/2, in0 = 2S+nx+2, N3 = 2 nx S, G = the
+ * CTAs of min(K, C) tiles of 32 (at most 148), up to alignment to 4 and 64 elements, the forward takes
+ *   8 (2 K + C (hidden + 1 + 2 S) + W + G Sc) bytes,  W = 3 (6 Hg^2 + 3 Hg) + 3 Hg gin + 2 Hg + 2 + in0 hidden
+ *                                                         + 2 hidden^2 + 2 hidden + (2 hidden + 1) N3,
+ *   Sc = 32 (4 B + 5 B hidden + 9 hidden + in0 + N3 + 18)   (per-CTA tile scratch),
+ * and the backward 8 ((K + C)(nx + 2) + G P) bytes more, P = nlc_model_grad_floats (per-CTA gradient partials).          */
+int64_t nlc_model_forward_f64_workspace_bytes(nlc_model_t m, int K, int n_t, int B);
+int nlc_model_forward_f64(nlc_model_t m, const double* params_dev, const double* obs_dev, const double* act_dev,
+                          const double* ts_dev, int K, int n_t, int B, double* out_dev, double* p_action_dev,
+                          void* workspace_dev, void* stream);
+int64_t nlc_model_backward_f64_workspace_bytes(nlc_model_t m, int K, int n_t, int B);
+int nlc_model_backward_f64(nlc_model_t m, const double* params_dev, const double* obs_dev, const double* act_dev,
+                           const double* ts_dev, int K, int n_t, int B, const double* grad_out_dev,
+                           double* grad_params_dev, double* grad_obs_dev, double* grad_act_dev,
+                           void* workspace_dev, void* stream);
 
 /* ReverseGRUEncoder.forward (w_nl.py:25-29) over every window of a K x L action history:
  * hist_dev [K][L][gru_in] env units, windows [t, t+B) for t in [0, T), L = B-1+T.

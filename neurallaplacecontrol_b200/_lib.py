@@ -82,6 +82,11 @@ SIGNATURES = {
     "nlc_model_backward_multi_workspace_bytes": (C.c_int64, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
     "nlc_model_backward_multi": (C.c_int, [C.c_void_p, _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, _fp, _fp, _fp, C.c_void_p,
                                            C.c_void_p]),
+    "nlc_model_forward_f64_workspace_bytes": (C.c_int64, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
+    "nlc_model_forward_f64": (C.c_int, [C.c_void_p, _fp, _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, _fp, C.c_void_p, C.c_void_p]),
+    "nlc_model_backward_f64_workspace_bytes": (C.c_int64, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
+    "nlc_model_backward_f64": (C.c_int, [C.c_void_p, _fp, _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, _fp, _fp, _fp, C.c_void_p,
+                                         C.c_void_p]),
     "nlc_encode_history": (C.c_int, [C.c_void_p, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_int, C.c_void_p]),
     "nlc_perturb": (C.c_int, [C.POINTER(MppiParams), _fp, _fp, C.c_int, _fp, C.c_uint64, C.c_uint64, _fp, _fp, _fp,
                               _fp, _fp, _fp, C.c_void_p]),

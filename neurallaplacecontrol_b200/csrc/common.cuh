@@ -129,6 +129,11 @@ struct ModelDev {
   float* state_inv_std; // [nx]   (1/std; 1 when normalize is off)
   float* act_mean;   // [gin]
   float* act_inv_std;// [gin]
+  // the same four in fp64, for the fp64 forward / backward (model_grad.cu), whose weights come per call from the caller
+  double* state_mean64;
+  double* state_inv_std64;
+  double* act_mean64;
+  double* act_inv_std64;
 };
 
 // float offsets inside ModelDev::enc2_c
@@ -280,6 +285,79 @@ __device__ __host__ __forceinline__ void philox4x32_10(uint32_t c[4], uint32_t k
     k0 += W0; k1 += W1;
   }
 }
+
+// ---------------------------------------------------------------------------------------------
+// fp64 counterparts of the fp32 helpers above, for the kernels templated on the scalar type
+// (model_grad.cu, the per-sample-time prep of rollout.cu).  They keep the same cancellation-free
+// forms on top of CUDA's fp64 libm (exp, tanh, tan, cos: <= 2 ulp).
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ double exp_acc(double x) { return exp(x); }
+__device__ __forceinline__ double sigmoid_acc(double x) { return 1.0 / (1.0 + exp(-x)); }
+__device__ __forceinline__ double tanh_acc(double x) { return tanh(x); }
+// tan((pi/2) sigmoid(2u)) through s = sigmoid(-2|u|) in (0, 1/2]: tan((pi/2) s) for u <= 0, cot((pi/2) s) for u > 0;
+// |u| clamped at 40 as in the fp32 form (a NaN stays NaN)
+__device__ __forceinline__ double sphere_radius(double u) {
+  const double au = fabs(u);
+  const double e = exp(-2.0 * (au > 40.0 ? 40.0 : au));
+  const double t = tan(1.5707963267948966 * (e / (1.0 + e)));
+  return u <= 0.0 ? t : 1.0 / t;
+}
+__device__ __forceinline__ double cos_reduced(double x) { return cos(x); }
+
+// Scalar-type-generic spellings of the libm calls and constants the templated kernels use: the float forms are exactly the
+// calls and literals of the fp32 kernels, so their fp32 instantiations compile to the same arithmetic.
+namespace rm {
+__device__ __forceinline__ float fma(float a, float b, float c) { return fmaf(a, b, c); }
+__device__ __forceinline__ double fma(double a, double b, double c) { return ::fma(a, b, c); }
+__device__ __forceinline__ float min(float a, float b) { return fminf(a, b); }
+__device__ __forceinline__ double min(double a, double b) { return fmin(a, b); }
+__device__ __forceinline__ float abs(float a) { return fabsf(a); }
+__device__ __forceinline__ double abs(double a) { return fabs(a); }
+__device__ __forceinline__ float rcp(float a) { return __frcp_rn(a); }
+__device__ __forceinline__ double rcp(double a) { return 1.0 / a; }
+__device__ __forceinline__ float exp(float a) { return expf(a); }
+__device__ __forceinline__ double exp(double a) { return ::exp(a); }
+__device__ __forceinline__ float atan(float a) { return atanf(a); }
+__device__ __forceinline__ double atan(double a) { return ::atan(a); }
+__device__ __forceinline__ float atan2(float a, float b) { return atan2f(a, b); }
+__device__ __forceinline__ double atan2(double a, double b) { return ::atan2(a, b); }
+__device__ __forceinline__ float sqrt(float a) { return sqrtf(a); }
+__device__ __forceinline__ double sqrt(double a) { return ::sqrt(a); }
+// 4 consecutive elements (16-byte aligned for float, 16-byte aligned pairs for double)
+__device__ __forceinline__ void ld4(const float* p, float v[4]) {
+  const float4 q = *reinterpret_cast<const float4*>(p);
+  v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+}
+__device__ __forceinline__ void ld4(const double* p, double v[4]) {
+  const double2 a = *reinterpret_cast<const double2*>(p), b = *reinterpret_cast<const double2*>(p + 2);
+  v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y;
+}
+__device__ __forceinline__ void ldg4(const float* p, float v[4]) {
+  const float4 q = __ldg(reinterpret_cast<const float4*>(p));
+  v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+}
+__device__ __forceinline__ void ldg4(const double* p, double v[4]) {
+  const double2 a = __ldg(reinterpret_cast<const double2*>(p)), b = __ldg(reinterpret_cast<const double2*>(p + 2));
+  v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y;
+}
+__device__ __forceinline__ void st4(float* p, const float v[4]) { *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]); }
+__device__ __forceinline__ void st4(double* p, const double v[4]) {
+  *reinterpret_cast<double2*>(p) = make_double2(v[0], v[1]);
+  *reinterpret_cast<double2*>(p + 2) = make_double2(v[2], v[3]);
+}
+}  // namespace rm
+
+// Constants of the Fourier ILT (torchlaplace defaults, oracle/ilt.py) in either precision: the float members are the
+// literals of the fp32 kernels.
+template <typename T> struct Real;
+template <> struct Real<float> {
+  static constexpr float pi = 3.14159265358979f, half_pi = 1.57079632679489662f, eps = 1.0e-6f, alpha = 1.0e-3f,
+                         ln_inv_tol = 4.605170185988091f;  // -ln(10 alpha)
+};
+template <> struct Real<double> {
+  static constexpr double pi = 3.141592653589793, half_pi = 1.5707963267948966, eps = 1.0e-6, alpha = 1.0e-3,
+                          ln_inv_tol = 4.605170185988091;
+};
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -208,6 +208,9 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
   size_t o_w2 = A.add((size_t)Hm * Hm), o_b2 = A.add(Hm), o_w3 = A.add((size_t)Hm * N3p), o_b3 = A.add(N3p);
   size_t o_phase = A.add(S), o_weight = A.add(S);
   size_t o_smean = A.add(nx), o_sinv = A.add(nx), o_amean = A.add(gin), o_ainv = A.add(gin);
+  // the same constants in fp64 (two floats per double; sections are 256-byte aligned)
+  size_t o_smean64 = A.add(2 * nx), o_sinv64 = A.add(2 * nx), o_amean64 = A.add(2 * gin), o_ainv64 = A.add(2 * gin);
+  auto put64 = [&](size_t off, size_t i, double v) { memcpy(A.data.data() + off + 2 * i, &v, sizeof(double)); };
   // tensor-core operand image of the three recurrent GRU matrices: fp16 hi/lo, UMMA canonical layout
   const size_t tc_halves = (size_t)3 * 2 * G3 * Hg;
   size_t o_enc2w = A.add(tc_halves / 2), o_enc2c = A.add(nlc::kE2Count), o_enc2x = A.add(2 * 256 * 8 / 2);
@@ -252,6 +255,8 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
   for (int i = 0; i < nx; ++i) {
     put(o_smean, i, d->normalize ? d->state_mean[i] : 0.0);
     put(o_sinv, i, d->normalize ? 1.0 / d->state_std[i] : 1.0);
+    put64(o_smean64, i, d->normalize ? d->state_mean[i] : 0.0);
+    put64(o_sinv64, i, d->normalize ? 1.0 / d->state_std[i] : 1.0);
   }
   for (int i = 0; i < gin; ++i) {
     // w_nl.py:121 (normalised) / :129 (actions / 3.0).  With encode_obs_time the extra channel is
@@ -263,6 +268,8 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
     }
     put(o_amean, i, mean);
     put(o_ainv, i, 1.0 / stdv);
+    put64(o_amean64, i, mean);
+    put64(o_ainv64, i, 1.0 / stdv);
   }
   if (Hm == 128) {  // (the tensor-core kernels are built for hidden_units = 128: other widths run on the fp32 kernels)
     // encode_tc2.cu operands: exponent scales folded (sigmoid(x) = 1/(1 + 2^(-log2e x)), tanh(x) = 2/(1 + 2^(-2 log2e x)) - 1)
@@ -391,6 +398,8 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
   m->d.w2_t = base + o_w2; m->d.b2 = base + o_b2; m->d.w3_t = base + o_w3; m->d.b3 = base + o_b3;
   m->d.ilt_phase = base + o_phase; m->d.ilt_weight = base + o_weight;
   m->d.state_mean = base + o_smean; m->d.state_inv_std = base + o_sinv; m->d.act_mean = base + o_amean; m->d.act_inv_std = base + o_ainv;
+  m->d.state_mean64 = reinterpret_cast<double*>(base + o_smean64); m->d.state_inv_std64 = reinterpret_cast<double*>(base + o_sinv64);
+  m->d.act_mean64 = reinterpret_cast<double*>(base + o_amean64); m->d.act_inv_std64 = reinterpret_cast<double*>(base + o_ainv64);
   rc = fold_prediction_time(m, d->dt);
   if (rc != NLC_OK) return fail(rc);
   *out = m;

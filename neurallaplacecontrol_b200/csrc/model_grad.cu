@@ -27,6 +27,13 @@
 //
 // Reads only the unfolded weights of ModelDev: b1_fold, ilt_phase, ilt_weight and the mlp2_* images belong to the last
 // prediction time a planner folded and are never touched here.
+//
+// fp64 (nlc_model_forward_f64 / nlc_model_backward_f64, the reference's training precision): the tile machinery below is
+// templated on the scalar type and instantiated a second time for double.  The weights then come per call from the
+// caller's fp64 parameter buffer (state_dict layout), which model_f64_weights_kernel rearranges into the workspace in the
+// layouts ModelDev holds (TileW); only shapes, flags, dt and the fp64 normalisation constants are read from the handle.
+// The fp64 forward is the recompute half of the tile steps (encoder, linear_out, MLP) followed by the ILT sum; the fp64
+// backward runs the two-stage form of nlc_model_backward_multi for every n_t (n_t = 1 included).
 #include <stddef.h>
 
 #include "common.cuh"
@@ -34,6 +41,8 @@
 namespace nlc {
 
 int launch_forward_ts_prep(nlc_model_s* m, const float* ts, int K, float* row_b1, float* row_tn, float* row_sph, cudaStream_t s);
+int launch_forward_ts_prep_f64(nlc_model_s* m, const double* b1_raw, const double* w1_full_t, const double* ts, int K, double* row_b1,
+                               double* row_tn, double* row_sph, cudaStream_t s);
 int encode_history_impl(nlc_model_t m, const float* hist_dev, int hist_ch, int K, int T, int B, float* p_dev, int math_mode,
                         cudaStream_t s);
 
@@ -55,6 +64,8 @@ struct GradShape {
   int s_xs, s_gate, s_h, s_gi, s_gh, s_x1, s_a1, s_a2, s_do, s_dz2, s_dz1, s_dh, s_dxt, s_rc, s_total;
   // transposed weight copies
   int w_hh0, w_ih1, w_hh1, w_2, w_3, w_total;
+  // fp64 only: the forward layouts of every weight (TileW), after the transposed copies (offsets from the image's start)
+  int f_wih0, f_bih0, f_bhh0, f_hh0t, f_ih1t, f_hh1t, f_bih1, f_bhh1, f_wout, f_bout, f_w1t, f_b1, f_w2t, f_b2, f_w3t, f_b3, f_total;
 };
 
 static GradShape make_shape(int nx, int nu, int gin, int H, int S, int B) {
@@ -93,118 +104,158 @@ static GradShape make_shape(int nx, int nu, int gin, int H, int S, int B) {
   o = 0;
   g.w_hh0 = take(G3 * Hg); g.w_ih1 = take(G3 * Hg); g.w_hh1 = take(G3 * Hg); g.w_2 = take(H * H); g.w_3 = take(g.N3p * H);
   g.w_total = (int)up64(o);
+  o = g.w_total;
+  g.f_wih0 = take(G3 * gin); g.f_bih0 = take(G3); g.f_bhh0 = take(G3); g.f_hh0t = take(Hg * G3); g.f_ih1t = take(Hg * G3);
+  g.f_hh1t = take(Hg * G3); g.f_bih1 = take(G3); g.f_bhh1 = take(G3); g.f_wout = take(2 * Hg); g.f_bout = take(2);
+  g.f_w1t = take(g.in0 * H); g.f_b1 = take(H); g.f_w2t = take(H * H); g.f_b2 = take(H); g.f_w3t = take(H * g.N3p); g.f_b3 = take(g.N3p);
+  g.f_total = (int)up64(o);
   return g;
 }
 
+// The weights the tile steps read, in ModelDev's layouts: the handle's fp32 arena, or (T = double) the image
+// model_f64_weights_kernel builds in the workspace from the caller's parameters.
+template <typename T>
+struct TileW {
+  const T *w_ih0, *b_ih0, *b_hh0, *w_hh0_t, *w_ih1_t, *w_hh1_t, *b_ih1, *b_hh1, *w_out, *b_out;
+  const T *w1_full_t, *b1_raw, *w2_t, *b2, *w3_t, *b3;
+  const T *state_mean, *state_inv_std, *act_mean, *act_inv_std;
+};
+
+static TileW<float> tile_w(const ModelDev& d) {
+  TileW<float> w;
+  w.w_ih0 = d.w_ih0; w.b_ih0 = d.b_ih0; w.b_hh0 = d.b_hh0; w.w_hh0_t = d.w_hh0_t; w.w_ih1_t = d.w_ih1_t; w.w_hh1_t = d.w_hh1_t;
+  w.b_ih1 = d.b_ih1; w.b_hh1 = d.b_hh1; w.w_out = d.w_out; w.b_out = d.b_out;
+  w.w1_full_t = d.w1_full_t; w.b1_raw = d.b1_raw; w.w2_t = d.w2_t; w.b2 = d.b2; w.w3_t = d.w3_t; w.b3 = d.b3;
+  w.state_mean = d.state_mean; w.state_inv_std = d.state_inv_std; w.act_mean = d.act_mean; w.act_inv_std = d.act_inv_std;
+  return w;
+}
+
+static TileW<double> tile_w_f64(const ModelDev& d, const GradShape& g, const double* img) {
+  TileW<double> w;
+  w.w_ih0 = img + g.f_wih0; w.b_ih0 = img + g.f_bih0; w.b_hh0 = img + g.f_bhh0; w.w_hh0_t = img + g.f_hh0t; w.w_ih1_t = img + g.f_ih1t;
+  w.w_hh1_t = img + g.f_hh1t; w.b_ih1 = img + g.f_bih1; w.b_hh1 = img + g.f_bhh1; w.w_out = img + g.f_wout; w.b_out = img + g.f_bout;
+  w.w1_full_t = img + g.f_w1t; w.b1_raw = img + g.f_b1; w.w2_t = img + g.f_w2t; w.b2 = img + g.f_b2; w.w3_t = img + g.f_w3t;
+  w.b3 = img + g.f_b3;
+  w.state_mean = d.state_mean64; w.state_inv_std = d.state_inv_std64; w.act_mean = d.act_mean64; w.act_inv_std = d.act_inv_std64;
+  return w;
+}
+
+template <typename T>
 struct GradArgs {
-  ModelDev m;
+  TileW<T> m;
   GradShape g;
-  const float* obs;       // [K][nx]
-  const float* act;       // [K][B][gin]
-  const float* gout;      // [K][nx]
-  const float* row_b1;    // [K][H]
-  const float* row_tn;    // [K]
-  const float* row_sph;   // [K][2S]
-  const float* wt;        // transposed weight copies
-  float* part;            // [grid][p_total]
-  float* scratch;         // [grid][s_total]
-  float* grad_obs;        // [K][nx] or null
-  float* grad_act;        // [K][B][gin] or null
+  const T* obs;       // [K][nx]
+  const T* act;       // [K][B][gin]
+  const T* gout;      // [K][nx]
+  const T* row_b1;    // [K][H]
+  const T* row_tn;    // [K]
+  const T* row_sph;   // [K][2S]
+  const T* wt;        // transposed weight copies
+  T* part;            // [grid][p_total]
+  T* scratch;         // [grid][s_total]
+  T* grad_obs;        // [K][nx] or null
+  T* grad_act;        // [K][B][gin] or null
   int K, n_tiles;
 };
 
 // ------------------------------------------------------------------------------------------------------------------
 // Tile products.  Rows are the kGradRows samples of the tile; every thread owns fixed 4 x 4 output blocks, so an output
 // element is always written by the same thread (repeated accumulating calls on one output need no barrier between them).
+// Everything from here to the kernels is templated on the scalar type T (float: the fp32 backward; double: the fp64
+// forward and backward).
 // ------------------------------------------------------------------------------------------------------------------
 enum { kEpiNone = 0, kEpiTanh = 1, kEpiDtanh = 2 };
 
 // C[m][n] (+)= sum_k A[m][k] W[k][n]  (+ bias[n]; kEpiTanh: tanh of it; kEpiDtanh: times 1 - aux[m][n]^2).
 // N, Kd, lda, ldw, ldc multiples of 4; W is read-only for the kernel's lifetime.
-template <int EPI>
-__device__ __forceinline__ void gemm_nn(const float* A, int lda, const float* __restrict__ W, int ldw, int Kd, int N, float* C, int ldc,
-                                        bool accumulate, const float* __restrict__ bias = nullptr, const float* aux = nullptr) {
+template <int EPI, typename T>
+__device__ __forceinline__ void gemm_nn(const T* A, int lda, const T* __restrict__ W, int ldw, int Kd, int N, T* C, int ldc,
+                                        bool accumulate, const T* __restrict__ bias = nullptr, const T* aux = nullptr) {
   const int CG = N / 4, items = (kGradRows / 4) * CG;
   for (int it = threadIdx.x; it < items; it += kGradThreads) {
     const int rg = it / CG, cg = it - rg * CG;
-    float c[4][4];
+    T c[4][4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (accumulate) v = *reinterpret_cast<const float4*>(C + (4 * rg + i) * ldc + 4 * cg);
-      else if (bias) v = *reinterpret_cast<const float4*>(bias + 4 * cg);
-      c[i][0] = v.x; c[i][1] = v.y; c[i][2] = v.z; c[i][3] = v.w;
+      if (accumulate) rm::ld4(C + (4 * rg + i) * ldc + 4 * cg, c[i]);
+      else if (bias) rm::ld4(bias + 4 * cg, c[i]);
+      else c[i][0] = c[i][1] = c[i][2] = c[i][3] = T(0);
     }
 #pragma unroll 2
     for (int k = 0; k < Kd; k += 4) {
-      float4 a[4];
+      T a[4][4];
 #pragma unroll
-      for (int i = 0; i < 4; ++i) a[i] = *reinterpret_cast<const float4*>(A + (4 * rg + i) * lda + k);
+      for (int i = 0; i < 4; ++i) rm::ld4(A + (4 * rg + i) * lda + k, a[i]);
 #pragma unroll
       for (int kk = 0; kk < 4; ++kk) {
-        const float4 w = __ldg(reinterpret_cast<const float4*>(W + (size_t)(k + kk) * ldw + 4 * cg));
+        T w[4];
+        rm::ldg4(W + (size_t)(k + kk) * ldw + 4 * cg, w);
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-          const float av = kk == 0 ? a[i].x : (kk == 1 ? a[i].y : (kk == 2 ? a[i].z : a[i].w));
-          c[i][0] = fmaf(av, w.x, c[i][0]);
-          c[i][1] = fmaf(av, w.y, c[i][1]);
-          c[i][2] = fmaf(av, w.z, c[i][2]);
-          c[i][3] = fmaf(av, w.w, c[i][3]);
+          const T av = a[i][kk];
+          c[i][0] = rm::fma(av, w[0], c[i][0]);
+          c[i][1] = rm::fma(av, w[1], c[i][1]);
+          c[i][2] = rm::fma(av, w[2], c[i][2]);
+          c[i][3] = rm::fma(av, w[3], c[i][3]);
         }
       }
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-      float* dst = C + (4 * rg + i) * ldc + 4 * cg;
+      T* dst = C + (4 * rg + i) * ldc + 4 * cg;
       if (EPI == kEpiTanh) {
         for (int j = 0; j < 4; ++j) c[i][j] = tanh_acc(c[i][j]);
       } else if (EPI == kEpiDtanh) {
-        const float4 y = *reinterpret_cast<const float4*>(aux + (4 * rg + i) * ldc + 4 * cg);
-        c[i][0] *= 1.0f - y.x * y.x; c[i][1] *= 1.0f - y.y * y.y; c[i][2] *= 1.0f - y.z * y.z; c[i][3] *= 1.0f - y.w * y.w;
+        T y[4];
+        rm::ld4(aux + (4 * rg + i) * ldc + 4 * cg, y);
+        c[i][0] *= T(1) - y[0] * y[0]; c[i][1] *= T(1) - y[1] * y[1]; c[i][2] *= T(1) - y[2] * y[2]; c[i][3] *= T(1) - y[3] * y[3];
       }
-      *reinterpret_cast<float4*>(dst) = make_float4(c[i][0], c[i][1], c[i][2], c[i][3]);
+      rm::st4(dst, c[i]);
     }
   }
 }
 
 // Weight gradient: P[k][n] += sum_{s in [s0, s1)} sum_m A_s[m][k] D_s[m][col(n)], A_s = A + (s - alag) sA, D_s = D + s sD,
 // col(n) = n + (n >= nsplit ? dshift : 0) (skips a gate slot of the saved GRU gradients).  Kd, N, nsplit multiples of 4.
-__device__ __forceinline__ void wgrad(float* P, int ldp, const float* A, int lda, int sA, int alag, const float* D, int ldd, int sD,
+template <typename T>
+__device__ __forceinline__ void wgrad(T* P, int ldp, const T* A, int lda, int sA, int alag, const T* D, int ldd, int sD,
                                       int s0, int s1, int Kd, int N, int nsplit, int dshift) {
   const int CG = N / 4, items = (Kd / 4) * CG;
   for (int it = threadIdx.x; it < items; it += kGradThreads) {
     const int kg = it / CG, cg = it - kg * CG;
     const int dc = 4 * cg + (4 * cg >= nsplit ? dshift : 0);
-    float c[4][4] = {};
+    T c[4][4] = {};
     for (int s = s0; s < s1; ++s) {
-      const float* As = A + (s - alag) * sA + 4 * kg;
-      const float* Ds = D + s * sD + dc;
+      const T* As = A + (s - alag) * sA + 4 * kg;
+      const T* Ds = D + s * sD + dc;
 #pragma unroll 4
       for (int m = 0; m < kGradRows; ++m) {
-        const float4 a = *reinterpret_cast<const float4*>(As + m * lda);
-        const float4 d = *reinterpret_cast<const float4*>(Ds + m * ldd);
-        const float av[4] = {a.x, a.y, a.z, a.w}, dv[4] = {d.x, d.y, d.z, d.w};
+        T av[4], dv[4];
+        rm::ld4(As + m * lda, av);
+        rm::ld4(Ds + m * ldd, dv);
 #pragma unroll
         for (int i = 0; i < 4; ++i)
 #pragma unroll
-          for (int j = 0; j < 4; ++j) c[i][j] = fmaf(av[i], dv[j], c[i][j]);
+          for (int j = 0; j < 4; ++j) c[i][j] = rm::fma(av[i], dv[j], c[i][j]);
       }
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-      float4* p = reinterpret_cast<float4*>(P + (4 * kg + i) * ldp + 4 * cg);
-      float4 v = *p;
-      v.x += c[i][0]; v.y += c[i][1]; v.z += c[i][2]; v.w += c[i][3];
-      *p = v;
+      T* p = P + (4 * kg + i) * ldp + 4 * cg;
+      T v[4];
+      rm::ld4(p, v);
+      v[0] += c[i][0]; v[1] += c[i][1]; v[2] += c[i][2]; v[3] += c[i][3];
+      rm::st4(p, v);
     }
   }
 }
 
 // Bias gradient: P[n] += sum_{s in [s0, s1)} sum_m D_s[m][col(n)]
-__device__ __forceinline__ void colsum(float* P, const float* D, int ldd, int sD, int s0, int s1, int N, int nsplit, int dshift) {
+template <typename T>
+__device__ __forceinline__ void colsum(T* P, const T* D, int ldd, int sD, int s0, int s1, int N, int nsplit, int dshift) {
   for (int n = threadIdx.x; n < N; n += kGradThreads) {
     const int dc = n + (n >= nsplit ? dshift : 0);
-    float acc = 0.0f;
+    T acc = T(0);
     for (int s = s0; s < s1; ++s)
       for (int m = 0; m < kGradRows; ++m) acc += D[s * sD + m * ldd + dc];
     P[n] += acc;
@@ -213,97 +264,115 @@ __device__ __forceinline__ void colsum(float* P, const float* D, int ldd, int sD
 
 // GRU cell forward (torch.nn.GRU, gate order r, z, n; the same expressions as encode_gru.cu gru_finish).  gi / gh are the
 // bias-free products (gh null: zero state); layer 0 (gin inputs) forms gi here from the step's window entry.
-__device__ __forceinline__ void gru_cell_fwd(const GradShape& g, const float* __restrict__ b_i, const float* __restrict__ b_h,
-                                             const float* __restrict__ w_ih0, const float* xs, const float* gi, const float* gh,
-                                             const float* hprev, float* gate, float* hout) {
+template <typename T>
+__device__ __forceinline__ void gru_cell_fwd(const GradShape& g, const T* __restrict__ b_i, const T* __restrict__ b_h,
+                                             const T* __restrict__ w_ih0, const T* xs, const T* gi, const T* gh,
+                                             const T* hprev, T* gate, T* hout) {
   const int Hg = g.Hg, G3 = g.G3;
   for (int i = threadIdx.x; i < kGradRows * Hg; i += kGradThreads) {
     const int m = i / Hg, u = i - m * Hg;
-    float gir, giz, gin_;
+    T gir, giz, gin_;
     if (gi) {
       gir = gi[m * G3 + u]; giz = gi[m * G3 + Hg + u]; gin_ = gi[m * G3 + 2 * Hg + u];
     } else {
-      float acc[3];
+      T acc[3];
 #pragma unroll
       for (int q = 0; q < 3; ++q) {
-        const float* w = w_ih0 + (q * Hg + u) * g.gin;
-        float a = 0.0f;
-        for (int v = 0; v < g.gin; ++v) a = fmaf(w[v], xs[m * 4 + v], a);
+        const T* w = w_ih0 + (q * Hg + u) * g.gin;
+        T a = T(0);
+        for (int v = 0; v < g.gin; ++v) a = rm::fma(w[v], xs[m * 4 + v], a);
         acc[q] = a;
       }
       gir = acc[0]; giz = acc[1]; gin_ = acc[2];
     }
-    const float ghr = gh ? gh[m * G3 + u] : 0.0f, ghz = gh ? gh[m * G3 + Hg + u] : 0.0f, ghn0 = gh ? gh[m * G3 + 2 * Hg + u] : 0.0f;
-    const float r = sigmoid_acc((gir + b_i[u]) + (ghr + b_h[u]));
-    const float z = sigmoid_acc((giz + b_i[Hg + u]) + (ghz + b_h[Hg + u]));
-    const float ghn = ghn0 + b_h[2 * Hg + u];
-    const float n = tanh_acc((gin_ + b_i[2 * Hg + u]) + r * ghn);
-    const float ho = hprev ? hprev[m * Hg + u] : 0.0f;
-    float* gt = gate + m * 4 * Hg;
+    const T ghr = gh ? gh[m * G3 + u] : T(0), ghz = gh ? gh[m * G3 + Hg + u] : T(0), ghn0 = gh ? gh[m * G3 + 2 * Hg + u] : T(0);
+    const T r = sigmoid_acc((gir + b_i[u]) + (ghr + b_h[u]));
+    const T z = sigmoid_acc((giz + b_i[Hg + u]) + (ghz + b_h[Hg + u]));
+    const T ghn = ghn0 + b_h[2 * Hg + u];
+    const T n = tanh_acc((gin_ + b_i[2 * Hg + u]) + r * ghn);
+    const T ho = hprev ? hprev[m * Hg + u] : T(0);
+    T* gt = gate + m * 4 * Hg;
     gt[u] = r; gt[Hg + u] = z; gt[2 * Hg + u] = n; gt[3 * Hg + u] = ghn;
-    hout[m * Hg + u] = fmaf(z, ho - n, n);
+    hout[m * Hg + u] = rm::fma(z, ho - n, n);
   }
 }
 
 // GRU cell backward: dh -> (dr_pre, dz_pre, dn_pre, d(W_hn h + b_hn)) in place of the saved gates, dh_prev's direct part.
-__device__ __forceinline__ void gru_cell_bwd(const GradShape& g, const float* dh, const float* hprev, float* gate, float* dh_prev) {
+template <typename T>
+__device__ __forceinline__ void gru_cell_bwd(const GradShape& g, const T* dh, const T* hprev, T* gate, T* dh_prev) {
   const int Hg = g.Hg;
   for (int i = threadIdx.x; i < kGradRows * Hg; i += kGradThreads) {
     const int m = i / Hg, u = i - m * Hg;
-    float* gt = gate + m * 4 * Hg;
-    const float r = gt[u], z = gt[Hg + u], n = gt[2 * Hg + u], ghn = gt[3 * Hg + u];
-    const float d = dh[m * Hg + u], ho = hprev ? hprev[m * Hg + u] : 0.0f;
-    const float dn = d * (1.0f - z) * (1.0f - n * n);
-    const float dr = dn * ghn * r * (1.0f - r);
-    const float dz = d * (ho - n) * z * (1.0f - z);
+    T* gt = gate + m * 4 * Hg;
+    const T r = gt[u], z = gt[Hg + u], n = gt[2 * Hg + u], ghn = gt[3 * Hg + u];
+    const T d = dh[m * Hg + u], ho = hprev ? hprev[m * Hg + u] : T(0);
+    const T dn = d * (T(1) - z) * (T(1) - n * n);
+    const T dr = dn * ghn * r * (T(1) - r);
+    const T dz = d * (ho - n) * z * (T(1) - z);
     gt[u] = dr; gt[Hg + u] = dz; gt[2 * Hg + u] = dn; gt[3 * Hg + u] = dn * r;
     dh_prev[m * Hg + u] = d * z;
   }
 }
 
-// The per-CTA scratch of a tile (GradShape s_* offsets).
+// The per-CTA scratch of a tile (GradShape s_* offsets, in elements of T).
+template <typename T>
 struct TileBufs {
-  float *xs, *gate, *hs, *gi, *gh, *x1, *a1, *a2, *dob, *dz2, *dz1, *dhb, *dxt, *rc;
+  T *xs, *gate, *hs, *gi, *gh, *x1, *a1, *a2, *dob, *dz2, *dz1, *dhb, *dxt, *rc;
 };
-__device__ __forceinline__ TileBufs tile_bufs(const GradShape& g, float* sc) {
-  TileBufs t;
+template <typename T>
+__device__ __forceinline__ TileBufs<T> tile_bufs(const GradShape& g, T* sc) {
+  TileBufs<T> t;
   t.xs = sc + g.s_xs; t.gate = sc + g.s_gate; t.hs = sc + g.s_h; t.gi = sc + g.s_gi; t.gh = sc + g.s_gh; t.x1 = sc + g.s_x1;
   t.a1 = sc + g.s_a1; t.a2 = sc + g.s_a2; t.dob = sc + g.s_do; t.dz2 = sc + g.s_dz2; t.dz1 = sc + g.s_dz1; t.dhb = sc + g.s_dh;
   t.dxt = sc + g.s_dxt; t.rc = sc + g.s_rc;
   return t;
 }
 // gate [l][st] at (l * B + st) * R * 4Hg, h [l][st] at (l * B + st) * R * Hg
-__device__ __forceinline__ float* tile_gate(const GradShape& g, const TileBufs& t, int l, int st) {
+template <typename T>
+__device__ __forceinline__ T* tile_gate(const GradShape& g, const TileBufs<T>& t, int l, int st) {
   return t.gate + (size_t)(l * g.B + st) * kGradRows * 4 * g.Hg;
 }
-__device__ __forceinline__ float* tile_h(const GradShape& g, const TileBufs& t, int l, int st) {
+template <typename T>
+__device__ __forceinline__ T* tile_h(const GradShape& g, const TileBufs<T>& t, int l, int st) {
   return t.hs + (size_t)(l * g.B + st) * kGradRows * g.Hg;
 }
 
 // Normalised window of samples k0 .. k0 + R - 1 (w_nl.py:121); rows past K repeat sample K - 1.
-__device__ __forceinline__ void tile_load_window(const GradShape& g, const ModelDev& md, const float* act, int k0, int K, float* xs) {
+template <typename T>
+__device__ __forceinline__ void tile_load_window(const GradShape& g, const TileW<T>& md, const T* act, int k0, int K, T* xs) {
   const int B = g.B, gin = g.gin, R = kGradRows;
   for (int i = threadIdx.x; i < B * R * 4; i += kGradThreads) {
     const int st = i / (R * 4), m = (i / 4) % R, u = i & 3;
     const int k = min(k0 + m, K - 1), j = B - 1 - st;  // step st reads entry B-1-st (reversed in time, w_nl.py:27)
-    xs[i] = u < gin ? (act[((size_t)k * B + j) * gin + u] - md.act_mean[u]) * md.act_inv_std[u] : 0.0f;
+    xs[i] = u < gin ? (act[((size_t)k * B + j) * gin + u] - md.act_mean[u]) * md.act_inv_std[u] : T(0);
   }
 }
 
 // Per-row Fourier constants pi t / T and exp(gamma t) / T of rows k0 .. k0 + R - 1 (rollout.cu rollout_nl_kernel: the same).
-__device__ __forceinline__ void tile_fourier_consts(const float* row_tn, int k0, int K, float* rc) {
+template <typename T>
+__device__ __forceinline__ void tile_fourier_consts(const T* row_tn, int k0, int K, T* rc) {
+  using C = Real<T>;
   const int R = kGradRows;
   for (int m = threadIdx.x; m < R; m += kGradThreads) {
-    const float tn = row_tn[min(k0 + m, K - 1)];
-    const float T = 2.0f * (tn + 1.0e-6f);
-    rc[m] = 3.14159265358979f * 1.0e-6f / T;
-    rc[R + m] = expf((1.0e-3f + 4.605170185988091f / T) * tn) / T;
+    const T tn = row_tn[min(k0 + m, K - 1)];
+    const T Tp = T(2) * (tn + C::eps);
+    rc[m] = C::pi * C::eps / Tp;
+    rc[R + m] = rm::exp((C::alpha + C::ln_inv_tol / Tp) * tn) / Tp;
   }
 }
 
+// Phase k pi t / T (the quarter turns exact, reduced to (-pi, pi] up to k delta) and Fourier weight of term kk of row m.
+template <typename T>
+__device__ __forceinline__ void ilt_term_consts(int kk, const T* rc, int m, T& ph, T& wt) {
+  using C = Real<T>;
+  const T quarter = (kk & 3) == 0 ? T(0) : ((kk & 3) == 1 ? C::half_pi : ((kk & 3) == 2 ? C::pi : -C::half_pi));
+  ph = quarter - (T)kk * rc[m];
+  wt = rc[kGradRows + m] * (kk == 0 ? T(0.5) : T(1));
+}
+
 // Encoder forward (w_nl.py:25-29) of the tile's windows, saving every cell.  Ends on a barrier.
-template <int H>
-__device__ __forceinline__ void tile_encoder_fwd(const GradShape& g, const ModelDev& md, const TileBufs& t) {
+template <int H, typename T>
+__device__ __forceinline__ void tile_encoder_fwd(const GradShape& g, const TileW<T>& md, const TileBufs<T>& t) {
   constexpr int Hg = H / 2, G3 = 3 * Hg;
   const int B = g.B;
   for (int st = 0; st < B; ++st) {
@@ -311,34 +380,61 @@ __device__ __forceinline__ void tile_encoder_fwd(const GradShape& g, const Model
       gemm_nn<kEpiNone>(tile_h(g, t, 0, st - 1), Hg, md.w_hh0_t, G3, Hg, G3, t.gh, G3, false);
       __syncthreads();
     }
-    gru_cell_fwd(g, md.b_ih0, md.b_hh0, md.w_ih0, t.xs + st * kGradRows * 4, nullptr, st > 0 ? t.gh : nullptr,
+    gru_cell_fwd(g, md.b_ih0, md.b_hh0, md.w_ih0, t.xs + st * kGradRows * 4, (const T*)nullptr, st > 0 ? t.gh : nullptr,
                  st > 0 ? tile_h(g, t, 0, st - 1) : nullptr, tile_gate(g, t, 0, st), tile_h(g, t, 0, st));
     __syncthreads();
     gemm_nn<kEpiNone>(tile_h(g, t, 0, st), Hg, md.w_ih1_t, G3, Hg, G3, t.gi, G3, false);
     if (st > 0) gemm_nn<kEpiNone>(tile_h(g, t, 1, st - 1), Hg, md.w_hh1_t, G3, Hg, G3, t.gh, G3, false);
     __syncthreads();
-    gru_cell_fwd(g, md.b_ih1, md.b_hh1, nullptr, nullptr, t.gi, st > 0 ? t.gh : nullptr, st > 0 ? tile_h(g, t, 1, st - 1) : nullptr,
-                 tile_gate(g, t, 1, st), tile_h(g, t, 1, st));
+    gru_cell_fwd(g, md.b_ih1, md.b_hh1, (const T*)nullptr, (const T*)nullptr, t.gi, st > 0 ? t.gh : nullptr,
+                 st > 0 ? tile_h(g, t, 1, st - 1) : nullptr, tile_gate(g, t, 1, st), tile_h(g, t, 1, st));
     __syncthreads();
   }
 }
 
-// Representation MLP forward (w_nl.py:55-63) from the first-layer input x1 and the Fourier constants rc, the ILT + sphere map
-// derivatives against gout, the MLP backward into the partial P, and the gradient of [obs_n | p_action] into dxt.  Rows
-// k0 .. k0 + R - 1 of row_b1 [K][H] and gout [K][nx]; rows past K get zero output gradients.  Ends on a barrier.
-template <int H>
-__device__ __forceinline__ void tile_mlp_fwd_bwd(const GradShape& g, const ModelDev& md, const float* wt, float* P, const TileBufs& t,
-                                                 const float* row_b1, const float* gout, int k0, int K) {
+// linear_out (w_nl.py:29) of the tile's last top-layer state -> the p_action columns of the MLP input x1.  No barrier.
+template <typename T>
+__device__ __forceinline__ void tile_linear_out(const GradShape& g, const TileW<T>& md, const TileBufs<T>& t) {
+  const int Hg = g.Hg, base = 2 * g.S + g.nx;
+  const T* h1last = tile_h(g, t, 1, g.B - 1);
+  for (int i = threadIdx.x; i < kGradRows * 2; i += kGradThreads) {
+    const int m = i >> 1, o = i & 1;
+    T acc = md.b_out[o];
+    for (int k = 0; k < Hg; ++k) acc = rm::fma(md.w_out[o * Hg + k], h1last[m * Hg + k], acc);
+    t.x1[m * g.in0p + base + o] = acc;
+  }
+}
+
+// First-layer input [theta_s | phi_s | obs_n | p_action | 0] of rows k0 .. k0 + R - 1 of a chunk whose row r is (sample
+// (r0 + r) / n_t, time (r0 + r) % n_t): sphere coordinates from row_sph [rows][2S], obs [K][nx] and p [K][2] per sample.
+template <typename T>
+__device__ __forceinline__ void tile_rows_input(const GradShape& g, const TileW<T>& md, const T* row_sph, const T* obs, const T* p,
+                                                long long r0, int rows, int n_t, int k0, T* x1) {
+  const int S = g.S, nx = g.nx, Lp = g.Lp, in0p = g.in0p;
+  for (int i = threadIdx.x; i < kGradRows * in0p; i += kGradThreads) {
+    const int m = i / in0p, j = i - m * in0p;
+    const int r = min(k0 + m, rows - 1);
+    const size_t k = (size_t)((r0 + r) / n_t);
+    T v = T(0);
+    if (j < 2 * S) v = row_sph[(size_t)r * 2 * S + j];
+    else if (j < 2 * S + nx) v = (obs[k * nx + (j - 2 * S)] - md.state_mean[j - 2 * S]) * md.state_inv_std[j - 2 * S];
+    else if (j < 2 * S + Lp) v = p[k * 2 + (j - 2 * S - nx)];
+    x1[i] = v;
+  }
+}
+
+// Representation MLP forward (w_nl.py:55-63) from the first-layer input x1: a1, a2 and the last layer's pre-activations
+// in dob.  Rows k0 .. k0 + R - 1 of row_b1 [K][H] (the s-columns, forward_ts_prep_kernel).  Ends on a barrier.
+template <int H, typename T>
+__device__ __forceinline__ void tile_mlp_fwd(const GradShape& g, const TileW<T>& md, const TileBufs<T>& t, const T* row_b1, int k0,
+                                             int K) {
   constexpr int R = kGradRows;
-  const int S = g.S, nx = g.nx, Lp = g.Lp, in0p = g.in0p, N3p = g.N3p, nP = nx * S;
-  const int tid = threadIdx.x;
-  const float* W2 = wt + g.w_2;  // [H][H]   (out, in)
-  const float* W3 = wt + g.w_3;  // [N3p][H] (paired output column, in)
-  float *x1 = t.x1, *a1 = t.a1, *a2 = t.a2, *dob = t.dob, *dz2 = t.dz2, *dz1 = t.dz1, *dxt = t.dxt, *rc = t.rc;
-  for (int i = tid; i < R * H; i += kGradThreads) {  // the s-columns are in row_b1 (forward_ts_prep_kernel)
+  const int S = g.S, Lp = g.Lp, in0p = g.in0p, N3p = g.N3p;
+  T *x1 = t.x1, *a1 = t.a1, *a2 = t.a2, *dob = t.dob;
+  for (int i = threadIdx.x; i < R * H; i += kGradThreads) {
     const int m = i / H, n = i - m * H;
-    float acc = row_b1[(size_t)min(k0 + m, K - 1) * H + n];
-    for (int j = 0; j < Lp; ++j) acc = fmaf(md.w1_full_t[(size_t)(2 * S + j) * H + n], x1[m * in0p + 2 * S + j], acc);
+    T acc = row_b1[(size_t)min(k0 + m, K - 1) * H + n];
+    for (int j = 0; j < Lp; ++j) acc = rm::fma(md.w1_full_t[(size_t)(2 * S + j) * H + n], x1[m * in0p + 2 * S + j], acc);
     a1[i] = tanh_acc(acc);
   }
   __syncthreads();
@@ -346,47 +442,81 @@ __device__ __forceinline__ void tile_mlp_fwd_bwd(const GradShape& g, const Model
   __syncthreads();
   gemm_nn<kEpiNone>(a2, H, md.w3_t, N3p, H, N3p, dob, N3p, false, md.b3);
   __syncthreads();
+}
+
+// The ILT of tile_mlp_fwd's output (w_nl.py:59-62 + the Fourier series, oracle/ilt.py): out[k0 + m][c] =
+// sum_k w_k rho_k cos(theta_k + a_k), k ascending, for the rows below K.  No barrier.
+template <typename T>
+__device__ __forceinline__ void tile_ilt_out(const GradShape& g, const TileBufs<T>& t, int k0, int K, T* out) {
+  using C = Real<T>;
+  const int S = g.S, nx = g.nx, N3p = g.N3p;
+  for (int i = threadIdx.x; i < kGradRows * nx; i += kGradThreads) {
+    const int m = i / nx, c = i - m * nx;
+    if (k0 + m >= K) continue;
+    const T* o = t.dob + m * N3p + 2 * c * S;
+    T acc = T(0);
+    for (int kk = 0; kk < S; ++kk) {
+      T ph, wt;
+      ilt_term_consts(kk, t.rc, m, ph, wt);
+      acc += wt * sphere_radius(o[2 * kk + 1]) * cos_reduced(C::pi * tanh_acc(o[2 * kk]) + ph);
+    }
+    out[(size_t)(k0 + m) * nx + c] = acc;
+  }
+}
+
+// After tile_mlp_fwd: the ILT + sphere map derivatives against gout, the MLP backward into the partial P, and the gradient
+// of [obs_n | p_action] into dxt.  Rows k0 .. k0 + R - 1 of gout [K][nx]; rows past K get zero output gradients.  Ends on
+// a barrier.
+template <int H, typename T>
+__device__ __forceinline__ void tile_mlp_bwd(const GradShape& g, const TileW<T>& md, const T* wt, T* P, const TileBufs<T>& t,
+                                             const T* gout, int k0, int K) {
+  using C = Real<T>;
+  constexpr int R = kGradRows;
+  const int S = g.S, nx = g.nx, Lp = g.Lp, in0p = g.in0p, N3p = g.N3p, nP = nx * S;
+  const int tid = threadIdx.x;
+  const T* W2 = wt + g.w_2;  // [H][H]   (out, in)
+  const T* W3 = wt + g.w_3;  // [N3p][H] (paired output column, in)
+  T *x1 = t.x1, *a1 = t.a1, *a2 = t.a2, *dob = t.dob, *dz2 = t.dz2, *dz1 = t.dz1, *dxt = t.dxt, *rc = t.rc;
   // ---- ILT + sphere map derivatives: Dx_c = sum_k w_k rho cos(theta + a_k), theta = pi tanh(u_t), rho = tan((pi/2) sigma(2 u_p)) ----
   for (int i = tid; i < R * (N3p / 2); i += kGradThreads) {
     const int m = i / (N3p / 2), pair = i - m * (N3p / 2);
-    float* o = dob + m * N3p + 2 * pair;
-    if (pair >= nP) { o[0] = 0.0f; o[1] = 0.0f; continue; }
+    T* o = dob + m * N3p + 2 * pair;
+    if (pair >= nP) { o[0] = T(0); o[1] = T(0); continue; }
     const int c = pair / S, kk = pair - c * S;
     const bool valid = k0 + m < K;
-    const float gc = valid ? gout[(size_t)(k0 + m) * nx + c] : 0.0f;
-    const float quarter = (kk & 3) == 0 ? 0.0f : ((kk & 3) == 1 ? 1.57079632679489662f : ((kk & 3) == 2 ? 3.14159265358979f : -1.57079632679489662f));
-    const float ph = quarter - (float)kk * rc[m];
-    const float wt = rc[R + m] * (kk == 0 ? 0.5f : 1.0f);
-    const float ut = o[0], up = o[1];
+    const T gc = valid ? gout[(size_t)(k0 + m) * nx + c] : T(0);
+    T ph, wk;
+    ilt_term_consts(kk, rc, m, ph, wk);
+    const T ut = o[0], up = o[1];
     // sech^2 u and sigma(2u) sigma(-2u) through e = exp(-2|u|): no cancellation in either tail (DESIGN.md 2.6)
-    const float et = exp_acc(-2.0f * fminf(fabsf(ut), 40.0f));
-    const float sech2 = 4.0f * et * __frcp_rn((1.0f + et) * (1.0f + et));
-    const float ep = exp_acc(-2.0f * fminf(fabsf(up), 40.0f));
-    const float ss = ep * __frcp_rn((1.0f + ep) * (1.0f + ep));
-    const float rho = sphere_radius(up);
-    const float arg = 3.14159265358979f * tanh_acc(ut) + ph;  // |arg| < 2 pi: cos_reduced's range
-    const float cs = cos_reduced(arg), sn = cos_reduced(arg - 1.57079632679489662f);
-    const float gw = gc * wt;
-    o[0] = -gw * rho * sn * 3.14159265358979f * sech2;
-    o[1] = gw * cs * 3.14159265358979f * fmaf(rho, rho * ss, ss);  // (1 + rho^2) ss without forming rho^2
+    const T et = exp_acc(T(-2) * rm::min(rm::abs(ut), T(40)));
+    const T sech2 = T(4) * et * rm::rcp((T(1) + et) * (T(1) + et));
+    const T ep = exp_acc(T(-2) * rm::min(rm::abs(up), T(40)));
+    const T ss = ep * rm::rcp((T(1) + ep) * (T(1) + ep));
+    const T rho = sphere_radius(up);
+    const T arg = C::pi * tanh_acc(ut) + ph;  // |arg| < 2 pi: cos_reduced's range
+    const T cs = cos_reduced(arg), sn = cos_reduced(arg - C::half_pi);
+    const T gw = gc * wk;
+    o[0] = -gw * rho * sn * C::pi * sech2;
+    o[1] = gw * cs * C::pi * rm::fma(rho, rho * ss, ss);  // (1 + rho^2) ss without forming rho^2
   }
   __syncthreads();
   // ---- MLP backward ----
   wgrad(P + g.p_w4, N3p, a2, H, 0, 0, dob, N3p, 0, 0, 1, H, N3p, N3p, 0);
   colsum(P + g.p_b4, dob, N3p, 0, 0, 1, N3p, N3p, 0);
-  gemm_nn<kEpiDtanh>(dob, N3p, W3, H, N3p, H, dz2, H, false, nullptr, a2);
+  gemm_nn<kEpiDtanh>(dob, N3p, W3, H, N3p, H, dz2, H, false, (const T*)nullptr, a2);
   __syncthreads();
   wgrad(P + g.p_w2, H, a1, H, 0, 0, dz2, H, 0, 0, 1, H, H, H, 0);
   colsum(P + g.p_b2, dz2, H, 0, 0, 1, H, H, 0);
-  gemm_nn<kEpiDtanh>(dz2, H, W2, H, H, H, dz1, H, false, nullptr, a1);
+  gemm_nn<kEpiDtanh>(dz2, H, W2, H, H, H, dz1, H, false, (const T*)nullptr, a1);
   __syncthreads();
   wgrad(P + g.p_w0, H, x1, in0p, 0, 0, dz1, H, 0, 0, 1, in0p, H, H, 0);
   colsum(P + g.p_b0, dz1, H, 0, 0, 1, H, H, 0);
   for (int i = tid; i < R * Lp; i += kGradThreads) {  // gradient of [obs_n | p_action]
     const int m = i / Lp, j = i - m * Lp;
-    const float* w = md.w1_full_t + (size_t)(2 * S + j) * H;
-    float acc = 0.0f;
-    for (int n = 0; n < H; ++n) acc = fmaf(dz1[m * H + n], w[n], acc);
+    const T* w = md.w1_full_t + (size_t)(2 * S + j) * H;
+    T acc = T(0);
+    for (int n = 0; n < H; ++n) acc = rm::fma(dz1[m * H + n], w[n], acc);
     dxt[m * 16 + j] = acc;
   }
   __syncthreads();
@@ -394,17 +524,17 @@ __device__ __forceinline__ void tile_mlp_fwd_bwd(const GradShape& g, const Model
 
 // From the gradient of [obs_n | p_action] in dxt: grad_obs, linear_out backward and BPTT through both GRU layers over the
 // reversed window (the saved cells of tile_encoder_fwd), grad_act, and the GRU weight gradients into the partial P.
-template <int H>
-__device__ __forceinline__ void tile_encoder_bwd(const GradShape& g, const ModelDev& md, const float* wt, float* P, const TileBufs& t,
-                                                 float* grad_obs, float* grad_act, int k0, int K) {
+template <int H, typename T>
+__device__ __forceinline__ void tile_encoder_bwd(const GradShape& g, const TileW<T>& md, const T* wt, T* P, const TileBufs<T>& t,
+                                                 T* grad_obs, T* grad_act, int k0, int K) {
   constexpr int Hg = H / 2, G3 = 3 * Hg, R = kGradRows;
   const int B = g.B, nx = g.nx, gin = g.gin;
   const int tid = threadIdx.x;
-  const float* W_hh0 = wt + g.w_hh0;  // [3Hg][Hg]
-  const float* W_ih1 = wt + g.w_ih1;
-  const float* W_hh1 = wt + g.w_hh1;
-  const float* dxt = t.dxt;
-  const float* h1last = tile_h(g, t, 1, B - 1);
+  const T* W_hh0 = wt + g.w_hh0;  // [3Hg][Hg]
+  const T* W_ih1 = wt + g.w_ih1;
+  const T* W_hh1 = wt + g.w_hh1;
+  const T* dxt = t.dxt;
+  const T* h1last = tile_h(g, t, 1, B - 1);
   if (grad_obs)
     for (int i = tid; i < R * nx; i += kGradThreads) {
       const int m = i / nx, c = i - m * nx;
@@ -412,31 +542,31 @@ __device__ __forceinline__ void tile_encoder_bwd(const GradShape& g, const Model
     }
   // ---- linear_out backward ----
   for (int i = tid; i < 2 * Hg + 2; i += kGradThreads) {
-    float acc = 0.0f;
+    T acc = T(0);
     if (i < 2 * Hg) {
       const int o = i / Hg, h = i - o * Hg;
-      for (int m = 0; m < R; ++m) acc = fmaf(dxt[m * 16 + nx + o], h1last[m * Hg + h], acc);
+      for (int m = 0; m < R; ++m) acc = rm::fma(dxt[m * 16 + nx + o], h1last[m * Hg + h], acc);
       P[g.p_wout + i] += acc;
     } else {
       for (int m = 0; m < R; ++m) acc += dxt[m * 16 + nx + (i - 2 * Hg)];
       P[g.p_bout + i - 2 * Hg] += acc;
     }
   }
-  float* dh0 = t.dhb;
-  float* dh1 = t.dhb + R * Hg;
-  float* dh0n = t.dhb + 2 * R * Hg;
-  float* dh1n = t.dhb + 3 * R * Hg;
+  T* dh0 = t.dhb;
+  T* dh1 = t.dhb + R * Hg;
+  T* dh0n = t.dhb + 2 * R * Hg;
+  T* dh1n = t.dhb + 3 * R * Hg;
   for (int i = tid; i < R * Hg; i += kGradThreads) {
     const int m = i / Hg, h = i - m * Hg;
-    dh1[i] = fmaf(dxt[m * 16 + nx], md.w_out[h], dxt[m * 16 + nx + 1] * md.w_out[Hg + h]);
-    dh0[i] = 0.0f;
+    dh1[i] = rm::fma(dxt[m * 16 + nx], md.w_out[h], dxt[m * 16 + nx + 1] * md.w_out[Hg + h]);
+    dh0[i] = T(0);
   }
   __syncthreads();
   // ---- BPTT over the reversed window: step B-1 (oldest entry) first ----
   for (int st = B - 1; st >= 0; --st) {
     gru_cell_bwd(g, dh1, st > 0 ? tile_h(g, t, 1, st - 1) : nullptr, tile_gate(g, t, 1, st), dh1n);
     __syncthreads();
-    const float* G1 = tile_gate(g, t, 1, st);
+    const T* G1 = tile_gate(g, t, 1, st);
     if (st > 0) {  // dh1_prev += [dr | dz] W_hh1[r,z] + dghn W_hh1[n]
       gemm_nn<kEpiNone>(G1, 4 * Hg, W_hh1, Hg, 2 * Hg, Hg, dh1n, Hg, true);
       gemm_nn<kEpiNone>(G1 + 3 * Hg, 4 * Hg, W_hh1 + 2 * Hg * Hg, Hg, Hg, Hg, dh1n, Hg, true);
@@ -445,7 +575,7 @@ __device__ __forceinline__ void tile_encoder_bwd(const GradShape& g, const Model
     __syncthreads();
     gru_cell_bwd(g, dh0, st > 0 ? tile_h(g, t, 0, st - 1) : nullptr, tile_gate(g, t, 0, st), dh0n);
     __syncthreads();
-    const float* G0 = tile_gate(g, t, 0, st);
+    const T* G0 = tile_gate(g, t, 0, st);
     if (st > 0) {
       gemm_nn<kEpiNone>(G0, 4 * Hg, W_hh0, Hg, 2 * Hg, Hg, dh0n, Hg, true);
       gemm_nn<kEpiNone>(G0 + 3 * Hg, 4 * Hg, W_hh0 + 2 * Hg * Hg, Hg, Hg, Hg, dh0n, Hg, true);
@@ -453,13 +583,13 @@ __device__ __forceinline__ void tile_encoder_bwd(const GradShape& g, const Model
     if (grad_act)
       for (int i = tid; i < R * gin; i += kGradThreads) {  // W_ih0^T dg_i, times the input scale
         const int m = i / gin, u = i - m * gin;
-        float acc = 0.0f;
-        for (int q = 0; q < G3; ++q) acc = fmaf(G0[m * 4 * Hg + q], md.w_ih0[q * gin + u], acc);
+        T acc = T(0);
+        for (int q = 0; q < G3; ++q) acc = rm::fma(G0[m * 4 * Hg + q], md.w_ih0[q * gin + u], acc);
         if (k0 + m < K) grad_act[((size_t)(k0 + m) * B + (B - 1 - st)) * gin + u] = acc * md.act_inv_std[u];
       }
     __syncthreads();
-    float* t0 = dh0; dh0 = dh0n; dh0n = t0;
-    float* t1 = dh1; dh1 = dh1n; dh1n = t1;
+    T* t0 = dh0; dh0 = dh0n; dh0n = t0;
+    T* t1 = dh1; dh1 = dh1n; dh1n = t1;
   }
   // ---- GRU weight gradients: products over (step, sample) rows ----
   const int sG = R * 4 * Hg, sH = R * Hg;
@@ -472,22 +602,22 @@ __device__ __forceinline__ void tile_encoder_bwd(const GradShape& g, const Model
   colsum(P + g.p_bhh0, tile_gate(g, t, 0, 0), 4 * Hg, sG, 0, B, G3, 2 * Hg, Hg);
   for (int i = tid; i < G3 * gin; i += kGradThreads) {
     const int q = i / gin, u = i - q * gin;
-    float acc = 0.0f;
+    T acc = T(0);
     for (int st = 0; st < B; ++st)
-      for (int m = 0; m < R; ++m) acc = fmaf(tile_gate(g, t, 0, st)[m * 4 * Hg + q], t.xs[(st * R + m) * 4 + u], acc);
+      for (int m = 0; m < R; ++m) acc = rm::fma(tile_gate(g, t, 0, st)[m * 4 * Hg + q], t.xs[(st * R + m) * 4 + u], acc);
     P[g.p_wih0 + i] += acc;
   }
 }
 
 template <int H>
-__global__ void __launch_bounds__(kGradThreads, 1) model_grad_tile_kernel(GradArgs a) {
+__global__ void __launch_bounds__(kGradThreads, 1) model_grad_tile_kernel(GradArgs<float> a) {
   const GradShape& g = a.g;
-  const ModelDev& md = a.m;
-  constexpr int Hg = H / 2, R = kGradRows;
-  const int B = g.B, S = g.S, nx = g.nx, in0p = g.in0p;
+  const TileW<float>& md = a.m;
+  constexpr int R = kGradRows;
+  const int S = g.S, nx = g.nx, in0p = g.in0p;
   const int tid = threadIdx.x;
   float* P = a.part + (size_t)blockIdx.x * g.p_total;
-  const TileBufs t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
+  const TileBufs<float> t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
 
   for (int i = tid; i < g.p_total; i += kGradThreads) P[i] = 0.0f;
 
@@ -507,69 +637,58 @@ __global__ void __launch_bounds__(kGradThreads, 1) model_grad_tile_kernel(GradAr
     tile_fourier_consts(a.row_tn, k0, a.K, t.rc);
     __syncthreads();
     tile_encoder_fwd<H>(g, md, t);
-    const float* h1last = tile_h(g, t, 1, B - 1);
-    for (int i = tid; i < R * 2; i += kGradThreads) {  // linear_out (w_nl.py:29) -> p_action columns of the MLP input
-      const int m = i >> 1, o = i & 1;
-      float acc = md.b_out[o];
-      for (int k = 0; k < Hg; ++k) acc = fmaf(md.w_out[o * Hg + k], h1last[m * Hg + k], acc);
-      t.x1[m * in0p + 2 * S + nx + o] = acc;
-    }
+    tile_linear_out(g, md, t);
     __syncthreads();
-    tile_mlp_fwd_bwd<H>(g, md, a.wt, P, t, a.row_b1, a.gout, k0, a.K);
+    tile_mlp_fwd<H>(g, md, t, a.row_b1, k0, a.K);
+    tile_mlp_bwd<H>(g, md, a.wt, P, t, a.gout, k0, a.K);
     tile_encoder_bwd<H>(g, md, a.wt, P, t, a.grad_obs, a.grad_act, k0, a.K);
   }
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// Several prediction times per sample (nlc_model_backward_multi): the K n_t rows (sample k, time j) = row k n_t + j share
-// sample k's encoder output, so the backward runs in two stages instead of the fused tile kernel:
+// Several prediction times per sample (nlc_model_backward_multi, and the fp64 backward for every n_t): the K n_t rows
+// (sample k, time j) = row k n_t + j share sample k's encoder output, so the backward runs in two stages instead of the
+// fused tile kernel:
 //   MLP/ILT stage over the rows, chunk by chunk (model_grad_multi_mlp_kernel), then a fixed-order sum of each sample's
 //   per-row gradient of [obs_n | p_action] over j (model_grad_multi_rowsum_kernel), then one encoder stage over the K
 //   samples (model_grad_multi_enc_kernel).  Both stages accumulate into the same per-CTA partials as the tile kernel.
 // ------------------------------------------------------------------------------------------------------------------
+template <typename T>
 struct MultiArgs {
-  ModelDev m;
+  TileW<T> m;
   GradShape g;
-  const float* obs;      // [K][nx]
-  const float* p;        // [K][2] encoder output
-  const float* gout;     // [rows][nx]   this chunk's rows of grad_out
-  const float* row_b1;   // [rows][H]
-  const float* row_tn;   // [rows]
-  const float* row_sph;  // [rows][2S]
-  const float* wt;
-  float* part;
-  float* scratch;
-  float* drow;           // [rows][Lp] gradient of [obs_n | p_action] per row
-  long long r0;          // global index of the chunk's first row
+  const T* obs;      // [K][nx]
+  const T* p;        // [K][2] encoder output
+  const T* gout;     // [rows][nx]   this chunk's rows of grad_out (the fp64 forward: its output rows)
+  const T* row_b1;   // [rows][H]
+  const T* row_tn;   // [rows]
+  const T* row_sph;  // [rows][2S]
+  const T* wt;
+  T* part;
+  T* scratch;
+  T* drow;           // [rows][Lp] gradient of [obs_n | p_action] per row
+  long long r0;      // global index of the chunk's first row
   int rows, n_t;
 };
 
-template <int H>
-__global__ void __launch_bounds__(kGradThreads, 1) model_grad_multi_mlp_kernel(MultiArgs a) {
+template <int H, typename T>
+__global__ void __launch_bounds__(kGradThreads, 1) model_grad_multi_mlp_kernel(MultiArgs<T> a) {
   const GradShape& g = a.g;
-  const ModelDev& md = a.m;
+  const TileW<T>& md = a.m;
   constexpr int R = kGradRows;
-  const int S = g.S, nx = g.nx, Lp = g.Lp, in0p = g.in0p;
+  const int Lp = g.Lp;
   const int tid = threadIdx.x;
-  float* P = a.part + (size_t)blockIdx.x * g.p_total;
-  const TileBufs t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
+  T* P = a.part + (size_t)blockIdx.x * g.p_total;
+  const TileBufs<T> t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
   const int n_tiles = (a.rows + R - 1) / R;
   for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
     const int k0 = tile * R;
     __syncthreads();  // the previous tile's last reads of the scratch are done
-    for (int i = tid; i < R * in0p; i += kGradThreads) {  // [theta_s | phi_s | obs_n | p_action | 0] of row r, sample (r0 + r) / n_t
-      const int m = i / in0p, j = i - m * in0p;
-      const int r = min(k0 + m, a.rows - 1);
-      const size_t k = (size_t)((a.r0 + r) / a.n_t);
-      float v = 0.0f;
-      if (j < 2 * S) v = a.row_sph[(size_t)r * 2 * S + j];
-      else if (j < 2 * S + nx) v = (a.obs[k * nx + (j - 2 * S)] - md.state_mean[j - 2 * S]) * md.state_inv_std[j - 2 * S];
-      else if (j < 2 * S + Lp) v = a.p[k * 2 + (j - 2 * S - nx)];
-      t.x1[i] = v;
-    }
+    tile_rows_input(g, md, a.row_sph, a.obs, a.p, a.r0, a.rows, a.n_t, k0, t.x1);
     tile_fourier_consts(a.row_tn, k0, a.rows, t.rc);
     __syncthreads();
-    tile_mlp_fwd_bwd<H>(g, md, a.wt, P, t, a.row_b1, a.gout, k0, a.rows);
+    tile_mlp_fwd<H>(g, md, t, a.row_b1, k0, a.rows);
+    tile_mlp_bwd<H>(g, md, a.wt, P, t, a.gout, k0, a.rows);
     for (int i = tid; i < R * Lp; i += kGradThreads) {
       const int m = i / Lp, j = i - m * Lp;
       if (k0 + m < a.rows) a.drow[(size_t)(k0 + m) * Lp + j] = t.dxt[m * 16 + j];
@@ -579,40 +698,85 @@ __global__ void __launch_bounds__(kGradThreads, 1) model_grad_multi_mlp_kernel(M
 
 // dsum[k] (+)= sum of drow over sample k's rows in this chunk, j ascending; a sample's first row starts its sum, so the
 // chunks in order give every sample the same sequential sum over j = 0 .. n_t - 1 whatever the chunk boundaries.
-__global__ void __launch_bounds__(256) model_grad_multi_rowsum_kernel(const float* __restrict__ drow, long long r0, int rows, int n_t,
-                                                                      int Lp, float* __restrict__ dsum) {
+template <typename T>
+__global__ void __launch_bounds__(256) model_grad_multi_rowsum_kernel(const T* __restrict__ drow, long long r0, int rows, int n_t,
+                                                                      int Lp, T* __restrict__ dsum) {
   const long long k_first = r0 / n_t, k_last = (r0 + rows - 1) / n_t;
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (k_last - k_first + 1) * Lp) return;
   const long long k = k_first + i / Lp;
   const int c = (int)(i % Lp);
   const long long j0 = k * n_t > r0 ? k * n_t : r0, j1 = (k + 1) * n_t < r0 + rows ? (k + 1) * n_t : r0 + rows;
-  float acc = j0 == k * n_t ? 0.0f : dsum[k * Lp + c];
+  T acc = j0 == k * n_t ? T(0) : dsum[k * Lp + c];
   for (long long r = j0; r < j1; ++r) acc += drow[(r - r0) * Lp + c];
   dsum[k * Lp + c] = acc;
 }
 
 // Encoder stage: tiles of kGradRows samples, the summed gradient of [obs_n | p_action] of each sample from dsum [K][Lp].
-template <int H>
-__global__ void __launch_bounds__(kGradThreads, 1) model_grad_multi_enc_kernel(GradArgs a, const float* __restrict__ dsum) {
+template <int H, typename T>
+__global__ void __launch_bounds__(kGradThreads, 1) model_grad_multi_enc_kernel(GradArgs<T> a, const T* __restrict__ dsum) {
   const GradShape& g = a.g;
-  const ModelDev& md = a.m;
+  const TileW<T>& md = a.m;
   constexpr int R = kGradRows;
   const int Lp = g.Lp;
   const int tid = threadIdx.x;
-  float* P = a.part + (size_t)blockIdx.x * g.p_total;
-  const TileBufs t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
+  T* P = a.part + (size_t)blockIdx.x * g.p_total;
+  const TileBufs<T> t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
   for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
     const int k0 = tile * R;
     __syncthreads();  // the previous tile's last reads of the scratch are done
     tile_load_window(g, md, a.act, k0, a.K, t.xs);
     for (int i = tid; i < R * Lp; i += kGradThreads) {  // rows past K repeat sample K - 1 in the window: zero gradient
       const int m = i / Lp, j = i - m * Lp;
-      t.dxt[m * 16 + j] = k0 + m < a.K ? dsum[(size_t)(k0 + m) * Lp + j] : 0.0f;
+      t.dxt[m * 16 + j] = k0 + m < a.K ? dsum[(size_t)(k0 + m) * Lp + j] : T(0);
     }
     __syncthreads();
     tile_encoder_fwd<H>(g, md, t);
     tile_encoder_bwd<H>(g, md, a.wt, P, t, a.grad_obs, a.grad_act, k0, a.K);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// fp64 forward: the recompute half of the tile steps.  model_f64_encode_kernel encodes tiles of kGradRows windows and
+// writes linear_out's p [K][2]; model_f64_rows_kernel runs the MLP and the ILT sum over a chunk's rows.
+// ------------------------------------------------------------------------------------------------------------------
+template <int H>
+__global__ void __launch_bounds__(kGradThreads, 1) model_f64_encode_kernel(GradArgs<double> a, double* __restrict__ p) {
+  const GradShape& g = a.g;
+  const TileW<double>& md = a.m;
+  constexpr int R = kGradRows;
+  const TileBufs<double> t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
+  for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
+    const int k0 = tile * R;
+    __syncthreads();  // the previous tile's last reads of the scratch are done
+    tile_load_window(g, md, a.act, k0, a.K, t.xs);
+    __syncthreads();
+    tile_encoder_fwd<H>(g, md, t);
+    tile_linear_out(g, md, t);
+    __syncthreads();
+    for (int i = threadIdx.x; i < R * 2; i += kGradThreads) {
+      const int m = i >> 1, o = i & 1;
+      if (k0 + m < a.K) p[(size_t)(k0 + m) * 2 + o] = t.x1[m * g.in0p + 2 * g.S + g.nx + o];
+    }
+  }
+}
+
+// a.gout is unused; out: this chunk's rows [rows][nx]
+template <int H>
+__global__ void __launch_bounds__(kGradThreads, 1) model_f64_rows_kernel(MultiArgs<double> a, double* __restrict__ out) {
+  const GradShape& g = a.g;
+  const TileW<double>& md = a.m;
+  constexpr int R = kGradRows;
+  const TileBufs<double> t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
+  const int n_tiles = (a.rows + R - 1) / R;
+  for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const int k0 = tile * R;
+    __syncthreads();  // the previous tile's last reads of the scratch are done
+    tile_rows_input(g, md, a.row_sph, a.obs, a.p, a.r0, a.rows, a.n_t, k0, t.x1);
+    tile_fourier_consts(a.row_tn, k0, a.rows, t.rc);
+    __syncthreads();
+    tile_mlp_fwd<H>(g, md, t, a.row_b1, k0, a.rows);
+    tile_ilt_out(g, t, k0, a.rows, out);
   }
 }
 
@@ -635,8 +799,54 @@ __global__ void __launch_bounds__(256) model_grad_wt_kernel(ModelDev m, GradShap
   }
 }
 
+// fp64: the weight image of one call from the caller's parameters prm (state_dict layout, GradShape o_* offsets) - the
+// row-major copies of model_grad_wt_kernel at w_*, and every weight in ModelDev's layout at f_* (TileW): the mirror
+// image of nlc_model_create's packing, without the fp32 rounding.
+__global__ void __launch_bounds__(256) model_f64_weights_kernel(GradShape g, const double* __restrict__ prm, double* __restrict__ img) {
+  const int Hg = g.Hg, G3 = g.G3, H = g.H, S = g.S, nx = g.nx, gin = g.gin, in0 = g.in0, N3 = g.N3, N3p = g.N3p;
+  const int i0 = blockIdx.x * blockDim.x + threadIdx.x, step = gridDim.x * blockDim.x;
+  // paired column col = 2 (c S + k) + part of the last layer <- state_dict row (part nx + c) S + k; -1: padding
+  auto w4_row = [&](int col) { return col < N3 ? ((col & 1) * nx + (col >> 1) / S) * S + (col >> 1) % S : -1; };
+  for (int i = i0; i < G3 * Hg; i += step) {  // [gate row q][unit k]: state_dict; _t [k][q]
+    const int q = i / Hg, k = i - q * Hg;
+    img[g.w_hh0 + i] = prm[g.o_whh0 + i]; img[g.w_ih1 + i] = prm[g.o_wih1 + i]; img[g.w_hh1 + i] = prm[g.o_whh1 + i];
+    img[g.f_hh0t + k * G3 + q] = prm[g.o_whh0 + i]; img[g.f_ih1t + k * G3 + q] = prm[g.o_wih1 + i];
+    img[g.f_hh1t + k * G3 + q] = prm[g.o_whh1 + i];
+  }
+  for (int i = i0; i < H * H; i += step) {  // W2 [out n][in k]
+    const int n = i / H, k = i - n * H;
+    img[g.w_2 + i] = prm[g.o_w2 + i];
+    img[g.f_w2t + k * H + n] = prm[g.o_w2 + i];
+  }
+  for (int i = i0; i < N3p * H; i += step) {  // W3 paired: [col][h] and [h][col]
+    const int col = i / H, h = i - col * H, src = w4_row(col);
+    const double v = src >= 0 ? prm[g.o_w4 + (size_t)src * H + h] : 0.0;
+    img[g.w_3 + i] = v;
+    img[g.f_w3t + (size_t)h * N3p + col] = v;
+  }
+  for (int i = i0; i < in0 * H; i += step) {  // W1 [n][in] -> [in][n]
+    const int n = i / in0, j = i - n * in0;
+    img[g.f_w1t + (size_t)j * H + n] = prm[g.o_w0 + i];
+  }
+  for (int i = i0; i < N3p; i += step) {
+    const int src = w4_row(i);
+    img[g.f_b3 + i] = src >= 0 ? prm[g.o_b4 + src] : 0.0;
+  }
+  for (int i = i0; i < G3 * gin; i += step) img[g.f_wih0 + i] = prm[g.o_wih0 + i];
+  for (int i = i0; i < G3; i += step) {
+    img[g.f_bih0 + i] = prm[g.o_bih0 + i]; img[g.f_bhh0 + i] = prm[g.o_bhh0 + i];
+    img[g.f_bih1 + i] = prm[g.o_bih1 + i]; img[g.f_bhh1 + i] = prm[g.o_bhh1 + i];
+  }
+  for (int i = i0; i < 2 * Hg + 2; i += step) {
+    if (i < 2 * Hg) img[g.f_wout + i] = prm[g.o_wout + i];
+    else img[g.f_bout + i - 2 * Hg] = prm[g.o_bout + i - 2 * Hg];
+  }
+  for (int i = i0; i < H; i += step) { img[g.f_b1 + i] = prm[g.o_b0 + i]; img[g.f_b2 + i] = prm[g.o_b2 + i]; }
+}
+
 // Sum of the per-CTA partials in CTA order, written in the state_dict layout (named_parameters() order).
-__global__ void __launch_bounds__(256) model_grad_reduce_kernel(GradShape g, const float* __restrict__ part, int n_part, float* out) {
+template <typename T>
+__global__ void __launch_bounds__(256) model_grad_reduce_kernel(GradShape g, const T* __restrict__ part, int n_part, T* out) {
   const int Hg = g.Hg, G3 = g.G3, H = g.H, S = g.S, nx = g.nx;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < g.o_total; i += gridDim.x * blockDim.x) {
     int src;
@@ -663,7 +873,7 @@ __global__ void __launch_bounds__(256) model_grad_reduce_kernel(GradShape g, con
       const int col = 2 * (c * S + k) + prt;
       src = bias ? g.p_b4 + col : g.p_w4 + h * g.N3p + col;
     }
-    float acc = 0.0f;
+    T acc = T(0);
     for (int c = 0; c < n_part; ++c) acc += part[(size_t)c * g.p_total + src];
     out[i] = acc;
   }
@@ -694,23 +904,25 @@ static GradWs ws_layout(const GradShape& g, int K) {
 
 // Several prediction times per sample: rows are walked in chunks of at most kMultiChunkRows (rollout.cu), so the per-row
 // buffers are bounded whatever K n_t is.
-// workspace (floats): p [K][2] | dsum [K][Lp] | row_b1 [C][H] | row_tn [C] | row_sph [C][2S] | drow [C][Lp] | weight copies |
-// partials [G] | scratch [G], C = min(K n_t, kMultiChunkRows), G = max(grid of C rows, grid of K samples)
+// workspace (elements of the scalar type): p [K][2] | dsum [K][Lp] | row_b1 [C][H] | row_tn [C] | row_sph [C][2S] |
+// drow [C][Lp] | weight copies | partials [G] | scratch [G], C = min(K n_t, kMultiChunkRows), G = max(grid of C rows, grid of
+// K samples).  fp64: the weight copies are followed by the forward layouts (f_total), and the forward (bwd = false) has no
+// dsum, drow or partials.
 struct MultiWs { size_t p, dsum, b1, tn, sph, drow, wt, part, scr, total; int C, Gm, Ge, G; };
-static MultiWs multi_ws_layout(const GradShape& g, int K, int n_t) {
+static MultiWs multi_ws_layout(const GradShape& g, int K, int n_t, bool f64 = false, bool bwd = true) {
   MultiWs w;
   const long long rows = (long long)K * n_t;
   w.C = rows < kMultiChunkRows ? (int)rows : kMultiChunkRows;
   w.Gm = grad_grid(w.C); w.Ge = grad_grid(K); w.G = w.Gm > w.Ge ? w.Gm : w.Ge;
   size_t o = 0;
   w.p = o; o += up64((size_t)K * 2);
-  w.dsum = o; o += up64((size_t)K * g.Lp);
+  w.dsum = o; o += bwd ? up64((size_t)K * g.Lp) : 0;
   w.b1 = o; o += up64((size_t)w.C * g.H);
   w.tn = o; o += up64(w.C);
   w.sph = o; o += up64((size_t)w.C * 2 * g.S);
-  w.drow = o; o += up64((size_t)w.C * g.Lp);
-  w.wt = o; o += g.w_total;
-  w.part = o; o += (size_t)w.G * g.p_total;
+  w.drow = o; o += bwd ? up64((size_t)w.C * g.Lp) : 0;
+  w.wt = o; o += f64 ? g.f_total : g.w_total;
+  w.part = o; o += bwd ? (size_t)w.G * g.p_total : 0;
   w.scr = o; o += (size_t)w.G * g.s_total;
   w.total = o;
   return w;
@@ -751,8 +963,8 @@ extern "C" int nlc_model_backward_ts(nlc_model_t m, const float* obs_dev, const 
   const int n_wt = 3 * g.G3 * g.Hg + g.H * g.H + g.N3p * g.H;
   model_grad_wt_kernel<<<(n_wt + 255) / 256, 256, 0, s>>>(m->d, g, ws + w.wt);
   NLC_LAUNCH_OK("model_grad_wt_kernel");
-  GradArgs a;
-  a.m = m->d; a.g = g; a.obs = obs_dev; a.act = act_dev; a.gout = grad_out_dev;
+  GradArgs<float> a;
+  a.m = tile_w(m->d); a.g = g; a.obs = obs_dev; a.act = act_dev; a.gout = grad_out_dev;
   a.row_b1 = ws + w.b1; a.row_tn = ws + w.tn; a.row_sph = ws + w.sph; a.wt = ws + w.wt;
   a.part = ws + w.part; a.scratch = ws + w.scr; a.grad_obs = grad_obs_dev; a.grad_act = grad_act_dev;
   a.K = K; a.n_tiles = (K + kGradRows - 1) / kGradRows;
@@ -760,7 +972,7 @@ extern "C" int nlc_model_backward_ts(nlc_model_t m, const float* obs_dev, const 
   if (m->Hm == 128) model_grad_tile_kernel<128><<<G, kGradThreads, 0, s>>>(a);
   else model_grad_tile_kernel<64><<<G, kGradThreads, 0, s>>>(a);
   NLC_LAUNCH_OK("model_grad_tile_kernel");
-  model_grad_reduce_kernel<<<(g.o_total + 255) / 256, 256, 0, s>>>(g, ws + w.part, G, grad_params_dev);
+  model_grad_reduce_kernel<float><<<(g.o_total + 255) / 256, 256, 0, s>>>(g, ws + w.part, G, grad_params_dev);
   NLC_LAUNCH_OK("model_grad_reduce_kernel");
   return NLC_OK;
 }
@@ -794,8 +1006,8 @@ extern "C" int nlc_model_backward_multi(nlc_model_t m, const float* obs_dev, con
   model_grad_wt_kernel<<<(n_wt + 255) / 256, 256, 0, s>>>(m->d, g, ws + w.wt);
   NLC_LAUNCH_OK("model_grad_wt_kernel");
   NLC_CUDA_OK(cudaMemsetAsync(ws + w.part, 0, (size_t)w.G * g.p_total * sizeof(float), s));
-  MultiArgs ma;
-  ma.m = m->d; ma.g = g; ma.obs = obs_dev; ma.p = ws + w.p; ma.row_b1 = ws + w.b1; ma.row_tn = ws + w.tn; ma.row_sph = ws + w.sph;
+  MultiArgs<float> ma;
+  ma.m = tile_w(m->d); ma.g = g; ma.obs = obs_dev; ma.p = ws + w.p; ma.row_b1 = ws + w.b1; ma.row_tn = ws + w.tn; ma.row_sph = ws + w.sph;
   ma.wt = ws + w.wt; ma.part = ws + w.part; ma.scratch = ws + w.scr; ma.drow = ws + w.drow; ma.n_t = n_t;
   const long long n_rows = (long long)K * n_t;
   for (long long r0 = 0; r0 < n_rows; r0 += w.C) {
@@ -803,22 +1015,139 @@ extern "C" int nlc_model_backward_multi(nlc_model_t m, const float* obs_dev, con
     rc = launch_forward_ts_prep(m, ts_dev + r0, rows, ws + w.b1, ws + w.tn, ws + w.sph, s);
     if (rc != NLC_OK) return rc;
     ma.gout = grad_out_dev + r0 * g.nx; ma.r0 = r0; ma.rows = rows;
-    if (m->Hm == 128) model_grad_multi_mlp_kernel<128><<<w.Gm, kGradThreads, 0, s>>>(ma);
-    else model_grad_multi_mlp_kernel<64><<<w.Gm, kGradThreads, 0, s>>>(ma);
+    if (m->Hm == 128) model_grad_multi_mlp_kernel<128, float><<<w.Gm, kGradThreads, 0, s>>>(ma);
+    else model_grad_multi_mlp_kernel<64, float><<<w.Gm, kGradThreads, 0, s>>>(ma);
     NLC_LAUNCH_OK("model_grad_multi_mlp_kernel");
     const long long n_sum = ((r0 + rows - 1) / n_t - r0 / n_t + 1) * g.Lp;
-    model_grad_multi_rowsum_kernel<<<(unsigned)((n_sum + 255) / 256), 256, 0, s>>>(ws + w.drow, r0, rows, n_t, g.Lp, ws + w.dsum);
+    model_grad_multi_rowsum_kernel<float><<<(unsigned)((n_sum + 255) / 256), 256, 0, s>>>(ws + w.drow, r0, rows, n_t, g.Lp, ws + w.dsum);
     NLC_LAUNCH_OK("model_grad_multi_rowsum_kernel");
   }
-  GradArgs a;
-  a.m = m->d; a.g = g; a.obs = obs_dev; a.act = act_dev; a.gout = nullptr;
+  GradArgs<float> a;
+  a.m = tile_w(m->d); a.g = g; a.obs = obs_dev; a.act = act_dev; a.gout = nullptr;
   a.row_b1 = nullptr; a.row_tn = nullptr; a.row_sph = nullptr; a.wt = ws + w.wt;
   a.part = ws + w.part; a.scratch = ws + w.scr; a.grad_obs = grad_obs_dev; a.grad_act = grad_act_dev;
   a.K = K; a.n_tiles = (K + kGradRows - 1) / kGradRows;
-  if (m->Hm == 128) model_grad_multi_enc_kernel<128><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
-  else model_grad_multi_enc_kernel<64><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
+  if (m->Hm == 128) model_grad_multi_enc_kernel<128, float><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
+  else model_grad_multi_enc_kernel<64, float><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
   NLC_LAUNCH_OK("model_grad_multi_enc_kernel");
-  model_grad_reduce_kernel<<<(g.o_total + 255) / 256, 256, 0, s>>>(g, ws + w.part, w.G, grad_params_dev);
+  model_grad_reduce_kernel<float><<<(g.o_total + 255) / 256, 256, 0, s>>>(g, ws + w.part, w.G, grad_params_dev);
   NLC_LAUNCH_OK("model_grad_reduce_kernel");
+  return NLC_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// fp64 forward and backward (NeuralLaplaceModel math_mode="fp64"): the weights are the caller's fp64 parameters params_dev
+// (nlc_model_grad_floats entries, the layout of grad_params_dev), rearranged per call into the workspace.
+// ---------------------------------------------------------------------------------------------------------------------
+namespace nlc {
+
+static int f64_check(const char* fn, nlc_model_t m, int K, int n_t, int B, const void* workspace_dev) {
+  NLC_REQUIRE(K >= 1 && n_t >= 1, NLC_ERR_ARG, "%s: K and n_t must be positive", fn);
+  NLC_REQUIRE((long long)K * n_t < (1LL << 31), NLC_ERR_SHAPE, "%s: K n_t = %lld rows, 2^31 or more", fn, (long long)K * n_t);
+  NLC_REQUIRE(B >= 1 && B <= 8, NLC_ERR_SHAPE, "%s: window length %d outside [1,8]", fn, B);
+  NLC_REQUIRE(((uintptr_t)workspace_dev & 15) == 0, NLC_ERR_ARG, "%s: workspace must be 16-byte aligned", fn);
+  return check_device_arch(m->device);
+}
+
+// The weight image, p [K][2] of the K windows (p_out when given, else the workspace's), and the launches of one chunk's prep.
+static int f64_encode(nlc_model_t m, const GradShape& g, const MultiWs& w, const double* params_dev, const double* act_dev, int K,
+                      double* ws, double* p, cudaStream_t s) {
+  const int n_img = g.N3p * g.H > g.in0 * g.H ? g.N3p * g.H : g.in0 * g.H;
+  model_f64_weights_kernel<<<(n_img + 255) / 256, 256, 0, s>>>(g, params_dev, ws + w.wt);
+  NLC_LAUNCH_OK("model_f64_weights_kernel");
+  GradArgs<double> a = {};
+  a.m = tile_w_f64(m->d, g, ws + w.wt); a.g = g; a.act = act_dev; a.wt = ws + w.wt; a.scratch = ws + w.scr;
+  a.K = K; a.n_tiles = (K + kGradRows - 1) / kGradRows;
+  if (m->Hm == 128) model_f64_encode_kernel<128><<<w.Ge, kGradThreads, 0, s>>>(a, p);
+  else model_f64_encode_kernel<64><<<w.Ge, kGradThreads, 0, s>>>(a, p);
+  NLC_LAUNCH_OK("model_f64_encode_kernel");
+  return NLC_OK;
+}
+
+}  // namespace nlc
+
+extern "C" int64_t nlc_model_forward_f64_workspace_bytes(nlc_model_t m, int K, int n_t, int B) {
+  if (!m || K < 1 || n_t < 1 || B < 1 || B > 8) return NLC_ERR_ARG;
+  if ((long long)K * n_t >= (1LL << 31)) return NLC_ERR_SHAPE;
+  return (int64_t)(multi_ws_layout(shape_of(m, B), K, n_t, true, false).total * sizeof(double));
+}
+
+extern "C" int nlc_model_forward_f64(nlc_model_t m, const double* params_dev, const double* obs_dev, const double* act_dev,
+                                     const double* ts_dev, int K, int n_t, int B, double* out_dev, double* p_action_dev,
+                                     void* workspace_dev, void* stream) {
+  NLC_REQUIRE(m && params_dev && obs_dev && act_dev && ts_dev && out_dev && workspace_dev, NLC_ERR_ARG,
+              "nlc_model_forward_f64: null pointer");
+  int rc = f64_check("nlc_model_forward_f64", m, K, n_t, B, workspace_dev);
+  if (rc != NLC_OK) return rc;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const GradShape g = shape_of(m, B);
+  const MultiWs w = multi_ws_layout(g, K, n_t, true, false);
+  double* ws = static_cast<double*>(workspace_dev);
+  double* p = p_action_dev ? p_action_dev : ws + w.p;
+  rc = f64_encode(m, g, w, params_dev, act_dev, K, ws, p, s);
+  if (rc != NLC_OK) return rc;
+  MultiArgs<double> ma = {};
+  ma.m = tile_w_f64(m->d, g, ws + w.wt); ma.g = g; ma.obs = obs_dev; ma.p = p; ma.row_b1 = ws + w.b1; ma.row_tn = ws + w.tn;
+  ma.row_sph = ws + w.sph; ma.wt = ws + w.wt; ma.scratch = ws + w.scr; ma.n_t = n_t;
+  const long long n_rows = (long long)K * n_t;
+  for (long long r0 = 0; r0 < n_rows; r0 += w.C) {
+    const int rows = (int)(n_rows - r0 < w.C ? n_rows - r0 : w.C);
+    rc = launch_forward_ts_prep_f64(m, ma.m.b1_raw, ma.m.w1_full_t, ts_dev + r0, rows, ws + w.b1, ws + w.tn, ws + w.sph, s);
+    if (rc != NLC_OK) return rc;
+    ma.r0 = r0; ma.rows = rows;
+    const int G = grad_grid(rows);
+    if (m->Hm == 128) model_f64_rows_kernel<128><<<G, kGradThreads, 0, s>>>(ma, out_dev + r0 * g.nx);
+    else model_f64_rows_kernel<64><<<G, kGradThreads, 0, s>>>(ma, out_dev + r0 * g.nx);
+    NLC_LAUNCH_OK("model_f64_rows_kernel");
+  }
+  return NLC_OK;
+}
+
+extern "C" int64_t nlc_model_backward_f64_workspace_bytes(nlc_model_t m, int K, int n_t, int B) {
+  if (!m || K < 1 || n_t < 1 || B < 1 || B > 8) return NLC_ERR_ARG;
+  if ((long long)K * n_t >= (1LL << 31)) return NLC_ERR_SHAPE;
+  return (int64_t)(multi_ws_layout(shape_of(m, B), K, n_t, true, true).total * sizeof(double));
+}
+
+extern "C" int nlc_model_backward_f64(nlc_model_t m, const double* params_dev, const double* obs_dev, const double* act_dev,
+                                      const double* ts_dev, int K, int n_t, int B, const double* grad_out_dev,
+                                      double* grad_params_dev, double* grad_obs_dev, double* grad_act_dev, void* workspace_dev,
+                                      void* stream) {
+  NLC_REQUIRE(m && params_dev && obs_dev && act_dev && ts_dev && grad_out_dev && grad_params_dev && workspace_dev, NLC_ERR_ARG,
+              "nlc_model_backward_f64: null pointer");
+  int rc = f64_check("nlc_model_backward_f64", m, K, n_t, B, workspace_dev);
+  if (rc != NLC_OK) return rc;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const GradShape g = shape_of(m, B);
+  const MultiWs w = multi_ws_layout(g, K, n_t, true, true);
+  double* ws = static_cast<double*>(workspace_dev);
+  rc = f64_encode(m, g, w, params_dev, act_dev, K, ws, ws + w.p, s);
+  if (rc != NLC_OK) return rc;
+  NLC_CUDA_OK(cudaMemsetAsync(ws + w.part, 0, (size_t)w.G * g.p_total * sizeof(double), s));
+  const TileW<double> tw = tile_w_f64(m->d, g, ws + w.wt);
+  MultiArgs<double> ma = {};
+  ma.m = tw; ma.g = g; ma.obs = obs_dev; ma.p = ws + w.p; ma.row_b1 = ws + w.b1; ma.row_tn = ws + w.tn; ma.row_sph = ws + w.sph;
+  ma.wt = ws + w.wt; ma.part = ws + w.part; ma.scratch = ws + w.scr; ma.drow = ws + w.drow; ma.n_t = n_t;
+  const long long n_rows = (long long)K * n_t;
+  for (long long r0 = 0; r0 < n_rows; r0 += w.C) {
+    const int rows = (int)(n_rows - r0 < w.C ? n_rows - r0 : w.C);
+    rc = launch_forward_ts_prep_f64(m, tw.b1_raw, tw.w1_full_t, ts_dev + r0, rows, ws + w.b1, ws + w.tn, ws + w.sph, s);
+    if (rc != NLC_OK) return rc;
+    ma.gout = grad_out_dev + r0 * g.nx; ma.r0 = r0; ma.rows = rows;
+    if (m->Hm == 128) model_grad_multi_mlp_kernel<128, double><<<w.Gm, kGradThreads, 0, s>>>(ma);
+    else model_grad_multi_mlp_kernel<64, double><<<w.Gm, kGradThreads, 0, s>>>(ma);
+    NLC_LAUNCH_OK("model_grad_multi_mlp_kernel<double>");
+    const long long n_sum = ((r0 + rows - 1) / n_t - r0 / n_t + 1) * g.Lp;
+    model_grad_multi_rowsum_kernel<double><<<(unsigned)((n_sum + 255) / 256), 256, 0, s>>>(ws + w.drow, r0, rows, n_t, g.Lp, ws + w.dsum);
+    NLC_LAUNCH_OK("model_grad_multi_rowsum_kernel<double>");
+  }
+  GradArgs<double> a = {};
+  a.m = tw; a.g = g; a.obs = obs_dev; a.act = act_dev; a.wt = ws + w.wt; a.part = ws + w.part; a.scratch = ws + w.scr;
+  a.grad_obs = grad_obs_dev; a.grad_act = grad_act_dev; a.K = K; a.n_tiles = (K + kGradRows - 1) / kGradRows;
+  if (m->Hm == 128) model_grad_multi_enc_kernel<128, double><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
+  else model_grad_multi_enc_kernel<64, double><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
+  NLC_LAUNCH_OK("model_grad_multi_enc_kernel<double>");
+  model_grad_reduce_kernel<double><<<(g.o_total + 255) / 256, 256, 0, s>>>(g, ws + w.part, w.G, grad_params_dev);
+  NLC_LAUNCH_OK("model_grad_reduce_kernel<double>");
   return NLC_OK;
 }

@@ -395,42 +395,55 @@ namespace nlc {
 // backward (model_grad.cu) multiplies into dW1.
 // row_obs (optional, [K][nx]) and row_p ([K][2]): row k's copy of obs and p of sample (r0 + k) / n_t, for rows that are
 // (sample, time) pairs (nlc_model_forward_multi)
-__global__ void __launch_bounds__(128) forward_ts_prep_kernel(ModelDev m, int kH, int S, int Lp, int norm_time, float dt, const float* __restrict__ ts,
-                                                              int K, float* __restrict__ row_b1, float* __restrict__ row_tn,
-                                                              float* __restrict__ row_sph, const float* __restrict__ obs,
-                                                              const float* __restrict__ p, long long r0, int n_t,
-                                                              float* __restrict__ row_obs, float* __restrict__ row_p) {
-  __shared__ float th[kMaxS], ph[kMaxS];
+// b1_raw [kH] and w1_full_t [2S+nx+2][kH] are the unfolded first layer; T = double is the fp64 forward / backward's form.
+template <typename T>
+__global__ void __launch_bounds__(128) forward_ts_prep_kernel(const T* __restrict__ b1_raw, const T* __restrict__ w1_full_t, int kH,
+                                                              int S, int Lp, int norm_time, T dt, const T* __restrict__ ts,
+                                                              int K, T* __restrict__ row_b1, T* __restrict__ row_tn,
+                                                              T* __restrict__ row_sph, const T* __restrict__ obs,
+                                                              const T* __restrict__ p, long long r0, int n_t,
+                                                              T* __restrict__ row_obs, T* __restrict__ row_p) {
+  using C = Real<T>;
+  __shared__ T th[kMaxS], ph[kMaxS];
   const int k = blockIdx.x, n = threadIdx.x;
   if (row_obs && n < Lp) {
     const size_t src = (size_t)((r0 + k) / n_t);
     if (n < Lp - 2) row_obs[(size_t)k * (Lp - 2) + n] = obs[src * (Lp - 2) + n];
     else row_p[(size_t)k * 2 + n - (Lp - 2)] = p[src * 2 + n - (Lp - 2)];
   }
-  float tn = ts[k];
-  if (norm_time) tn = tn / (dt * 8.0f);  // w_nl.py:123
-  const float T = 2.0f * (tn + 1.0e-6f);
-  const float gamma = 1.0e-3f + 4.605170185988091f / T;
+  T tn = ts[k];
+  if (norm_time) tn = tn / (dt * T(8));  // w_nl.py:123
+  const T Tp = T(2) * (tn + C::eps);
+  const T gamma = C::alpha + C::ln_inv_tol / Tp;
   for (int j = n; j < S; j += kH) {  // oracle/ilt.py: fourier_s_points + complex_to_sphere
-    const float im = 3.14159265358979f * (float)j / T;
-    th[j] = atan2f(im, gamma);
+    const T im = C::pi * (T)j / Tp;
+    th[j] = rm::atan2(im, gamma);
     // phi = asin((r^2-1)/(r^2+1)) = 2 atan(r) - pi/2 (the asin form cancels for large r)
-    ph[j] = 2.0f * atanf(sqrtf(fmaf(gamma, gamma, im * im))) - 1.57079632679489662f;
+    ph[j] = T(2) * rm::atan(rm::sqrt(rm::fma(gamma, gamma, im * im))) - C::half_pi;
     if (row_sph) { row_sph[(size_t)k * 2 * S + j] = th[j]; row_sph[(size_t)k * 2 * S + S + j] = ph[j]; }
   }
   __syncthreads();
-  float acc = m.b1_raw[n];
-  for (int j = 0; j < S; ++j) acc = fmaf(m.w1_full_t[(size_t)j * kH + n], th[j], acc);
-  for (int j = 0; j < S; ++j) acc = fmaf(m.w1_full_t[(size_t)(S + j) * kH + n], ph[j], acc);
+  T acc = b1_raw[n];
+  for (int j = 0; j < S; ++j) acc = rm::fma(w1_full_t[(size_t)j * kH + n], th[j], acc);
+  for (int j = 0; j < S; ++j) acc = rm::fma(w1_full_t[(size_t)(S + j) * kH + n], ph[j], acc);
   row_b1[(size_t)k * kH + n] = acc;
   if (n == 0) row_tn[k] = tn;
 }
 
 static int launch_prep(nlc_model_s* m, const float* ts, int K, float* row_b1, float* row_tn, float* row_sph, const float* obs,
                        const float* p, long long r0, int n_t, float* row_obs, float* row_p, cudaStream_t s) {
-  forward_ts_prep_kernel<<<K, m->Hm, 0, s>>>(m->d, m->Hm, m->S, m->nx + 2, m->normalize && m->normalize_time, (float)m->dt, ts, K, row_b1,
-                                             row_tn, row_sph, obs, p, r0, n_t, row_obs, row_p);
+  forward_ts_prep_kernel<float><<<K, m->Hm, 0, s>>>(m->d.b1_raw, m->d.w1_full_t, m->Hm, m->S, m->nx + 2, m->normalize && m->normalize_time,
+                                                    (float)m->dt, ts, K, row_b1, row_tn, row_sph, obs, p, r0, n_t, row_obs, row_p);
   NLC_LAUNCH_OK("forward_ts_prep_kernel");
+  return NLC_OK;
+}
+
+// fp64 form (model_grad.cu): first layer from the caller's fp64 weights, dt and the time normalisation in fp64
+int launch_forward_ts_prep_f64(nlc_model_s* m, const double* b1_raw, const double* w1_full_t, const double* ts, int K, double* row_b1,
+                               double* row_tn, double* row_sph, cudaStream_t s) {
+  forward_ts_prep_kernel<double><<<K, m->Hm, 0, s>>>(b1_raw, w1_full_t, m->Hm, m->S, m->nx + 2, m->normalize && m->normalize_time,
+                                                     m->dt, ts, K, row_b1, row_tn, row_sph, nullptr, nullptr, 0, 1, nullptr, nullptr);
+  NLC_LAUNCH_OK("forward_ts_prep_kernel<double>");
   return NLC_OK;
 }
 

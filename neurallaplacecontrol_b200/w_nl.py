@@ -74,6 +74,7 @@ class NeuralLaplaceModel(nn.Module):
         self._cuda_device = torch.device(device) if device is not None else None
         self._handle = None
         self._handle_key = None
+        self._handle_bkey = None
         self._handle_ts = None
 
     # ---- device handle -------------------------------------------------------------------------------------------
@@ -87,7 +88,17 @@ class NeuralLaplaceModel(nn.Module):
             self.__dict__["_fp_tensors"] = ts
         return tuple((v._version, v.data_ptr()) for v in ts)
 
+    def _buffer_key(self):
+        """(version, address) of the buffers (state_mean, state_std, action_mean, action_std, dt) and the device: all of the
+        handle that math_mode="fp64" reads, whose weights come per call."""
+        bs = self.__dict__.get("_fp_buffers")
+        if bs is None:
+            bs = list(self.buffers())
+            self.__dict__["_fp_buffers"] = bs
+        return tuple((v._version, v.data_ptr()) for v in bs), str(self._device())
+
     def _apply(self, fn, *a, **k):
+        self.__dict__["_fp_buffers"] = None
         self.__dict__["_fp_tensors"] = None
         for m in self.modules():
             m.__dict__["_fp_tensors"] = None
@@ -96,6 +107,7 @@ class NeuralLaplaceModel(nn.Module):
     def __setattr__(self, name, value):
         if isinstance(value, (torch.Tensor, nn.Module)):
             self.__dict__["_fp_tensors"] = None
+            self.__dict__["_fp_buffers"] = None
         super().__setattr__(name, value)
 
     def _device(self):
@@ -143,7 +155,15 @@ class NeuralLaplaceModel(nn.Module):
         dev = self._device()
         _lib.check(lib.nlc_model_create(C.byref(h), C.byref(d), dev.index if dev.index is not None else 0), "nlc_model_create")
         self._handle, self._handle_key, self._handle_ts = h, key, float(sd["dt"])
+        self._handle_bkey = self._buffer_key()
         return h
+
+    def _handle_f64(self):
+        """The handle for math_mode="fp64": any live handle built with the current buffers and device serves, however the
+        parameters changed since (an optimizer step does not rebuild it); otherwise ``handle()``."""
+        if self._handle is not None and self._handle_bkey == self._buffer_key():
+            return self._handle
+        return self.handle()
 
     def _free(self):
         if self._handle is not None:
@@ -173,7 +193,11 @@ class NeuralLaplaceModel(nn.Module):
         does: ``torch.squeeze`` of a (K, n_t, nx) result, each sample's history encoded once (``nlc_model_forward_multi``).
 
         In grad mode, when a parameter or an input requires grad, the output carries a ``grad_fn`` like the reference
-        module's: its backward runs ``nlc_model_backward_ts`` (``nlc_model_backward_multi`` for (K, n_t) times; fp32 CUDA cores).  The forward values are the same either way."""
+        module's: its backward runs ``nlc_model_backward_ts`` (``nlc_model_backward_multi`` for (K, n_t) times; fp32 CUDA cores).  The forward values are the same either way.
+
+        ``math_mode="fp64"`` runs every form, forward and backward, in fp64 (``nlc_model_forward_f64`` /
+        ``nlc_model_backward_f64``), the precision the reference trains in: the parameters go to the kernels per call as one
+        flat fp64 tensor, so an optimizer step needs no repacking of the device handle."""
         if torch.is_grad_enabled():
             if torch.is_tensor(ts_pred) and ts_pred.requires_grad:
                 raise NotImplementedError("NeuralLaplaceModel: gradients with respect to ts_pred are not provided")
@@ -184,13 +208,15 @@ class NeuralLaplaceModel(nn.Module):
         out, _ = self._forward_kernels(in_batch_obs, in_batch_action, ts_pred)
         return torch.squeeze(out.to(in_batch_obs.dtype))
 
-    def _inputs(self, in_batch_obs, in_batch_action, ts_pred):
+    def _inputs(self, in_batch_obs, in_batch_action, ts_pred, dtype=torch.float32):
         dev = self._device()
-        obs = in_batch_obs.detach().to(device=dev, dtype=torch.float32).contiguous()
-        act = in_batch_action.detach().to(device=dev, dtype=torch.float32)
+        obs = in_batch_obs.detach().to(device=dev, dtype=dtype).contiguous()
+        act = in_batch_action.detach().to(device=dev, dtype=dtype)
         if act.dim() == 2:
             act = act.unsqueeze(1)
         act = act.contiguous()
+        if dtype == torch.float64 and not torch.is_tensor(ts_pred):
+            ts_pred = torch.as_tensor(ts_pred, dtype=torch.float64)  # a Python float keeps its fp64 value
         ts = torch.as_tensor(ts_pred).detach().to(device=dev, dtype=torch.float64)
         if ts.dim() == 2 and ts.shape[1] >= 2:  # several times per sample: (K, n_t), a 2-D tensor of its own
             if ts.shape[0] != act.shape[0]:
@@ -203,7 +229,9 @@ class NeuralLaplaceModel(nn.Module):
 
     def _forward_kernels(self, in_batch_obs, in_batch_action, ts_pred):
         """(K, nx) or, for (K, n_t) times, (K, n_t, nx) fp32 output of the forward kernels and the prepared inputs
-        (device, obs, act, ts)."""
+        (device, obs, act, ts); fp64, and the prepared inputs with the flat parameters, in math_mode="fp64"."""
+        if self.math_mode == "fp64":
+            return self._forward_f64(in_batch_obs, in_batch_action, ts_pred)
         dev, obs, act, ts = self._inputs(in_batch_obs, in_batch_action, ts_pred)
         K, B = act.shape[0], act.shape[1]
         lib = _lib.load()
@@ -239,9 +267,50 @@ class NeuralLaplaceModel(nn.Module):
                 self.last_p_action = scratch.view(-1)[:2 * K].view(K, 2)
         return out, (dev, obs, act, ts)
 
+    def _forward_f64(self, in_batch_obs, in_batch_action, ts_pred):
+        """``nlc_model_forward_f64``: (K, nx) or (K, n_t, nx) fp64 output and (device, obs, act, ts (K, n_t), flat parameters,
+        n_t given) for the backward."""
+        dev, obs, act, ts = self._inputs(in_batch_obs, in_batch_action, ts_pred, torch.float64)
+        K, B = act.shape[0], act.shape[1]
+        multi = ts.dim() == 2
+        ts2 = (ts if multi else ts.expand(K).reshape(K, 1)).to(torch.float64).contiguous()  # a uniform time becomes per sample
+        n_t = ts2.shape[1]
+        # one flat fp64 tensor in named_parameters() order (one host-to-device copy for CPU parameters)
+        params = torch.cat([p.detach().reshape(-1) for p in self.parameters()]).to(device=dev, dtype=torch.float64)
+        lib = _lib.load()
+        out = torch.empty((K, n_t, self.output_dim), dtype=torch.float64, device=dev)
+        p_action = torch.empty((K, 2), dtype=torch.float64, device=dev)
+        with torch.cuda.device(dev):
+            h = self._handle_f64()
+            ws = torch.empty(int(lib.nlc_model_forward_f64_workspace_bytes(h, K, n_t, B)), dtype=torch.uint8, device=dev)
+            _lib.check(lib.nlc_model_forward_f64(h, params.data_ptr(), obs.data_ptr(), act.data_ptr(), ts2.data_ptr(), K, n_t, B,
+                                                 out.data_ptr(), p_action.data_ptr(), ws.data_ptr(), _lib.current_stream_ptr()),
+                       "nlc_model_forward_f64")
+        self.last_p_action = p_action
+        return (out if multi else out.view(K, self.output_dim)), (dev, obs, act, ts2, params, multi)
+
+    def _backward_f64(self, prepared, grad_out, need_obs, need_act):
+        dev, obs, act, ts, params, multi = prepared
+        K, B, n_t = act.shape[0], act.shape[1], ts.shape[1]
+        lib = _lib.load()
+        g = grad_out.detach().to(device=dev, dtype=torch.float64).reshape(K, n_t, self.output_dim).contiguous()
+        grad_params = torch.empty_like(params)
+        g_obs = torch.empty_like(obs) if need_obs else None
+        g_act = torch.empty_like(act) if need_act else None
+        with torch.cuda.device(dev):
+            h = self._handle_f64()
+            ws = torch.empty(int(lib.nlc_model_backward_f64_workspace_bytes(h, K, n_t, B)), dtype=torch.uint8, device=dev)
+            _lib.check(lib.nlc_model_backward_f64(h, params.data_ptr(), obs.data_ptr(), act.data_ptr(), ts.data_ptr(), K, n_t, B,
+                                                  g.data_ptr(), grad_params.data_ptr(), _lib.ptr(g_obs), _lib.ptr(g_act),
+                                                  ws.data_ptr(), _lib.current_stream_ptr()), "nlc_model_backward_f64")
+        return grad_params, g_obs, g_act
+
     def _backward_kernels(self, prepared, grad_out, need_obs, need_act):
-        """fp32 gradients from ``nlc_model_backward_ts`` (``nlc_model_backward_multi`` for (K, n_t) times): (flat parameter
-        gradients in named_parameters() order, each in its state_dict layout; d obs (K, nx) or None; d act (K, B, gin) or None)."""
+        """fp32 gradients from ``nlc_model_backward_ts`` (``nlc_model_backward_multi`` for (K, n_t) times), fp64 ones from
+        ``nlc_model_backward_f64`` when the forward ran in math_mode="fp64": (flat parameter gradients in named_parameters()
+        order, each in its state_dict layout; d obs (K, nx) or None; d act (K, B, gin) or None)."""
+        if len(prepared) == 6:
+            return self._backward_f64(prepared, grad_out, need_obs, need_act)
         dev, obs, act, ts = prepared
         K, B = act.shape[0], act.shape[1]
         lib = _lib.load()
