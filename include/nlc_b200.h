@@ -13,7 +13,7 @@
  *
  * Arithmetic: fp32 on the device (the reference runs fp64 on the CPU, mppi_with_model.py:65,101);
  * host-side constant folding is done in fp64 and rounded once.  The model's fp64 entry points
- * (nlc_model_forward_f64 / nlc_model_backward_f64) compute in fp64 throughout.
+ * (nlc_model_forward_f64 / nlc_model_backward_f64) and the fp64 planner (nlc_planner_f64_*) compute in fp64 throughout.
  */
 #ifndef NLC_B200_H
 #define NLC_B200_H
@@ -357,6 +357,60 @@ int nlc_planner_exchange_status(nlc_planner_t p, int* connected, int* status);
  * after the step as usual).  Without injected noise the whole step is one CUDA-graph launch.          */
 int nlc_planner_command_host(nlc_planner_t p, const double* state_host, const double* action_buffer_host,
                              const float* noise_in_dev, double* action_host, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * fp64 planner: MPPIDelay.command (mppi_delay.py:193-224) in fp64 throughout, the precision the reference plans in
+ * (its model is .double(), train_utils.py:267; its noise_sigma is fp64, mppi_with_model.py:66-70).  A handle of its own,
+ * single shard, direct launches on the caller's stream.  All tensors are C-contiguous fp64.
+ *   stage 1  roll U, U[-1] = u_init; perturbed = U + noise, the null sample, bound(perturbed u_scale)/u_scale,
+ *            noise = perturbed - U, hist and actions: round-to-nearest fp64 operations in the reference's order, so these
+ *            tensors are bit-identical to the reference's for the same noise;
+ *   model    the K T history windows through the fp64 encoder, then per tile of 32 samples the whole horizon: fp64 MLP,
+ *            Fourier ILT at dt (the arithmetic of nlc_model_forward_f64 at a uniform time), state += delta, running cost;
+ *            analytic dynamics: one fp64 Euler step (oracle.py:11-224) per step instead;
+ *   stage 4  beta = min c, w = exp(-(1/lambda)(c - beta)), eta = sum w, U[t] += sum_k (w_k/eta) noise[k][t]: fixed-order
+ *            sums, so two calls on the same inputs give bit-identical results.
+ * On-device sampler (noise_in_dev NULL): Philox4x32-10, key = seed, counter = (idx_lo, idx_hi, call_lo, call_hi) with
+ * idx = k T + t and the call index counting this planner's control steps (as nlc_perturb).  Of the four output words
+ * (x0, x1, x2, x3): u1 = (2 ((x0 >> 6) 2^26 + (x1 >> 6)) + 1) 2^-53 and u2 likewise from (x2, x3) - 53-bit uniforms in
+ * (0, 1), never 0 or 1 - and z0 = r cos(2 pi u2), z1 = r sin(2 pi u2), r = sqrt(-2 log u1) (fp64 sincospi).  nu > 2 takes
+ * z2, z3 from a second block, counter word 3 = call_hi ^ 0x80000000.  noise[u] = mu[u] + sum_{v <= u} L[u][v] z[v]
+ * (fp64 FMAs, v ascending), L = sigma_chol.
+ * ------------------------------------------------------------------------------------------------ */
+typedef struct nlc_planner_f64_s* nlc_planner_f64_t;
+
+typedef struct {
+  /* K, T, nu, B, nx, env, state_constraint, dynamics, delay, keep_states, seed, sample_null_action, noise_abs_cost,
+   * has_bounds are read from base; its float values (lambda_, u_scale, bounds, sigma, mu, u_init, goal_x, dt), k_offset,
+   * k_total, shard_index and math_mode are ignored; n_shards must be 1 (else NLC_ERR_UNSUPPORTED).                     */
+  nlc_planner_desc base;
+  double lambda_, u_scale, dt, goal_x;
+  double u_min[4], u_max[4];
+  double sigma_inv[16], sigma_chol[16], noise_mu[4], u_init[4];  /* [nu][nu] row-major; sigma_chol lower triangular */
+} nlc_planner_f64_desc;
+
+/* model: NULL for analytic dynamics.  The model handle supplies shapes, flags and the fp64 normalisation constants; the
+ * planner takes a reference on it (as nlc_planner_create).  B in [1, 8], T nu <= 256.                               */
+int nlc_planner_f64_create(nlc_planner_f64_t* out, nlc_model_t model, const nlc_planner_f64_desc* d, int device);
+int nlc_planner_f64_destroy(nlc_planner_f64_t p);
+/* The model's 16 parameters, fp64 on the device, in the layout of nlc_model_backward_f64's params_dev: rearranged into the
+ * planner's own weight image (and the first layer folded at dt) on `stream`; later commands use them until the next call.
+ * Required before the first command of a Neural Laplace planner.                                                    */
+int nlc_planner_f64_set_params(nlc_planner_f64_t p, const double* params_dev, void* stream);
+/* host fp64 [T][nu]; synchronous                                                                                     */
+int nlc_planner_f64_set_U(nlc_planner_f64_t p, const double* U_host);
+int nlc_planner_f64_get_U(nlc_planner_f64_t p, double* U_host);
+/* Device buffers as in nlc_planner_buffer (NLC_BUF_U .. NLC_BUF_ACTION_BUFFER, without the triples), sizes in doubles:
+ * WEIGHTS holds w = exp(-(1/lambda)(c - beta)) (cost_total_non_zero), STATS (beta, eta).                            */
+int nlc_planner_f64_buffer(nlc_planner_f64_t p, int which, void** dev_ptr, int64_t* n_doubles);
+/* One control step on device inputs: state_dev [nx] (state_per_sample 0) or [K][nx] (1), action_buffer_dev [B][nu],
+ * noise_in_dev [K][T][nu] or NULL (the on-device sampler).  The action [nu] = U[0] u_scale lands in NLC_BUF_ACTION.  */
+int nlc_planner_f64_command(nlc_planner_f64_t p, const double* state_dev, int state_per_sample, const double* action_buffer_dev,
+                            const double* noise_in_dev, void* stream);
+/* The same with host buffers (state [nx], action_buffer [B][nu]) and the on-device sampler: copies in, one control step,
+ * the action [nu] copied back to action_host; synchronises the stream.                                              */
+int nlc_planner_f64_command_host(nlc_planner_f64_t p, const double* state_host, const double* action_buffer_host,
+                                 double* action_host, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Instance-batched planning and the closed loop (BASELINE config 5; the caller side of the path,

@@ -62,6 +62,13 @@ class PlannerDesc(C.Structure):
                 ("shard_index", C.c_int32), ("math_mode", C.c_int32), ("keep_states", C.c_int32), ("seed", C.c_uint64)]
 
 
+class PlannerF64Desc(C.Structure):
+    """``nlc_planner_f64_desc``: the fp32 planner's descriptor for shapes and flags, and the fp64 values beside it."""
+    _fields_ = [("base", PlannerDesc), ("lambda_", C.c_double), ("u_scale", C.c_double), ("dt", C.c_double), ("goal_x", C.c_double),
+                ("u_min", C.c_double * 4), ("u_max", C.c_double * 4), ("sigma_inv", C.c_double * 16),
+                ("sigma_chol", C.c_double * 16), ("noise_mu", C.c_double * 4), ("u_init", C.c_double * 4)]
+
+
 # name -> (restype, argtypes); also the list the CPU test checks against include/nlc_b200.h
 SIGNATURES = {
     "nlc_last_error": (C.c_char_p, []),
@@ -112,6 +119,14 @@ SIGNATURES = {
     "nlc_planner_exchange_connect": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "nlc_planner_exchange_status": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "nlc_planner_command_host": (C.c_int, [C.c_void_p, _dp, _dp, _fp, _dp, C.c_void_p]),
+    "nlc_planner_f64_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.POINTER(PlannerF64Desc), C.c_int]),
+    "nlc_planner_f64_destroy": (C.c_int, [C.c_void_p]),
+    "nlc_planner_f64_set_params": (C.c_int, [C.c_void_p, _fp, C.c_void_p]),
+    "nlc_planner_f64_set_U": (C.c_int, [C.c_void_p, _dp]),
+    "nlc_planner_f64_get_U": (C.c_int, [C.c_void_p, _dp]),
+    "nlc_planner_f64_buffer": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),
+    "nlc_planner_f64_command": (C.c_int, [C.c_void_p, _fp, C.c_int, _fp, _fp, C.c_void_p]),
+    "nlc_planner_f64_command_host": (C.c_int, [C.c_void_p, _dp, _dp, _dp, C.c_void_p]),
     "nlc_batch_planner_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.POINTER(PlannerDesc), C.c_int,
                                            C.POINTER(C.c_uint64), C.c_int]),
     "nlc_batch_planner_destroy": (C.c_int, [C.c_void_p]),

@@ -128,4 +128,91 @@ __device__ __forceinline__ void env_analytic_step(const nlc_rollout_opts& o, flo
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// fp64 forms for the fp64 planner (planner_f64.cu, model_grad.cu plan_f64_rollout_kernel): the reference's expressions in
+// its own evaluation order (oracle/costs.py, oracle/dynamics.py), acrobot through atan2 / sincos as the reference does.
+// goal_x and dt come in fp64 (the float opts cannot hold dt = 0.05 exactly).
+// ---------------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ double trig2angle(double c, double s) {  // base_env.py:297-301
+  const double C = c * c + s * s;
+  c = c / C; s = s / C;
+  return atan2(s / C, c / C);
+}
+
+__device__ __forceinline__ double env_running_cost(int env, int state_constraint, double goal_x, const double* s, const double* u,
+                                                   int nu) {
+  double ac = 0.0;
+  for (int i = 0; i < nu; ++i) ac = ac + u[i] * u[i];
+  if (env == NLC_ENV_PENDULUM) {
+    const double om = 1.0 - s[0];
+    const double state_reward = -(om * om + s[1] * s[1]);
+    const double reward = state_reward + 0.01 * (-(s[2] * s[2]));
+    return -(reward + (-0.01 * ac));
+  } else if (env == NLC_ENV_CARTPOLE) {
+    const double ex = (s[0] + s[3]) - goal_x;
+    const double ey = s[2] - 1.0;
+    const double state_reward = state_constraint ? -((ex * ex + exp(ex * 10.0 + 7.0)) + ey * ey) : -(ex * ex + ey * ey);
+    const double vel = -(s[1] * s[1]) - s[4] * s[4];
+    const double reward = state_reward + 0.01 * vel;
+    return -(reward + (-0.01 * ac));
+  } else {
+    const double th1 = trig2angle(s[0], s[1]);
+    const double th2 = trig2angle(s[2], s[3]);
+    const double vel = -(s[4] * s[4]) - s[5] * s[5];
+    double s1, c1, s12, c12;
+    sincos(th1, &s1, &c1);
+    sincos(th1 + th2, &s12, &c12);
+    const double p2x = -c1 - c12, p2y = s1 + s12;
+    const double dx = (p2x - 1.0) - 1.0;
+    const double state_reward = -(dx * dx) - p2y * p2y;
+    const double reward = state_reward + 0.1 * vel;
+    return -(reward + (-1e-4 * ac));
+  }
+}
+
+__device__ __forceinline__ void env_analytic_step(int env, double ts, double* s, const double* u) {
+  if (env == NLC_ENV_PENDULUM) {
+    const double th = trig2angle(s[0], s[1]);
+    const double thdot = s[2];
+    const double uu = fmin(fmax(u[0], -2.0), 2.0);
+    const double newth = th + thdot * ts;
+    const double newthdot = thdot + (-15.0 * sin(th + 3.141592653589793) + 3.0 * uu) * ts;
+    double sn, cs;
+    sincos(newth, &sn, &cs);
+    s[0] = cs; s[1] = sn; s[2] = newthdot;
+  } else if (env == NLC_ENV_CARTPOLE) {
+    const double x = s[0], x_dot = s[1], theta_dot = s[4];
+    const double C = s[2] * s[2] + s[3] * s[3];
+    const double costheta = s[2] / C, sintheta = s[3] / C;
+    const double theta = atan2(sintheta / C, costheta / C);
+    const double force = fmin(fmax(u[0], -3.0), 3.0) * 3.0;
+    const double total_mass = 0.1 + 1.0, pml = 0.1 * 1.0;
+    const double temp = (force + pml * theta_dot * theta_dot * sintheta) / total_mass;
+    const double thetaacc = (9.8 * sintheta - costheta * temp) / (1.0 * (4.0 / 3.0 - 0.1 * costheta * costheta / total_mass));
+    const double xacc = temp - pml * thetaacc * costheta / total_mass;
+    const double new_theta = theta + theta_dot * ts;
+    double sn, cs;
+    sincos(new_theta, &sn, &cs);
+    s[0] = x + x_dot * ts; s[1] = x_dot + xacc * ts; s[2] = cs; s[3] = sn; s[4] = theta_dot + thetaacc * ts;
+  } else {
+    const double th1 = trig2angle(s[0], s[1]);
+    const double th2 = trig2angle(s[2], s[3]);
+    const double d1_ = s[4], d2_ = s[5];
+    const double a0 = fmin(fmax(u[0], -5.0), 5.0), a1 = fmin(fmax(u[1], -5.0), 5.0);
+    const double c2 = cos(th2), s2 = sin(th2);
+    // m1 = m2 = l1 = I1 = I2 = 1, lc1 = lc2 = 0.5, g = 9.8 (oracle/dynamics.py)
+    const double d1 = 0.25 + (1.0 + 0.25 + 1.0 * c2) + 1.0 + 1.0;
+    const double d2 = (0.25 + 0.5 * c2) + 1.0;
+    const double phi2 = 0.5 * 9.8 * cos(th1 + th2 - 1.5707963267948966);
+    const double phi1 = -0.5 * (d2_ * d2_) * s2 - 1.0 * d2_ * d1_ * s2 + (0.5 + 1.0) * 9.8 * cos(th1 - 1.5707963267948966) + phi2;
+    const double dd2 = (a0 + d2 / d1 * phi1 - 0.5 * (d1_ * d1_) * s2 - phi2) / (0.25 + 1.0 - d2 * d2 / d1);
+    const double dd1 = -(a1 + d2 * dd2 + phi1) / d1;
+    const double n1 = th1 + d1_ * ts, n2 = th2 + d2_ * ts;
+    double sa, ca, sb, cb;
+    sincos(n1, &sa, &ca);
+    sincos(n2, &sb, &cb);
+    s[0] = ca; s[1] = sa; s[2] = cb; s[3] = sb; s[4] = d1_ + dd1 * ts; s[5] = d2_ + dd2 * ts;
+  }
+}
+
 }  // namespace nlc

@@ -34,9 +34,12 @@
 // layouts ModelDev holds (TileW); only shapes, flags, dt and the fp64 normalisation constants are read from the handle.
 // The fp64 forward is the recompute half of the tile steps (encoder, linear_out, MLP) followed by the ILT sum; the fp64
 // backward runs the two-stage form of nlc_model_backward_multi for every n_t (n_t = 1 included).
+//
+// The fp64 planner (planner_f64.cu) runs its history encoder and rollout on the same tile steps: plan_f64_* at the end.
 #include <stddef.h>
 
 #include "common.cuh"
+#include "env_cost.cuh"
 
 namespace nlc {
 
@@ -1151,3 +1154,172 @@ extern "C" int nlc_model_backward_f64(nlc_model_t m, const double* params_dev, c
   NLC_LAUNCH_OK("model_grad_reduce_kernel<double>");
   return NLC_OK;
 }
+
+// ---------------------------------------------------------------------------------------------------------------------
+// The fp64 planner's model stages (nlc_planner_f64_*, planner_f64.cu): the tile steps above over a control step's K T
+// history windows (plan_f64_encode_kernel) and its K rollouts (plan_f64_rollout_kernel).  The weights are the image
+// model_f64_weights_kernel builds from the caller's parameters, the s-point columns of the first layer are folded at the
+// planner's dt by forward_ts_prep_kernel<double> - the arithmetic of nlc_model_forward_f64 at a uniform time, so a step of
+// the rollout equals that forward bit for bit.
+// ---------------------------------------------------------------------------------------------------------------------
+namespace nlc {
+
+struct PlanF64Args {
+  TileW<double> m;
+  GradShape g;
+  const double* hist;       // [K][L][hist_ch] env units, L = B - 1 + T
+  int hist_ch;              // channels stored per entry: an encode_obs_time model's time channel is synthesised
+  const double* p;          // [K][T][2] encoder outputs
+  const double* state0;     // [nx] (sps = 0) or [K][nx] (sps = 1)
+  int sps;
+  const double* row_b1;     // [H] first-layer bias with the s-point columns folded at dt
+  const double* row_tn;     // [1] the (normalised) prediction time
+  const double* pert_cost;  // [K]
+  int env, state_constraint;
+  double goal_x;
+  double* p_out;            // [K][T][2]
+  double* cost;             // [K]
+  double* states;           // [K][T][nx] or null
+  double* scratch;          // [grid][s_total]
+  int K, T;
+};
+
+// Window w = k T + t is hist[k][t : t + B] (mppi_delay.py:261-288), read in the order of tile_load_window.
+template <int H>
+__global__ void __launch_bounds__(kGradThreads, 1) plan_f64_encode_kernel(PlanF64Args a) {
+  const GradShape& g = a.g;
+  const TileW<double>& md = a.m;
+  constexpr int R = kGradRows;
+  const TileBufs<double> t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
+  const long long n_win = (long long)a.K * a.T;
+  const long long n_tiles = (n_win + R - 1) / R;
+  const int B = g.B, gin = g.gin, L = B - 1 + a.T;
+  for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const long long w0 = tile * R;
+    __syncthreads();  // the previous tile's last reads of the scratch are done
+    for (int i = threadIdx.x; i < B * R * 4; i += kGradThreads) {
+      const int st = i / (R * 4), m = (i / 4) % R, u = i & 3;
+      const long long w = w0 + m < n_win ? w0 + m : n_win - 1;
+      const long long k = w / a.T;
+      const int tt = (int)(w - k * a.T), j = B - 1 - st;
+      double v = 0.0;
+      if (u < gin) {
+        const double x = u < a.hist_ch ? a.hist[((size_t)k * L + tt + j) * a.hist_ch + u] : (double)(B - 1 - j);
+        v = (x - md.act_mean[u]) * md.act_inv_std[u];
+      }
+      t.xs[i] = v;
+    }
+    __syncthreads();
+    tile_encoder_fwd<H>(g, md, t);
+    tile_linear_out(g, md, t);
+    __syncthreads();
+    for (int i = threadIdx.x; i < R * 2; i += kGradThreads) {
+      const int m = i >> 1, o = i & 1;
+      if (w0 + m < n_win) a.p_out[(size_t)(w0 + m) * 2 + o] = t.x1[m * g.in0p + 2 * g.S + g.nx + o];
+    }
+  }
+}
+
+// A tile of kGradRows samples through the whole horizon: per step the model (tile_rows_input's first-layer input,
+// tile_mlp_fwd, tile_ilt_out's sum), state += delta, and the running cost (mppi_delay.py:232-313).
+template <int H>
+__global__ void __launch_bounds__(kGradThreads, 1) plan_f64_rollout_kernel(PlanF64Args a) {
+  using C = Real<double>;
+  const GradShape& g = a.g;
+  const TileW<double>& md = a.m;
+  constexpr int R = kGradRows;
+  const int S = g.S, nx = g.nx, nu = g.nu, Lp = g.Lp, in0p = g.in0p, N3p = g.N3p, T = a.T, B = g.B, L = B - 1 + T;
+  __shared__ double st[R][kMaxNx], dl[R][kMaxNx], acc[R];
+  const TileBufs<double> t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
+  const int n_tiles = (a.K + R - 1) / R;
+  for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const int k0 = tile * R;
+    __syncthreads();  // the previous tile's last reads of the scratch and of st / acc are done
+    for (int i = threadIdx.x; i < R * nx; i += kGradThreads) {
+      const int m = i / nx, c = i - m * nx, k = min(k0 + m, a.K - 1);
+      st[m][c] = a.state0[(size_t)(a.sps ? k : 0) * nx + c];
+    }
+    for (int m = threadIdx.x; m < R; m += kGradThreads) acc[m] = 0.0;
+    tile_fourier_consts(a.row_tn, 0, 1, t.rc);
+    __syncthreads();
+    for (int tt = 0; tt < T; ++tt) {
+      for (int i = threadIdx.x; i < R * Lp; i += kGradThreads) {
+        const int m = i / Lp, j = i - m * Lp;
+        const size_t k = (size_t)min(k0 + m, a.K - 1);
+        t.x1[m * in0p + 2 * S + j] = j < nx ? (st[m][j] - md.state_mean[j]) * md.state_inv_std[j] : a.p[(k * T + tt) * 2 + (j - nx)];
+      }
+      __syncthreads();
+      tile_mlp_fwd<H>(g, md, t, a.row_b1, 0, 1);
+      for (int i = threadIdx.x; i < R * nx; i += kGradThreads) {
+        const int m = i / nx, c = i - m * nx;
+        const double* o = t.dob + m * N3p + 2 * c * S;
+        double d = 0.0;
+        for (int kk = 0; kk < S; ++kk) {
+          double ph, wt;
+          ilt_term_consts(kk, t.rc, m, ph, wt);
+          d += wt * sphere_radius(o[2 * kk + 1]) * cos_reduced(C::pi * tanh_acc(o[2 * kk]) + ph);
+        }
+        dl[m][c] = d;
+      }
+      __syncthreads();
+      for (int m = threadIdx.x; m < R; m += kGradThreads) {
+        const int k = min(k0 + m, a.K - 1);
+        for (int c = 0; c < nx; ++c) st[m][c] = st[m][c] + dl[m][c];
+        acc[m] = acc[m] + env_running_cost(a.env, a.state_constraint, a.goal_x, st[m], a.hist + ((size_t)k * L + tt + B - 1) * nu, nu);
+        if (a.states && k0 + m < a.K)
+          for (int c = 0; c < nx; ++c) a.states[((size_t)k * T + tt) * nx + c] = st[m][c];
+      }
+      __syncthreads();
+    }
+    for (int m = threadIdx.x; m < R; m += kGradThreads)
+      if (k0 + m < a.K) a.cost[k0 + m] = acc[m] + a.pert_cost[k0 + m];
+  }
+}
+
+static int plan_f64_grid(long long rows) { return rows >= (long long)kGradGridCap * kGradRows ? kGradGridCap : (int)((rows + kGradRows - 1) / kGradRows); }
+
+// Doubles of the weight image (model_f64_weights_kernel's layout) and of the per-CTA tile scratch of the two kernels.
+size_t plan_f64_image_doubles(nlc_model_t m) { return shape_of(m, 1).f_total; }
+size_t plan_f64_scratch_doubles(nlc_model_t m, int B, int K, int T) {
+  return (size_t)plan_f64_grid((long long)K * T) * shape_of(m, B).s_total;  // the encoder's grid: at least the rollout's
+}
+
+// The weight image of params_dev and the first-layer bias row_b1 [H] / time row_tn [1] at the prediction time ts_dev [1].
+int plan_f64_set_params(nlc_model_t m, const double* params_dev, const double* ts_dev, double* img, double* row_b1, double* row_tn,
+                        cudaStream_t s) {
+  const GradShape g = shape_of(m, 1);
+  const int n_img = g.N3p * g.H > g.in0 * g.H ? g.N3p * g.H : g.in0 * g.H;
+  model_f64_weights_kernel<<<(n_img + 255) / 256, 256, 0, s>>>(g, params_dev, img);
+  NLC_LAUNCH_OK("model_f64_weights_kernel");
+  const TileW<double> w = tile_w_f64(m->d, g, img);
+  return launch_forward_ts_prep_f64(m, w.b1_raw, w.w1_full_t, ts_dev, 1, row_b1, row_tn, nullptr, s);
+}
+
+int plan_f64_encode(nlc_model_t m, int B, const double* img, const double* hist, int hist_ch, int K, int T, double* p_out,
+                    double* scratch, cudaStream_t s) {
+  PlanF64Args a = {};
+  a.g = shape_of(m, B); a.m = tile_w_f64(m->d, a.g, img);
+  a.hist = hist; a.hist_ch = hist_ch; a.p_out = p_out; a.scratch = scratch; a.K = K; a.T = T;
+  const int G = plan_f64_grid((long long)K * T);
+  if (m->Hm == 128) plan_f64_encode_kernel<128><<<G, kGradThreads, 0, s>>>(a);
+  else plan_f64_encode_kernel<64><<<G, kGradThreads, 0, s>>>(a);
+  NLC_LAUNCH_OK("plan_f64_encode_kernel");
+  return NLC_OK;
+}
+
+int plan_f64_rollout(nlc_model_t m, int B, const double* img, const double* row_b1, const double* row_tn, const double* state0, int sps,
+                     const double* hist, const double* p, const double* pert_cost, int K, int T, int env, int state_constraint,
+                     double goal_x, double* cost, double* states, double* scratch, cudaStream_t s) {
+  PlanF64Args a = {};
+  a.g = shape_of(m, B); a.m = tile_w_f64(m->d, a.g, img);
+  a.hist = hist; a.p = p; a.state0 = state0; a.sps = sps; a.row_b1 = row_b1; a.row_tn = row_tn; a.pert_cost = pert_cost;
+  a.env = env; a.state_constraint = state_constraint; a.goal_x = goal_x; a.cost = cost; a.states = states; a.scratch = scratch;
+  a.K = K; a.T = T;
+  const int G = plan_f64_grid(K);
+  if (m->Hm == 128) plan_f64_rollout_kernel<128><<<G, kGradThreads, 0, s>>>(a);
+  else plan_f64_rollout_kernel<64><<<G, kGradThreads, 0, s>>>(a);
+  NLC_LAUNCH_OK("plan_f64_rollout_kernel");
+  return NLC_OK;
+}
+
+}  // namespace nlc

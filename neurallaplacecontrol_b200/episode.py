@@ -37,6 +37,8 @@ class BatchedMPPIDelay:
     def __init__(self, dynamics, running_cost, nx, noise_sigma, n_instances, seeds=None, U_init=None, **kw):
         if "process_group" in kw and kw["process_group"] is not None:
             raise NotImplementedError("BatchedMPPIDelay shards by instance: give each rank its own instances")
+        if kw.get("math_mode") == "fp64":
+            raise NotImplementedError("BatchedMPPIDelay has no fp64 mode: plan each instance with MPPIDelay(math_mode='fp64')")
         self.I = int(n_instances)
         self.seeds = list(range(self.I)) if seeds is None else [int(s) for s in seeds]
         if len(self.seeds) != self.I:

@@ -18,7 +18,17 @@ Differences a caller can see, all deliberate:
   ``torch.distributed`` group (one exchange of the (beta, eta, W) triple per control step), ``seed`` keys the
   on-device Philox sampler, ``math_mode`` selects the contraction arithmetic (default ``"tc_split3"``: tcgen05 tensor
   cores, fp16 hi/lo split operands, fp32 accumulate - fp32-class, the 1e-4 bound; ``"fp32"`` = CUDA-core FFMA anchor;
-  ``"tc_fp16"`` = single pass, 2e-2 bound), ``keep_states`` can drop the ``states`` trajectory output.
+  ``"tc_fp16"`` = single pass, 2e-2 bound; ``"fp64"`` = the whole control step in fp64, see below), ``keep_states`` can
+  drop the ``states`` trajectory output.
+
+``math_mode="fp64"`` plans at the reference's own precision (its model is ``.double()``, ``train_utils.py:267``, and its
+``noise_sigma`` fp64): the object is an fp64 planner (``nlc_planner_f64_*``) whose kernels compute every stage in fp64 -
+stage 1 bit-identical to the reference for the same noise, the model as ``NeuralLaplaceModel(math_mode="fp64")`` computes it,
+fixed-order softmax sums.  It works whatever the model's own ``math_mode``: before every control step the model's parameters
+go to the device as one flat fp64 tensor when they changed (``_fingerprint``), so an optimizer step between two commands is
+planned with.  Post-call attributes are fp64 CUDA tensors (zero-copy views), injected noise is kept in fp64.  It plans on one
+GPU: ``process_group`` / ``shard``, ``get_rollouts``, ``set_inputs`` / ``step`` and ``BatchedMPPIDelay`` raise
+``NotImplementedError``.
 
 Noise injection for parity tests works as on the reference: replace ``planner.noise_dist.sample`` with a callable
 returning the ``(K, T, nu)`` tensor (it is called once per ``command`` with ``(K, T)``, ``mppi_delay.py:319``).
@@ -43,8 +53,8 @@ _NULL_CTX = contextlib.nullcontext()
 class _DevView:
     """Zero-copy torch view of a raw device buffer through ``__cuda_array_interface__``."""
 
-    def __init__(self, ptr, shape):
-        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": "<f4", "data": (int(ptr), False), "version": 2}
+    def __init__(self, ptr, shape, typestr="<f4"):
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (int(ptr), False), "version": 2}
 
 
 def _bound_vector(x, nu, name):
@@ -62,6 +72,11 @@ def _bound_vector(x, nu, name):
 
 
 class MPPIDelay:
+    def __new__(cls, *args, **kw):
+        if cls is MPPIDelay and kw.get("math_mode") == "fp64":
+            cls = _MPPIDelayF64  # a planner object of its own (nlc_planner_f64_*): see its docstring
+        return super().__new__(cls)
+
     def __init__(self, dynamics, running_cost, nx, noise_sigma, num_samples=100, horizon=15, device="cpu",
                  terminal_state_cost=None, lambda_=1.0, noise_mu=None, u_min=None, u_max=None, u_init=None,
                  U_init=None, u_scale=1, u_per_command=1, step_dependent_dynamics=False, rollout_samples=1,
@@ -566,3 +581,191 @@ class MPPIDelay:
             _lib.check(self._lib.nlc_rollout_cost(mh, C.byref(ro), st.data_ptr(), 1, p.data_ptr(), hist.data_ptr(), None, n, self.T, 1,
                                                   self.nu, cost.data_ptr(), states.data_ptr(), fp32, stream), "nlc_rollout_cost")
         return states.to(self.dtype)
+
+
+class _MPPIDelayF64(MPPIDelay):
+    """``MPPIDelay(..., math_mode="fp64")``: the control step on the fp64 planner handle (``nlc_planner_f64_*``), single shard,
+    direct launches on the current stream (host inputs: one C call that copies in, plans and copies the action back)."""
+
+    def __init__(self, *args, process_group=None, shard=None, **kw):
+        if process_group is not None or shard is not None:
+            raise NotImplementedError("math_mode='fp64' plans on one GPU: K sharding (process_group / shard) is not implemented")
+        super().__init__(*args, **kw)
+        self._params_key = None
+        self._params_dev = None
+
+    def _desc_f64(self, B):
+        d = _lib.PlannerF64Desc()
+        b = d.base
+        mp = b.mppi
+        mp.K, mp.T, mp.nu, mp.B, mp.k_offset, mp.k_total = self.K, self.T, self.nu, B, 0, self.K
+        mp.has_bounds = int(self._bounds is not None)
+        mp.sample_null_action, mp.noise_abs_cost = int(self.sample_null_action), int(self.noise_abs_cost)
+        ro = b.rollout
+        ro.env = _lib.ENV_IDS[self.running_cost.env_name]
+        ro.state_constraint, ro.dynamics, ro.delay = int(self.running_cost.state_constraint), self.F.kind, int(self.F.delay)
+        b.nx, b.n_shards, b.shard_index, b.keep_states, b.seed = self.nx, 1, 0, int(self.keep_states), self.seed
+        d.lambda_, d.u_scale, d.dt, d.goal_x = float(self.lambda_), float(self.u_scale), float(self.F.dt), float(self.running_cost.goal_x)
+        if self._bounds is not None:
+            for i in range(self.nu):
+                d.u_min[i], d.u_max[i] = self._bounds[0][i], self._bounds[1][i]
+        sinv = self.noise_sigma_inv.to(torch.float64).reshape(self.nu, self.nu)
+        chol = torch.linalg.cholesky(self.noise_sigma.to(torch.float64).reshape(self.nu, self.nu))
+        for i in range(self.nu):
+            d.noise_mu[i] = float(self.noise_mu.reshape(-1)[i])
+            d.u_init[i] = float(torch.as_tensor(self.u_init).reshape(-1)[i])
+            for j in range(self.nu):
+                d.sigma_inv[i * self.nu + j], d.sigma_chol[i * self.nu + j] = float(sinv[i, j]), float(chol[i, j])
+        return d
+
+    def _ensure(self, B):
+        """The fp64 planner for a B-entry action buffer, rebuilt when the model's handle is a new one (its buffers or device
+        changed); its weights come separately (``_push_params``)."""
+        model_h = None
+        if isinstance(self.F, NLDynamics):
+            if self.F.model._cuda_device is None:
+                self.F.model._cuda_device = self.d
+            with self._on_device():
+                model_h = self.F.model._handle_f64()
+        key = None if model_h is None else model_h.value
+        if self._handle is not None and self._handle_B == B and self._handle_model == key:
+            return self._handle
+        self._destroy()
+        h = C.c_void_p()
+        _lib.check(self._lib.nlc_planner_f64_create(C.byref(h), model_h, C.byref(self._desc_f64(B)), self.d.index), "nlc_planner_f64_create")
+        self._handle, self._handle_B, self._handle_model, self._views = h, B, key, {}
+        self._U_dirty = True
+        self._params_key = None
+        return h
+
+    def _push_params(self, h, stream):
+        """The model's parameters as one flat fp64 tensor (named_parameters() order, the ``_forward_f64`` layout), sent only
+        when they changed since the last control step."""
+        if not isinstance(self.F, NLDynamics):
+            return
+        model = self.F.model
+        key = model._fingerprint()
+        if key == self._params_key:
+            return
+        params = torch.cat([p.detach().reshape(-1) for p in model.parameters()]).to(device=self.d, dtype=torch.float64)
+        _lib.check(self._lib.nlc_planner_f64_set_params(h, params.data_ptr(), stream), "nlc_planner_f64_set_params")
+        self._params_dev, self._params_key = params, key
+
+    def _destroy(self):
+        if self._handle is not None:
+            self._sync_U_to_host()
+            self._lib.nlc_planner_f64_destroy(self._handle)
+            self._handle = None
+            self._views = {}
+
+    def __del__(self):
+        try:
+            if self._handle is not None:
+                self._lib.nlc_planner_f64_destroy(self._handle)
+        except Exception:
+            pass
+
+    def _buf(self, which, shape):
+        """fp64 CUDA tensor aliasing one of the fp64 planner's device buffers."""
+        key = (which, tuple(shape))
+        if key not in self._views:
+            p, n = C.c_void_p(), C.c_int64()
+            _lib.check(self._lib.nlc_planner_f64_buffer(self._handle, which, C.byref(p), C.byref(n)), "nlc_planner_f64_buffer")
+            if p.value is None or n.value == 0:
+                return None
+            assert int(np.prod(shape)) == n.value, (which, shape, n.value)
+            self._views[key] = torch.as_tensor(_DevView(p.value, shape, "<f8"), device=self.d)
+        return self._views[key]
+
+    def _sync_U_to_host(self):
+        if self._handle is not None and not self._U_dirty:
+            arr = np.empty(self.T * self.nu, dtype=np.float64)
+            _lib.check(self._lib.nlc_planner_f64_get_U(self._handle, arr.ctypes.data_as(C.POINTER(C.c_double))), "nlc_planner_f64_get_U")
+            self._U_host = torch.from_numpy(arr).reshape(self.T, self.nu).clone()
+
+    def _push_U(self):
+        if self._U_dirty:
+            ptr, keep = _lib.as_double_array(self._U_host.numpy())
+            _lib.check(self._lib.nlc_planner_f64_set_U(self._handle, ptr), "nlc_planner_f64_set_U")
+            self._U_dirty = False
+
+    @property
+    def cost_total_non_zero(self):
+        """exp(-(1/lambda)(c - beta)) (mppi_delay.py:210-211)."""
+        return self._after(_lib.BUF_WEIGHTS, (self.K,))
+
+    @property
+    def omega(self):
+        nz = self.cost_total_non_zero
+        return None if nz is None else (1.0 / self._buf(_lib.BUF_STATS, (2,))[1]) * nz
+
+    def _injected_noise(self):
+        fn = self.noise_dist.__dict__.get("sample")
+        if fn is None:
+            return None
+        nz = torch.as_tensor(fn((self.K, self.T)))
+        if tuple(nz.shape) != (self.K, self.T, self.nu):
+            raise ValueError(f"injected noise must have shape {(self.K, self.T, self.nu)}, got {tuple(nz.shape)}")
+        return nz.to(device=self.d, dtype=torch.float64).contiguous()
+
+    def command(self, state, action_buffer):
+        """:param state: (nx) or (K x nx) current state; :param action_buffer: (B x nu) past actions, env units.
+        :returns action: (nu) best action (``mppi_delay.py:193-224``), ``(u_per_command, nu)`` for ``u_per_command > 1``."""
+        action_buffer = torch.as_tensor(action_buffer)
+        if self.encode_obs_time:
+            action_buffer = action_buffer[:, :self.nu]  # the time column is not read by the analytic dynamics (oracle.py:23)
+        B = action_buffer.shape[0]
+        h = self._ensure(B)
+        self._push_U()
+        if not torch.is_tensor(state):
+            state = torch.tensor(np.asarray(state))
+        self.state = state.to(dtype=self.dtype)
+        noise = self._injected_noise()
+        per_sample = state.dim() == 2 and state.shape[0] != 1
+        with self._on_device():
+            stream = _lib.current_stream_ptr()
+            self._push_params(h, stream)
+            if not per_sample and noise is None and not state.is_cuda and not action_buffer.is_cuda:
+                sp, k1 = _lib.as_double_array(state.detach().reshape(-1).numpy())
+                bp, k2 = _lib.as_double_array(action_buffer.detach().reshape(-1).numpy())
+                out = np.empty(self.nu, dtype=np.float64)
+                _lib.check(self._lib.nlc_planner_f64_command_host(h, sp, bp, out.ctypes.data_as(C.POINTER(C.c_double)), stream),
+                           "nlc_planner_f64_command_host")
+                self.last_action_host = out
+            else:
+                if per_sample and state.shape[0] != self.K:
+                    raise ValueError("per-sample states must have K rows")
+                st = (state if per_sample else state.reshape(-1)).to(device=self.d, dtype=torch.float64).contiguous()
+                ab = action_buffer.reshape(B, self.nu).to(device=self.d, dtype=torch.float64).contiguous()
+                _lib.check(self._lib.nlc_planner_f64_command(h, st.data_ptr(), int(per_sample), ab.data_ptr(), _lib.ptr(noise), stream),
+                           "nlc_planner_f64_command")
+                self.last_action_host = None
+        self._calls += 1
+        return self._first_actions(self._buf(_lib.BUF_ACTION, (self.nu,)).to(self.dtype, copy=True))
+
+    def _unsupported(self, what):
+        raise NotImplementedError(f"{what} is not implemented for math_mode='fp64' (single-GPU command() only)")
+
+    def set_inputs(self, state, action_buffer):
+        self._unsupported("set_inputs / step (the resident-input graph step)")
+
+    def step(self):
+        self._unsupported("set_inputs / step (the resident-input graph step)")
+
+    def get_rollouts(self, state, num_rollouts=1):
+        self._unsupported("get_rollouts")
+
+    def _begin(self, state, action_buffer):
+        self._unsupported("the sharded control step")
+
+    def _finish(self):
+        self._unsupported("the sharded control step")
+
+    def overlap_status(self):
+        return False, 0
+
+    def exchange_status(self):
+        return False, 0
+
+    shard_triple = property(lambda self: self._unsupported("the sharded control step"))
+    all_triples = property(lambda self: self._unsupported("the sharded control step"))
