@@ -441,6 +441,12 @@ int nlc_batch_planner_command(nlc_batch_planner_t p, const float* state_dev, con
  * state_dev [I][nx] and action_buffer_dev [I][B][nu] are updated in place.                          */
 int nlc_env_step(const nlc_rollout_opts* o, float* state_dev, float* action_buffer_dev, const float* action_dev,
                  int I, int B, int nu, float* reward_dev, void* stream);
+/* nlc_env_step in fp64, for the closed loop around the fp64 planner: the same buffer roll and delayed action, the Euler step
+ * and reward in fp64 with the reference's evaluation order (the fp64 planner's analytic dynamics and running cost, default
+ * cost options).  dt is a double: the float nlc_rollout_opts.dt cannot hold 0.05 exactly.  env is an nlc_env, delay in
+ * [0, B), B in [1, 8], nu that of env; reward_dev [I] may be NULL.  The argument checks run before any CUDA call.       */
+int nlc_env_step_f64(int env, int delay, double dt, double* state_dev, double* action_buffer_dev, const double* action_dev,
+                     int I, int B, int nu, double* reward_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Generic Fourier-series inverse Laplace transform (torchlaplace's Fourier ILT as called from

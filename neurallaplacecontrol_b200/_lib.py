@@ -134,6 +134,7 @@ SIGNATURES = {
     "nlc_batch_planner_buffer": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),
     "nlc_batch_planner_command": (C.c_int, [C.c_void_p, _fp, _fp, _fp, _fp, C.c_void_p]),
     "nlc_env_step": (C.c_int, [C.POINTER(RolloutOpts), _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_void_p]),
+    "nlc_env_step_f64": (C.c_int, [C.c_int, C.c_int, C.c_double, _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_void_p]),
     "nlc_ilt_fourier": (C.c_int, [_fp, _fp, C.c_int, C.c_int64, C.c_int, C.c_int, _fp, C.c_void_p]),
     "nlc_selftest_umma_gemm_ts": (C.c_int, [_fp, _fp, C.c_int, C.c_int, C.c_int, C.c_int, _fp, C.c_void_p]),
     "nlc_selftest_umma_gemm": (C.c_int, [_fp, _fp, C.c_int, C.c_int, C.c_int, C.c_int, _fp, C.c_void_p]),

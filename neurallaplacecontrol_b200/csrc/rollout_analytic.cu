@@ -67,6 +67,27 @@ __global__ void env_step_kernel(nlc_rollout_opts o, float* __restrict__ state, f
   if (reward) reward[i] = -env_running_cost(o, s, at, nu);
 }
 
+// env_step_kernel in fp64 (the closed loop around the fp64 planner): the same buffer roll and delayed action, the fp64 Euler
+// step and running cost of env_cost.cuh that the fp64 planner's analytic rollout uses, dt in fp64.
+template <int NX>
+__global__ void env_step_f64_kernel(int env, int delay, double dt, double* __restrict__ state, double* __restrict__ abuf,
+                                    const double* __restrict__ action, int I, int B, int nu, double* __restrict__ reward) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= I) return;
+  double* b = abuf + (size_t)i * B * nu;
+  for (int j = 0; j + 1 < B; ++j)
+    for (int u = 0; u < nu; ++u) b[j * nu + u] = b[(j + 1) * nu + u];
+  for (int u = 0; u < nu; ++u) b[(B - 1) * nu + u] = action[(size_t)i * nu + u];
+  const double* at = b + (size_t)(B - 1 - delay) * nu;
+  double s[NX];
+#pragma unroll
+  for (int c = 0; c < NX; ++c) s[c] = state[(size_t)i * NX + c];
+  env_analytic_step(env, dt, s, at);
+#pragma unroll
+  for (int c = 0; c < NX; ++c) state[(size_t)i * NX + c] = s[c];
+  if (reward) reward[i] = -env_running_cost(env, 0, 0.0, s, at, nu);
+}
+
 }  // namespace nlc
 
 extern "C" int nlc_env_step(const nlc_rollout_opts* o, float* state_dev, float* action_buffer_dev, const float* action_dev,
@@ -88,5 +109,27 @@ extern "C" int nlc_env_step(const nlc_rollout_opts* o, float* state_dev, float* 
   else if (o->env == NLC_ENV_CARTPOLE) env_step_kernel<5><<<grid, 128, 0, s>>>(*o, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
   else env_step_kernel<6><<<grid, 128, 0, s>>>(*o, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
   NLC_LAUNCH_OK("env_step_kernel");
+  return NLC_OK;
+}
+
+extern "C" int nlc_env_step_f64(int env, int delay, double dt, double* state_dev, double* action_buffer_dev, const double* action_dev,
+                                int I, int B, int nu, double* reward_dev, void* stream) {
+  using namespace nlc;
+  NLC_REQUIRE(state_dev && action_buffer_dev && action_dev, NLC_ERR_ARG, "nlc_env_step_f64: null pointer");
+  NLC_REQUIRE(I >= 1 && B >= 1 && B <= 8, NLC_ERR_ARG, "nlc_env_step_f64: I >= 1 and 1 <= B <= 8 required");
+  NLC_REQUIRE(env >= NLC_ENV_PENDULUM && env <= NLC_ENV_ACROBOT, NLC_ERR_ARG, "unknown env id %d", env);
+  NLC_REQUIRE(delay >= 0 && delay < B, NLC_ERR_ARG, "nlc_env_step_f64: delay %d outside the %d-entry action buffer", delay, B);
+  const int env_nu[3] = {1, 1, 2};
+  NLC_REQUIRE(nu == env_nu[env], NLC_ERR_SHAPE, "env %d takes nu=%d actions, got %d", env, env_nu[env], nu);
+  int dev = 0;
+  NLC_CUDA_OK(cudaGetDevice(&dev));
+  int rc = check_device_arch(dev);
+  if (rc != NLC_OK) return rc;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int grid = (I + 127) / 128;
+  if (env == NLC_ENV_PENDULUM) env_step_f64_kernel<3><<<grid, 128, 0, s>>>(env, delay, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
+  else if (env == NLC_ENV_CARTPOLE) env_step_f64_kernel<5><<<grid, 128, 0, s>>>(env, delay, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
+  else env_step_f64_kernel<6><<<grid, 128, 0, s>>>(env, delay, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
+  NLC_LAUNCH_OK("env_step_f64_kernel");
   return NLC_OK;
 }

@@ -8,9 +8,10 @@ of one environment share every kernel launch and nothing leaves the device insid
 * :class:`BatchedMPPIDelay` - ``I`` independent ``MPPIDelay`` objects (own control sequence, action buffer, sampler seed):
   stage 1 and stage 4 per instance, ONE encoder launch and ONE rollout launch over all ``I*K`` samples
   (``nlc_batch_planner_*``).  Instance ``i`` reproduces a stand-alone ``MPPIDelay(..., seed=seeds[i])``.
-* :func:`env_step` - ``step_env`` for ``I`` instances on the device (``nlc_env_step``; dynamics as stated by the
-  reference's ``oracle.py:11-224``, golden-pinned in ``tests/golden/env_step_*.npz``).
-* :func:`run_closed_loop` - ``loop()`` for ``I`` instances; returns the reference's result keys per instance.
+* :func:`env_step` - ``step_env`` for ``I`` instances on the device (``nlc_env_step``, or ``nlc_env_step_f64`` on fp64
+  tensors; dynamics as stated by the reference's ``oracle.py:11-224``, golden-pinned in ``tests/golden/env_step_*.npz``).
+* :func:`run_closed_loop` - ``loop()`` for ``I`` instances of a ``BatchedMPPIDelay``, or in fp64 over one
+  ``MPPIDelay(math_mode="fp64")`` per instance; returns the reference's result keys per instance.
 
 Everything computes in ``libnlc_b200.so``; there is no CPU fallback.
 """
@@ -24,7 +25,7 @@ import torch
 
 from . import _lib
 from .closures import NLDynamics
-from .planners.mppi_delay import MPPIDelay, _DevView
+from .planners.mppi_delay import MPPIDelay, _DevView, _MPPIDelayF64
 
 
 class BatchedMPPIDelay:
@@ -38,7 +39,8 @@ class BatchedMPPIDelay:
         if "process_group" in kw and kw["process_group"] is not None:
             raise NotImplementedError("BatchedMPPIDelay shards by instance: give each rank its own instances")
         if kw.get("math_mode") == "fp64":
-            raise NotImplementedError("BatchedMPPIDelay has no fp64 mode: plan each instance with MPPIDelay(math_mode='fp64')")
+            raise NotImplementedError("BatchedMPPIDelay has no fp64 mode: plan each instance with MPPIDelay(math_mode='fp64') "
+                                      "and drive them with run_closed_loop([planner_0, planner_1, ...], ...)")
         self.I = int(n_instances)
         self.seeds = list(range(self.I)) if seeds is None else [int(s) for s in seeds]
         if len(self.seeds) != self.I:
@@ -157,41 +159,102 @@ class BatchedMPPIDelay:
 
 
 def env_step(env_name, states, action_buffers, actions, action_delay, dt=0.05, rewards=None):
-    """``step_env`` (``mppi_with_model.py:193-216``) for I instances, in place on fp32 CUDA tensors: ``action_buffers``
+    """``step_env`` (``mppi_with_model.py:193-216``) for I instances, in place on CUDA tensors: ``action_buffers``
     (I, B, nu) is rolled and receives ``actions`` (I, nu) (``get_action``, ``:25-28``), ``states`` (I, nx) advances by
-    one Euler step of the true dynamics driven by the delayed action, ``rewards`` (I) receives the step reward."""
-    for t in (states, action_buffers, actions):
-        if not (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous()):
-            raise TypeError("env_step works in place on contiguous fp32 CUDA tensors (no CPU fallback)")
+    one Euler step of the true dynamics driven by the delayed action, ``rewards`` (I) receives the step reward.
+
+    All tensors (``rewards`` if given) are contiguous and either all fp32 (``nlc_env_step``) or all fp64
+    (``nlc_env_step_f64``: the reference's own precision and evaluation order, ``dt`` kept in fp64); anything else raises
+    ``TypeError``.  In both precisions this is the Euler step of the reference's ``oracle.py``, NOT the reference
+    environment's integrator (see :func:`run_closed_loop`)."""
+    tensors = [t for t in (states, action_buffers, actions, rewards) if t is not None]
+    dtype = states.dtype
+    if dtype not in (torch.float32, torch.float64) or not all(t.is_cuda and t.dtype == dtype and t.is_contiguous() for t in tensors):
+        raise TypeError("env_step works in place on contiguous CUDA tensors, all fp32 or all fp64 (no CPU fallback)")
     I, B, nu = action_buffers.shape
-    ro = _lib.RolloutOpts()
-    ro.env, ro.state_constraint, ro.goal_x, ro.dynamics, ro.delay, ro.dt = _lib.ENV_IDS[env_name], 0, 0.0, _lib.DYN_ANALYTIC_DELAY, int(action_delay), float(dt)
     with torch.cuda.device(states.device):
+        if dtype == torch.float64:
+            _lib.check(_lib.load().nlc_env_step_f64(_lib.ENV_IDS[env_name], int(action_delay), float(dt), states.data_ptr(),
+                                                    action_buffers.data_ptr(), actions.data_ptr(), I, B, nu, _lib.ptr(rewards),
+                                                    _lib.current_stream_ptr()), "nlc_env_step_f64")
+            return
+        ro = _lib.RolloutOpts()
+        ro.env, ro.state_constraint, ro.goal_x, ro.dynamics, ro.delay, ro.dt = _lib.ENV_IDS[env_name], 0, 0.0, _lib.DYN_ANALYTIC_DELAY, int(action_delay), float(dt)
         _lib.check(_lib.load().nlc_env_step(C.byref(ro), states.data_ptr(), action_buffers.data_ptr(), actions.data_ptr(), I, B, nu,
                                             _lib.ptr(rewards), _lib.current_stream_ptr()), "nlc_env_step")
 
 
-def run_closed_loop(planner: BatchedMPPIDelay, env_name, states0, action_delay, n_steps, dt=0.05, noise_fn=None):
-    """``loop()`` of ``mppi_with_model.py:244-317`` for ``planner.I`` instances: zero action buffers (``:245``), then
+class _F64Instances:
+    """One ``MPPIDelay(math_mode="fp64")`` per instance behind the ``command`` of :class:`BatchedMPPIDelay`: a control step
+    plans every instance in turn on the device (``nlc_planner_f64_command``) and stacks the actions."""
+
+    def __init__(self, planners):
+        self.planners = list(planners)
+        if not self.planners:
+            raise ValueError("run_closed_loop needs at least one planner")
+        for p in self.planners:
+            if not isinstance(p, _MPPIDelayF64):
+                raise TypeError("a list of planners must hold MPPIDelay(math_mode='fp64') objects, one per instance "
+                                "(fp32 instances are batched by BatchedMPPIDelay)")
+        p0 = self.planners[0]
+        for p in self.planners:
+            if (p.nx, p.nu, p.B, p.d) != (p0.nx, p0.nu, p0.B, p0.d):
+                raise ValueError("the planners of one closed loop must share nx, nu, the action buffer size and the device")
+            if p.u_per_command != 1:
+                raise ValueError("the closed loop applies one action per command: u_per_command must be 1")
+        self.I, self.nx, self.nu, self.B, self.d, self.K, self.T = len(self.planners), p0.nx, p0.nu, p0.B, p0.d, p0.K, p0.T
+
+    def command(self, states, action_buffers, noise=None):
+        """``states`` (I, nx), ``action_buffers`` (I, B, nu) fp64 on the device; ``noise`` optional (I, K, T, nu): instance
+        i's slice goes in through its planner's ``noise_dist.sample`` for this call only.  Returns the actions (I, nu)."""
+        actions = []
+        for i, p in enumerate(self.planners):
+            if noise is None:
+                actions.append(p.command(states[i], action_buffers[i]))
+                continue
+            saved = p.noise_dist.__dict__.get("sample")
+            p.noise_dist.sample = lambda shape, nz=noise[i]: nz
+            try:
+                actions.append(p.command(states[i], action_buffers[i]))
+            finally:
+                if saved is None:
+                    del p.noise_dist.sample
+                else:
+                    p.noise_dist.sample = saved
+        return torch.stack(actions)
+
+
+def run_closed_loop(planner, env_name, states0, action_delay, n_steps, dt=0.05, noise_fn=None):
+    """``loop()`` of ``mppi_with_model.py:244-317`` for I instances: zero action buffers (``:245``), then
     ``n_steps`` x (command, step_env); rewards accumulate on the device.
+
+    ``planner`` is a :class:`BatchedMPPIDelay` (``I = planner.I``; fp32 state, buffers and rewards), or a list / tuple of
+    ``MPPIDelay(math_mode="fp64")`` objects, one per instance (``I = len(planner)``; they share ``nx``, ``nu``, the action
+    buffer size and the device, and take ``u_per_command == 1``): then the state, the buffers and the rewards are fp64 like
+    the reference's loop, each instance plans on its own planner and one fp64 ``env_step`` advances them all.
+    ``roll_outs`` / ``time_steps`` of the result are those of the first planner.
 
     NOT the reference environment's integrator: ``env_step`` takes ONE EXPLICIT EULER step of the dynamics as the
     reference's ``oracle.py`` states them (what its "oracle" planner model uses), whereas the reference's gym envs
     integrate the same right-hand side with ``torchdiffeq.odeint`` (``base_env.py:136-173``, dopri5 by default).
-    Closed-loop rewards are therefore those of the Euler-discretised plant, not the reference environment's.  ``noise_fn(it)`` may return injected noise for
-    step ``it`` (parity tests).  Returns the reference's result keys (``:289-302``) with per-instance arrays."""
+    Closed-loop rewards are therefore those of the Euler-discretised plant, not the reference environment's.  ``noise_fn(it)`` may return injected noise
+    (I, K, T, nu) for step ``it`` (parity tests).  Returns the reference's result keys (``:289-302``) with per-instance arrays."""
+    if isinstance(planner, (list, tuple)):
+        planner, dtype = _F64Instances(planner), torch.float64
+    else:
+        dtype = torch.float32
     I, B, nu, dev = planner.I, planner.B, planner.nu, planner.d
-    states = torch.as_tensor(states0).to(device=dev, dtype=torch.float32).reshape(I, planner.nx).clone()
-    bufs = torch.zeros(I, B, nu, dtype=torch.float32, device=dev)
-    total = torch.zeros(I, dtype=torch.float32, device=dev)
-    reward = torch.zeros(I, dtype=torch.float32, device=dev)
+    states = torch.as_tensor(states0).to(device=dev, dtype=dtype).reshape(I, planner.nx).clone()
+    bufs = torch.zeros(I, B, nu, dtype=dtype, device=dev)
+    total = torch.zeros(I, dtype=dtype, device=dev)
+    reward = torch.zeros(I, dtype=dtype, device=dev)
     elapsed = 0.0
     for it in range(int(n_steps)):
         t0 = time.perf_counter()
         actions = planner.command(states, bufs, None if noise_fn is None else noise_fn(it))
         torch.cuda.synchronize(dev)
         elapsed += time.perf_counter() - t0  # the reference's bracket (:255-264) around command()
-        env_step(env_name, states, bufs, actions.to(torch.float32).contiguous(), action_delay, dt, reward)
+        env_step(env_name, states, bufs, actions.to(dtype).contiguous(), action_delay, dt, reward)
         total += reward
     torch.cuda.synchronize(dev)
     tot = total.double().cpu().numpy()
