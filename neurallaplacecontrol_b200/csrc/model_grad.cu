@@ -35,7 +35,8 @@
 // The fp64 forward is the recompute half of the tile steps (encoder, linear_out, MLP) followed by the ILT sum; the fp64
 // backward runs the two-stage form of nlc_model_backward_multi for every n_t (n_t = 1 included).
 //
-// The fp64 planner (planner_f64.cu) runs its history encoder and rollout on the same tile steps: plan_f64_* at the end.
+// The fp64 planner (planner_f64.cu) runs its history encoder and rollout on the same tile steps (at the end); that encoder
+// also encodes the fp64 model's windows.
 #include <stddef.h>
 
 #include "common.cuh"
@@ -43,9 +44,10 @@
 
 namespace nlc {
 
-int launch_forward_ts_prep(nlc_model_s* m, const float* ts, int K, float* row_b1, float* row_tn, float* row_sph, cudaStream_t s);
-int launch_forward_ts_prep_f64(nlc_model_s* m, const double* b1_raw, const double* w1_full_t, const double* ts, int K, double* row_b1,
-                               double* row_tn, double* row_sph, cudaStream_t s);
+template <typename T>
+int launch_forward_ts_prep(nlc_model_s* m, const T* b1_raw, const T* w1_full_t, const T* ts, int K, T* row_b1, T* row_tn, T* row_sph,
+                           cudaStream_t s, const T* obs = nullptr, const T* p = nullptr, long long r0 = 0, int n_t = 1,
+                           T* row_obs = nullptr, T* row_p = nullptr);
 int encode_history_impl(nlc_model_t m, const float* hist_dev, int hist_ch, int K, int T, int B, float* p_dev, int math_mode,
                         cudaStream_t s);
 
@@ -740,30 +742,9 @@ __global__ void __launch_bounds__(kGradThreads, 1) model_grad_multi_enc_kernel(G
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// fp64 forward: the recompute half of the tile steps.  model_f64_encode_kernel encodes tiles of kGradRows windows and
-// writes linear_out's p [K][2]; model_f64_rows_kernel runs the MLP and the ILT sum over a chunk's rows.
+// fp64 forward: the recompute half of the tile steps.  f64_encode_kernel (below, shared with the fp64 planner) encodes the
+// K windows into linear_out's p [K][2]; model_f64_rows_kernel runs the MLP and the ILT sum over a chunk's rows.
 // ------------------------------------------------------------------------------------------------------------------
-template <int H>
-__global__ void __launch_bounds__(kGradThreads, 1) model_f64_encode_kernel(GradArgs<double> a, double* __restrict__ p) {
-  const GradShape& g = a.g;
-  const TileW<double>& md = a.m;
-  constexpr int R = kGradRows;
-  const TileBufs<double> t = tile_bufs(g, a.scratch + (size_t)blockIdx.x * g.s_total);
-  for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
-    const int k0 = tile * R;
-    __syncthreads();  // the previous tile's last reads of the scratch are done
-    tile_load_window(g, md, a.act, k0, a.K, t.xs);
-    __syncthreads();
-    tile_encoder_fwd<H>(g, md, t);
-    tile_linear_out(g, md, t);
-    __syncthreads();
-    for (int i = threadIdx.x; i < R * 2; i += kGradThreads) {
-      const int m = i >> 1, o = i & 1;
-      if (k0 + m < a.K) p[(size_t)(k0 + m) * 2 + o] = t.x1[m * g.in0p + 2 * g.S + g.nx + o];
-    }
-  }
-}
-
 // a.gout is unused; out: this chunk's rows [rows][nx]
 template <int H>
 __global__ void __launch_bounds__(kGradThreads, 1) model_f64_rows_kernel(MultiArgs<double> a, double* __restrict__ out) {
@@ -931,6 +912,68 @@ static MultiWs multi_ws_layout(const GradShape& g, int K, int n_t, bool f64 = fa
   return w;
 }
 
+// The argument checks of the (K, n_t) entry points, fn naming the entry point in the messages.
+static int multi_check(const char* fn, nlc_model_t m, int K, int n_t, int B, const void* workspace_dev) {
+  NLC_REQUIRE(K >= 1 && n_t >= 1, NLC_ERR_ARG, "%s: K and n_t must be positive", fn);
+  NLC_REQUIRE((long long)K * n_t < (1LL << 31), NLC_ERR_SHAPE, "%s: K n_t = %lld rows, 2^31 or more", fn, (long long)K * n_t);
+  NLC_REQUIRE(B >= 1 && B <= 8, NLC_ERR_SHAPE, "%s: window length %d outside [1,8]", fn, B);
+  NLC_REQUIRE(((uintptr_t)workspace_dev & 15) == 0, NLC_ERR_ARG, "%s: workspace must be 16-byte aligned", fn);
+  return check_device_arch(m->device);
+}
+
+// Bytes of multi_ws_layout, or the error code of arguments the entry point would reject.
+static int64_t multi_ws_bytes(nlc_model_t m, int K, int n_t, int B, bool f64, bool bwd) {
+  if (!m || K < 1 || n_t < 1 || B < 1 || B > 8) return NLC_ERR_ARG;
+  if ((long long)K * n_t >= (1LL << 31)) return NLC_ERR_SHAPE;
+  return (int64_t)(multi_ws_layout(shape_of(m, B), K, n_t, f64, bwd).total * (f64 ? sizeof(double) : sizeof(float)));
+}
+
+// fp64: the weight image img (GradShape w_* and f_* offsets) of the caller's parameters params_dev.
+static int f64_weight_image(const GradShape& g, const double* params_dev, double* img, cudaStream_t s) {
+  const int n_img = g.N3p * g.H > g.in0 * g.H ? g.N3p * g.H : g.in0 * g.H;
+  model_f64_weights_kernel<<<(n_img + 255) / 256, 256, 0, s>>>(g, params_dev, img);
+  NLC_LAUNCH_OK("model_f64_weights_kernel");
+  return NLC_OK;
+}
+
+// with the fp64 planner's stages at the end of this file
+int encode_windows_f64(nlc_model_t m, int B, const double* img, const double* hist, int hist_ch, int K, int T, double* p_out,
+                       double* scratch, cudaStream_t s);
+
+// The two stages of the backward and the reduction, once the workspace holds p [K][2] at w.p and the weight copies at w.wt
+// (tw: the weights the tile steps read).
+template <typename T>
+static int backward_two_stage(nlc_model_t m, const GradShape& g, const MultiWs& w, const TileW<T>& tw, T* ws, const T* obs_dev,
+                              const T* act_dev, const T* ts_dev, int K, int n_t, const T* grad_out_dev, T* grad_params_dev,
+                              T* grad_obs_dev, T* grad_act_dev, cudaStream_t s) {
+  NLC_CUDA_OK(cudaMemsetAsync(ws + w.part, 0, (size_t)w.G * g.p_total * sizeof(T), s));
+  MultiArgs<T> ma = {};
+  ma.m = tw; ma.g = g; ma.obs = obs_dev; ma.p = ws + w.p; ma.row_b1 = ws + w.b1; ma.row_tn = ws + w.tn; ma.row_sph = ws + w.sph;
+  ma.wt = ws + w.wt; ma.part = ws + w.part; ma.scratch = ws + w.scr; ma.drow = ws + w.drow; ma.n_t = n_t;
+  const long long n_rows = (long long)K * n_t;
+  for (long long r0 = 0; r0 < n_rows; r0 += w.C) {
+    const int rows = (int)(n_rows - r0 < w.C ? n_rows - r0 : w.C);
+    const int rc = launch_forward_ts_prep(m, tw.b1_raw, tw.w1_full_t, ts_dev + r0, rows, ws + w.b1, ws + w.tn, ws + w.sph, s);
+    if (rc != NLC_OK) return rc;
+    ma.gout = grad_out_dev + r0 * g.nx; ma.r0 = r0; ma.rows = rows;
+    if (m->Hm == 128) model_grad_multi_mlp_kernel<128, T><<<w.Gm, kGradThreads, 0, s>>>(ma);
+    else model_grad_multi_mlp_kernel<64, T><<<w.Gm, kGradThreads, 0, s>>>(ma);
+    NLC_LAUNCH_OK("model_grad_multi_mlp_kernel");
+    const long long n_sum = ((r0 + rows - 1) / n_t - r0 / n_t + 1) * g.Lp;
+    model_grad_multi_rowsum_kernel<T><<<(unsigned)((n_sum + 255) / 256), 256, 0, s>>>(ws + w.drow, r0, rows, n_t, g.Lp, ws + w.dsum);
+    NLC_LAUNCH_OK("model_grad_multi_rowsum_kernel");
+  }
+  GradArgs<T> a = {};
+  a.m = tw; a.g = g; a.obs = obs_dev; a.act = act_dev; a.wt = ws + w.wt; a.part = ws + w.part; a.scratch = ws + w.scr;
+  a.grad_obs = grad_obs_dev; a.grad_act = grad_act_dev; a.K = K; a.n_tiles = (K + kGradRows - 1) / kGradRows;
+  if (m->Hm == 128) model_grad_multi_enc_kernel<128, T><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
+  else model_grad_multi_enc_kernel<64, T><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
+  NLC_LAUNCH_OK("model_grad_multi_enc_kernel");
+  model_grad_reduce_kernel<T><<<(g.o_total + 255) / 256, 256, 0, s>>>(g, ws + w.part, w.G, grad_params_dev);
+  NLC_LAUNCH_OK("model_grad_reduce_kernel");
+  return NLC_OK;
+}
+
 }  // namespace nlc
 
 using namespace nlc;
@@ -961,7 +1004,7 @@ extern "C" int nlc_model_backward_ts(nlc_model_t m, const float* obs_dev, const 
   const GradShape g = shape_of(m, B);
   const GradWs w = ws_layout(g, K);
   float* ws = static_cast<float*>(workspace_dev);
-  rc = launch_forward_ts_prep(m, ts_dev, K, ws + w.b1, ws + w.tn, ws + w.sph, s);
+  rc = launch_forward_ts_prep(m, m->d.b1_raw, m->d.w1_full_t, ts_dev, K, ws + w.b1, ws + w.tn, ws + w.sph, s);
   if (rc != NLC_OK) return rc;
   const int n_wt = 3 * g.G3 * g.Hg + g.H * g.H + g.N3p * g.H;
   model_grad_wt_kernel<<<(n_wt + 255) / 256, 256, 0, s>>>(m->d, g, ws + w.wt);
@@ -981,9 +1024,7 @@ extern "C" int nlc_model_backward_ts(nlc_model_t m, const float* obs_dev, const 
 }
 
 extern "C" int64_t nlc_model_backward_multi_workspace_bytes(nlc_model_t m, int K, int n_t, int B) {
-  if (!m || K < 1 || n_t < 1 || B < 1 || B > 8) return NLC_ERR_ARG;
-  if ((long long)K * n_t >= (1LL << 31)) return NLC_ERR_SHAPE;
-  return (int64_t)(multi_ws_layout(shape_of(m, B), K, n_t).total * sizeof(float));
+  return multi_ws_bytes(m, K, n_t, B, false, true);
 }
 
 extern "C" int nlc_model_backward_multi(nlc_model_t m, const float* obs_dev, const float* act_dev, const float* ts_dev, int K, int n_t,
@@ -991,12 +1032,7 @@ extern "C" int nlc_model_backward_multi(nlc_model_t m, const float* obs_dev, con
                                         float* grad_act_dev, void* workspace_dev, void* stream) {
   NLC_REQUIRE(m && obs_dev && act_dev && ts_dev && grad_out_dev && grad_params_dev && workspace_dev, NLC_ERR_ARG,
               "nlc_model_backward_multi: null pointer");
-  NLC_REQUIRE(K >= 1 && n_t >= 1, NLC_ERR_ARG, "nlc_model_backward_multi: K and n_t must be positive");
-  NLC_REQUIRE((long long)K * n_t < (1LL << 31), NLC_ERR_SHAPE, "nlc_model_backward_multi: K n_t = %lld rows, 2^31 or more",
-              (long long)K * n_t);
-  NLC_REQUIRE(B >= 1 && B <= 8, NLC_ERR_SHAPE, "nlc_model_backward_multi: window length %d outside [1,8]", B);
-  NLC_REQUIRE(((uintptr_t)workspace_dev & 15) == 0, NLC_ERR_ARG, "nlc_model_backward_multi: workspace must be 16-byte aligned");
-  int rc = check_device_arch(m->device);
+  int rc = multi_check("nlc_model_backward_multi", m, K, n_t, B, workspace_dev);
   if (rc != NLC_OK) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const GradShape g = shape_of(m, B);
@@ -1008,71 +1044,17 @@ extern "C" int nlc_model_backward_multi(nlc_model_t m, const float* obs_dev, con
   const int n_wt = 3 * g.G3 * g.Hg + g.H * g.H + g.N3p * g.H;
   model_grad_wt_kernel<<<(n_wt + 255) / 256, 256, 0, s>>>(m->d, g, ws + w.wt);
   NLC_LAUNCH_OK("model_grad_wt_kernel");
-  NLC_CUDA_OK(cudaMemsetAsync(ws + w.part, 0, (size_t)w.G * g.p_total * sizeof(float), s));
-  MultiArgs<float> ma;
-  ma.m = tile_w(m->d); ma.g = g; ma.obs = obs_dev; ma.p = ws + w.p; ma.row_b1 = ws + w.b1; ma.row_tn = ws + w.tn; ma.row_sph = ws + w.sph;
-  ma.wt = ws + w.wt; ma.part = ws + w.part; ma.scratch = ws + w.scr; ma.drow = ws + w.drow; ma.n_t = n_t;
-  const long long n_rows = (long long)K * n_t;
-  for (long long r0 = 0; r0 < n_rows; r0 += w.C) {
-    const int rows = (int)(n_rows - r0 < w.C ? n_rows - r0 : w.C);
-    rc = launch_forward_ts_prep(m, ts_dev + r0, rows, ws + w.b1, ws + w.tn, ws + w.sph, s);
-    if (rc != NLC_OK) return rc;
-    ma.gout = grad_out_dev + r0 * g.nx; ma.r0 = r0; ma.rows = rows;
-    if (m->Hm == 128) model_grad_multi_mlp_kernel<128, float><<<w.Gm, kGradThreads, 0, s>>>(ma);
-    else model_grad_multi_mlp_kernel<64, float><<<w.Gm, kGradThreads, 0, s>>>(ma);
-    NLC_LAUNCH_OK("model_grad_multi_mlp_kernel");
-    const long long n_sum = ((r0 + rows - 1) / n_t - r0 / n_t + 1) * g.Lp;
-    model_grad_multi_rowsum_kernel<float><<<(unsigned)((n_sum + 255) / 256), 256, 0, s>>>(ws + w.drow, r0, rows, n_t, g.Lp, ws + w.dsum);
-    NLC_LAUNCH_OK("model_grad_multi_rowsum_kernel");
-  }
-  GradArgs<float> a;
-  a.m = tile_w(m->d); a.g = g; a.obs = obs_dev; a.act = act_dev; a.gout = nullptr;
-  a.row_b1 = nullptr; a.row_tn = nullptr; a.row_sph = nullptr; a.wt = ws + w.wt;
-  a.part = ws + w.part; a.scratch = ws + w.scr; a.grad_obs = grad_obs_dev; a.grad_act = grad_act_dev;
-  a.K = K; a.n_tiles = (K + kGradRows - 1) / kGradRows;
-  if (m->Hm == 128) model_grad_multi_enc_kernel<128, float><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
-  else model_grad_multi_enc_kernel<64, float><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
-  NLC_LAUNCH_OK("model_grad_multi_enc_kernel");
-  model_grad_reduce_kernel<float><<<(g.o_total + 255) / 256, 256, 0, s>>>(g, ws + w.part, w.G, grad_params_dev);
-  NLC_LAUNCH_OK("model_grad_reduce_kernel");
-  return NLC_OK;
+  return backward_two_stage(m, g, w, tile_w(m->d), ws, obs_dev, act_dev, ts_dev, K, n_t, grad_out_dev, grad_params_dev, grad_obs_dev,
+                            grad_act_dev, s);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
 // fp64 forward and backward (NeuralLaplaceModel math_mode="fp64"): the weights are the caller's fp64 parameters params_dev
-// (nlc_model_grad_floats entries, the layout of grad_params_dev), rearranged per call into the workspace.
+// (nlc_model_grad_floats entries, the layout of grad_params_dev), rearranged per call into the workspace.  The K windows
+// are encoded by the fp64 planner's encoder at T = 1 (a window per sample, hist = act).
 // ---------------------------------------------------------------------------------------------------------------------
-namespace nlc {
-
-static int f64_check(const char* fn, nlc_model_t m, int K, int n_t, int B, const void* workspace_dev) {
-  NLC_REQUIRE(K >= 1 && n_t >= 1, NLC_ERR_ARG, "%s: K and n_t must be positive", fn);
-  NLC_REQUIRE((long long)K * n_t < (1LL << 31), NLC_ERR_SHAPE, "%s: K n_t = %lld rows, 2^31 or more", fn, (long long)K * n_t);
-  NLC_REQUIRE(B >= 1 && B <= 8, NLC_ERR_SHAPE, "%s: window length %d outside [1,8]", fn, B);
-  NLC_REQUIRE(((uintptr_t)workspace_dev & 15) == 0, NLC_ERR_ARG, "%s: workspace must be 16-byte aligned", fn);
-  return check_device_arch(m->device);
-}
-
-// The weight image, p [K][2] of the K windows (p_out when given, else the workspace's), and the launches of one chunk's prep.
-static int f64_encode(nlc_model_t m, const GradShape& g, const MultiWs& w, const double* params_dev, const double* act_dev, int K,
-                      double* ws, double* p, cudaStream_t s) {
-  const int n_img = g.N3p * g.H > g.in0 * g.H ? g.N3p * g.H : g.in0 * g.H;
-  model_f64_weights_kernel<<<(n_img + 255) / 256, 256, 0, s>>>(g, params_dev, ws + w.wt);
-  NLC_LAUNCH_OK("model_f64_weights_kernel");
-  GradArgs<double> a = {};
-  a.m = tile_w_f64(m->d, g, ws + w.wt); a.g = g; a.act = act_dev; a.wt = ws + w.wt; a.scratch = ws + w.scr;
-  a.K = K; a.n_tiles = (K + kGradRows - 1) / kGradRows;
-  if (m->Hm == 128) model_f64_encode_kernel<128><<<w.Ge, kGradThreads, 0, s>>>(a, p);
-  else model_f64_encode_kernel<64><<<w.Ge, kGradThreads, 0, s>>>(a, p);
-  NLC_LAUNCH_OK("model_f64_encode_kernel");
-  return NLC_OK;
-}
-
-}  // namespace nlc
-
 extern "C" int64_t nlc_model_forward_f64_workspace_bytes(nlc_model_t m, int K, int n_t, int B) {
-  if (!m || K < 1 || n_t < 1 || B < 1 || B > 8) return NLC_ERR_ARG;
-  if ((long long)K * n_t >= (1LL << 31)) return NLC_ERR_SHAPE;
-  return (int64_t)(multi_ws_layout(shape_of(m, B), K, n_t, true, false).total * sizeof(double));
+  return multi_ws_bytes(m, K, n_t, B, true, false);
 }
 
 extern "C" int nlc_model_forward_f64(nlc_model_t m, const double* params_dev, const double* obs_dev, const double* act_dev,
@@ -1080,14 +1062,16 @@ extern "C" int nlc_model_forward_f64(nlc_model_t m, const double* params_dev, co
                                      void* workspace_dev, void* stream) {
   NLC_REQUIRE(m && params_dev && obs_dev && act_dev && ts_dev && out_dev && workspace_dev, NLC_ERR_ARG,
               "nlc_model_forward_f64: null pointer");
-  int rc = f64_check("nlc_model_forward_f64", m, K, n_t, B, workspace_dev);
+  int rc = multi_check("nlc_model_forward_f64", m, K, n_t, B, workspace_dev);
   if (rc != NLC_OK) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const GradShape g = shape_of(m, B);
   const MultiWs w = multi_ws_layout(g, K, n_t, true, false);
   double* ws = static_cast<double*>(workspace_dev);
   double* p = p_action_dev ? p_action_dev : ws + w.p;
-  rc = f64_encode(m, g, w, params_dev, act_dev, K, ws, p, s);
+  rc = f64_weight_image(g, params_dev, ws + w.wt, s);
+  if (rc != NLC_OK) return rc;
+  rc = encode_windows_f64(m, B, ws + w.wt, act_dev, g.gin, K, 1, p, ws + w.scr, s);
   if (rc != NLC_OK) return rc;
   MultiArgs<double> ma = {};
   ma.m = tile_w_f64(m->d, g, ws + w.wt); ma.g = g; ma.obs = obs_dev; ma.p = p; ma.row_b1 = ws + w.b1; ma.row_tn = ws + w.tn;
@@ -1095,7 +1079,7 @@ extern "C" int nlc_model_forward_f64(nlc_model_t m, const double* params_dev, co
   const long long n_rows = (long long)K * n_t;
   for (long long r0 = 0; r0 < n_rows; r0 += w.C) {
     const int rows = (int)(n_rows - r0 < w.C ? n_rows - r0 : w.C);
-    rc = launch_forward_ts_prep_f64(m, ma.m.b1_raw, ma.m.w1_full_t, ts_dev + r0, rows, ws + w.b1, ws + w.tn, ws + w.sph, s);
+    rc = launch_forward_ts_prep(m, ma.m.b1_raw, ma.m.w1_full_t, ts_dev + r0, rows, ws + w.b1, ws + w.tn, ws + w.sph, s);
     if (rc != NLC_OK) return rc;
     ma.r0 = r0; ma.rows = rows;
     const int G = grad_grid(rows);
@@ -1107,9 +1091,7 @@ extern "C" int nlc_model_forward_f64(nlc_model_t m, const double* params_dev, co
 }
 
 extern "C" int64_t nlc_model_backward_f64_workspace_bytes(nlc_model_t m, int K, int n_t, int B) {
-  if (!m || K < 1 || n_t < 1 || B < 1 || B > 8) return NLC_ERR_ARG;
-  if ((long long)K * n_t >= (1LL << 31)) return NLC_ERR_SHAPE;
-  return (int64_t)(multi_ws_layout(shape_of(m, B), K, n_t, true, true).total * sizeof(double));
+  return multi_ws_bytes(m, K, n_t, B, true, true);
 }
 
 extern "C" int nlc_model_backward_f64(nlc_model_t m, const double* params_dev, const double* obs_dev, const double* act_dev,
@@ -1118,46 +1100,24 @@ extern "C" int nlc_model_backward_f64(nlc_model_t m, const double* params_dev, c
                                       void* stream) {
   NLC_REQUIRE(m && params_dev && obs_dev && act_dev && ts_dev && grad_out_dev && grad_params_dev && workspace_dev, NLC_ERR_ARG,
               "nlc_model_backward_f64: null pointer");
-  int rc = f64_check("nlc_model_backward_f64", m, K, n_t, B, workspace_dev);
+  int rc = multi_check("nlc_model_backward_f64", m, K, n_t, B, workspace_dev);
   if (rc != NLC_OK) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const GradShape g = shape_of(m, B);
   const MultiWs w = multi_ws_layout(g, K, n_t, true, true);
   double* ws = static_cast<double*>(workspace_dev);
-  rc = f64_encode(m, g, w, params_dev, act_dev, K, ws, ws + w.p, s);
+  rc = f64_weight_image(g, params_dev, ws + w.wt, s);
   if (rc != NLC_OK) return rc;
-  NLC_CUDA_OK(cudaMemsetAsync(ws + w.part, 0, (size_t)w.G * g.p_total * sizeof(double), s));
-  const TileW<double> tw = tile_w_f64(m->d, g, ws + w.wt);
-  MultiArgs<double> ma = {};
-  ma.m = tw; ma.g = g; ma.obs = obs_dev; ma.p = ws + w.p; ma.row_b1 = ws + w.b1; ma.row_tn = ws + w.tn; ma.row_sph = ws + w.sph;
-  ma.wt = ws + w.wt; ma.part = ws + w.part; ma.scratch = ws + w.scr; ma.drow = ws + w.drow; ma.n_t = n_t;
-  const long long n_rows = (long long)K * n_t;
-  for (long long r0 = 0; r0 < n_rows; r0 += w.C) {
-    const int rows = (int)(n_rows - r0 < w.C ? n_rows - r0 : w.C);
-    rc = launch_forward_ts_prep_f64(m, tw.b1_raw, tw.w1_full_t, ts_dev + r0, rows, ws + w.b1, ws + w.tn, ws + w.sph, s);
-    if (rc != NLC_OK) return rc;
-    ma.gout = grad_out_dev + r0 * g.nx; ma.r0 = r0; ma.rows = rows;
-    if (m->Hm == 128) model_grad_multi_mlp_kernel<128, double><<<w.Gm, kGradThreads, 0, s>>>(ma);
-    else model_grad_multi_mlp_kernel<64, double><<<w.Gm, kGradThreads, 0, s>>>(ma);
-    NLC_LAUNCH_OK("model_grad_multi_mlp_kernel<double>");
-    const long long n_sum = ((r0 + rows - 1) / n_t - r0 / n_t + 1) * g.Lp;
-    model_grad_multi_rowsum_kernel<double><<<(unsigned)((n_sum + 255) / 256), 256, 0, s>>>(ws + w.drow, r0, rows, n_t, g.Lp, ws + w.dsum);
-    NLC_LAUNCH_OK("model_grad_multi_rowsum_kernel<double>");
-  }
-  GradArgs<double> a = {};
-  a.m = tw; a.g = g; a.obs = obs_dev; a.act = act_dev; a.wt = ws + w.wt; a.part = ws + w.part; a.scratch = ws + w.scr;
-  a.grad_obs = grad_obs_dev; a.grad_act = grad_act_dev; a.K = K; a.n_tiles = (K + kGradRows - 1) / kGradRows;
-  if (m->Hm == 128) model_grad_multi_enc_kernel<128, double><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
-  else model_grad_multi_enc_kernel<64, double><<<w.Ge, kGradThreads, 0, s>>>(a, ws + w.dsum);
-  NLC_LAUNCH_OK("model_grad_multi_enc_kernel<double>");
-  model_grad_reduce_kernel<double><<<(g.o_total + 255) / 256, 256, 0, s>>>(g, ws + w.part, w.G, grad_params_dev);
-  NLC_LAUNCH_OK("model_grad_reduce_kernel<double>");
-  return NLC_OK;
+  rc = encode_windows_f64(m, B, ws + w.wt, act_dev, g.gin, K, 1, ws + w.p, ws + w.scr, s);
+  if (rc != NLC_OK) return rc;
+  return backward_two_stage(m, g, w, tile_w_f64(m->d, g, ws + w.wt), ws, obs_dev, act_dev, ts_dev, K, n_t, grad_out_dev,
+                            grad_params_dev, grad_obs_dev, grad_act_dev, s);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
 // The fp64 planner's model stages (nlc_planner_f64_*, planner_f64.cu): the tile steps above over a control step's K T
-// history windows (plan_f64_encode_kernel) and its K rollouts (plan_f64_rollout_kernel).  The weights are the image
+// history windows (f64_encode_kernel, which also encodes the fp64 model's windows) and its K rollouts
+// (plan_f64_rollout_kernel).  The weights are the image
 // model_f64_weights_kernel builds from the caller's parameters, the s-point columns of the first layer are folded at the
 // planner's dt by forward_ts_prep_kernel<double> - the arithmetic of nlc_model_forward_f64 at a uniform time, so a step of
 // the rollout equals that forward bit for bit.
@@ -1184,9 +1144,10 @@ struct PlanF64Args {
   int K, T;
 };
 
-// Window w = k T + t is hist[k][t : t + B] (mppi_delay.py:261-288), read in the order of tile_load_window.
+// Window w = k T + t is hist[k][t : t + B] (mppi_delay.py:261-288), read in the order of tile_load_window.  With T = 1,
+// hist = act and hist_ch = gin these are the model's windows act [K][B][gin], read as tile_load_window reads them.
 template <int H>
-__global__ void __launch_bounds__(kGradThreads, 1) plan_f64_encode_kernel(PlanF64Args a) {
+__global__ void __launch_bounds__(kGradThreads, 1) f64_encode_kernel(PlanF64Args a) {
   const GradShape& g = a.g;
   const TileW<double>& md = a.m;
   constexpr int R = kGradRows;
@@ -1288,22 +1249,21 @@ size_t plan_f64_scratch_doubles(nlc_model_t m, int B, int K, int T) {
 int plan_f64_set_params(nlc_model_t m, const double* params_dev, const double* ts_dev, double* img, double* row_b1, double* row_tn,
                         cudaStream_t s) {
   const GradShape g = shape_of(m, 1);
-  const int n_img = g.N3p * g.H > g.in0 * g.H ? g.N3p * g.H : g.in0 * g.H;
-  model_f64_weights_kernel<<<(n_img + 255) / 256, 256, 0, s>>>(g, params_dev, img);
-  NLC_LAUNCH_OK("model_f64_weights_kernel");
+  const int rc = f64_weight_image(g, params_dev, img, s);
+  if (rc != NLC_OK) return rc;
   const TileW<double> w = tile_w_f64(m->d, g, img);
-  return launch_forward_ts_prep_f64(m, w.b1_raw, w.w1_full_t, ts_dev, 1, row_b1, row_tn, nullptr, s);
+  return launch_forward_ts_prep<double>(m, w.b1_raw, w.w1_full_t, ts_dev, 1, row_b1, row_tn, nullptr, s);
 }
 
-int plan_f64_encode(nlc_model_t m, int B, const double* img, const double* hist, int hist_ch, int K, int T, double* p_out,
-                    double* scratch, cudaStream_t s) {
+int encode_windows_f64(nlc_model_t m, int B, const double* img, const double* hist, int hist_ch, int K, int T, double* p_out,
+                       double* scratch, cudaStream_t s) {
   PlanF64Args a = {};
   a.g = shape_of(m, B); a.m = tile_w_f64(m->d, a.g, img);
   a.hist = hist; a.hist_ch = hist_ch; a.p_out = p_out; a.scratch = scratch; a.K = K; a.T = T;
   const int G = plan_f64_grid((long long)K * T);
-  if (m->Hm == 128) plan_f64_encode_kernel<128><<<G, kGradThreads, 0, s>>>(a);
-  else plan_f64_encode_kernel<64><<<G, kGradThreads, 0, s>>>(a);
-  NLC_LAUNCH_OK("plan_f64_encode_kernel");
+  if (m->Hm == 128) f64_encode_kernel<128><<<G, kGradThreads, 0, s>>>(a);
+  else f64_encode_kernel<64><<<G, kGradThreads, 0, s>>>(a);
+  NLC_LAUNCH_OK("f64_encode_kernel");
   return NLC_OK;
 }
 

@@ -2,7 +2,7 @@
 // plans in.  A handle of its own beside nlc_planner_t: no tensor cores, no encoder beside the rollout, no device exchange, no
 // graphs and no mapped staging - one fixed sequence of direct launches per control step:
 //   plan_f64_perturb_kernel           stage 1 (warp per sample, lanes over the horizon, as perturb_kernel)
-//   plan_f64_encode_kernel            the K T history windows through the fp64 encoder     } model_grad.cu (the tile steps
+//   f64_encode_kernel                 the K T history windows through the fp64 encoder     } model_grad.cu (the tile steps
 //   plan_f64_rollout_kernel           tiles of 32 samples through the whole horizon         }  of the fp64 model)
 //   (plan_f64_rollout_analytic_kernel instead of both for the analytic dynamics)
 //   plan_f64_softmax_kernel           beta, w = exp(-(1/lambda)(c - beta)), eta              } stage 4: fixed-order sums,
@@ -21,8 +21,8 @@ size_t plan_f64_image_doubles(nlc_model_t m);
 size_t plan_f64_scratch_doubles(nlc_model_t m, int B, int K, int T);
 int plan_f64_set_params(nlc_model_t m, const double* params_dev, const double* ts_dev, double* img, double* row_b1, double* row_tn,
                         cudaStream_t s);
-int plan_f64_encode(nlc_model_t m, int B, const double* img, const double* hist, int hist_ch, int K, int T, double* p_out,
-                    double* scratch, cudaStream_t s);
+int encode_windows_f64(nlc_model_t m, int B, const double* img, const double* hist, int hist_ch, int K, int T, double* p_out,
+                       double* scratch, cudaStream_t s);
 int plan_f64_rollout(nlc_model_t m, int B, const double* img, const double* row_b1, const double* row_tn, const double* state0, int sps,
                      const double* hist, const double* p, const double* pert_cost, int K, int T, int env, int state_constraint,
                      double goal_x, double* cost, double* states, double* scratch, cudaStream_t s);
@@ -405,7 +405,7 @@ extern "C" int nlc_planner_f64_command(nlc_planner_f64_t p, const double* state_
   int rc = perturb_f64(p, noise_in_dev, action_buffer_dev, s);
   if (rc != NLC_OK) return rc;
   if (p->model) {
-    rc = plan_f64_encode(p->model, B, p->img, p->hist, nu, K, T, p->p, p->scratch, s);
+    rc = encode_windows_f64(p->model, B, p->img, p->hist, nu, K, T, p->p, p->scratch, s);
     if (rc != NLC_OK) return rc;
     rc = plan_f64_rollout(p->model, B, p->img, p->row_b1, p->row_tn, state_dev, state_per_sample, p->hist, p->p, p->pert_cost, K, T,
                           b.rollout.env, b.rollout.state_constraint, p->d.goal_x, p->cost_total, p->states, p->scratch, s);

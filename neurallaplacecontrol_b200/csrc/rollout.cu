@@ -430,26 +430,21 @@ __global__ void __launch_bounds__(128) forward_ts_prep_kernel(const T* __restric
   if (n == 0) row_tn[k] = tn;
 }
 
-static int launch_prep(nlc_model_s* m, const float* ts, int K, float* row_b1, float* row_tn, float* row_sph, const float* obs,
-                       const float* p, long long r0, int n_t, float* row_obs, float* row_p, cudaStream_t s) {
-  forward_ts_prep_kernel<float><<<K, m->Hm, 0, s>>>(m->d.b1_raw, m->d.w1_full_t, m->Hm, m->S, m->nx + 2, m->normalize && m->normalize_time,
-                                                    (float)m->dt, ts, K, row_b1, row_tn, row_sph, obs, p, r0, n_t, row_obs, row_p);
+// b1_raw / w1_full_t: the handle's fp32 first layer, or (T = double, model_grad.cu) the one of the caller's fp64 weight image;
+// dt and the time normalisation are then in fp64 too.
+template <typename T>
+int launch_forward_ts_prep(nlc_model_s* m, const T* b1_raw, const T* w1_full_t, const T* ts, int K, T* row_b1, T* row_tn, T* row_sph,
+                           cudaStream_t s, const T* obs = nullptr, const T* p = nullptr, long long r0 = 0, int n_t = 1,
+                           T* row_obs = nullptr, T* row_p = nullptr) {
+  forward_ts_prep_kernel<T><<<K, m->Hm, 0, s>>>(b1_raw, w1_full_t, m->Hm, m->S, m->nx + 2, m->normalize && m->normalize_time, (T)m->dt,
+                                                ts, K, row_b1, row_tn, row_sph, obs, p, r0, n_t, row_obs, row_p);
   NLC_LAUNCH_OK("forward_ts_prep_kernel");
   return NLC_OK;
 }
-
-// fp64 form (model_grad.cu): first layer from the caller's fp64 weights, dt and the time normalisation in fp64
-int launch_forward_ts_prep_f64(nlc_model_s* m, const double* b1_raw, const double* w1_full_t, const double* ts, int K, double* row_b1,
-                               double* row_tn, double* row_sph, cudaStream_t s) {
-  forward_ts_prep_kernel<double><<<K, m->Hm, 0, s>>>(b1_raw, w1_full_t, m->Hm, m->S, m->nx + 2, m->normalize && m->normalize_time,
-                                                     m->dt, ts, K, row_b1, row_tn, row_sph, nullptr, nullptr, 0, 1, nullptr, nullptr);
-  NLC_LAUNCH_OK("forward_ts_prep_kernel<double>");
-  return NLC_OK;
-}
-
-int launch_forward_ts_prep(nlc_model_s* m, const float* ts, int K, float* row_b1, float* row_tn, float* row_sph, cudaStream_t s) {
-  return launch_prep(m, ts, K, row_b1, row_tn, row_sph, nullptr, nullptr, 0, 1, nullptr, nullptr, s);
-}
+template int launch_forward_ts_prep(nlc_model_s*, const float*, const float*, const float*, int, float*, float*, float*, cudaStream_t,
+                                    const float*, const float*, long long, int, float*, float*);
+template int launch_forward_ts_prep(nlc_model_s*, const double*, const double*, const double*, int, double*, double*, double*,
+                                    cudaStream_t, const double*, const double*, long long, int, double*, double*);
 
 // The MLP + Fourier ILT of K rows with per-row obs [K][nx], encoder output p [K][2] and prepared row_b1 / row_tn; mm is
 // NLC_MATH_FP32 or NLC_MATH_TC_SPLIT3.
@@ -504,7 +499,7 @@ extern "C" int nlc_model_forward_ts(nlc_model_t m, const float* obs_dev, const f
   const int mm = math_mode == NLC_MATH_TC_FP16 ? NLC_MATH_TC_SPLIT3 : math_mode;
   int rc = encode_history_impl(m, act_dev, m->gin, K, 1, B, p_action, mm, s);
   if (rc != NLC_OK) return rc;
-  rc = launch_forward_ts_prep(m, ts_dev, K, row_b1, row_tn, nullptr, s);
+  rc = launch_forward_ts_prep<float>(m, m->d.b1_raw, m->d.w1_full_t, ts_dev, K, row_b1, row_tn, nullptr, s);
   if (rc != NLC_OK) return rc;
   return forward_rows(m, obs_dev, p_action, act_dev, row_b1, row_tn, K, B, out_dev, mm, s);
 }
@@ -537,7 +532,8 @@ extern "C" int nlc_model_forward_multi(nlc_model_t m, const float* obs_dev, cons
   const long long n_rows = (long long)K * n_t;
   for (long long r0 = 0; r0 < n_rows; r0 += w.C) {
     const int rows = (int)(n_rows - r0 < w.C ? n_rows - r0 : w.C);
-    rc = launch_prep(m, ts_dev + r0, rows, ws + w.b1, ws + w.tn, nullptr, obs_dev, p, r0, n_t, ws + w.obs, ws + w.rp, s);
+    rc = launch_forward_ts_prep<float>(m, m->d.b1_raw, m->d.w1_full_t, ts_dev + r0, rows, ws + w.b1, ws + w.tn, nullptr, s, obs_dev, p,
+                                       r0, n_t, ws + w.obs, ws + w.rp);
     if (rc != NLC_OK) return rc;
     rc = forward_rows(m, ws + w.obs, ws + w.rp, act_dev, ws + w.b1, ws + w.tn, rows, B, out_dev + r0 * m->nx, mm, s);
     if (rc != NLC_OK) return rc;

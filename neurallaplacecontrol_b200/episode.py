@@ -20,12 +20,10 @@ from __future__ import annotations
 import ctypes as C
 import time
 
-import numpy as np
 import torch
 
 from . import _lib
-from .closures import NLDynamics
-from .planners.mppi_delay import MPPIDelay, _DevView, _MPPIDelayF64
+from .planners.mppi_delay import MPPIDelay, _MPPIDelayF64, _buffer_view
 
 
 class BatchedMPPIDelay:
@@ -34,6 +32,7 @@ class BatchedMPPIDelay:
     Constructor arguments are ``MPPIDelay``'s (``planners/mppi_delay.py:64-90``) plus ``n_instances``, ``seeds``
     (one sampler seed per instance, default ``range(n_instances)``) and ``U_init`` of shape ``(T, nu)`` (shared) or
     ``(I, T, nu)``.  ``process_group`` is not accepted: a batch is sharded by instance, never by sample (SURVEY 8e)."""
+    _c_buffer, _typestr = "nlc_batch_planner_buffer", "<f4"
 
     def __init__(self, dynamics, running_cost, nx, noise_sigma, n_instances, seeds=None, U_init=None, **kw):
         if "process_group" in kw and kw["process_group"] is not None:
@@ -65,17 +64,13 @@ class BatchedMPPIDelay:
     def _ensure(self, B):
         # the packed model is re-fetched on every call (see MPPIDelay._ensure): a rebuilt or re-folded model handle
         # must never be planned on silently
-        model_h = None
-        if isinstance(self._tpl.F, NLDynamics):
-            if self._tpl.F.model._cuda_device is None:
-                self._tpl.F.model._cuda_device = self.d
-            model_h = self._tpl.F.model.set_prediction_time(self._tpl.F.dt)
+        model_h = self._tpl._model_handle()
         key = None if model_h is None else model_h.value
         if self._handle is not None and self._handle_B == B and self._handle_model == key:
             return self._handle
         self._destroy()
         self._handle_model = key
-        d, model_h = self._tpl._desc(B, self.K, 0, self.K, 1, 0)
+        d = self._tpl._desc(B, self.K, 0, self.K, 1, 0)
         seeds = (C.c_uint64 * self.I)(*self.seeds)
         h = C.c_void_p()
         _lib.check(self._lib.nlc_batch_planner_create(C.byref(h), model_h, C.byref(d), self.I, seeds, self.d.index), "nlc_batch_planner_create")
@@ -109,16 +104,7 @@ class BatchedMPPIDelay:
         except Exception:
             pass
 
-    def _buf(self, which, shape):
-        key = (which, tuple(shape))
-        if key not in self._views:
-            p, n = C.c_void_p(), C.c_int64()
-            _lib.check(self._lib.nlc_batch_planner_buffer(self._handle, which, C.byref(p), C.byref(n)), "nlc_batch_planner_buffer")
-            if p.value is None or n.value == 0:
-                return None
-            assert int(np.prod(shape)) == n.value, (which, shape, n.value)
-            self._views[key] = torch.as_tensor(_DevView(p.value, shape), device=self.d)
-        return self._views[key]
+    _buf = _buffer_view
 
     def _after(self, which, shape):
         return None if self._handle is None or self._calls == 0 else self._buf(which, shape)

@@ -57,6 +57,20 @@ class _DevView:
         self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (int(ptr), False), "version": 2}
 
 
+def _buffer_view(planner, which, shape):
+    """CUDA tensor aliasing one of a planner handle's device buffers, through the planner's ``_c_buffer`` C function and
+    in its ``_typestr`` element type; cached in ``planner._views``, None for a buffer the handle does not keep."""
+    key = (which, tuple(shape))
+    if key not in planner._views:
+        p, n = C.c_void_p(), C.c_int64()
+        _lib.check(getattr(planner._lib, planner._c_buffer)(planner._handle, which, C.byref(p), C.byref(n)), planner._c_buffer)
+        if p.value is None or n.value == 0:
+            return None
+        assert int(np.prod(shape)) == n.value, (which, shape, n.value)
+        planner._views[key] = torch.as_tensor(_DevView(p.value, shape, planner._typestr), device=planner.d)
+    return planner._views[key]
+
+
 def _bound_vector(x, nu, name):
     """Bound per action dimension: a scalar (what the reference's callers pass, mppi_with_model.py:227-228) or ``nu`` values.
     With a ``(nu,)`` tensor the reference's ``_bound_action`` (``mppi_delay.py:347-356``: slices of the T axis, ``torch.min``
@@ -72,6 +86,10 @@ def _bound_vector(x, nu, name):
 
 
 class MPPIDelay:
+    # the handle's C functions and element type (_MPPIDelayF64: nlc_planner_f64_*, fp64)
+    _c_destroy, _c_buffer, _c_get_U, _c_set_U = "nlc_planner_destroy", "nlc_planner_buffer", "nlc_planner_get_U", "nlc_planner_set_U"
+    _elem, _typestr = torch.float32, "<f4"
+
     def __new__(cls, *args, **kw):
         if cls is MPPIDelay and kw.get("math_mode") == "fp64":
             cls = _MPPIDelayF64  # a planner object of its own (nlc_planner_f64_*): see its docstring
@@ -196,6 +214,32 @@ class MPPIDelay:
         return buf.cpu()
 
     # ---- device handle ---------------------------------------------------------------------------------------
+    def _model_handle(self):
+        """The packed model's handle (None for the analytic dynamics), on this planner's device when the model has not been
+        given one."""
+        if not isinstance(self.F, NLDynamics):
+            return None
+        if self.F.model._cuda_device is None:
+            self.F.model._cuda_device = self.d
+        return self._fetch_handle(self.F.model)
+
+    def _fetch_handle(self, model):
+        return model.set_prediction_time(self.F.dt)
+
+    def _fill_sampling(self, x):
+        """The bounds and sampler values ``u_min`` / ``u_max``, ``noise_mu``, ``u_init``, ``sigma_inv`` and ``sigma_chol`` of
+        a descriptor (``nlc_mppi_params`` or ``nlc_planner_f64_desc``)."""
+        if self._bounds is not None:
+            for i in range(self.nu):
+                x.u_min[i], x.u_max[i] = self._bounds[0][i], self._bounds[1][i]
+        sinv = self.noise_sigma_inv.to(torch.float64).reshape(self.nu, self.nu)
+        chol = torch.linalg.cholesky(self.noise_sigma.to(torch.float64).reshape(self.nu, self.nu))
+        for i in range(self.nu):
+            x.noise_mu[i] = float(self.noise_mu.reshape(-1)[i])
+            x.u_init[i] = float(torch.as_tensor(self.u_init).reshape(-1)[i])
+            for j in range(self.nu):
+                x.sigma_inv[i * self.nu + j], x.sigma_chol[i * self.nu + j] = float(sinv[i, j]), float(chol[i, j])
+
     def _desc(self, B, K_local, k_offset, k_total, n_shards, shard_index):
         """``nlc_planner_desc`` of this planner's options (shared with the instance-batched planner)."""
         d = _lib.PlannerDesc()
@@ -204,18 +248,8 @@ class MPPIDelay:
         mp.k_offset, mp.k_total = k_offset, k_total
         mp.lambda_, mp.u_scale = float(self.lambda_), float(self.u_scale)
         mp.has_bounds = int(self.u_max is not None)
-        if self._bounds is not None:
-            for i in range(self.nu):
-                mp.u_min[i], mp.u_max[i] = self._bounds[0][i], self._bounds[1][i]
         mp.sample_null_action, mp.noise_abs_cost = int(self.sample_null_action), int(self.noise_abs_cost)
-        sinv = self.noise_sigma_inv.to(torch.float64).reshape(self.nu, self.nu)
-        chol = torch.linalg.cholesky(self.noise_sigma.to(torch.float64).reshape(self.nu, self.nu))
-        for i in range(self.nu):
-            mp.noise_mu[i] = float(self.noise_mu.reshape(-1)[i])
-            mp.u_init[i] = float(torch.as_tensor(self.u_init).reshape(-1)[i])
-            for j in range(self.nu):
-                mp.sigma_inv[i * self.nu + j] = float(sinv[i, j])
-                mp.sigma_chol[i * self.nu + j] = float(chol[i, j])
+        self._fill_sampling(mp)
         ro = d.rollout
         ro.env = _lib.ENV_IDS[self.running_cost.env_name]
         ro.state_constraint = int(self.running_cost.state_constraint)
@@ -227,12 +261,7 @@ class MPPIDelay:
         d.math_mode = _lib.MATH_MODES[self.math_mode]
         d.keep_states = int(self.keep_states)
         d.seed = self.seed
-        model_h = None
-        if isinstance(self.F, NLDynamics):
-            if self.F.model._cuda_device is None:
-                self.F.model._cuda_device = self.d
-            model_h = self.F.model.set_prediction_time(self.F.dt)
-        return d, model_h
+        return d
 
     def _ensure(self, B):
         """The device planner for a B-entry action buffer.  The packed model is re-fetched on EVERY call: the model
@@ -240,28 +269,23 @@ class MPPIDelay:
         constants when ``forward`` ran at another prediction time, and the planner must never roll out on a stale
         or re-folded handle - so the prediction time is folded back to this planner's ``dt`` and the planner handle
         is recreated when the model handle is a new one."""
-        model_h = None
-        if isinstance(self.F, NLDynamics):
-            if self.F.model._cuda_device is None:
-                self.F.model._cuda_device = self.d
-            model_h = self.F.model.set_prediction_time(self.F.dt)
+        model_h = self._model_handle()
         key = None if model_h is None else model_h.value
         if self._handle is not None and self._handle_B == B and self._handle_model == key:
             return self._handle
         self._destroy()
-        d, model_h = self._desc(B, self.K_local, self.k_offset, self.K, self.G, self.rank)
+        d = self._desc(B, self.K_local, self.k_offset, self.K, self.G, self.rank)
         h = C.c_void_p()
         _lib.check(self._lib.nlc_planner_create(C.byref(h), model_h, C.byref(d), self.d.index), "nlc_planner_create")
-        self._handle, self._handle_B, self._views = h, B, {}
-        self._handle_model = None if model_h is None else model_h.value
+        self._handle, self._handle_B, self._handle_model, self._views = h, B, key, {}
         self._U_dirty = True
         self._exchange = False
         if self.G > 1 and self.process_group is not None:
-            self._connect_exchange(h)
+            self._connect_exchange(h, model_h)
         return self._handle
 
     # ---- device-side exchange of the shard triples (include/nlc_b200.h: nlc_planner_exchange_*) ----------------------------
-    def _connect_exchange(self, h):
+    def _connect_exchange(self, h, model_h):
         """Map every rank's mailbox into this process through CUDA IPC (one all-gather of the 64-byte handles, at handle
         creation only).  From then on a control step exchanges the triples on the device and is ONE graph launch.  If any
         rank cannot map a peer (no P2P between the GPUs, ``NLC_NO_DEVICE_EXCHANGE=1``) every rank falls back to the
@@ -289,7 +313,7 @@ class MPPIDelay:
         else:
             # a half-connected group would deadlock in the device-side poll: drop the handle and keep the collective path
             # (a connected handle cannot be disconnected, so it is rebuilt; nothing has been planned with it yet)
-            d, model_h = self._desc(self._handle_B, self.K_local, self.k_offset, self.K, self.G, self.rank)
+            d = self._desc(self._handle_B, self.K_local, self.k_offset, self.K, self.G, self.rank)
             self._lib.nlc_planner_destroy(h)
             h2 = C.c_void_p()
             _lib.check(self._lib.nlc_planner_create(C.byref(h2), model_h, C.byref(d), self.d.index), "nlc_planner_create")
@@ -322,39 +346,29 @@ class MPPIDelay:
     def _destroy(self):
         if self._handle is not None:
             self._sync_U_to_host()
-            self._lib.nlc_planner_destroy(self._handle)
+            getattr(self._lib, self._c_destroy)(self._handle)
             self._handle = None
             self._views = {}
 
     def __del__(self):
         try:
             if self._handle is not None:
-                self._lib.nlc_planner_destroy(self._handle)
+                getattr(self._lib, self._c_destroy)(self._handle)
         except Exception:
             pass
 
-    def _buf(self, which, shape):
-        """fp32 CUDA tensor aliasing one of the planner's device buffers."""
-        key = (which, tuple(shape))
-        if key not in self._views:
-            p, n = C.c_void_p(), C.c_int64()
-            _lib.check(self._lib.nlc_planner_buffer(self._handle, which, C.byref(p), C.byref(n)), "nlc_planner_buffer")
-            if p.value is None or n.value == 0:
-                return None
-            assert int(np.prod(shape)) == n.value, (which, shape, n.value)
-            self._views[key] = torch.as_tensor(_DevView(p.value, shape), device=self.d)
-        return self._views[key]
+    _buf = _buffer_view
 
     def _sync_U_to_host(self):
         if self._handle is not None and not self._U_dirty:
             arr = np.empty(self.T * self.nu, dtype=np.float64)
-            _lib.check(self._lib.nlc_planner_get_U(self._handle, arr.ctypes.data_as(C.POINTER(C.c_double))), "nlc_planner_get_U")
+            _lib.check(getattr(self._lib, self._c_get_U)(self._handle, arr.ctypes.data_as(C.POINTER(C.c_double))), self._c_get_U)
             self._U_host = torch.from_numpy(arr).reshape(self.T, self.nu).clone()
 
     def _push_U(self):
         if self._U_dirty:
             ptr, keep = _lib.as_double_array(self._U_host.numpy())
-            _lib.check(self._lib.nlc_planner_set_U(self._handle, ptr), "nlc_planner_set_U")
+            _lib.check(getattr(self._lib, self._c_set_U)(self._handle, ptr), self._c_set_U)
             self._U_dirty = False
 
     # ---- the reference's attributes ------------------------------------------------------------------------------
@@ -406,7 +420,7 @@ class MPPIDelay:
         if tuple(nz.shape) != (self.K, self.T, self.nu):
             raise ValueError(f"injected noise must have shape {(self.K, self.T, self.nu)}, got {tuple(nz.shape)}")
         nz = nz[self.k_offset:self.k_offset + self.K_local]  # bit-exact sample indexing: global k = offset + local k
-        return nz.to(device=self.d, dtype=torch.float32).contiguous()
+        return nz.to(device=self.d, dtype=self._elem).contiguous()
 
     def command(self, state, action_buffer):
         """:param state: (nx) or (K x nx) current state; :param action_buffer: (B x nu) past actions, env units.
@@ -561,10 +575,7 @@ class MPPIDelay:
             state = state.repeat(n, 1)
         if state.shape[0] != n:
             raise ValueError("state must be (nx) or (num_rollouts, nx)")
-        model = self.F.model
-        if model._cuda_device is None:
-            model._cuda_device = self.d
-        mh = model.set_prediction_time(self.F.dt)
+        mh = self._model_handle()
         U = self.U.to(device=self.d, dtype=torch.float32).reshape(self.T, self.nu)
         hist = (float(self.u_scale) * U).reshape(1, self.T, self.nu).repeat(n, 1, 1).contiguous()  # B = 1: L = T
         st = state.to(device=self.d, dtype=torch.float32).contiguous()
@@ -586,6 +597,9 @@ class MPPIDelay:
 class _MPPIDelayF64(MPPIDelay):
     """``MPPIDelay(..., math_mode="fp64")``: the control step on the fp64 planner handle (``nlc_planner_f64_*``), single shard,
     direct launches on the current stream (host inputs: one C call that copies in, plans and copies the action back)."""
+    _c_destroy, _c_buffer = "nlc_planner_f64_destroy", "nlc_planner_f64_buffer"
+    _c_get_U, _c_set_U = "nlc_planner_f64_get_U", "nlc_planner_f64_set_U"
+    _elem, _typestr = torch.float64, "<f8"
 
     def __init__(self, *args, process_group=None, shard=None, **kw):
         if process_group is not None or shard is not None:
@@ -606,27 +620,17 @@ class _MPPIDelayF64(MPPIDelay):
         ro.state_constraint, ro.dynamics, ro.delay = int(self.running_cost.state_constraint), self.F.kind, int(self.F.delay)
         b.nx, b.n_shards, b.shard_index, b.keep_states, b.seed = self.nx, 1, 0, int(self.keep_states), self.seed
         d.lambda_, d.u_scale, d.dt, d.goal_x = float(self.lambda_), float(self.u_scale), float(self.F.dt), float(self.running_cost.goal_x)
-        if self._bounds is not None:
-            for i in range(self.nu):
-                d.u_min[i], d.u_max[i] = self._bounds[0][i], self._bounds[1][i]
-        sinv = self.noise_sigma_inv.to(torch.float64).reshape(self.nu, self.nu)
-        chol = torch.linalg.cholesky(self.noise_sigma.to(torch.float64).reshape(self.nu, self.nu))
-        for i in range(self.nu):
-            d.noise_mu[i] = float(self.noise_mu.reshape(-1)[i])
-            d.u_init[i] = float(torch.as_tensor(self.u_init).reshape(-1)[i])
-            for j in range(self.nu):
-                d.sigma_inv[i * self.nu + j], d.sigma_chol[i * self.nu + j] = float(sinv[i, j]), float(chol[i, j])
+        self._fill_sampling(d)
         return d
+
+    def _fetch_handle(self, model):
+        with self._on_device():
+            return model._handle_f64()
 
     def _ensure(self, B):
         """The fp64 planner for a B-entry action buffer, rebuilt when the model's handle is a new one (its buffers or device
         changed); its weights come separately (``_push_params``)."""
-        model_h = None
-        if isinstance(self.F, NLDynamics):
-            if self.F.model._cuda_device is None:
-                self.F.model._cuda_device = self.d
-            with self._on_device():
-                model_h = self.F.model._handle_f64()
+        model_h = self._model_handle()
         key = None if model_h is None else model_h.value
         if self._handle is not None and self._handle_B == B and self._handle_model == key:
             return self._handle
@@ -651,44 +655,6 @@ class _MPPIDelayF64(MPPIDelay):
         _lib.check(self._lib.nlc_planner_f64_set_params(h, params.data_ptr(), stream), "nlc_planner_f64_set_params")
         self._params_dev, self._params_key = params, key
 
-    def _destroy(self):
-        if self._handle is not None:
-            self._sync_U_to_host()
-            self._lib.nlc_planner_f64_destroy(self._handle)
-            self._handle = None
-            self._views = {}
-
-    def __del__(self):
-        try:
-            if self._handle is not None:
-                self._lib.nlc_planner_f64_destroy(self._handle)
-        except Exception:
-            pass
-
-    def _buf(self, which, shape):
-        """fp64 CUDA tensor aliasing one of the fp64 planner's device buffers."""
-        key = (which, tuple(shape))
-        if key not in self._views:
-            p, n = C.c_void_p(), C.c_int64()
-            _lib.check(self._lib.nlc_planner_f64_buffer(self._handle, which, C.byref(p), C.byref(n)), "nlc_planner_f64_buffer")
-            if p.value is None or n.value == 0:
-                return None
-            assert int(np.prod(shape)) == n.value, (which, shape, n.value)
-            self._views[key] = torch.as_tensor(_DevView(p.value, shape, "<f8"), device=self.d)
-        return self._views[key]
-
-    def _sync_U_to_host(self):
-        if self._handle is not None and not self._U_dirty:
-            arr = np.empty(self.T * self.nu, dtype=np.float64)
-            _lib.check(self._lib.nlc_planner_f64_get_U(self._handle, arr.ctypes.data_as(C.POINTER(C.c_double))), "nlc_planner_f64_get_U")
-            self._U_host = torch.from_numpy(arr).reshape(self.T, self.nu).clone()
-
-    def _push_U(self):
-        if self._U_dirty:
-            ptr, keep = _lib.as_double_array(self._U_host.numpy())
-            _lib.check(self._lib.nlc_planner_f64_set_U(self._handle, ptr), "nlc_planner_f64_set_U")
-            self._U_dirty = False
-
     @property
     def cost_total_non_zero(self):
         """exp(-(1/lambda)(c - beta)) (mppi_delay.py:210-211)."""
@@ -698,15 +664,6 @@ class _MPPIDelayF64(MPPIDelay):
     def omega(self):
         nz = self.cost_total_non_zero
         return None if nz is None else (1.0 / self._buf(_lib.BUF_STATS, (2,))[1]) * nz
-
-    def _injected_noise(self):
-        fn = self.noise_dist.__dict__.get("sample")
-        if fn is None:
-            return None
-        nz = torch.as_tensor(fn((self.K, self.T)))
-        if tuple(nz.shape) != (self.K, self.T, self.nu):
-            raise ValueError(f"injected noise must have shape {(self.K, self.T, self.nu)}, got {tuple(nz.shape)}")
-        return nz.to(device=self.d, dtype=torch.float64).contiguous()
 
     def command(self, state, action_buffer):
         """:param state: (nx) or (K x nx) current state; :param action_buffer: (B x nu) past actions, env units.

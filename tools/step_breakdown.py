@@ -35,7 +35,7 @@ def main():
     buf = torch.zeros(B, nu, dtype=torch.float64, device=dev)
     planner.command(state, buf)  # creates the handle and buffers
     lib, h = _lib.load(), planner._handle
-    d, mh = planner._desc(B, K, 0, K, 1, 0)
+    d, mh = planner._desc(B, K, 0, K, 1, 0), planner._model_handle()
     mp, ro, mode = d.mppi, d.rollout, d.math_mode
     g = lambda which, shape: planner._buf(which, shape)  # noqa: E731
     U, noise, pert, hist = g(_lib.BUF_U, (H, nu)), g(_lib.BUF_NOISE, (K, H, nu)), g(_lib.BUF_PERTURBED, (K, H, nu)), g(_lib.BUF_HIST, (K, B - 1 + H, nu))
