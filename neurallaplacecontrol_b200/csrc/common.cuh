@@ -102,17 +102,16 @@ struct ModelDev {
   // rollout_tc2.cu: representation MLP with -2 log2(e) folded into every layer (all three feed tanh-like maps):
   // mlp2_w1 [2 (hi,lo)][128 x 16]  first layer on the tensor cores, K = [obs_n | p_action | 1 (folded bias) | 0..]
   //                                 (re-packed by nlc_model_set_prediction_time: the bias depends on the s-points);
-  // mlp2_w2 [2][128 x 128]; mlp2_w3 [2][N3t x 128] pair-permuted; mlp2_c = [b2 (128) | b3 (256)] scaled
+  // mlp2_w2 [2][128 x 128], mlp2_b2 [128] scaled;
+  // mlp2_w3 [2 (hi,lo)][N3u x 128], mlp2_b3 [N3u] scaled, in the GROUP-UNIFORM column order (rollout_tc2.cu: every column
+  // group of a tile runs the SAME L3 epilogue code): column = 32 j + 8 cg + 2 i + {theta, phi}; regular unit j < NX (S-1)/16:
+  // channel j / upc, term 16 (j % upc) + cg + 4 i (upc = (S-1)/16); last unit: the channels' last terms k = S-1, pair i =
+  // channel cg + 4 i (zero columns where that channel does not exist)
   void* mlp2_w1;
   void* mlp2_w2;
+  float* mlp2_b2;
   void* mlp2_w3;
-  float* mlp2_c;
-  // the ping-pong rollout's own W3 image and biases, in the GROUP-UNIFORM column order (rollout_tc2.cu: every column group of
-  // a tile runs the SAME L3 epilogue code): column = 32 j + 8 cg + 2 i + {theta, phi}; regular unit j < NX (S-1)/16: channel
-  // j / upc, term 16 (j % upc) + cg + 4 i (upc = (S-1)/16); last unit: the channels' last terms k = S-1, pair i = channel
-  // cg + 4 i (zero columns where that channel does not exist).  mlp2_w3u [2 (hi,lo)][N3u x 128], mlp2_cu [N3u] scaled biases.
-  void* mlp2_w3u;
-  float* mlp2_cu;
+  float* mlp2_b3;
   // ---- representation MLP (w_nl.py:32-63) --------------------------------------------------
   float* w1_full_t; // [2S+nx+2][Hm]  unfolded first layer (per-sample-time forward)
   float* b1_raw;    // [Hm]
@@ -164,8 +163,8 @@ struct ModelHost {  // fp64 copies kept for re-folding at another prediction tim
 
 struct nlc_model_s {
   int device;
-  int nx, nu, gin, Hm, Hg, S, N3, N3p, N3t;  // N3t: N3 rounded up to the MMA's N granularity (16)
-  int N3u;                                   // columns of the group-uniform W3 image (0: none packed)
+  int nx, nu, gin, Hm, Hg, S, N3, N3p;
+  int N3u;  // columns of the group-uniform W3 image (0: none packed)
   int normalize, normalize_time, encode_obs_time;
   double dt, ts_pred, t_norm;
   nlc::ModelDev d;

@@ -32,7 +32,6 @@
 //              layers; warp 16: MMA issue.  544 threads -> 96 registers per thread (the register file is allocated in
 //              units of 4 warps: 104 would not launch).
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "f32x2.cuh"
@@ -88,18 +87,18 @@ __device__ __forceinline__ void ldtm8p(uint32_t taddr, f2_t (&v)[4]) {
 //   pr, pz = -log2e (W_r. + b_r), -log2e (W_z. + b_z);   gi, gh = -2 log2e (W_in x + b_in), -2 log2e (W_hn h + b_hn)
 //   r = 1/(1 + 2^pr), z = 1/(1 + 2^pz) through ONE reciprocal of the product;  n = 2/(1 + 2^(gi + r gh)) - 1;
 //   h' = n + z (h - n).   Arguments of ex2 are clamped so that the shared-reciprocal product stays finite.
-//   RZ == kGateTanhApprox: the single-pass fp16 mode's accuracy class - three tanh.approx (|error| <= 2^-10.99) per unit and
+//   kAccurate (fp32-class mode): the (r, z) reciprocal by Newton (rcp2<3>), the n reciprocal by Newton when kNewtonN, else MUFU.
+//   !kAccurate: the single-pass fp16 mode's accuracy class - three tanh.approx (|error| <= 2^-10.99) per unit and
 //   almost no arithmetic: sigmoid(x) = 0.5 tanh(x/2) + 0.5, with x/2 = -pr / (2 log2e) recovered from the folded scale.
-constexpr int kGateTanhApprox = 9;
 __device__ __forceinline__ float mufu_tanh(float x) { float y; asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 
 //   kClampRZ: clamp the (r, z) exponents at 60 so that the shared-reciprocal product (1 + 2^pr)(1 + 2^pz) stays finite.  Not
 //   needed (and compiled out) when the pre-activations are provably inside +-60 - layer 1, whose inputs are hidden states in
 //   (-1, 1): the bound is the L1 norm of the weight rows, checked when the model is packed (model.cu: enc_l1_bounded).
 //   The n exponent needs no clamp with the MUFU reciprocal: 2^x = inf gives rcp = 0, n = -1, h - n = h + 1, all exact limits.
-template <int RZ, int NN, bool kClampRZ>
+template <bool kAccurate, bool kNewtonN, bool kClampRZ>
 __device__ __forceinline__ f2_t gru_pair(f2_t pr, f2_t pz, f2_t gi, f2_t gh, f2_t h_old) {
-  if (RZ == kGateTanhApprox) {
+  if (!kAccurate) {
     const f2_t c = pk2(-0.34657359027997264f, -0.34657359027997264f);  // -1 / (2 log2 e)
     const f2_t half = pk2(0.5f, 0.5f);
     float a0, a1, b0, b1, x0, x1;
@@ -118,13 +117,13 @@ __device__ __forceinline__ f2_t gru_pair(f2_t pr, f2_t pz, f2_t gi, f2_t gh, f2_
   if (kClampRZ) { a0 = fminf(a0, 60.0f); a1 = fminf(a1, 60.0f); b0 = fminf(b0, 60.0f); b1 = fminf(b1, 60.0f); }
   const f2_t da = add2(pk2(mufu_ex2(a0), mufu_ex2(a1)), one);
   const f2_t db = add2(pk2(mufu_ex2(b0), mufu_ex2(b1)), one);
-  const f2_t inv = rcp2<RZ>(mul2(da, db));
+  const f2_t inv = rcp2<3>(mul2(da, db));
   const f2_t r = mul2(db, inv), z = mul2(da, inv);
   float x0, x1;
   upk2(fma2(r, gh, gi), x0, x1);
-  if (NN != 0) { x0 = fminf(x0, 120.0f); x1 = fminf(x1, 120.0f); }  // the Newton reciprocal needs a finite argument
+  if (kNewtonN) { x0 = fminf(x0, 120.0f); x1 = fminf(x1, 120.0f); }  // the Newton reciprocal needs a finite argument
   const f2_t dn = add2(pk2(mufu_ex2(x0), mufu_ex2(x1)), one);
-  const f2_t invn = rcp2<NN>(dn);
+  const f2_t invn = rcp2<kNewtonN ? 3 : 0>(dn);
   const f2_t n = fma2(pk2(2.0f, 2.0f), invn, pk2(-1.0f, -1.0f));
   const f2_t hm = fma2(pk2(-2.0f, -2.0f), invn, add2(h_old, one));  // h - n = (h + 1) - 2 invn
   return fma2(z, hm, n);
@@ -203,7 +202,9 @@ struct Smem {
   uint32_t tmem_base;
 };
 
-template <bool kSplit3, int GIN, int RZ, int NN, bool kClamp1, bool kTrace = false>
+// kSplit3: the fp32-class mode (split-3 products, Newton (r, z) reciprocals, Newton for one n-pair in four); else the
+// single-pass fp16 mode with tanh.approx gates
+template <bool kSplit3, int GIN, bool kClamp1, bool kTrace = false>
 __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   Smem& s = *reinterpret_cast<Smem*>(smem_raw);
@@ -393,11 +394,11 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
       tmem_ld_wait();
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
-        // NN = 1 / 2: the n-gate reciprocal by Newton for one / two of the four pairs of a chunk, MUFU for the others.  The MUFU
-        // pipe (70 % busy) and the FMA pipe / issue slots are balanced at one in four: 2.18 ms at config 4 against 2.23 (none),
-        // 2.21 (two) and 2.29 ms (all four by Newton)
-        if ((NN == 1 && i == 0) || (NN == 2 && (i & 1) == 0)) h0r[4 * c + i] = gru_pair<RZ, 3, true>(gr[i], gz[i], gn[i], gh[i], h0r[4 * c + i]);
-        else h0r[4 * c + i] = gru_pair<RZ, (NN == 1 || NN == 2) ? 0 : NN, true>(gr[i], gz[i], gn[i], gh[i], h0r[4 * c + i]);
+        // fp32-class: the n-gate reciprocal by Newton for the first of the four pairs of a chunk, MUFU for the others.  The
+        // MUFU pipe (70 % busy) and the FMA pipe / issue slots are balanced at one in four: 2.18 ms at config 4 against 2.23
+        // (none), 2.21 (two) and 2.29 ms (all four by Newton)
+        if (kSplit3 && i == 0) h0r[4 * c + i] = gru_pair<kSplit3, true, true>(gr[i], gz[i], gn[i], gh[i], h0r[4 * c + i]);
+        else h0r[4 * c + i] = gru_pair<kSplit3, false, true>(gr[i], gz[i], gn[i], gh[i], h0r[4 * c + i]);
       }
     }
     if (store) {
@@ -483,8 +484,8 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
         tmem_ld_wait();
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-          if ((NN == 1 && i == 0) || (NN == 2 && (i & 1) == 0)) h1r[4 * c + i] = gru_pair<RZ, 3, kClamp1>(gr[i], gz[i], gn[i], gh[i], h1r[4 * c + i]);
-          else h1r[4 * c + i] = gru_pair<RZ, (NN == 1 || NN == 2) ? 0 : NN, kClamp1>(gr[i], gz[i], gn[i], gh[i], h1r[4 * c + i]);
+          if (kSplit3 && i == 0) h1r[4 * c + i] = gru_pair<kSplit3, true, kClamp1>(gr[i], gz[i], gn[i], gh[i], h1r[4 * c + i]);
+          else h1r[4 * c + i] = gru_pair<kSplit3, false, kClamp1>(gr[i], gz[i], gn[i], gh[i], h1r[4 * c + i]);
         }
         if (st + 1 < B) {  // MMA B(st), the last reader of the h1 image, has completed (bar_b above): store chunk by chunk
           const f2_t (&hc)[4] = *reinterpret_cast<const f2_t(*)[4]>(&h1r[4 * c]);
@@ -568,23 +569,16 @@ int launch_encode_tc2(nlc_model_s* m, const float* hist, int hist_ch, int K, int
   a.m = m->d;
   a.trace = g_enc_trace;
   const int smem = (int)sizeof(Smem) + 128;
-  // fp32-class mode: Newton (3 steps) for the (r, z) reciprocal; for n, Newton for one pair in four and MUFU for the rest ("31");
+  // fp32-class mode: Newton (3 steps) for the (r, z) reciprocal; for n, Newton for one pair in four and MUFU for the rest;
   // single-pass fp16 mode: three tanh.approx per unit (that mode's accuracy class, 2e-2 bound).
-  // NLC_ENC_RCP=<rz><nn> (00, 30, 31, 32, 33) overrides the fp32-class choice for measurements.
-  static const int rcp_sel = [] { const char* e = getenv("NLC_ENC_RCP"); return (e && e[0] && e[1]) ? (e[0] - '0') * 10 + (e[1] - '0') : 31; }();
   void (*kern)(Args);
   // layer-1 (r, z) clamps are compiled out when the packed weights prove |pre-activation| * log2(e) < 60 (model.cu)
   const bool c1 = !m->enc_l1_bounded;
-#define NLC_ENC_PICK(S3, RZ_, NN_, TR) \
-  (m->gin == 1 ? (c1 ? encode_tc2_kernel<S3, 1, RZ_, NN_, true, TR> : encode_tc2_kernel<S3, 1, RZ_, NN_, false, TR>) \
-               : (c1 ? encode_tc2_kernel<S3, 2, RZ_, NN_, true, TR> : encode_tc2_kernel<S3, 2, RZ_, NN_, false, TR>))
-  if (!split3) kern = m->gin == 1 ? encode_tc2_kernel<false, 1, kGateTanhApprox, 0, true> : encode_tc2_kernel<false, 2, kGateTanhApprox, 0, true>;
-  else if (rcp_sel == 0) kern = NLC_ENC_PICK(true, 0, 0, false);
-  else if (rcp_sel == 33) kern = NLC_ENC_PICK(true, 3, 3, false);
-  else if (rcp_sel == 30) kern = NLC_ENC_PICK(true, 3, 0, false);
-  else if (rcp_sel == 32) kern = NLC_ENC_PICK(true, 3, 2, false);
-  else kern = NLC_ENC_PICK(true, 3, 1, false);
-  if (a.trace && split3) kern = NLC_ENC_PICK(true, 3, 1, true);
+#define NLC_ENC_PICK(TR) \
+  (m->gin == 1 ? (c1 ? encode_tc2_kernel<true, 1, true, TR> : encode_tc2_kernel<true, 1, false, TR>) \
+               : (c1 ? encode_tc2_kernel<true, 2, true, TR> : encode_tc2_kernel<true, 2, false, TR>))
+  if (!split3) kern = m->gin == 1 ? encode_tc2_kernel<false, 1, true> : encode_tc2_kernel<false, 2, true>;
+  else kern = a.trace ? NLC_ENC_PICK(true) : NLC_ENC_PICK(false);
 #undef NLC_ENC_PICK
   NLC_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   long long n_tiles = ready ? (long long)a.tiles_per_t * T : (a.rows + kRows - 1) / kRows;

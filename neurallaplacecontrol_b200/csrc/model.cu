@@ -168,7 +168,7 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
                         d->enc_out_w, d->enc_out_b, d->mlp_w0, d->mlp_b0, d->mlp_w2, d->mlp_b2, d->mlp_w4, d->mlp_b4};
   for (const void* p : ptrs) NLC_REQUIRE(p != nullptr, NLC_ERR_ARG, "null weight pointer in nlc_model_desc");
 
-  const int Hg = Hm / 2, G3 = 3 * Hg, L = nx + 2, in0 = 2 * S + L, N3 = 2 * nx * S, N3p = (N3 + 3) / 4 * 4, N3t = (N3 + 15) / 16 * 16;
+  const int Hg = Hm / 2, G3 = 3 * Hg, L = nx + 2, in0 = 2 * S + L, N3 = 2 * nx * S, N3p = (N3 + 3) / 4 * 4;
   {
     // Every parameter must be finite.  Besides being meaningless otherwise, the tensor-core encoder's [x | 1] operand
     // block lets the zero half of its A side multiply neighbouring (weight) data of the B side (encode_tc2.cu): that
@@ -186,7 +186,7 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
   }
   nlc_model_s* m = new nlc_model_s();
   memset(&m->d, 0, sizeof(m->d));
-  m->device = device; m->nx = nx; m->nu = nu; m->gin = gin; m->Hm = Hm; m->Hg = Hg; m->S = S; m->N3 = N3; m->N3p = N3p; m->N3t = N3t;
+  m->device = device; m->nx = nx; m->nu = nu; m->gin = gin; m->Hm = Hm; m->Hg = Hg; m->S = S; m->N3 = N3; m->N3p = N3p;
   m->normalize = d->normalize; m->normalize_time = d->normalize_time; m->encode_obs_time = d->encode_obs_time;
   m->dt = d->dt; m->arena = nullptr; m->refs = 0; m->destroy_requested = false;
   {
@@ -214,14 +214,13 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
   // tensor-core operand image of the three recurrent GRU matrices: fp16 hi/lo, UMMA canonical layout
   const size_t tc_halves = (size_t)3 * 2 * G3 * Hg;
   size_t o_enc2w = A.add(tc_halves / 2), o_enc2c = A.add(nlc::kE2Count), o_enc2x = A.add(2 * 256 * 8 / 2);
-  size_t o_m2w1 = A.add((size_t)2 * Hm * 16 / 2), o_m2w2 = A.add((size_t)2 * Hm * Hm / 2), o_m2w3 = A.add((size_t)2 * N3t * Hm / 2);
-  size_t o_m2c = A.add(128 + 416);  // b2 | b3 (up to 416 (theta, phi) columns: rollout_tc2.cu kMaxN3)
-  // group-uniform W3 image of the ping-pong rollout: 32 columns per unit, NX (S-1)/16 regular units + 1 unit of last terms
+  size_t o_m2w1 = A.add((size_t)2 * Hm * 16 / 2), o_m2w2 = A.add((size_t)2 * Hm * Hm / 2), o_m2b2 = A.add(128);
+  // group-uniform W3 image of the tensor-core rollout: 32 columns per unit, NX (S-1)/16 regular units + 1 unit of last terms
   const int gu_upc = (S - 1) % 16 == 0 ? (S - 1) / 16 : 0;
   const int gu_units = gu_upc ? nx * gu_upc + 1 : 0;
   const int N3u = (Hm == 128 && gu_units >= 1 && gu_units <= 13) ? 32 * gu_units : 0;  // <= 416 columns (rollout_tc2.cu kMaxN3)
   m->N3u = N3u;
-  size_t o_m2w3u = A.add((size_t)2 * (N3u ? N3u : 16) * Hm / 2), o_m2cu = A.add(N3u ? N3u : 16);
+  size_t o_m2w3 = A.add((size_t)2 * (N3u ? N3u : 16) * Hm / 2), o_m2b3 = A.add(N3u ? N3u : 16);
 
   for (int i = 0; i < G3 * gin; ++i) put(o_w_ih0, i, d->gru_w_ih_l0[i]);
   for (int i = 0; i < G3; ++i) {
@@ -338,39 +337,28 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
     for (int i = 0; i < 2; ++i) put(o_enc2c, nlc::kE2Bout + i, d->enc_out_b[i]);
   }
 
-  if (N3t <= 416 && Hm == 128) {  // rollout_tc2.cu operands: -2 log2(e) folded
+  if (N3u) {  // rollout_tc2.cu operands: -2 log2(e) folded
     const double cN = -2.0 * 1.4426950408889634;
     std::vector<double> w2s((size_t)Hm * Hm);
     for (size_t i = 0; i < w2s.size(); ++i) w2s[i] = cN * d->mlp_w2[i];
     uint16_t* w2i = reinterpret_cast<uint16_t*>(A.data.data() + o_m2w2);
     nlc::tc_pack_weight_split(w2s.data(), Hm, Hm, w2i, w2i + (size_t)Hm * Hm);
-    std::vector<double> w3p((size_t)N3t * Hm, 0.0);
-    for (int c = 0; c < nx; ++c)
-      for (int k = 0; k < S; ++k)
-        for (int part = 0; part < 2; ++part) {
-          const int src = (part * nx + c) * S + k, dst = 2 * (c * S + k) + part;
-          for (int h = 0; h < Hm; ++h) w3p[(size_t)dst * Hm + h] = cN * d->mlp_w4[(size_t)src * Hm + h];
-          put(o_m2c, 128 + dst, cN * d->mlp_b4[src]);
-        }
-    uint16_t* w3i = reinterpret_cast<uint16_t*>(A.data.data() + o_m2w3);
-    nlc::tc_pack_weight_split(w3p.data(), N3t, Hm, w3i, w3i + (size_t)N3t * Hm);
-    if (N3u) {  // the same rows in the group-uniform order (see ModelDev::mlp2_w3u)
-      std::vector<double> w3u((size_t)N3u * Hm, 0.0);
-      const int kJ = nx * gu_upc;
-      for (int col = 0; col < N3u; ++col) {
-        const int j = col / 32, cgp = (col % 32) / 8, i = (col % 8) / 2, part = col % 2;
-        int c, k;
-        if (j < kJ) { c = j / gu_upc; k = 16 * (j % gu_upc) + cgp + 4 * i; }
-        else { c = cgp + 4 * i; k = S - 1; }
-        if (c >= nx) continue;  // no such channel: zero weights and bias (its Fourier weight is zeroed in the kernel too)
-        const int src = (part * nx + c) * S + k;
-        for (int h = 0; h < Hm; ++h) w3u[(size_t)col * Hm + h] = cN * d->mlp_w4[(size_t)src * Hm + h];
-        put(o_m2cu, col, cN * d->mlp_b4[src]);
-      }
-      uint16_t* w3ui = reinterpret_cast<uint16_t*>(A.data.data() + o_m2w3u);
-      nlc::tc_pack_weight_split(w3u.data(), N3u, Hm, w3ui, w3ui + (size_t)N3u * Hm);
+    // the third layer's rows in the group-uniform order (see ModelDev::mlp2_w3)
+    std::vector<double> w3u((size_t)N3u * Hm, 0.0);
+    const int kJ = nx * gu_upc;
+    for (int col = 0; col < N3u; ++col) {
+      const int j = col / 32, cgp = (col % 32) / 8, i = (col % 8) / 2, part = col % 2;
+      int c, k;
+      if (j < kJ) { c = j / gu_upc; k = 16 * (j % gu_upc) + cgp + 4 * i; }
+      else { c = cgp + 4 * i; k = S - 1; }
+      if (c >= nx) continue;  // no such channel: zero weights and bias (its Fourier weight is zeroed in the kernel too)
+      const int src = (part * nx + c) * S + k;
+      for (int h = 0; h < Hm; ++h) w3u[(size_t)col * Hm + h] = cN * d->mlp_w4[(size_t)src * Hm + h];
+      put(o_m2b3, col, cN * d->mlp_b4[src]);
     }
-    for (int n = 0; n < Hm; ++n) put(o_m2c, n, cN * d->mlp_b2[n]);
+    uint16_t* w3ui = reinterpret_cast<uint16_t*>(A.data.data() + o_m2w3);
+    nlc::tc_pack_weight_split(w3u.data(), N3u, Hm, w3ui, w3ui + (size_t)N3u * Hm);
+    for (int n = 0; n < Hm; ++n) put(o_m2b2, n, cN * d->mlp_b2[n]);
   }
 
   m->h.w0 = new double[(size_t)Hm * in0];
@@ -392,8 +380,8 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
   m->d.w_hh0_t = base + o_hh0; m->d.w_ih1_t = base + o_ih1; m->d.w_hh1_t = base + o_hh1;
   m->d.b_ih1 = base + o_b_ih1; m->d.b_hh1 = base + o_b_hh1; m->d.w_out = base + o_wout; m->d.b_out = base + o_bout;
   m->d.enc2_w = base + o_enc2w; m->d.enc2_c = base + o_enc2c; m->d.enc2_x = base + o_enc2x;
-  m->d.mlp2_w1 = base + o_m2w1; m->d.mlp2_w2 = base + o_m2w2; m->d.mlp2_w3 = base + o_m2w3; m->d.mlp2_c = base + o_m2c;
-  m->d.mlp2_w3u = base + o_m2w3u; m->d.mlp2_cu = base + o_m2cu;
+  m->d.mlp2_w1 = base + o_m2w1; m->d.mlp2_w2 = base + o_m2w2; m->d.mlp2_b2 = base + o_m2b2;
+  m->d.mlp2_w3 = base + o_m2w3; m->d.mlp2_b3 = base + o_m2b3;
   m->d.w1_full_t = base + o_w1full; m->d.b1_raw = base + o_b1raw; m->d.w1x_t = base + o_w1x; m->d.b1_fold = base + o_b1f;
   m->d.w2_t = base + o_w2; m->d.b2 = base + o_b2; m->d.w3_t = base + o_w3; m->d.b3 = base + o_b3;
   m->d.ilt_phase = base + o_phase; m->d.ilt_weight = base + o_weight;

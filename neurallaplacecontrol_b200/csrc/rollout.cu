@@ -278,11 +278,18 @@ int launch_rollout_tc2(nlc_model_s* m, const nlc_rollout_opts* o, const float* s
                        const float* row_tn = nullptr);
 bool rollout_has_tensor_core_form(const nlc_model_s* m);
 
-// planner.cu: can the rollout of this plan run BESIDE its history encoder (one-tile tcgen05 form on ceil(K/128) SMs, polling the
-// encoder's per-step readiness counters)?
+// NLC_ROLLOUT_TILES=1 or 3 forces the tensor-core rollout's form (1: one tile per CTA, 3: ping-pong) - the parity tests run
+// both; anything else leaves the choice to the plan size.  Read at every call.  A forced form also keeps the planner's plain
+// sequence (no rollout beside the encoder).
+static int forced_rollout_form() {
+  const char* f = getenv("NLC_ROLLOUT_TILES");
+  return (f && (f[0] == '1' || f[0] == '3')) ? f[0] - '0' : 0;
+}
+
+// planner.cu: can the rollout of this plan run BESIDE its history encoder (the one-tile tcgen05 form on ceil(K/128) SMs or the
+// ping-pong form on fewer, polling the encoder's per-step readiness counters)?
 bool rollout_can_overlap(const nlc_model_s* m, int K, int T, int math_mode) {
   static const bool off = [] { const char* e = getenv("NLC_NO_OVERLAP"); return e && e[0] == '1'; }();
-  const char* f = getenv("NLC_ROLLOUT_TILES");  // a forced kernel form (parity tests) keeps the plain sequence
   // up to 74 tiles the encoder keeps at least half the SMs for the whole step; beyond, the planner runs the first part of the
   // encoder alone and the rest beside the rollout (planner.cu) - worth it while the rollout leaves the encoder >= 8 SMs.
   // Ping-pong plans of two passes per CTA (up to 560 tiles; config 4 on one GPU: 512 tiles = 128 CTAs x 2 passes, 20 SMs to
@@ -290,7 +297,7 @@ bool rollout_can_overlap(const nlc_model_s* m, int K, int T, int math_mode) {
   // rollout: the last pass starts ~T steps after the fork, which leaves the encoder time for those steps.
   const int n_tiles = (K + 127) / 128;
   const bool pp_form = 2 * m->nx * m->S <= 256;  // shapes with a ping-pong instantiation (rollout_tc2.cu launch_one)
-  return !off && !(f && f[0]) && math_mode != NLC_MATH_FP32 && rollout_has_tensor_core_form(m) && T >= 2 &&
+  return !off && !forced_rollout_form() && math_mode != NLC_MATH_FP32 && rollout_has_tensor_core_form(m) && T >= 2 &&
          (pp_form ? (n_tiles <= 140 || (pp_overlap_iters(n_tiles) <= 2 && pp_overlap_grid(n_tiles) <= 140)) : n_tiles <= 140);
 }
 // The overlapped rollout's form: one tile per CTA on n_tiles SMs (9.5 us per step), or - from 89 tiles - the ping-pong form on
@@ -317,11 +324,9 @@ static int launch_rollout(nlc_model_s* m, const nlc_rollout_opts* o, const float
                           float* delta_out, int math_mode, cudaStream_t stream) {
   if (math_mode != NLC_MATH_FP32 && rollout_has_tensor_core_form(m)) {
     // rollout_tc2.cu: beyond one wave of 128-sample tiles the ping-pong form (two tiles per CTA, all 16 warps alternating
-    // between them: form 3), below that one tile on all 16 warps (form 1: the step latency is then all that matters).
-    // NLC_ROLLOUT_TILES=1|2|3 forces a form (2 = two free-running 8-warp groups, the ping-pong form's predecessor);
-    // read at every call: the parity tests run all three.
-    const char* f = getenv("NLC_ROLLOUT_TILES");
-    const int tiles = (f && (f[0] == '1' || f[0] == '2' || f[0] == '3')) ? f[0] - '0' : ((K + 127) / 128 > 148 ? 3 : 1);
+    // between them: form 3), below that one tile on all 16 warps (form 1: the step latency is then all that matters)
+    const int forced = forced_rollout_form();
+    const int tiles = forced ? forced : ((K + 127) / 128 > 148 ? 3 : 1);
     int rc = launch_rollout_tc2(m, o, state, sps, p, hist, pert_cost, K, T, B, nu, cost, states, delta_out,
                                 math_mode == NLC_MATH_TC_SPLIT3, tiles, stream);
     if (rc != NLC_ERR_UNSUPPORTED) return rc;

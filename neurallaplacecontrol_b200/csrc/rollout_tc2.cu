@@ -1,30 +1,24 @@
 // Stages 2+3 for the Neural Laplace dynamics, representation MLP on the 5th-generation tensor cores
-// (rollout.cu is the fp32 CUDA-core anchor).  Three forms of one recurrence, chosen by plan size in rollout.cu:
-//   rollout_pp_kernel            "ping-pong": two 128-sample tiles per CTA, all 16 epilogue warps on one tile's phase at a
-//                                time + a dedicated MMA warp - plans beyond one wave of tiles (documented at the kernel)
-//   rollout_tc2_kernel<kTiles=1> one tile per CTA on all 16 warps - plans within one wave: the step latency is what counts
-//   rollout_tc2_kernel<kTiles=2> two free-running 8-warp groups - the ping-pong form's predecessor, kept for comparison
-//                                (NLC_ROLLOUT_TILES=2) and as the second opinion of the parity suite
+// (rollout.cu is the fp32 CUDA-core anchor).  Two forms of one recurrence, chosen by plan size in rollout.cu:
+//   rollout_pp_kernel   "ping-pong": two 128-sample tiles per CTA, all 16 epilogue warps on one tile's phase at a time + a
+//                       dedicated MMA warp - plans beyond one wave of tiles (documented at the kernel)
+//   rollout_tc2_kernel  one tile per CTA on all 16 warps - plans within one wave, where the step latency is what counts, and
+//                       every plan of the shapes whose W3 does not fit shared memory (streamed, see the kernel)
 //
 // Same recurrence as rollout.cu: state <- state + ILT(MLP([s | obs_n | p_action])), cost += running_cost, whole horizon in
 // one launch, state in registers.  The recurrence is a strict chain per sample (L1 -> L2 -> L3 -> ILT -> next step), so
-// inside ONE tile the tensor pipe and the CUDA cores can only alternate; the first form measured 22.7 k clocks per step
-// = MUFU time + issue time + MMA time, nothing overlapping.  In the two-group form every CTA runs TWO independent tiles
-// ("groups" of 8 warps = 128 samples each) that share the weight images in shared memory and otherwise never synchronise
-// with each other: one group's MMAs and barrier round trips run under the other group's epilogues.  (Holding the two groups
-// exactly half a step apart with named barriers was tried: 29.5 k instead of 31.3 k clocks per step in the trace, but
-// slower end to end - tools/trace_rollout.py shows long transients with every phase stretched - so they run free.)
+// inside ONE tile the tensor pipe and the CUDA cores can only alternate: the one-tile form's first version measured 22.7 k
+// clocks per step = MUFU time + issue time + MMA time, nothing overlapping.  It overlaps what it can by splitting products
+// (kSplitK, kSplitD below); beyond one wave the ping-pong form covers each tile's products with the other tile's epilogues.
 //
-//   per step and group      A1 = [obs_n | p_action | 1] as a K = 16 operand (TMEM)          (one thread per sample)
+//   per step                A1 = [obs_n | p_action | 1] as a K = 16 operand (TMEM)          (one thread per sample)
 //     M1  D = A1 W1^T       N = 128, K = 16   the first layer WITH its folded bias on the tensor cores
 //     E1  tanh -> A         hidden activations re-written as the fp16 hi/lo A operand in TMEM (tcgen05.st)
 //     M2  D = A W2^T        N = 128, K = 128
 //     E2  + b2, tanh -> A
-//     M3a D = A W3[:N3a]^T  the (theta, phi) pre-activations in two column halves so that A (128 columns) and D
-//     E3a                   (128 columns) of BOTH groups fit the 512 TMEM columns
-//     M3b / E3b             second half (skipped when 2 nx S <= 128)
-//     E3: sphere -> complex map, Fourier weights, fixed-order sum over the terms; the two column groups of a sample
-//     exchange partial sums through shared memory; residual add; running cost (overlapped with M3a)
+//     M3  D = A W3^T        the (theta, phi) pre-activations, in the group-uniform column order (l3_units_gu)
+//     E3: sphere -> complex map, Fourier weights, fixed-order sum over the terms; the four column groups of a sample
+//     exchange partial sums through shared memory; residual add; running cost (overlapped with M3)
 //
 //   -2 log2(e) is folded into all three layers on the host (model.cu): tanh(x) = 2 / (1 + 2^x') - 1 with x' = -2 log2e x,
 //   the reciprocals are Newton iterations on the FMA pipe in packed fp32x2 (f32x2.cuh); per (channel, term) pair the
@@ -32,11 +26,11 @@
 //   NLC_MATH_TC_SPLIT3: operands split hi+lo in fp16, D += A_hi B_hi + A_lo B_hi + A_hi B_lo (fp32-class);
 //   NLC_MATH_TC_FP16  : single pass, tanh.approx (the stated looser bound).
 //
-//   Samples are dealt to the 2 x gridDim groups in contiguous ranges (multiples of 32 rows), each walked in tiles of up
+//   One-tile form: samples are dealt to the CTAs in contiguous ranges (multiples of 32 rows), each walked in tiles of up
 //   to 128 rows: a plan that is not a whole number of waves ends on partially filled tiles instead of an idle wave.
-//   Threads (two-group form): group g = warps 8g .. 8g+7; warp w of a group owns TMEM lanes 32 (w & 3).. (its 32 samples)
-//   and column half w >> 2.  After a group barrier its first warp issues the group's MMAs under elect.sync: the group waits
-//   for that product anyway, so the issuing thread being held by the MMA queue costs nothing (unlike in the encoder).
+//   Warp w owns TMEM lanes 32 (w & 3).. (its 32 samples) and column group w >> 2.  After a CTA barrier warp 0 issues the
+//   MMAs under elect.sync: the tile waits for that product anyway, so the issuing thread being held by the MMA queue costs
+//   nothing (unlike in the encoder).
 #include <cuda_fp16.h>
 #include <stdlib.h>
 
@@ -57,7 +51,7 @@ constexpr int kRows = 128, kH = 128;
 constexpr uint32_t kLbo = 128, kSbo = (kH / 8) * 128;  // K = 128 operand images
 constexpr uint32_t kSbo16 = (16 / 8) * 128;             // K = 16 (first layer)
 constexpr uint32_t kColA = 0, kColD = 128, kGroupCols = 256, kTmemCols = 512;
-constexpr int kGroupThreads = 256, kThreads = 2 * kGroupThreads;
+constexpr int kThreads = 512;
 
 struct Args {
   ModelDev m;
@@ -107,25 +101,23 @@ __device__ __forceinline__ void wait_windows_ready(const Args& a, int t, int lan
 // W1 (2 x 4 KB), W2 (2 x 32 KB), W3 (2 x N3t x 256 B) -> shared memory; bulk copies of at most 32 KB each.  with_w3 = false:
 // W3 is streamed half by half instead (load_w3_rows)
 __device__ __forceinline__ void load_weight_images(const ModelDev& m, unsigned char* w1_img, unsigned char* w2_img, unsigned char* w3_img,
-                                                   int N3t, uint64_t* bar, bool with_w3 = true, const void* w3_src = nullptr) {
-  if (!w3_src) w3_src = m.mlp2_w3;
+                                                   int N3t, uint64_t* bar, bool with_w3 = true) {
   const uint32_t b1 = 2 * kH * 16 * 2, b2 = 2 * kH * kH * 2, b3 = with_w3 ? 2u * (uint32_t)N3t * kH * 2 : 0u;
   mbar_expect_tx(bar, b1 + b2 + b3);
   bulk_g2s(w1_img, m.mlp2_w1, b1, bar);
   for (uint32_t o = 0; o < b2; o += 32768) bulk_g2s(w2_img + o, static_cast<const unsigned char*>(m.mlp2_w2) + o, 32768, bar);
   for (uint32_t o = 0; o < b3; o += 32768) {
     const uint32_t n = b3 - o < 32768 ? b3 - o : 32768;
-    bulk_g2s(w3_img + o, static_cast<const unsigned char*>(w3_src) + o, n, bar);
+    bulk_g2s(w3_img + o, static_cast<const unsigned char*>(m.mlp2_w3) + o, n, bar);
   }
 }
 // Rows [row0, row0 + nrows) of W3 (output columns of the third layer; multiples of 8, so whole 8-row groups of the K-major
-// image = contiguous bytes), hi and lo image, into a buffer that holds n_buf rows of each.  Issued by one thread.  (The
-// streamed form is a one-tile form: the group-uniform image.)
+// image = contiguous bytes), hi and lo image, into a buffer that holds n_buf rows of each.  Issued by one thread.
 __device__ __forceinline__ void load_w3_rows(const ModelDev& m, unsigned char* w3_buf, int row0, int nrows, int N3t, int n_buf, uint64_t* bar) {
   const uint32_t bytes = (uint32_t)nrows * kH * 2;
   mbar_expect_tx(bar, 2 * bytes);
   for (int img = 0; img < 2; ++img) {
-    const unsigned char* src = static_cast<const unsigned char*>(m.mlp2_w3u) + ((size_t)img * N3t + row0) * kH * 2;
+    const unsigned char* src = static_cast<const unsigned char*>(m.mlp2_w3) + ((size_t)img * N3t + row0) * kH * 2;
     unsigned char* dst = w3_buf + (size_t)img * n_buf * kH * 2;
     for (uint32_t o = 0; o < bytes; o += 32768) bulk_g2s(dst + o, src + o, bytes - o < 32768 ? bytes - o : 32768, bar);
   }
@@ -139,7 +131,7 @@ struct SmemTail {  // after the weight images
   alignas(16) float b3[kMaxN3];
   float phase[kMaxS], weight[kMaxS];
   float smean[kMaxNx], sinv[kMaxNx];
-  alignas(16) float exch[4][kRows * kMaxNx];     // [tile * column groups + column group] partial ILT sums
+  alignas(16) float exch[4][kRows * kMaxNx];     // [column group] partial ILT sums
   alignas(8) uint64_t done[2];
   uint32_t tmem_base;
 };
@@ -337,63 +329,8 @@ __device__ __forceinline__ void l3_two_pairs(f2_t th, f2_t ph, float phase0, flo
   t1 = (w1 * rad1) * mufu_cos(fmaf(3.14159265358979f, y1, phase1));
 }
 
-// L3 epilogue of one 16-column chunk (8 pairs); kChunk = chunk index in the full N3t column space, kCol0 = first chunk
-// of the half that currently sits in the D region
-// kPerRow: the sample has its own prediction time - phase_k = k pi t/T = k (pi/2 - rd) reduced to (-pi, pi] with the quarter turns
-// exact, weight_k = rs (k == 0 ? 1/2 : 1), rd = pi eps / T and rs = exp(gamma t) / T of that sample (oracle/ilt.py)
-template <int NX, int S, int kChunk, int kCol0, bool kAccurate, int kRcp, bool kPerRow = false>
-__device__ __forceinline__ void l3_chunk(uint32_t tD, const float* __restrict__ b3, const float* __restrict__ phase,
-                                         const float* __restrict__ weight, float (&delta)[NX], float rd = 0.0f, float rs = 0.0f) {
-  f2_t v[8];
-  ldtm16p(tD + 16 * (kChunk - kCol0), v);
-  tmem_ld_wait();
-  f2_t bb[8];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const float4 t = *reinterpret_cast<const float4*>(b3 + 16 * kChunk + 4 * i);
-    bb[2 * i] = pk2(t.x, t.y);
-    bb[2 * i + 1] = pk2(t.z, t.w);
-  }
-#pragma unroll
-  for (int i = 0; i < 8; i += 2) {
-    constexpr int dummy = 0; (void)dummy;
-    const int p0 = 8 * kChunk + i, p1 = p0 + 1;
-    if (p0 < NX * S) {
-      // v[i] = (theta', phi') of pair p0, v[i+1] of pair p1: regroup into (theta0, theta1), (phi0, phi1)
-      const f2_t s0 = add2(v[i], bb[i]), s1 = add2(v[i + 1], bb[i + 1]);
-      float th0, ph0, th1, ph1;
-      upk2(s0, th0, ph0);
-      upk2(s1, th1, ph1);
-      const int ch0 = p0 / S, k0 = p0 - ch0 * S;
-      const int ch1 = (p1 < NX * S) ? p1 / S : ch0, k1 = (p1 < NX * S) ? p1 - ch1 * S : k0;
-      float t0, t1;
-      if (kPerRow) {
-        const float q0 = (k0 & 3) == 0 ? 0.0f : ((k0 & 3) == 1 ? 1.57079632679489662f : ((k0 & 3) == 2 ? 3.14159265358979f : -1.57079632679489662f));
-        const float q1 = (k1 & 3) == 0 ? 0.0f : ((k1 & 3) == 1 ? 1.57079632679489662f : ((k1 & 3) == 2 ? 3.14159265358979f : -1.57079632679489662f));
-        l3_two_pairs<kAccurate, kRcp>(pk2(th0, th1), pk2(ph0, ph1), fmaf(-(float)k0, rd, q0), fmaf(-(float)k1, rd, q1),
-                                      k0 == 0 ? 0.5f * rs : rs, k1 == 0 ? 0.5f * rs : rs, t0, t1);
-      } else {
-        l3_two_pairs<kAccurate, kRcp>(pk2(th0, th1), pk2(ph0, ph1), phase[k0], phase[k1], weight[k0], weight[k1], t0, t1);
-      }
-      delta[ch0] += t0;
-      if (p1 < NX * S) delta[ch1] += t1;
-    }
-  }
-}
-// chunks kChunk, kChunk + kStride, ... < kEnd (the column groups of a sample take chunks round-robin)
-template <int NX, int S, int kChunk, int kEnd, int kCol0, bool kAccurate, int kRcp, int kStride, bool kPerRow = false>
-struct L3Loop {
-  static __device__ __forceinline__ void run(uint32_t tD, const float* b3, const float* phase, const float* weight, float (&delta)[NX],
-                                             float rd = 0.0f, float rs = 0.0f) {
-    if constexpr (kChunk < kEnd) {
-      l3_chunk<NX, S, kChunk, kCol0, kAccurate, kRcp, kPerRow>(tD, b3, phase, weight, delta, rd, rs);
-      L3Loop<NX, S, kChunk + kStride, kEnd, kCol0, kAccurate, kRcp, kStride, kPerRow>::run(tD, b3, phase, weight, delta, rd, rs);
-    }
-  }
-};
-
-// Ping-pong and one-tile forms: a thread reads its (theta, phi) columns in UNITS of 8 columns (4 pairs), and all of its units of
-// a phase (up to four) are loaded before the first is used - one TMEM round trip per phase instead of one per chunk.
+// A thread reads its (theta, phi) columns in UNITS of 8 columns (4 pairs), and all of its units of a phase (up to four) are
+// loaded before the first is used - one TMEM round trip per phase instead of one per 16-column chunk.
 __device__ __forceinline__ void ldtm8q(uint32_t taddr, f2_t (&v)[4]) {
   uint32_t r[8];
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
@@ -403,14 +340,15 @@ __device__ __forceinline__ void ldtm8q(uint32_t taddr, f2_t (&v)[4]) {
 #pragma unroll
   for (int i = 0; i < 4; ++i) v[i] = pk2u(r[2 * i], r[2 * i + 1]);
 }
-// GROUP-UNIFORM units (ping-pong form, ModelDev::mlp2_w3u): unit j = 32 columns, 8 per column group, so that the four column
-// groups of a sample run the SAME instructions on different addresses - the four warps of an SM sub-partition are the four
-// column groups of one row quarter, and with a code variant per group each sub-partition walked four copies of the unrolled
+// GROUP-UNIFORM units (ModelDev::mlp2_w3): unit j = 32 columns, 8 per column group, so that the four column groups of a
+// sample run the SAME instructions on different addresses - the four warps of an SM sub-partition are the four column
+// groups of one row quarter, and with a code variant per group each sub-partition walked four copies of the unrolled
 // epilogue (47 KB; a tenth of the warp stalls were instruction fetches).  Regular unit j < NX upc (upc = (S-1)/16): channel
 // j / upc (compile time), terms 16 (j % upc) + cg + 4 i; the last unit holds the terms k = S-1 of channels cg and cg + 4.
 // tDcg, b3cg, phasecg, weightcg: the D region / bias / Fourier tables offset by this thread's column group (8 cg, 8 cg, cg, cg).
-// kPerRow: the sample's own prediction time (see l3_chunk) - k & 3 = cg for the regular units (their terms are cg + a multiple
-// of 4), 0 for the last (S - 1 is a multiple of 16).
+// kPerRow: the sample has its own prediction time - phase_k = k pi t/T = k (pi/2 - rd) reduced to (-pi, pi] with the quarter
+// turns exact, weight_k = rs (k == 0 ? 1/2 : 1), rd = pi eps / T and rs = exp(gamma t) / T of that sample (oracle/ilt.py);
+// k & 3 = cg for the regular units (their terms are cg + a multiple of 4), 0 for the last (S - 1 is a multiple of 16).
 template <int NX, int S, int kJ0, int kJ1, bool kAccurate, int kRcp, bool kPerRow = false>
 __device__ __forceinline__ void l3_units_gu(uint32_t tDcg, const float* __restrict__ b3cg, const float* __restrict__ phasecg,
                                             const float* __restrict__ weightcg, int cg, float (&delta)[NX], float rd = 0.0f,
@@ -474,42 +412,28 @@ struct PPShape {  // columns of the group-uniform W3 image: model.cu packs N3u =
   static constexpr int kUnits = NX * ((S - 1) / 16) + 1, N3u = 32 * kUnits;
 };
 
-template <int NX, int S, bool kSplit3, int kRcp, int kTiles, bool kPerRow = false>
+template <int NX, int S, bool kSplit3, int kRcp, bool kPerRow = false>
 __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
-  static_assert(!kPerRow || kTiles == 1, "per-sample prediction times: one-tile form");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int Lp = NX + 2;
-  // kGU (one tile): the (theta, phi) columns in the GROUP-UNIFORM order (l3_units_gu: one L3 epilogue code for all four column
-  // groups), counted in "chunks" of 16 columns like the natural order of the two-tile form - a unit is two chunks
-  constexpr bool kGU = kTiles == 1;
-  constexpr int kUnits = PPShape<NX, S>::kUnits;
-  constexpr int N3t = kGU ? PPShape<NX, S>::N3u : (2 * NX * S + 15) / 16 * 16;
-  constexpr int kChunks = N3t / 16;
-  // kTiles == 2: two 128-sample tiles per CTA, 8 warps and 256 TMEM columns each, two column groups per tile, L3 in two
-  // column halves.  kTiles == 1 (plans of at most one wave of tiles, where the step latency is all that matters): one
-  // tile, all 16 warps on it in four column groups, L3 in one piece (A 128 + D up to 256 columns), (theta, phi) columns in
-  // the group-uniform order.
-  constexpr int kCG = 4 / kTiles;                                   // column groups per tile
-  constexpr int kGroupWarps = 4 * kCG, kGroupT = 32 * kGroupWarps;  // warps / threads per tile
-  constexpr int kColsPerThread = kH / kCG, kC16 = kColsPerThread / 16;
-  // kStream (one tile, more than 256 (theta, phi) columns: S = 33 with nx >= 5, the reference class default w_nl.py:73): L3 in
+  // the (theta, phi) columns in the GROUP-UNIFORM order (l3_units_gu: one L3 epilogue code for all four column groups)
+  constexpr int kUnits = PPShape<NX, S>::kUnits, N3t = PPShape<NX, S>::N3u;
+  // One tile, all 16 warps on it in four column groups of 32 hidden units, L3 in one piece (A 128 + D up to 256 columns).
+  // kStream (more than 256 (theta, phi) columns: S = 33 with nx >= 5, the reference class default w_nl.py:73): L3 in
   // two column halves of at most 256 columns, and W3 - which no longer fits shared memory next to W1 and W2 - streamed: one
   // buffer of N3a rows, reloaded by TMA bulk copies (L2-resident source) as soon as the product that read it has completed,
   // each load hidden under the epilogue that follows.
-  constexpr bool kStream = kTiles == 1 && N3t > 256;
-  constexpr int kUnitsA = kStream ? (kUnits + 1) / 2 : kUnits;        // (kGU) units in the first column half
-  constexpr int kChunksA = kGU ? 2 * kUnitsA : (N3t <= 128 ? kChunks : (kChunks + 1) / 2);  // chunks in the first column half
-  constexpr int N3a = 16 * kChunksA, N3b = N3t - N3a;
+  constexpr bool kStream = N3t > 256;
+  constexpr int kUnitsA = kStream ? (kUnits + 1) / 2 : kUnits;        // units in the first column half
+  constexpr int N3a = 32 * kUnitsA, N3b = N3t - N3a;
   constexpr int N3buf = kStream ? N3a : N3t;                          // rows of W3 resident at a time
-  // kSplitD (one tile, resident W3): the L3 product is issued as TWO products into disjoint column ranges of the accumulator,
+  // kSplitD (resident W3): the L3 product is issued as TWO products into disjoint column ranges of the accumulator,
   // each with its own completion barrier, so the epilogue of the first half's columns runs while the second half is still
   // on the tensor pipe - in this form nothing else covers the products (strict chain per sample)
-  constexpr bool kSplitD = kTiles == 1 && !kStream && kChunks >= 8;
-  constexpr bool kSplitK = kTiles == 1;                               // M2 / M3 issued in two K-halves (hidden_split)
-  constexpr int kUnitsH = kSplitD ? (kUnits + 1) / 2 : kUnits;        // (kGU) units of the first product
-  constexpr int kChunksH = kGU ? 2 * kUnitsH : kChunks;               // chunks of the first product
-  constexpr int N3h = 16 * kChunksH;
-  static_assert((kTiles == 1 ? (N3a <= 256 && N3b <= 256) : (N3a <= 128 && N3b <= 128 && N3t <= 256)) && N3t <= kMaxN3 && Lp + 1 <= 16, "tile shape");
+  constexpr bool kSplitD = !kStream && N3t >= 128;
+  constexpr int kUnitsH = kSplitD ? (kUnits + 1) / 2 : kUnits;        // units of the first product
+  constexpr int N3h = 32 * kUnitsH;
+  static_assert(N3a <= 256 && N3b <= 256 && N3t <= kMaxN3 && Lp + 1 <= 16, "tile shape");
   unsigned char* w1_img = smem_raw;                                   // [hi | lo] 128 x 16 halves = 4 KB each
   unsigned char* w2_img = w1_img + 2 * kH * 16 * 2;                   // [hi | lo] 32 KB each
   unsigned char* w3_img = w2_img + 2 * kH * kH * 2;                   // [hi | lo] N3buf * 256 B each
@@ -517,17 +441,17 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
   {
-    // weight images by TMA bulk copies (one issuing thread, counted on bar_w): only the MMA-issuing warps wait for them, so the
+    // weight images by TMA bulk copies (one issuing thread, counted on bar_w): only the MMA-issuing warp waits for them, so the
     // load runs under the TMEM allocation and the first operand's preparation - prologue latency is what small plans pay for
     if (warp == 0 && elect_one()) {  // (elect.sync, not tid == 0: the copies' operands then stay in uniform registers)
       mbar_init(&s.bar_w, 1);
       mbar_init(&s.bar_w3, 1);
       mbar_fence_init();
-      load_weight_images(a.m, w1_img, w2_img, w3_img, N3t, &s.bar_w, !kStream, kGU ? a.m.mlp2_w3u : a.m.mlp2_w3);
+      load_weight_images(a.m, w1_img, w2_img, w3_img, N3t, &s.bar_w, !kStream);
       if (kStream) load_w3_rows(a.m, w3_img, 0, N3a, N3t, N3buf, &s.bar_w3);
     }
-    for (int i = tid; i < kH; i += kThreads) s.b2[i] = a.m.mlp2_c[i];
-    for (int i = tid; i < kMaxN3; i += kThreads) s.b3[i] = i < N3t ? (kGU ? a.m.mlp2_cu[i] : a.m.mlp2_c[128 + i]) : 0.0f;
+    for (int i = tid; i < kH; i += kThreads) s.b2[i] = a.m.mlp2_b2[i];
+    for (int i = tid; i < kMaxN3; i += kThreads) s.b3[i] = i < N3t ? a.m.mlp2_b3[i] : 0.0f;
     for (int i = tid; i < S; i += kThreads) { s.phase[i] = a.m.ilt_phase[i]; s.weight[i] = a.m.ilt_weight[i]; }
     if (tid < NX) { s.smean[tid] = a.m.state_mean[tid]; s.sinv[tid] = a.m.state_inv_std[tid]; }
     if (tid == 0) {
@@ -542,77 +466,64 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
   fence_after_sync();
   const uint32_t tmem = s.tmem_base;
 
-  // samples of this group: a contiguous range, a multiple of 32 rows long (except at the very end of the plan)
-  const int g = warp / kGroupWarps;
-  const int n_slots = kTiles * gridDim.x, slot = kTiles * blockIdx.x + g;
+  // samples of this CTA: a contiguous range, a multiple of 32 rows long (except at the very end of the plan)
+  const int n_slots = gridDim.x, slot = blockIdx.x;
   const int per_slot = ((a.K + n_slots - 1) / n_slots + 31) / 32 * 32;
   const long long r_begin_ll = (long long)slot * per_slot;
   const int r_begin = (int)(r_begin_ll < a.K ? r_begin_ll : a.K);
   const int r_end = (r_begin + per_slot < a.K) ? r_begin + per_slot : a.K;
-  const uint32_t tg = tmem + kGroupCols * g;
-  uint64_t* done = &s.done[g];
+  uint64_t* done = &s.done[0];
 
   {
-    // =====================================  epilogue warps of group g  =====================================
-    const int wl = warp % kGroupWarps, q = wl & 3, cg = wl >> 2;
+    // =====================================  the 16 epilogue warps  =====================================
+    const int q = warp & 3, cg = warp >> 2;
     const int row = 32 * q + lane;
-    const uint32_t tlane = tg + ((uint32_t)(32 * q) << 16);
+    const uint32_t tlane = tmem + ((uint32_t)(32 * q) << 16);
     const uint32_t tA = tlane + kColA, tD = tlane + kColD;
     const uint32_t w1_hi = smem_u32(w1_img), w1_lo = w1_hi + kH * 16 * 2;
     const uint32_t w2_hi = smem_u32(w2_img), w2_lo = w2_hi + kH * kH * 2;
     const uint32_t w3_hi = smem_u32(w3_img), w3_lo = w3_hi + (uint32_t)N3buf * kH * 2;
-    const uint32_t w3b_off = kStream ? 0u : (uint32_t)(N3a / 8) * kSbo;
     uint32_t n = 0, n_w3 = 0, n_b = 0;  // products waited for; W3 halves waited for (issuing warp only); second L3 halves (kSplitD)
     bool active_w = false;              // (hidden_split) this warp has live samples in the current tile
     int tstep = 0;
     auto mark = [&](int ev) {
       if (a.trace && blockIdx.x == 0 && lane == 0 && tstep < 104) a.trace[(tstep * 16 + warp) * 8 + ev] = clock64();
     };
-    // hand-off to the tensor pipe: every warp of the group has finished its TMEM stores / loads (group barrier), then
-    // one thread issues product `ev` of the step.  The group waits for that product anyway (strict chain per sample),
-    // so the issuing warp being held by the MMA queue costs nothing; the other group keeps the CUDA cores busy.
-    if (wl == 0) mbar_wait(&s.bar_w, 0);  // the issuing warp: weight images landed
+    // hand-off to the tensor pipe: every warp has finished its TMEM stores / loads (CTA barrier), then one thread issues
+    // product `ev` of the step (0: M1, 3: the second column half of M3 with W3 streamed).  The tile waits for that product
+    // anyway (strict chain per sample), so the issuing warp being held by the MMA queue costs nothing.
+    if (warp == 0) mbar_wait(&s.bar_w, 0);  // the issuing warp: weight images landed
     auto issue = [&](int ev) {
       tmem_st_wait();
       fence_before_sync();
-      asm volatile("bar.sync %0, %1;" ::"r"(1 + g), "n"(kGroupT) : "memory");
-      if (kStream && wl == 0 && ev >= 2) { mbar_wait(&s.bar_w3, n_w3 & 1); ++n_w3; }  // this half of W3 has landed
-      if (wl == 0 && elect_one()) {
+      asm volatile("bar.sync %0, %1;" ::"r"(1), "n"(kThreads) : "memory");
+      if (kStream && warp == 0 && ev == 3) { mbar_wait(&s.bar_w3, n_w3 & 1); ++n_w3; }  // this half of W3 has landed
+      if (warp == 0 && elect_one()) {
         fence_after_sync();
-        if (ev == 0) issue_gemm_ts<kSplit3>(tg + kColD, tg + kColA, w1_hi, w1_lo, kH, 1, kSbo16);
-        else if (ev == 1) issue_gemm_ts<kSplit3>(tg + kColD, tg + kColA, w2_hi, w2_lo, kH, kH / 16, kSbo);
-        else if (ev == 2 && kSplitD) {
-          issue_gemm_ts<kSplit3>(tg + kColD, tg + kColA, w3_hi, w3_lo, N3h, kH / 16, kSbo);
-          mma_commit(done);  // first half: the epilogue starts on it while the second half computes
-          issue_gemm_ts<kSplit3>(tg + kColD + N3h, tg + kColA, w3_hi + (uint32_t)(N3h / 8) * kSbo, w3_lo + (uint32_t)(N3h / 8) * kSbo,
-                                 N3t - N3h, kH / 16, kSbo);
-          mma_commit(&s.done[1]);
-        }
-        else if (ev == 2) issue_gemm_ts<kSplit3>(tg + kColD, tg + kColA, w3_hi, w3_lo, N3a, kH / 16, kSbo);
-        else issue_gemm_ts<kSplit3>(tg + kColD, tg + kColA, w3_hi + w3b_off, w3_lo + w3b_off, N3b, kH / 16, kSbo);
-        if (!(ev == 2 && kSplitD)) mma_commit(done);
+        if (ev == 0) issue_gemm_ts<kSplit3>(tmem + kColD, tmem + kColA, w1_hi, w1_lo, kH, 1, kSbo16);
+        else issue_gemm_ts<kSplit3>(tmem + kColD, tmem + kColA, w3_hi, w3_lo, N3b, kH / 16, kSbo);  // (the buffer holds that half)
+        mma_commit(done);
       }
       __syncwarp();
     };
-    // kSplitK (one tile, four column groups): products M2 and M3 in two K-halves (issue_gemm_ts_half).  half 0 = the K-steps
-    // fed by every thread's first 16 activation columns (even steps: thread columns 32 cg .. 32 cg + 15 are K-step 2 cg),
-    // half 1 = the rest and the commit(s).
+    // products M2 and M3 in two K-halves (issue_gemm_ts_half).  half 0 = the K-steps fed by every thread's first 16
+    // activation columns (even steps: thread columns 32 cg .. 32 cg + 15 are K-step 2 cg), half 1 = the rest and the commit(s).
     auto issue_k = [&](int ev, int half) {
       tmem_st_wait();
       fence_before_sync();
-      asm volatile("bar.sync %0, %1;" ::"r"(1 + g), "n"(kGroupT) : "memory");
-      if (kStream && wl == 0 && ev >= 2 && half == 0) { mbar_wait(&s.bar_w3, n_w3 & 1); ++n_w3; }  // this half of W3 has landed
-      if (wl == 0 && elect_one()) {
+      asm volatile("bar.sync %0, %1;" ::"r"(1), "n"(kThreads) : "memory");
+      if (kStream && warp == 0 && ev >= 2 && half == 0) { mbar_wait(&s.bar_w3, n_w3 & 1); ++n_w3; }  // this half of W3 has landed
+      if (warp == 0 && elect_one()) {
         fence_after_sync();
-        if (ev == 1) issue_gemm_ts_half<kSplit3>(tg + kColD, tg + kColA, w2_hi, w2_lo, kH, kH / 16, kSbo, half);
+        if (ev == 1) issue_gemm_ts_half<kSplit3>(tmem + kColD, tmem + kColA, w2_hi, w2_lo, kH, kH / 16, kSbo, half);
         else if (kSplitD) {
-          issue_gemm_ts_half<kSplit3>(tg + kColD, tg + kColA, w3_hi, w3_lo, N3h, kH / 16, kSbo, half);
+          issue_gemm_ts_half<kSplit3>(tmem + kColD, tmem + kColA, w3_hi, w3_lo, N3h, kH / 16, kSbo, half);
           if (half == 1) mma_commit(done);  // first column half: the epilogue starts on it while the second half computes
-          issue_gemm_ts_half<kSplit3>(tg + kColD + N3h, tg + kColA, w3_hi + (uint32_t)(N3h / 8) * kSbo, w3_lo + (uint32_t)(N3h / 8) * kSbo,
+          issue_gemm_ts_half<kSplit3>(tmem + kColD + N3h, tmem + kColA, w3_hi + (uint32_t)(N3h / 8) * kSbo, w3_lo + (uint32_t)(N3h / 8) * kSbo,
                                       N3t - N3h, kH / 16, kSbo, half);
           if (half == 1) mma_commit(&s.done[1]);
         } else {
-          issue_gemm_ts_half<kSplit3>(tg + kColD, tg + kColA, w3_hi, w3_lo, N3a, kH / 16, kSbo, half);
+          issue_gemm_ts_half<kSplit3>(tmem + kColD, tmem + kColA, w3_hi, w3_lo, N3a, kH / 16, kSbo, half);
         }
         if (half == 1 && !(ev == 2 && kSplitD)) mma_commit(done);
       }
@@ -622,11 +533,11 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
       mbar_wait_sleep(done, n & 1); ++n;
       fence_after_sync();
     };
-    // hidden-layer epilogue of the one-tile form with the K-split hand-off: both 16-column chunks of this thread are read
-    // BEFORE the first half of the next product may overwrite the accumulator; kBias: 0 none, 1 b2, 2 per-sample first-layer bias
+    // hidden-layer epilogue with the K-split hand-off: both 16-column chunks of this thread are read BEFORE the first half of
+    // the next product may overwrite the accumulator; bias_kind: 0 none, 1 b2, 2 per-sample first-layer bias
     auto hidden_split = [&](int ev_next, int bias_kind, int kk) {
       f2_t va[8], vb[8];
-      const int n0 = kColsPerThread * cg;
+      const int n0 = 32 * cg;
       if (active_w) {
         ldtm16p(tD + n0, va);
         ldtm16p(tD + n0 + 16, vb);
@@ -676,7 +587,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
       }
       {
         // (__ldcg: p may be written by the encoder kernel while this kernel runs - never through a stale L1 line)
-        if (kTiles == 1 && a.ready) wait_windows_ready(a, 0, lane);
+        if (a.ready) wait_windows_ready(a, 0, lane);
         const float2 pv = __ldcg(reinterpret_cast<const float2*>(a.p + ((size_t)kk * a.T) * 2));
         in[NX] = pv.x; in[NX + 1] = pv.y;
       }
@@ -691,7 +602,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
 
       for (int t = 0; t < a.T; ++t) {
         float2 pnext = make_float2(0.f, 0.f);
-        if (!(kTiles == 1 && a.ready) && t + 1 < a.T) pnext = __ldcg(reinterpret_cast<const float2*>(a.p + ((size_t)kk * a.T + t + 1) * 2));
+        if (!a.ready && t + 1 < a.T) pnext = __ldcg(reinterpret_cast<const float2*>(a.p + ((size_t)kk * a.T + t + 1) * 2));
 
         // ---------------- A1 = [in | 1 | 0..] as the K = 16 operand (one thread per sample) ----------------
         if (cg == 0 && active) {
@@ -714,70 +625,16 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
         // ---------------- E1: tanh -> A ----------------
         wait_mma();
         mark(1);
-        if constexpr (kSplitK) {
-          active_w = active;
-          hidden_split(1, kPerRow ? 2 : 0, kk);
-          mark(2);
-        } else {
-        if (active) {
-#pragma unroll
-          for (int c16 = 0; c16 < kC16; ++c16) {
-            const int n0 = kColsPerThread * cg + 16 * c16;
-            f2_t v[8];
-            ldtm16p(tD + n0, v);
-            tmem_ld_wait();
-            if (kPerRow) {  // + (-2 log2 e) x this sample's first-layer bias (the accumulator carries the folded scale)
-              const float4* bp = reinterpret_cast<const float4*>(a.row_b1 + (size_t)kk * kH + n0);
-#pragma unroll
-              for (int i = 0; i < 4; ++i) {
-                const float4 b = __ldg(bp + i);
-                const f2_t c = pk2(-2.8853900817779268f, -2.8853900817779268f);
-                v[2 * i] = fma2(pk2(b.x, b.y), c, v[2 * i]);
-                v[2 * i + 1] = fma2(pk2(b.z, b.w), c, v[2 * i + 1]);
-              }
-            }
-            tanh16_scaled<kSplit3, kRcp / 10>(v);
-            uint32_t ph[8], pl[8];
-            pack16<kSplit3>(v, ph, pl);
-            tmem_st8(tA + n0 / 2, ph);
-            if (kSplit3) tmem_st8(tA + 64 + n0 / 2, pl);
-          }
-        }
+        active_w = active;
+        hidden_split(1, kPerRow ? 2 : 0, kk);
         mark(2);
-        issue(1);
-        }
         // ---------------- E2: + b2, tanh -> A ----------------
         wait_mma();
         mark(3);
-        if constexpr (kSplitK) {
-          hidden_split(2, 1, kk);
-          mark(4);
-        } else {
-        if (active) {
-#pragma unroll
-          for (int c16 = 0; c16 < kC16; ++c16) {
-            const int n0 = kColsPerThread * cg + 16 * c16;
-            f2_t v[8];
-            ldtm16p(tD + n0, v);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              const float4 b = *reinterpret_cast<const float4*>(s.b2 + n0 + 4 * i);
-              v[2 * i] = add2(v[2 * i], pk2(b.x, b.y));
-              v[2 * i + 1] = add2(v[2 * i + 1], pk2(b.z, b.w));
-            }
-            tanh16_scaled<kSplit3, kRcp / 10>(v);
-            uint32_t ph[8], pl[8];
-            pack16<kSplit3>(v, ph, pl);
-            tmem_st8(tA + n0 / 2, ph);
-            if (kSplit3) tmem_st8(tA + 64 + n0 / 2, pl);
-          }
-        }
+        hidden_split(2, 1, kk);
         mark(4);
-        issue(2);
-        }
         // overlapped form: the next step's encoder output, polled for and loaded under the L3 product
-        if (kTiles == 1 && a.ready && t + 1 < a.T) {
+        if (a.ready && t + 1 < a.T) {
           wait_windows_ready(a, t + 1, lane);
           pnext = __ldcg(reinterpret_cast<const float2*>(a.p + ((size_t)kk * a.T + t + 1) * 2));
         }
@@ -791,7 +648,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
         wait_mma();
         mark(5);
         // the first half's product has read the W3 buffer: the second half streams in under this epilogue
-        if (kStream && wl == 0 && elect_one()) load_w3_rows(a.m, w3_img, N3a, N3b, N3t, N3buf, &s.bar_w3);
+        if (kStream && warp == 0 && elect_one()) load_w3_rows(a.m, w3_img, N3a, N3b, N3t, N3buf, &s.bar_w3);
         const uint32_t tDcg = tD + 8 * cg;
         const float *b3cg = s.b3 + 8 * cg, *phcg = s.phase + cg, *wtcg = s.weight + cg;
         if constexpr (kSplitD) {
@@ -800,49 +657,38 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
           mbar_wait_sleep(&s.done[1], n_b & 1); ++n_b;
           fence_after_sync();
           if (active) L3GU<NX, S, kUnitsH, kUnits, 0, kSplit3, kRcp % 10, kPerRow>::run(tDcg, b3cg, phcg, wtcg, cg, delta, rd, rs);
-        } else if constexpr (kGU) {
+        } else {
           if (active) L3GU<NX, S, 0, kUnitsA, 0, kSplit3, kRcp % 10, kPerRow>::run(tDcg, b3cg, phcg, wtcg, cg, delta, rd, rs);
-        } else if (active) {
-          if (cg == 0) L3Loop<NX, S, 0, kChunksA, 0, kSplit3, kRcp % 10, kCG, kPerRow>::run(tD, s.b3, s.phase, s.weight, delta, rd, rs);
-          else L3Loop<NX, S, 1, kChunksA, 0, kSplit3, kRcp % 10, kCG, kPerRow>::run(tD, s.b3, s.phase, s.weight, delta, rd, rs);
         }
-        if (N3b > 0) {
+        if constexpr (kStream) {
           mark(6);
           issue(3);
           wait_mma();
           mark(7);
           // ... and the first half again for the next step (or the next tile), under this epilogue and the next step's E1 / E2
-          if (kStream && wl == 0 && elect_one()) load_w3_rows(a.m, w3_img, 0, N3a, N3t, N3buf, &s.bar_w3);
-          if (active) {
-            if constexpr (kGU) {  // (streamed W3) the second half's units, now in column 0.. of the D region
-              L3GU<NX, S, kUnitsA, kUnits, kUnitsA, kSplit3, kRcp % 10, kPerRow>::run(tDcg, b3cg, phcg, wtcg, cg, delta, rd, rs);
-            } else {
-              constexpr int kFirstB0 = kChunksA + (kChunksA & 1);        // first chunk >= kChunksA with even index
-              constexpr int kFirstB1 = kChunksA + 1 - (kChunksA & 1);    // ... with odd index
-              if (cg == 0) L3Loop<NX, S, kFirstB0, kChunks, kChunksA, kSplit3, kRcp % 10, 2>::run(tD, s.b3, s.phase, s.weight, delta);
-              else L3Loop<NX, S, kFirstB1, kChunks, kChunksA, kSplit3, kRcp % 10, 2>::run(tD, s.b3, s.phase, s.weight, delta);
-            }
-          }
+          if (warp == 0 && elect_one()) load_w3_rows(a.m, w3_img, 0, N3a, N3t, N3buf, &s.bar_w3);
+          // the second half's units, now in column 0.. of the D region
+          if (active) L3GU<NX, S, kUnitsA, kUnits, kUnitsA, kSplit3, kRcp % 10, kPerRow>::run(tDcg, b3cg, phcg, wtcg, cg, delta, rd, rs);
         }
 #pragma unroll
-        for (int c = 0; c < NX; ++c) s.exch[g * kCG + cg][row * NX + c] = delta[c];
-        asm volatile("bar.sync %0, %1;" ::"r"(1 + g), "n"(kGroupT) : "memory");
+        for (int c = 0; c < NX; ++c) s.exch[cg][row * NX + c] = delta[c];
+        asm volatile("bar.sync %0, %1;" ::"r"(1), "n"(kThreads) : "memory");
         // every thread of a sample adds the partials in the same order: the replicated state stays bit-identical
 #pragma unroll
         for (int c = 0; c < NX; ++c) {
-          float d = s.exch[g * kCG][row * NX + c];
+          float d = s.exch[0][row * NX + c];
 #pragma unroll
-          for (int j = 1; j < kCG; ++j) d += s.exch[g * kCG + j][row * NX + c];
+          for (int j = 1; j < 4; ++j) d += s.exch[j][row * NX + c];
           st[c] += d;                                             // mppi_with_model.py:121
           in[c] = (st[c] - s.smean[c]) * s.sinv[c];
-          if (cg == kCG - 1 && live) {
+          if (cg == 3 && live) {
             if (a.states) a.states[((size_t)kk * a.T + t) * NX + c] = st[c];
             if (a.delta_out) a.delta_out[(size_t)kk * NX + c] = d;
           }
         }
         in[NX] = pnext.x; in[NX + 1] = pnext.y;
         ++tstep;
-        // exch is rewritten only after the next step's MMA round trips, which need every warp of the group
+        // exch is rewritten only after the next step's MMA round trips, which need every warp
       }
       if (cg == 0 && live && a.cost_total) {
         cost_acc += env_running_cost_fast(a.o, st, a.hist + ((size_t)kk * a.L + (a.T - 1) + a.B - 1) * a.nu, a.nu);
@@ -850,22 +696,22 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
       }
     }
     // the last streamed half (requested for a step that never comes) must have landed before the CTA's shared memory goes
-    if (kStream && wl == 0) mbar_wait(&s.bar_w3, n_w3 & 1);
+    if (kStream && warp == 0) mbar_wait(&s.bar_w3, n_w3 & 1);
   }
   fence_before_sync();
   __syncthreads();
   if (warp == 0) tmem_dealloc(tmem, kTmemCols);
 }
 
-
 // ======================================  ping-pong form  ======================================
-// Two 128-sample tiles per CTA again, but ALL 16 warps work on ONE tile's epilogue at a time and alternate between the
-// tiles phase by phase:
+// Two 128-sample tiles per CTA, and ALL 16 warps work on ONE tile's epilogue at a time and alternate between the tiles
+// phase by phase:
 //     E1x E1y  E2x E2y  E3ax E3ay  E3bx E3by  Ux Uy        (x, y = the two tiles;  U = state update + next A1)
 // Every product (M2, M3a, M3b, M1 of the next step) is issued at the end of its tile's phase and has the whole following
 // phase of the OTHER tile to complete, so the CUDA cores never wait for the tensor pipe and every SM sub-partition always
-// has its four warps in the same instruction mix.  The free-running two-group form above leaves each tile with two warps
-// per sub-partition (latency-bound epilogues: 33.5 k clocks per step of a tile pair at config 4, issue slots 40 % busy).
+// has its four warps in the same instruction mix.  Its predecessor ran the two tiles as two free-running 8-warp groups,
+// which left each tile two warps per sub-partition (latency-bound epilogues: 33.5 k clocks per step of a tile pair at
+// config 4, issue slots 40 % busy).
 //   hand-off   a dedicated MMA warp (warp 16): an epilogue warp arrives on the tile's NAMED barrier (bar.arrive: it does not
 //              block) after its TMEM stores and moves on to the other tile's phase; the MMA warp waits for the 16 arrivals
 //              (bar.sync), issues the product under elect.sync and commits it to the mbarrier done[tile], which the epilogue
@@ -920,10 +766,10 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
     if (warp == 0 && elect_one()) {  // weight images by TMA bulk copies; only the MMA warp waits for them (see rollout_tc2_kernel)
       mbar_init(&s.bar_w, 1);
       mbar_fence_init();
-      load_weight_images(a.m, w1_img, w2_img, w3_img, N3t, &s.bar_w, true, a.m.mlp2_w3u);
+      load_weight_images(a.m, w1_img, w2_img, w3_img, N3t, &s.bar_w);
     }
-    for (int i = tid; i < kH; i += kThreadsPP) s.b2[i] = a.m.mlp2_c[i];
-    for (int i = tid; i < 256; i += kThreadsPP) s.b3[i] = i < N3t ? a.m.mlp2_cu[i] : 0.0f;
+    for (int i = tid; i < kH; i += kThreadsPP) s.b2[i] = a.m.mlp2_b2[i];
+    for (int i = tid; i < 256; i += kThreadsPP) s.b3[i] = i < N3t ? a.m.mlp2_b3[i] : 0.0f;
     for (int i = tid; i < S; i += kThreadsPP) { s.phase[i] = a.m.ilt_phase[i]; s.weight[i] = a.m.ilt_weight[i]; }
     if (tid < NX) { s.smean[tid] = a.m.state_mean[tid]; s.sinv[tid] = a.m.state_inv_std[tid]; }
     for (int i = tid; i < 2 * 2 * kRows * 2; i += kThreadsPP) (&s.stage_u[0][0][0][0])[i] = 0.0f;
@@ -1280,38 +1126,37 @@ static int launch_pp(const Args& a, cudaStream_t stream) {
   return NLC_OK;
 }
 
-template <int NX, int S, bool kSplit3, int kRcp, int kTiles, bool kPerRow = false>
+template <int NX, int S, bool kSplit3, int kRcp, bool kPerRow = false>
 static int launch_one_t(const Args& a, cudaStream_t stream) {
-  constexpr int kUnits = PPShape<NX, S>::kUnits;
-  constexpr int N3t = kTiles == 1 ? PPShape<NX, S>::N3u : (2 * NX * S + 15) / 16 * 16;
-  constexpr int N3buf = (kTiles == 1 && N3t > 256) ? 32 * ((kUnits + 1) / 2) : N3t;  // streamed W3: one half resident
+  constexpr int kUnits = PPShape<NX, S>::kUnits, N3t = PPShape<NX, S>::N3u;
+  constexpr int N3buf = N3t > 256 ? 32 * ((kUnits + 1) / 2) : N3t;  // streamed W3: one half resident
   const size_t smem = 2 * (size_t)kH * 16 * 2 + 2 * (size_t)kH * kH * 2 + 2 * (size_t)N3buf * kH * 2 + sizeof(SmemTail) + 128;
   NLC_REQUIRE(smem <= 227 * 1024, NLC_ERR_SHAPE, "tcgen05 rollout: %zu bytes of shared memory needed", smem);
-  auto kern = rollout_tc2_kernel<NX, S, kSplit3, kRcp, kTiles, kPerRow>;
+  auto kern = rollout_tc2_kernel<NX, S, kSplit3, kRcp, kPerRow>;
   NLC_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  // one tile slot per 32..128 samples: enough CTAs to give every slot at least one warp of samples, at most one per SM
-  int grid = (a.K + 32 * kTiles - 1) / (32 * kTiles);
+  // one tile per 32..128 samples: enough CTAs to give every tile at least one warp of samples, at most one per SM
+  int grid = (a.K + 31) / 32;
   if (grid > 148) grid = 148;
   // overlapped planner step: whole 128-sample tiles on as few SMs as possible - the encoder runs on the others
-  if (kTiles == 1 && a.ready) grid = (a.K + kRows - 1) / kRows;
+  if (a.ready) grid = (a.K + kRows - 1) / kRows;
   kern<<<grid, kThreads, smem, stream>>>(a);
   NLC_LAUNCH_OK("rollout_tc2_kernel");
   return NLC_OK;
 }
 
-// two tiles per CTA once the plan is more than one wave of 128-sample tiles, else one tile on all 16 warps
+// tiles == 3: the ping-pong form (plans of more than one wave of 128-sample tiles), else one tile on all 16 warps
 template <int NX, int S, bool kSplit3, int kRcp>
 static int launch_one(const Args& a, int tiles, cudaStream_t stream) {
   if (a.row_b1) {  // per-sample prediction times: the one-tile form's kPerRow instantiation (fp32-class arithmetic only)
-    if constexpr (kSplit3) return launch_one_t<NX, S, true, kRcp, 1, true>(a, stream);
+    if constexpr (kSplit3) return launch_one_t<NX, S, true, kRcp, true>(a, stream);
     else return NLC_ERR_UNSUPPORTED;
   }
   if constexpr (2 * NX * S > 256) {
-    // more (theta, phi) columns than two tiles' accumulators hold: the one-tile form with W3 streamed, whatever the plan size
-    return launch_one_t<NX, S, kSplit3, kRcp, 1>(a, stream);
+    // more (theta, phi) columns than the ping-pong form's accumulators hold: the one-tile form with W3 streamed, whatever
+    // the plan size
+    return launch_one_t<NX, S, kSplit3, kRcp>(a, stream);
   } else {
-    if (tiles == 3) return launch_pp<NX, S, kSplit3, kRcp>(a, stream);
-    return tiles == 1 ? launch_one_t<NX, S, kSplit3, kRcp, 1>(a, stream) : launch_one_t<NX, S, kSplit3, kRcp, 2>(a, stream);
+    return tiles == 3 ? launch_pp<NX, S, kSplit3, kRcp>(a, stream) : launch_one_t<NX, S, kSplit3, kRcp>(a, stream);
   }
 }
 
@@ -1334,7 +1179,7 @@ int launch_rollout_tc2(nlc_model_s* m, const nlc_rollout_opts* o, const float* s
   a.row_b1 = row_b1; a.row_tn = row_tn;
   NLC_REQUIRE(!row_b1 || (row_tn && split3 && !ready), NLC_ERR_ARG, "rollout: per-sample times need row_tn and the fp32-class tensor-core mode");
   if (2 * m->nx * m->S > 256) tiles_per_cta = 1;
-  NLC_REQUIRE(tiles_per_cta == 2 || m->N3u == 32 * (m->nx * ((m->S - 1) / 16) + 1), NLC_ERR_SHAPE,
+  NLC_REQUIRE(m->N3u == 32 * (m->nx * ((m->S - 1) / 16) + 1), NLC_ERR_SHAPE,
               "tcgen05 rollout: the model holds no group-uniform W3 image for nx=%d S=%d", m->nx, m->S);
   NLC_REQUIRE(!ready || (status && ((tiles_per_cta == 1 && (K + 127) / 128 <= 148) || tiles_per_cta == 3)), NLC_ERR_ARG,
               "rollout: the overlapped forms are the one-tile form of plans within one wave and the ping-pong form");
@@ -1343,7 +1188,7 @@ int launch_rollout_tc2(nlc_model_s* m, const nlc_rollout_opts* o, const float* s
   a.trace = g_roll_trace;
   // reciprocal flavour of the fp32-class epilogues: Newton on the FMA pipe for both the MLP tanh and the L3 pair ("33").
   // Ping-pong form at config 4: 1.412 ms; MUFU for the L3 pair ("30") 1.447, for the tanh ("03") 1.427, for both ("00") 1.466
-  // (round 2; round 1 measured 1.71 vs 1.85 ms with the two-group form, profiles/r1_rollout_sweep.md)
+  // (round 2; round 1 measured 1.71 vs 1.85 ms with the ping-pong form's two-group predecessor, profiles/r1_rollout_sweep.md)
 #define NLC_RT2_CASE(NX_, S_)                                                                \
   if (m->nx == NX_ && m->S == S_) {                                                          \
     if (!split3) return rt2::launch_one<NX_, S_, false, 0>(a, tiles_per_cta, stream);        \

@@ -5,9 +5,8 @@ CUDA events for each kernel form / measurement ablation given on the command lin
     python tools/bench_encoder.py [--env oderl-acrobot] [--K 65536] [--H 50] [--math tc_split3] VARIANT ...
 
 A VARIANT is a comma-separated list of NAME=VALUE environment settings applied before each timing (any name works as a
-label for repeated runs; NLC_ENC_RCP is latched at first use, so one reciprocal flavour per process).  The NLC_ENC_ABLATE
-bit mask behind profiles/r1_encoder_ablation.md was removed from the production kernel after those measurements (its
-run-time tests cost instructions in the hot loop).
+label for repeated runs).  The NLC_ENC_ABLATE bit mask behind profiles/r1_encoder_ablation.md and the NLC_ENC_RCP
+reciprocal flavours of DESIGN.md §3a were removed from the production kernel after those measurements.
 """
 import argparse
 import json

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Rollout microbenchmark (representation MLP + Fourier ILT + cost over the horizon, encoder output given), timed alone
 with CUDA events over a sweep of K.     python tools/bench_rollout.py [--env oderl-acrobot] [--H 50] [--math tc_split3] K ...
-NLC_ROLLOUT_TILES=1|2 in the environment forces the tiles-per-CTA form (default: by plan size)."""
+NLC_ROLLOUT_TILES=1|3 in the environment forces the one-tile or the ping-pong form (default: by plan size)."""
 import argparse
 import ctypes as C
 import json

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
-"""Timeline of the rollout kernel's first CTA (clock64 per warp at the phase boundaries), forms 1 and 2 of rollout_tc2.cu
-(NLC_ROLLOUT_TILES, default here 2); the ping-pong form has its own tool, trace_rollout_pp.py.  Measurement tool only."""
+"""Timeline of the rollout kernel's first CTA (clock64 per warp at the phase boundaries), the one-tile form of
+rollout_tc2.cu (forced here with NLC_ROLLOUT_TILES=1); the ping-pong form has its own tool, trace_rollout_pp.py.
+Measurement tool only."""
 import ctypes as C
 import os
 import sys
@@ -16,11 +17,11 @@ from neurallaplacecontrol_b200 import _lib  # noqa: E402
 from _util import DT, S_TERMS, weights  # noqa: E402
 from oracle import costs  # noqa: E402
 
-EV = ["A1 written", "M1 done", "E1 done", "M2 done", "E2 done", "M3a done", "E3a done", "M3b done"]
+EV = ["A1 written", "M1 done", "E1 done", "M2 done", "E2 done", "M3(a) done", "E3a done", "M3b done"]
 
 
 def main():
-    os.environ.setdefault("NLC_ROLLOUT_TILES", "2")
+    os.environ["NLC_ROLLOUT_TILES"] = "1"
     torch.set_grad_enabled(False)
     dev = torch.device("cuda", 0)
     env = "oderl-acrobot"
@@ -50,25 +51,19 @@ def main():
                                         cost.data_ptr(), states.data_ptr(), mode, _lib.current_stream_ptr()))
     torch.cuda.synchronize()
     tr = trace.cpu().numpy().reshape(104, 16, 8).astype(np.int64)
-    for g in range(2):
-        w = slice(8 * g, 8 * g + 8)
-        t0 = tr[4, w, 0].min()
-        print(f"group {g}: per event min/median/max over the 8 warps, clocks relative to step 4")
-        prev = None
-        for s in (4, 5, 6, 7, 24, 25, 26, 27, 28):
-            row = []
-            for e in range(8):
-                v = tr[s, w, e]
-                v = v[v > 0]
-                row.append("-" if len(v) == 0 else f"{v.min() - tr[s, w, 0].min():6d}/{int(np.median(v)) - tr[s, w, 0].min():6d}/{v.max() - tr[s, w, 0].min():6d}")
-            start = tr[s, w, 0].min()
-            t0 = start
-            print(f" step {s:2d} | " + " | ".join(row))
-    for g in range(2):
-        st = [int(tr[s_, 8 * g:8 * g + 8, 0].min()) for s_ in range(104)]
-        tails = [int(np.median(tr[s_ + 1, 8 * g:8 * g + 8, 0])) - int(np.median(tr[s_, 8 * g:8 * g + 8, 7])) for s_ in range(103)]
-        print(f"group {g} tail (last product done -> next A1 written) (k clk):", [round(x / 1e3, 1) for x in tails])
-        print(f"group {g} step durations (k clk):", [round((st[i + 1] - st[i]) / 1e3, 1) for i in range(103)])
+    print("per event min/median/max over the 16 warps, clocks relative to the step's first A1")
+    for s in (4, 5, 6, 7, 24, 25, 26, 27, 28):
+        row = []
+        for e in range(8):
+            v = tr[s, :, e]
+            v = v[v > 0]
+            row.append("-" if len(v) == 0 else f"{v.min() - tr[s, :, 0].min():6d}/{int(np.median(v)) - tr[s, :, 0].min():6d}/{v.max() - tr[s, :, 0].min():6d}")
+        print(f" step {s:2d} | " + " | ".join(row))
+    last = max(e for e in range(8) if (tr[:, :, e] > 0).any())  # the step's last product: M3 (resident W3) or M3b (streamed)
+    st = [int(tr[s_, :, 0].min()) for s_ in range(104)]
+    tails = [int(np.median(tr[s_ + 1, :, 0])) - int(np.median(tr[s_, :, last])) for s_ in range(103)]
+    print("tail (last product done -> next A1 written) (k clk):", [round(x / 1e3, 1) for x in tails])
+    print("step durations (k clk):", [round((st[i + 1] - st[i]) / 1e3, 1) for i in range(103)])
     print("events:", ", ".join(f"{i}={n}" for i, n in enumerate(EV)))
 
 
