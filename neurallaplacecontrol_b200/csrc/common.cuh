@@ -95,15 +95,16 @@ struct ModelDev {
   // columns); and the matching fp32 constants (biases, layer-0 input weights, output layer), layout kE2* below
   void* enc2_w;
   float* enc2_c;
-  // input/bias blocks of the two GRU layers, [2 layers][256 accumulator columns][8 halves] =
+  // input/bias blocks of the two GRU layers, [2 layers][4 Hg accumulator columns][8 halves] =
   // [W0_hi W0_hi W0_lo | W1_hi W1_hi W1_lo | b_hi b_lo]: all three split-3 terms of W_ih0 x + b in ONE K = 16 MMA against
   // the operand block [x0_hi x0_lo x0_hi | x1_hi x1_lo x1_hi | 1 1 | 0 x 8]   (layer 1: biases only)
   void* enc2_x;
   // rollout_tc2.cu: representation MLP with -2 log2(e) folded into every layer (all three feed tanh-like maps):
-  // mlp2_w1 [2 (hi,lo)][128 x 16]  first layer on the tensor cores, K = [obs_n | p_action | 1 (folded bias) | 0..]
+  // (Hm = 128 or 64; packed at both widths)
+  // mlp2_w1 [2 (hi,lo)][Hm x 16]   first layer on the tensor cores, K = [obs_n | p_action | 1 (folded bias) | 0..]
   //                                 (re-packed by nlc_model_set_prediction_time: the bias depends on the s-points);
-  // mlp2_w2 [2][128 x 128], mlp2_b2 [128] scaled;
-  // mlp2_w3 [2 (hi,lo)][N3u x 128], mlp2_b3 [N3u] scaled, in the GROUP-UNIFORM column order (rollout_tc2.cu: every column
+  // mlp2_w2 [2][Hm x Hm], mlp2_b2 [Hm] scaled;
+  // mlp2_w3 [2 (hi,lo)][N3u x Hm], mlp2_b3 [N3u] scaled, in the GROUP-UNIFORM column order (rollout_tc2.cu: every column
   // group of a tile runs the SAME L3 epilogue code): column = 32 j + 8 cg + 2 i + {theta, phi}; regular unit j < NX (S-1)/16:
   // channel j / upc, term 16 (j % upc) + cg + 4 i (upc = (S-1)/16); last unit: the channels' last terms k = S-1, pair i =
   // channel cg + 4 i (zero columns where that channel does not exist)

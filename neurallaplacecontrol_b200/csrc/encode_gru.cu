@@ -19,7 +19,6 @@
 namespace nlc {
 
 constexpr int kEncRows = 64;
-constexpr int kHg = 64;   // GRU width of the tensor-core encoder (hidden_units = 128); the fp32 kernel below is a template on it
 
 struct EncArgs {
   const float* hist;  // [K][L][gin] env units
@@ -237,7 +236,7 @@ int encode_history_impl(nlc_model_t m, const float* hist_dev, int hist_ch, int K
     case NLC_MATH_TC_SPLIT3:
     case NLC_MATH_TC_FP16:
       // shapes without a tensor-core instantiation run on the fp32 kernel
-      if (B < 2 || B * m->gin > 8 || m->gin > 2 || m->Hg != kHg) {
+      if (B < 2 || B * m->gin > 8 || m->gin > 2) {
         if ((long long)K * T >= 4096)
           warn_once(kWarnEncoderFfma, "encoder: window length %d x input width %d has no tcgen05 instantiation; %lld windows run on the "
                     "fp32 CUDA-core kernel", B, m->gin, (long long)K * T);
@@ -251,7 +250,7 @@ int encode_history_impl(nlc_model_t m, const float* hist_dev, int hist_ch, int K
 // Does (model, window length, math mode) run on the tcgen05 encoder?  (planner.cu: only then can the encoder publish per-step
 // readiness to a rollout kernel running beside it.)
 bool encoder_is_tensor_core(nlc_model_t m, int B, int math_mode) {
-  return math_mode != NLC_MATH_FP32 && !(B < 2 || B * m->gin > 8 || m->gin > 2) && m->Hg == kHg;
+  return math_mode != NLC_MATH_FP32 && !(B < 2 || B * m->gin > 8 || m->gin > 2);
 }
 
 // The planner's overlapped form: step-major tile order over the samples from k_sub on, ready[t] counts finished warps of step t

@@ -23,14 +23,17 @@
 //
 //   operands   fp16 hi (+ lo) images, K-major no-swizzle canonical layout; NLC_MATH_TC_SPLIT3: A_hi B_hi + A_lo B_hi +
 //              A_hi B_lo, fp32 accumulate (fp32-class);  NLC_MATH_TC_FP16: A_hi B_hi only.
-//   TMEM       D0[256] = [r | z | hn | in] of layer 0;  D1[256] = [in | r | z | hn] of layer 1: all 512 columns.
+//   widths     a template on the GRU width HG: 64 (hidden_units = 128) or 32 (hidden_units = 64, the reference class
+//              default).  Every product and image below scales with HG; the thread layout and the schedule do not.
+//   TMEM       D0[4 HG] = [r | z | hn | in] of layer 0;  D1[4 HG] = [in | r | z | hn] of layer 1: 512 columns at HG = 64,
+//              256 at HG = 32.
 //   schedule   layer 0 runs one cell ahead of layer 1, so every MMA burst runs under the other layer's gate epilogue:
 //                 epi A(s+1) || MMA B(s)   ->   epi B(s) || MMA A(s+2)   ->   ...        (tiles software-pipelined)
 //   barriers   bar_a / bar_b: MMA A / B complete (tcgen05.commit);  h0_ready / h1_ready: all 16 epilogue warps stored
 //              their operand slice and finished reading their accumulator columns.
-//   threads    epilogue warp w < 16: TMEM lanes 32 (w & 3).. (its 32 windows), hidden units 16 (w >> 2).. +15 of both
-//              layers; warp 16: MMA issue.  544 threads -> 96 registers per thread (the register file is allocated in
-//              units of 4 warps: 104 would not launch).
+//   threads    epilogue warp w < 16: TMEM lanes 32 (w & 3).. (its 32 windows), hidden units HG/4 (w >> 2).. + HG/4 - 1
+//              of both layers (16 at HG = 64, 8 at HG = 32); warp 16: MMA issue.  544 threads -> 96 registers per thread
+//              (the register file is allocated in units of 4 warps: 104 would not launch).
 #include <cuda_fp16.h>
 
 #include "common.cuh"
@@ -43,11 +46,23 @@ using namespace umma;
 
 namespace enc2 {
 
-constexpr int kRows = 128, kHg = 64, kG3 = 192, kThreads = 512;
-constexpr uint32_t kOpBytes = kRows * kHg * 2;  // one fp16 A-operand image (16 KB)
-constexpr uint32_t kWBytes = kG3 * kHg * 2;     // one fp16 weight image (24 KB)
-constexpr uint32_t kLbo = 128, kSbo = (kHg / 8) * 128;
-constexpr uint32_t kColD0 = 0, kColD1 = 256, kTmemCols = 512;  // D0 = [r | z | hn | in], D1 = [in | r | z | hn]
+constexpr int kRows = 128, kThreads = 512;
+constexpr uint32_t kLbo = 128;
+// shapes of the GRU width HG (64 or 32); the sizes in the comments are those of HG = 64
+template <int HG>
+struct Geo {
+  static constexpr int kHg = HG, kG3 = 3 * HG;
+  static constexpr int kUnits = HG / 4;                          // hidden units per thread and layer
+  static constexpr uint32_t kOpBytes = kRows * kHg * 2;          // one fp16 A-operand image (16 KB)
+  static constexpr uint32_t kWBytes = kG3 * kHg * 2;             // one fp16 weight image (24 KB)
+  static constexpr uint32_t kSbo = (kHg / 8) * 128;
+  static constexpr uint32_t kColD0 = 0, kColD1 = 4 * HG, kTmemCols = 8 * HG;  // D0 = [r | z | hn | in], D1 = [in | r | z | hn]
+  // layer 0's [x | 1] block: one extra K block of the layer-0 state image (see below)
+  static constexpr int kKx = kHg + 16;
+  static constexpr uint32_t kSboX = (kKx / 8) * 128;             // 8-row-group stride of the K = 80 image
+  static constexpr uint32_t kH0HiBytes = kRows * kKx * 2;        // 20 KB
+  static constexpr uint32_t kWxBytes = 4 * HG * 8 * 2;           // B side of the block: [4 HG][8] halves (4 KB)
+};
 
 struct Args {
   const float* hist;
@@ -153,19 +168,20 @@ __device__ __forceinline__ void store_operand8(unsigned char* img_hi, uint32_t s
   if (kSplit3) *reinterpret_cast<uint4*>(img_lo + (uint32_t)(row >> 3) * sbo_lo + in_group) = make_uint4(pl[0], pl[1], pl[2], pl[3]);
 }
 
-// D[128 x 192] += A[128 x 64] * B[192 x 64]^T : 4 (x3) MMA instructions.  The hi and lo images of A may have different
-// 8-row-group strides (the layer-0 state image carries an extra K block, see Smem)
-template <bool kSplit3>
-__device__ __forceinline__ void issue_gemm192(uint32_t d_tmem, uint32_t a_hi, uint32_t a_hi_sbo, uint32_t a_lo, uint32_t a_lo_sbo,
+// D[128 x 3 HG] += A[128 x HG] * B[3 HG x HG]^T : HG / 16 (x3) MMA instructions (N = 192 at HG = 64, 96 at HG = 32).  The hi
+// and lo images of A may have different 8-row-group strides (the layer-0 state image carries an extra K block, see Smem)
+template <int HG, bool kSplit3>
+__device__ __forceinline__ void issue_gemm_g3(uint32_t d_tmem, uint32_t a_hi, uint32_t a_hi_sbo, uint32_t a_lo, uint32_t a_lo_sbo,
                                               uint32_t b_hi, uint32_t b_lo) {
-  const uint32_t idesc = idesc_f16_f32(kRows, kG3);
+  using G = Geo<HG>;
+  const uint32_t idesc = idesc_f16_f32(kRows, G::kG3);
 #pragma unroll
-  for (int ks = 0; ks < kHg / 16; ++ks) {
+  for (int ks = 0; ks < G::kHg / 16; ++ks) {
     const uint32_t off = ks * 2 * kLbo;  // 16 K-elements = two core matrices
-    mma_f16_ss(d_tmem, smem_desc(a_hi + off, kLbo, a_hi_sbo), smem_desc(b_hi + off, kLbo, kSbo), idesc, 1u);
+    mma_f16_ss(d_tmem, smem_desc(a_hi + off, kLbo, a_hi_sbo), smem_desc(b_hi + off, kLbo, G::kSbo), idesc, 1u);
     if (kSplit3) {
-      mma_f16_ss(d_tmem, smem_desc(a_lo + off, kLbo, a_lo_sbo), smem_desc(b_hi + off, kLbo, kSbo), idesc, 1u);
-      mma_f16_ss(d_tmem, smem_desc(a_hi + off, kLbo, a_hi_sbo), smem_desc(b_lo + off, kLbo, kSbo), idesc, 1u);
+      mma_f16_ss(d_tmem, smem_desc(a_lo + off, kLbo, a_lo_sbo), smem_desc(b_hi + off, kLbo, G::kSbo), idesc, 1u);
+      mma_f16_ss(d_tmem, smem_desc(a_hi + off, kLbo, a_hi_sbo), smem_desc(b_lo + off, kLbo, G::kSbo), idesc, 1u);
     }
   }
 }
@@ -181,20 +197,18 @@ constexpr int kBarH0 = 2, kBarH1 = 3;             // named barriers: layer-0 / l
 //   B block (per column)  [W0_hi W0_hi W0_lo | W1_hi W1_hi W1_lo | b_hi b_lo | 0 ...]
 // so one K = 16 MMA with accumulate = 0 writes  W_ih0 x + b  (all three split terms at once) into D0 = [r | z | hn | in]
 // and the hidden products accumulate on top: no input FMAs, no bias loads, no accumulator re-arm in the layer-0 epilogue.
-constexpr int kKx = kHg + 16;
-constexpr uint32_t kSboX = (kKx / 8) * 128;       // 8-row-group stride of the K = 80 image
-constexpr uint32_t kH0HiBytes = kRows * kKx * 2;  // 20 KB
-// The B side of that block stores only its first 8 K-elements ([256][8] halves, 4 KB): the A side's second 8 are zeros
-// for ever, so the descriptor lets the second core matrix alias the next row group's (finite) data - 0 x finite = 0.
-constexpr uint32_t kWxBytes = 256 * 8 * 2;
-constexpr int kC2Wout = 0, kC2Bout = 128, kC2Count = 136;  // shared-memory constants: the output layer
+// The B side of that block stores only its first 8 K-elements ([4 HG][8] halves, Geo::kWxBytes): the A side's second 8 are
+// zeros for ever, so the descriptor lets the second core matrix alias the next row group's (finite) data - 0 x finite = 0.
+constexpr int kC2Wout = 0, kC2Bout = 128, kC2Count = 136;  // shared-memory constants: the output layer ([2][HG] weights, bias)
 
+template <int HG>
 struct Smem {
-  alignas(128) unsigned char w[3][2][kWBytes];   // [W_hh0, W_ih1 (n|r|z), W_hh1][hi, lo]
-  alignas(128) unsigned char wx[2][kWxBytes + 128];  // input/bias blocks: layer 0 rows in D0 order, layer 1 in D1 order; + zero pad
-  alignas(128) unsigned char h0_hi[kH0HiBytes];  // layer-0 state, K = 64 + the [x | 1] block
-  alignas(128) unsigned char h0_lo[kOpBytes];
-  alignas(128) unsigned char h1[2][kOpBytes];
+  using G = Geo<HG>;
+  alignas(128) unsigned char w[3][2][G::kWBytes];   // [W_hh0, W_ih1 (n|r|z), W_hh1][hi, lo]
+  alignas(128) unsigned char wx[2][G::kWxBytes + 128];  // input/bias blocks: layer 0 rows in D0 order, layer 1 in D1 order; + zero pad
+  alignas(128) unsigned char h0_hi[G::kH0HiBytes];  // layer-0 state, K = HG + the [x | 1] block
+  alignas(128) unsigned char h0_lo[G::kOpBytes];
+  alignas(128) unsigned char h1[2][G::kOpBytes];
   alignas(16) float c[kC2Count];
   alignas(16) float pout[3][kRows * 2];
   alignas(8) uint64_t bar_w;                 // weight images landed (TMA bulk copies)
@@ -204,14 +218,17 @@ struct Smem {
 
 // kSplit3: the fp32-class mode (split-3 products, Newton (r, z) reciprocals, Newton for one n-pair in four); else the
 // single-pass fp16 mode with tanh.approx gates
-template <bool kSplit3, int GIN, bool kClamp1, bool kTrace = false>
+template <int HG, bool kSplit3, int GIN, bool kClamp1, bool kTrace = false>
 __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
+  using G = Geo<HG>;
+  constexpr int kHg = G::kHg, kU = G::kUnits;
+  constexpr uint32_t kSbo = G::kSbo, kSboX = G::kSboX, kColD0 = G::kColD0, kColD1 = G::kColD1, kTmemCols = G::kTmemCols;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  Smem& s = *reinterpret_cast<Smem*>(smem_raw);
+  Smem<HG>& s = *reinterpret_cast<Smem<HG>*>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int q = warp & 3, grp = warp >> 2;
   const int row = 32 * q + lane;   // window within the tile == TMEM lane
-  const int ubase = 16 * grp;      // first of the 16 hidden units (per layer) this thread owns
+  const int ubase = kU * grp;      // first of the kU hidden units (per layer) this thread owns
   const int B = a.B;
   int tstep = 0;
   auto mark = [&](int ev) {  // compiled in for tools/trace_encoder.py only: the tests cost instructions in the hot loop
@@ -219,23 +236,23 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
   };
 
   {
-    // The weight images (144 KB + the two input/bias blocks) come in by TMA bulk copies issued by ONE thread and counted on
+    // The weight images (144 KB at HG = 64, 36 KB at HG = 32, + the two input/bias blocks) come in by TMA bulk copies issued by ONE thread and counted on
     // an mbarrier that only the MMA warp waits for - no other thread ever reads them - so the load runs under the TMEM
     // allocation, the zero fills and the first window fetch instead of in front of them.
     if (warp == 0 && elect_one()) {  // (elect.sync, not tid == 0: the copies' operands then stay in uniform registers)
       mbar_init(&s.bar_w, 1);
       mbar_fence_init();
-      mbar_expect_tx(&s.bar_w, (uint32_t)(3 * 2 * kWBytes + 2 * kWxBytes));
+      mbar_expect_tx(&s.bar_w, (uint32_t)(3 * 2 * G::kWBytes + 2 * G::kWxBytes));
       const unsigned char* src = reinterpret_cast<const unsigned char*>(a.m.enc2_w);
-      for (int i = 0; i < 6; ++i) bulk_g2s(&s.w[0][0][0] + (size_t)i * kWBytes, src + (size_t)i * kWBytes, kWBytes, &s.bar_w);
+      for (int i = 0; i < 6; ++i) bulk_g2s(&s.w[0][0][0] + (size_t)i * G::kWBytes, src + (size_t)i * G::kWBytes, G::kWBytes, &s.bar_w);
       const unsigned char* sx = reinterpret_cast<const unsigned char*>(a.m.enc2_x);
-      for (int l = 0; l < 2; ++l) bulk_g2s(s.wx[l], sx + (size_t)l * kWxBytes, kWxBytes, &s.bar_w);
+      for (int l = 0; l < 2; ++l) bulk_g2s(s.wx[l], sx + (size_t)l * G::kWxBytes, G::kWxBytes, &s.bar_w);
     }
     for (int i = tid; i < 2 * 8; i += blockDim.x)  // the zero pad behind each input/bias block
-      reinterpret_cast<uint4*>(s.wx[i >> 3] + kWxBytes)[i & 7] = make_uint4(0u, 0u, 0u, 0u);
+      reinterpret_cast<uint4*>(s.wx[i >> 3] + G::kWxBytes)[i & 7] = make_uint4(0u, 0u, 0u, 0u);
     uint4* dz = reinterpret_cast<uint4*>(s.h0_hi);  // the second half of the [x | 1] block stays zero for ever
-    for (int i = tid; i < (int)(kH0HiBytes / 16); i += blockDim.x) dz[i] = make_uint4(0u, 0u, 0u, 0u);
-    for (int i = tid; i < 128; i += blockDim.x) s.c[kC2Wout + i] = a.m.enc2_c[kE2Wout + i];
+    for (int i = tid; i < (int)(G::kH0HiBytes / 16); i += blockDim.x) dz[i] = make_uint4(0u, 0u, 0u, 0u);
+    for (int i = tid; i < 2 * kHg; i += blockDim.x) s.c[kC2Wout + i] = a.m.enc2_c[kE2Wout + i];
     if (tid < 2) s.c[kC2Bout + tid] = a.m.enc2_c[kE2Bout + tid];
     if (tid == 0) {
       mbar_init(&s.bar_a, 1); mbar_init(&s.bar_b, 1); mbar_init(&s.bar_h0, 1);
@@ -275,8 +292,8 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
     auto issue_a = [&](bool with_hidden) {
       if (elect_one()) {
         fence_after_sync();
-        mma_f16_ss(tmem + kColD0, smem_desc(a_h0_hi + 8 * kLbo, kLbo, kSboX), smem_desc(w_x0, kLbo, 128), idesc_f16_f32(kRows, 256), 0u);
-        if (with_hidden) issue_gemm192<kSplit3>(tmem + kColD0, a_h0_hi, kSboX, a_h0_lo, kSbo, w_hh0_hi, w_hh0_lo);
+        mma_f16_ss(tmem + kColD0, smem_desc(a_h0_hi + (kHg / 8) * kLbo, kLbo, kSboX), smem_desc(w_x0, kLbo, 128), idesc_f16_f32(kRows, 4 * kHg), 0u);
+        if (with_hidden) issue_gemm_g3<HG, kSplit3>(tmem + kColD0, a_h0_hi, kSboX, a_h0_lo, kSbo, w_hh0_hi, w_hh0_lo);
         mma_commit(&s.bar_a);
       }
       __syncwarp();
@@ -285,12 +302,12 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
       if (elect_one()) {
         fence_after_sync();
         // biases first (accumulate = 0 over all of D1 = [in | r | z | hn]): the 1-columns of the [x | 1] block
-        mma_f16_ss(tmem + kColD1, smem_desc(a_h0_hi + 8 * kLbo, kLbo, kSboX), smem_desc(w_x1, kLbo, 128), idesc_f16_f32(kRows, 256), 0u);
-        issue_gemm192<kSplit3>(tmem + kColD1, a_h0_hi, kSboX, a_h0_lo, kSbo, w_ih1_hi, w_ih1_lo);
+        mma_f16_ss(tmem + kColD1, smem_desc(a_h0_hi + (kHg / 8) * kLbo, kLbo, kSboX), smem_desc(w_x1, kLbo, 128), idesc_f16_f32(kRows, 4 * kHg), 0u);
+        issue_gemm_g3<HG, kSplit3>(tmem + kColD1, a_h0_hi, kSboX, a_h0_lo, kSbo, w_ih1_hi, w_ih1_lo);
         // everything that reads the layer-0 state image is issued: the layer-0 epilogue may overwrite it as soon as THIS much
         // has completed (half a product earlier than bar_b), so its operand stores interleave with its gate math
         mma_commit(&s.bar_h0);
-        if (with_h1) issue_gemm192<kSplit3>(tmem + kColD1 + 64, a_h1_hi, kSbo, a_h1_lo, kSbo, w_hh1_hi, w_hh1_lo);
+        if (with_h1) issue_gemm_g3<HG, kSplit3>(tmem + kColD1 + kHg, a_h1_hi, kSbo, a_h1_lo, kSbo, w_hh1_hi, w_hh1_lo);
         mma_commit(&s.bar_b);
       }
       __syncwarp();
@@ -324,7 +341,7 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
   for (int v = 0; v < GIN; ++v) { amean[v] = a.m.act_mean[v]; ainv[v] = a.m.act_inv_std[v]; }
 
   uint32_t n_a = 0, n_b = 0, n_h0 = 0;  // waits completed on bar_a / bar_b / bar_h0
-  f2_t h0r[8], h1r[8];
+  f2_t h0r[kU / 2], h1r[kU / 2];
   // raw window entry of the FOLLOWING layer-0 cell (threads with grp == 0 feed the operand).  It is normalised only when it is
   // written into the operand, a whole gate epilogue after the load was issued: nothing waits for global memory
   float xraw[GIN] = {};
@@ -374,23 +391,23 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
     uint32_t w[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) { const __half2 p2 = __halves2half2(hv[2 * i], hv[2 * i + 1]); w[i] = *reinterpret_cast<const uint32_t*>(&p2); }
-    *reinterpret_cast<uint4*>(s.h0_hi + (uint32_t)(row >> 3) * kSboX + 8 * kLbo + (uint32_t)(row & 7) * 16) = make_uint4(w[0], w[1], w[2], w[3]);
+    *reinterpret_cast<uint4*>(s.h0_hi + (uint32_t)(row >> 3) * kSboX + (kHg / 8) * kLbo + (uint32_t)(row & 7) * 16) = make_uint4(w[0], w[1], w[2], w[3]);
   };
   // layer-0 cell: complete pre-activations come out of D0 = [r | z | hn | in]; with `store` the new state goes into the layer-0
   // state image (after `wait_h0`: see below).
   auto cell_a = [&](bool from_zero, bool store, bool wait_h0) {
     if (from_zero) {  // cell 0 of a window: h = 0 (one uniform branch instead of a select per use)
 #pragma unroll
-      for (int i = 0; i < 8; ++i) h0r[i] = 0ull;
+      for (int i = 0; i < kU / 2; ++i) h0r[i] = 0ull;
     }
 #pragma unroll
-    for (int c = 0; c < 2; ++c) {
+    for (int c = 0; c < kU / 8; ++c) {
       const int u0 = ubase + 8 * c;
       f2_t gr[4], gz[4], gh[4], gn[4];
       ldtm8p(tlane + kColD0 + u0, gr);
-      ldtm8p(tlane + kColD0 + 64 + u0, gz);
-      ldtm8p(tlane + kColD0 + 128 + u0, gh);
-      ldtm8p(tlane + kColD0 + 192 + u0, gn);
+      ldtm8p(tlane + kColD0 + kHg + u0, gz);
+      ldtm8p(tlane + kColD0 + 2 * kHg + u0, gh);
+      ldtm8p(tlane + kColD0 + 3 * kHg + u0, gn);
       tmem_ld_wait();
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
@@ -407,7 +424,7 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
       // issued, later than one chunk's math (waiting after the first chunk showed up as 8.8 % of all stall samples).
       if (wait_h0) { mbar_wait_sleep(&s.bar_h0, n_h0 & 1); ++n_h0; }
 #pragma unroll
-      for (int c = 0; c < 2; ++c) {
+      for (int c = 0; c < kU / 8; ++c) {
         const f2_t (&hc)[4] = *reinterpret_cast<const f2_t(*)[4]>(&h0r[4 * c]);
         store_operand8<kSplit3>(s.h0_hi, kSboX, s.h0_lo, kSbo, row, ubase + 8 * c, hc);
       }
@@ -468,19 +485,19 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
       // ======== layer-1 epilogue B(st)  ||  MMA A ========
       if (st == 0) {
 #pragma unroll
-        for (int i = 0; i < 8; ++i) h1r[i] = 0ull;
+        for (int i = 0; i < kU / 2; ++i) h1r[i] = 0ull;
       }
       mbar_wait_sleep(&s.bar_b, n_b & 1); ++n_b;
       fence_after_sync();
       mark(4);
 #pragma unroll
-      for (int c = 0; c < 2; ++c) {
+      for (int c = 0; c < kU / 8; ++c) {
         const int u0 = ubase + 8 * c;
         f2_t gn[4], gr[4], gz[4], gh[4];
         ldtm8p(tlane + kColD1 + u0, gn);
-        ldtm8p(tlane + kColD1 + 64 + u0, gr);
-        ldtm8p(tlane + kColD1 + 128 + u0, gz);
-        ldtm8p(tlane + kColD1 + 192 + u0, gh);
+        ldtm8p(tlane + kColD1 + kHg + u0, gr);
+        ldtm8p(tlane + kColD1 + 2 * kHg + u0, gz);
+        ldtm8p(tlane + kColD1 + 3 * kHg + u0, gh);
         tmem_ld_wait();
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
@@ -501,7 +518,7 @@ __global__ void __launch_bounds__(kThreadsAll, 1) encode_tc2_kernel(Args a) {
         // ---------------- linear_out on the top layer's last state (w_nl.py:29) ----------------
         float o0 = 0.f, o1 = 0.f;
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
+        for (int i = 0; i < kU / 2; ++i) {
           float x0, x1;
           upk2(h1r[i], x0, x1);
           const float2 wa = *reinterpret_cast<const float2*>(cst + kC2Wout + ubase + 2 * i);
@@ -556,6 +573,7 @@ int launch_encode_tc2(nlc_model_s* m, const float* hist, int hist_ch, int K, int
   NLC_REQUIRE(B * m->gin <= 8, NLC_ERR_SHAPE, "tcgen05 encoder: window_length * input_width = %d exceeds 8", B * m->gin);
   NLC_REQUIRE(B >= 2, NLC_ERR_SHAPE, "tcgen05 encoder: window_length must be >= 2");
   NLC_REQUIRE(m->gin == 1 || m->gin == 2, NLC_ERR_SHAPE, "tcgen05 encoder: GRU input width %d has no instantiation", m->gin);
+  NLC_REQUIRE(m->Hg == 64 || m->Hg == 32, NLC_ERR_SHAPE, "tcgen05 encoder: GRU width %d has no instantiation", m->Hg);
   NLC_REQUIRE(!ready || (k_sub >= 0 && k_sub < K && ((long long)k_sub * T) % kRows == 0 && (!with_head || tile_begin == 0)), NLC_ERR_ARG,
               "tcgen05 encoder: bad step-major sub-plan (first sample %d of %d)", k_sub, K);
   Args a;
@@ -568,17 +586,23 @@ int launch_encode_tc2(nlc_model_s* m, const float* hist, int hist_ch, int K, int
   a.head_tiles = ready && with_head ? (int)((long long)k_sub * T / kRows) : 0;
   a.m = m->d;
   a.trace = g_enc_trace;
-  const int smem = (int)sizeof(Smem) + 128;
+  const int smem = (int)(m->Hg == 32 ? sizeof(Smem<32>) : sizeof(Smem<64>)) + 128;
   // fp32-class mode: Newton (3 steps) for the (r, z) reciprocal; for n, Newton for one pair in four and MUFU for the rest;
   // single-pass fp16 mode: three tanh.approx per unit (that mode's accuracy class, 2e-2 bound).
   void (*kern)(Args);
   // layer-1 (r, z) clamps are compiled out when the packed weights prove |pre-activation| * log2(e) < 60 (model.cu)
   const bool c1 = !m->enc_l1_bounded;
-#define NLC_ENC_PICK(TR) \
-  (m->gin == 1 ? (c1 ? encode_tc2_kernel<true, 1, true, TR> : encode_tc2_kernel<true, 1, false, TR>) \
-               : (c1 ? encode_tc2_kernel<true, 2, true, TR> : encode_tc2_kernel<true, 2, false, TR>))
-  if (!split3) kern = m->gin == 1 ? encode_tc2_kernel<false, 1, true> : encode_tc2_kernel<false, 2, true>;
-  else kern = a.trace ? NLC_ENC_PICK(true) : NLC_ENC_PICK(false);
+#define NLC_ENC_PICK(HG, TR) \
+  (m->gin == 1 ? (c1 ? encode_tc2_kernel<HG, true, 1, true, TR> : encode_tc2_kernel<HG, true, 1, false, TR>) \
+               : (c1 ? encode_tc2_kernel<HG, true, 2, true, TR> : encode_tc2_kernel<HG, true, 2, false, TR>))
+  if (m->Hg == 32) {  // hidden_units = 64 (the clock64 timeline is measured at the 128 width only)
+    if (!split3) kern = m->gin == 1 ? encode_tc2_kernel<32, false, 1, true> : encode_tc2_kernel<32, false, 2, true>;
+    else kern = NLC_ENC_PICK(32, false);
+  } else if (!split3) {
+    kern = m->gin == 1 ? encode_tc2_kernel<64, false, 1, true> : encode_tc2_kernel<64, false, 2, true>;
+  } else {
+    kern = a.trace ? NLC_ENC_PICK(64, true) : NLC_ENC_PICK(64, false);
+  }
 #undef NLC_ENC_PICK
   NLC_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   long long n_tiles = ready ? (long long)a.tiles_per_t * T : (a.rows + kRows - 1) / kRows;

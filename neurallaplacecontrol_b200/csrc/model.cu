@@ -218,7 +218,7 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
   // group-uniform W3 image of the tensor-core rollout: 32 columns per unit, NX (S-1)/16 regular units + 1 unit of last terms
   const int gu_upc = (S - 1) % 16 == 0 ? (S - 1) / 16 : 0;
   const int gu_units = gu_upc ? nx * gu_upc + 1 : 0;
-  const int N3u = (Hm == 128 && gu_units >= 1 && gu_units <= 13) ? 32 * gu_units : 0;  // <= 416 columns (rollout_tc2.cu kMaxN3)
+  const int N3u = (gu_units >= 1 && gu_units <= 13) ? 32 * gu_units : 0;  // <= 416 columns (rollout_tc2.cu kMaxN3)
   m->N3u = N3u;
   size_t o_m2w3 = A.add((size_t)2 * (N3u ? N3u : 16) * Hm / 2), o_m2b3 = A.add(N3u ? N3u : 16);
 
@@ -270,7 +270,7 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
     put64(o_amean64, i, mean);
     put64(o_ainv64, i, 1.0 / stdv);
   }
-  if (Hm == 128) {  // (the tensor-core kernels are built for hidden_units = 128: other widths run on the fp32 kernels)
+  {  // both widths (hidden_units 128 and 64) have tensor-core encoder and rollout kernels
     // encode_tc2.cu operands: exponent scales folded (sigmoid(x) = 1/(1 + 2^(-log2e x)), tanh(x) = 2/(1 + 2^(-2 log2e x)) - 1)
     const double cR = -1.4426950408889634, cN = 2.0 * cR;
     auto gate_scale = [&](int row) { return row < 2 * Hg ? cR : cN; };
@@ -298,17 +298,17 @@ extern "C" int nlc_model_create(nlc_model_t* out, const nlc_model_desc* d, int d
       for (int v = 0; v < gin; ++v)
         for (int u = 0; u < Hg; ++u)
           put(o_enc2c, nlc::kE2Wih0 + (size_t)(g * nlc::kMaxNu + v) * Hg + u, (g < 2 ? cR : cN) * d->gru_w_ih_l0[(size_t)(g * Hg + u) * gin + v]);
-    if (gin <= 2) {  // the [x | 1] blocks of the tensor-core encoder (encode_tc2.cu): [layer][256 rows][8 halves]
+    if (gin <= 2) {  // the [x | 1] blocks of the tensor-core encoder (encode_tc2.cu): [layer][4 Hg rows][8 halves]
       uint16_t* wx = reinterpret_cast<uint16_t*>(A.data.data() + o_enc2x);
       auto split = [](double v, uint16_t& hi, uint16_t& lo) {
         __half h = __float2half_rn((float)v);
         __half l = __float2half_rn((float)(v - (double)__half2float(h)));
         hi = *reinterpret_cast<uint16_t*>(&h); lo = *reinterpret_cast<uint16_t*>(&l);
       };
-      for (int row = 0; row < 256; ++row) {
+      for (int row = 0; row < 4 * Hg; ++row) {
         const int blk = row / Hg, u = row % Hg;
-        uint16_t* r0 = wx + (size_t)row * 8;          // layer 0, accumulator order [r | z | hn | in]
-        uint16_t* r1 = wx + (size_t)(256 + row) * 8;  // layer 1, accumulator order [in | r | z | hn]: biases only
+        uint16_t* r0 = wx + (size_t)row * 8;             // layer 0, accumulator order [r | z | hn | in]
+        uint16_t* r1 = wx + (size_t)(4 * Hg + row) * 8;  // layer 1, accumulator order [in | r | z | hn]: biases only
         for (int k = 0; k < 8; ++k) r0[k] = r1[k] = 0;
         {
           // r, z: W_ih0 x + b_ih + b_hh;  hn: b_hh[n] only;  in: W_ih0[n] x + b_ih[n]

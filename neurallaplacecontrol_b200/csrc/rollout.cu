@@ -295,9 +295,10 @@ bool rollout_can_overlap(const nlc_model_s* m, int K, int T, int math_mode) {
   // Ping-pong plans of two passes per CTA (up to 560 tiles; config 4 on one GPU: 512 tiles = 128 CTAs x 2 passes, 20 SMs to
   // spare) encode the first pass's samples before the fork and only the last steps of the last pass's samples beside the
   // rollout: the last pass starts ~T steps after the fork, which leaves the encoder time for those steps.
+  // The schedule and its constants were measured at hidden_units = 128; hidden-64 plans run the encoder, then the rollout.
   const int n_tiles = (K + 127) / 128;
   const bool pp_form = 2 * m->nx * m->S <= 256;  // shapes with a ping-pong instantiation (rollout_tc2.cu launch_one)
-  return !off && !forced_rollout_form() && math_mode != NLC_MATH_FP32 && rollout_has_tensor_core_form(m) && T >= 2 &&
+  return !off && !forced_rollout_form() && math_mode != NLC_MATH_FP32 && m->Hm == 128 && rollout_has_tensor_core_form(m) && T >= 2 &&
          (pp_form ? (n_tiles <= 140 || (pp_overlap_iters(n_tiles) <= 2 && pp_overlap_grid(n_tiles) <= 140)) : n_tiles <= 140);
 }
 // The overlapped rollout's form: one tile per CTA on n_tiles SMs (9.5 us per step), or - from 89 tiles - the ping-pong form on

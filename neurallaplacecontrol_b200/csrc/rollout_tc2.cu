@@ -47,10 +47,15 @@ using namespace umma;
 
 namespace rt2 {
 
-constexpr int kRows = 128, kH = 128;
-constexpr uint32_t kLbo = 128, kSbo = (kH / 8) * 128;  // K = 128 operand images
+// Both kernels are templates on the MLP width H: 128 (config.py:37) or 64 (the reference class default, w_nl.py:71).  At H = 64
+// every thread owns 16 hidden units instead of 32 (one 16-column chunk), the A operand takes H / 2 TMEM columns per image,
+// the accumulator region starts at column H, and W3 (at most 106 KB) always stays resident.  The sizes in the comments are
+// those of H = 128.
+constexpr int kRows = 128, kMaxH = 128;
+constexpr uint32_t kLbo = 128;
+template <int H> constexpr uint32_t kSboH = (H / 8) * 128;  // K = H operand images
 constexpr uint32_t kSbo16 = (16 / 8) * 128;             // K = 16 (first layer)
-constexpr uint32_t kColA = 0, kColD = 128, kGroupCols = 256, kTmemCols = 512;
+constexpr uint32_t kColA = 0, kGroupCols = 256, kTmemCols = 512;  // the accumulator region starts at column H (A: hi | lo)
 constexpr int kThreads = 512;
 
 struct Args {
@@ -100,12 +105,14 @@ __device__ __forceinline__ void wait_windows_ready(const Args& a, int t, int lan
 
 // W1 (2 x 4 KB), W2 (2 x 32 KB), W3 (2 x N3t x 256 B) -> shared memory; bulk copies of at most 32 KB each.  with_w3 = false:
 // W3 is streamed half by half instead (load_w3_rows)
+template <int kH>
 __device__ __forceinline__ void load_weight_images(const ModelDev& m, unsigned char* w1_img, unsigned char* w2_img, unsigned char* w3_img,
                                                    int N3t, uint64_t* bar, bool with_w3 = true) {
   const uint32_t b1 = 2 * kH * 16 * 2, b2 = 2 * kH * kH * 2, b3 = with_w3 ? 2u * (uint32_t)N3t * kH * 2 : 0u;
+  constexpr uint32_t kChunk2 = 2 * kH * kH * 2 < 32768 ? 2 * kH * kH * 2 : 32768;
   mbar_expect_tx(bar, b1 + b2 + b3);
   bulk_g2s(w1_img, m.mlp2_w1, b1, bar);
-  for (uint32_t o = 0; o < b2; o += 32768) bulk_g2s(w2_img + o, static_cast<const unsigned char*>(m.mlp2_w2) + o, 32768, bar);
+  for (uint32_t o = 0; o < b2; o += kChunk2) bulk_g2s(w2_img + o, static_cast<const unsigned char*>(m.mlp2_w2) + o, kChunk2, bar);
   for (uint32_t o = 0; o < b3; o += 32768) {
     const uint32_t n = b3 - o < 32768 ? b3 - o : 32768;
     bulk_g2s(w3_img + o, static_cast<const unsigned char*>(m.mlp2_w3) + o, n, bar);
@@ -113,6 +120,7 @@ __device__ __forceinline__ void load_weight_images(const ModelDev& m, unsigned c
 }
 // Rows [row0, row0 + nrows) of W3 (output columns of the third layer; multiples of 8, so whole 8-row groups of the K-major
 // image = contiguous bytes), hi and lo image, into a buffer that holds n_buf rows of each.  Issued by one thread.
+template <int kH>
 __device__ __forceinline__ void load_w3_rows(const ModelDev& m, unsigned char* w3_buf, int row0, int nrows, int N3t, int n_buf, uint64_t* bar) {
   const uint32_t bytes = (uint32_t)nrows * kH * 2;
   mbar_expect_tx(bar, 2 * bytes);
@@ -127,7 +135,7 @@ constexpr int kMaxN3 = 416;  // (theta, phi) columns of the largest instantiatio
 struct SmemTail {  // after the weight images
   alignas(8) uint64_t bar_w;
   alignas(8) uint64_t bar_w3;   // streamed W3 halves (instantiations whose W3 does not fit shared memory)
-  alignas(16) float b2[kH];
+  alignas(16) float b2[kMaxH];
   alignas(16) float b3[kMaxN3];
   float phase[kMaxS], weight[kMaxS];
   float smean[kMaxNx], sinv[kMaxNx];
@@ -217,15 +225,15 @@ __device__ __forceinline__ void ldtm16p(uint32_t taddr, f2_t (&v)[8]) {
   for (int i = 0; i < 8; ++i) v[i] = pk2u(r[2 * i], r[2 * i + 1]);
 }
 
-// D[128 x N] = A[128 x Kdim] (TMEM, hi at a_tmem, lo at a_tmem + 64) * B[N x Kdim]^T (smem image, K-major)
-template <bool kSplit3>
+// D[128 x N] = A[128 x Kdim] (TMEM, hi at a_tmem, lo at a_tmem + kALo = H / 2) * B[N x Kdim]^T (smem image, K-major)
+template <bool kSplit3, int kALo>
 __device__ __forceinline__ void issue_gemm_ts(uint32_t d_tmem, uint32_t a_tmem, uint32_t b_hi, uint32_t b_lo, int N, int ksteps, uint32_t sbo) {
   const uint32_t idesc = idesc_f16_f32(kRows, N);
   for (int ks = 0; ks < ksteps; ++ks) {
     const uint32_t boff = ks * 2 * kLbo;
     mma_f16_ts(d_tmem, a_tmem + 8 * ks, smem_desc(b_hi + boff, kLbo, sbo), idesc, ks > 0 ? 1u : 0u);
     if (kSplit3) {
-      mma_f16_ts(d_tmem, a_tmem + 64 + 8 * ks, smem_desc(b_hi + boff, kLbo, sbo), idesc, 1u);
+      mma_f16_ts(d_tmem, a_tmem + kALo + 8 * ks, smem_desc(b_hi + boff, kLbo, sbo), idesc, 1u);
       mma_f16_ts(d_tmem, a_tmem + 8 * ks, smem_desc(b_lo + boff, kLbo, sbo), idesc, 1u);
     }
   }
@@ -234,15 +242,16 @@ __device__ __forceinline__ void issue_gemm_ts(uint32_t d_tmem, uint32_t a_tmem, 
 // Every second K-step of the same product (kHalf = 0: steps 0, 2, ..; 1: steps 1, 3, ..): the one-tile form issues a layer's
 // product in two halves, the first as soon as the first 16 of every thread's 32 activation columns are in TMEM, so that half
 // of the product runs under the second half of the epilogue that feeds it (strict chain per sample: nothing else covers it).
-template <bool kSplit3>
+// kParts = 1 (H = 64: a thread's 16 columns are one K-step): `half` 0 is the whole product.
+template <bool kSplit3, int kALo, int kParts = 2>
 __device__ __forceinline__ void issue_gemm_ts_half(uint32_t d_tmem, uint32_t a_tmem, uint32_t b_hi, uint32_t b_lo, int N, int ksteps, uint32_t sbo,
                                                    int half) {
   const uint32_t idesc = idesc_f16_f32(kRows, N);
-  for (int ks = half; ks < ksteps; ks += 2) {
+  for (int ks = half; ks < ksteps; ks += kParts) {
     const uint32_t boff = ks * 2 * kLbo;
     mma_f16_ts(d_tmem, a_tmem + 8 * ks, smem_desc(b_hi + boff, kLbo, sbo), idesc, ks > 0 ? 1u : 0u);
     if (kSplit3) {
-      mma_f16_ts(d_tmem, a_tmem + 64 + 8 * ks, smem_desc(b_hi + boff, kLbo, sbo), idesc, 1u);
+      mma_f16_ts(d_tmem, a_tmem + kALo + 8 * ks, smem_desc(b_hi + boff, kLbo, sbo), idesc, 1u);
       mma_f16_ts(d_tmem, a_tmem + 8 * ks, smem_desc(b_lo + boff, kLbo, sbo), idesc, 1u);
     }
   }
@@ -253,7 +262,7 @@ __device__ __forceinline__ void issue_gemm_ts_half(uint32_t d_tmem, uint32_t a_t
 // that spilled 246 words under the small budget); inside, fully unrolled with the descriptors advanced by immediates
 // (a rolled loop that rebuilt them issued one MMA per ~130 clocks: the MMAs, not the epilogues, then set the step time).
 // Called by the whole (converged) warp; ONE thread chosen by elect.sync issues and commits (tc_umma.cuh: elect_one).
-template <int kSteps, bool kSplit3>
+template <int kSteps, bool kSplit3, int kALo>
 __device__ __noinline__ void issue_gemm_ts_fn(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_hi_desc, uint64_t b_lo_desc, uint32_t idesc,
                                               uint64_t* done) {
   if (elect_one()) {
@@ -263,7 +272,7 @@ __device__ __noinline__ void issue_gemm_ts_fn(uint32_t d_tmem, uint32_t a_tmem, 
       const uint64_t off = (uint64_t)(ks * 2 * kLbo >> 4);  // the start-address field counts 16-byte units
       mma_f16_ts(d_tmem, a_tmem + 8 * ks, b_hi_desc + off, idesc, ks > 0 ? 1u : 0u);
       if (kSplit3) {
-        mma_f16_ts(d_tmem, a_tmem + 64 + 8 * ks, b_hi_desc + off, idesc, 1u);
+        mma_f16_ts(d_tmem, a_tmem + kALo + 8 * ks, b_hi_desc + off, idesc, 1u);
         mma_f16_ts(d_tmem, a_tmem + 8 * ks, b_lo_desc + off, idesc, 1u);
       }
     }
@@ -412,18 +421,21 @@ struct PPShape {  // columns of the group-uniform W3 image: model.cu packs N3u =
   static constexpr int kUnits = NX * ((S - 1) / 16) + 1, N3u = 32 * kUnits;
 };
 
-template <int NX, int S, bool kSplit3, int kRcp, bool kPerRow = false>
+template <int H, int NX, int S, bool kSplit3, int kRcp, bool kPerRow = false>
 __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int Lp = NX + 2;
+  constexpr int kH = H, kChunks = H / 64;  // 16-column chunks of hidden units per thread
+  constexpr uint32_t kSbo = kSboH<H>, kALo = H / 2, kColD = H;
   // the (theta, phi) columns in the GROUP-UNIFORM order (l3_units_gu: one L3 epilogue code for all four column groups)
   constexpr int kUnits = PPShape<NX, S>::kUnits, N3t = PPShape<NX, S>::N3u;
-  // One tile, all 16 warps on it in four column groups of 32 hidden units, L3 in one piece (A 128 + D up to 256 columns).
-  // kStream (more than 256 (theta, phi) columns: S = 33 with nx >= 5, the reference class default w_nl.py:73): L3 in
-  // two column halves of at most 256 columns, and W3 - which no longer fits shared memory next to W1 and W2 - streamed: one
+  // One tile, all 16 warps on it in four column groups of H / 4 hidden units, L3 in one piece (A 128 + D up to 256 columns).
+  // kStream (H = 128 with more than 256 (theta, phi) columns: S = 33 with nx >= 5, the reference class default w_nl.py:73): L3
+  // in two column halves of at most 256 columns, and W3 - which no longer fits shared memory next to W1 and W2 - streamed: one
   // buffer of N3a rows, reloaded by TMA bulk copies (L2-resident source) as soon as the product that read it has completed,
-  // each load hidden under the epilogue that follows.
-  constexpr bool kStream = N3t > 256;
+  // each load hidden under the epilogue that follows.  At H = 64 W3 (<= 106 KB) stays resident and the accumulator region
+  // (from column 64) holds all of its up to 416 columns: L3 is then always the two kSplitD products of <= 256 columns.
+  constexpr bool kStream = H == 128 && N3t > 256;
   constexpr int kUnitsA = kStream ? (kUnits + 1) / 2 : kUnits;        // units in the first column half
   constexpr int N3a = 32 * kUnitsA, N3b = N3t - N3a;
   constexpr int N3buf = kStream ? N3a : N3t;                          // rows of W3 resident at a time
@@ -433,7 +445,9 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
   constexpr bool kSplitD = !kStream && N3t >= 128;
   constexpr int kUnitsH = kSplitD ? (kUnits + 1) / 2 : kUnits;        // units of the first product
   constexpr int N3h = 32 * kUnitsH;
-  static_assert(N3a <= 256 && N3b <= 256 && N3t <= kMaxN3 && Lp + 1 <= 16, "tile shape");
+  static_assert((kStream ? N3a <= 256 && N3b <= 256 : N3h <= 256 && N3t - N3h <= 256) && N3t <= kMaxN3 && Lp + 1 <= 16,
+                "tile shape");
+  static_assert(kColD + (kStream ? N3a : N3t) <= kTmemCols, "accumulator columns");
   unsigned char* w1_img = smem_raw;                                   // [hi | lo] 128 x 16 halves = 4 KB each
   unsigned char* w2_img = w1_img + 2 * kH * 16 * 2;                   // [hi | lo] 32 KB each
   unsigned char* w3_img = w2_img + 2 * kH * kH * 2;                   // [hi | lo] N3buf * 256 B each
@@ -447,8 +461,8 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
       mbar_init(&s.bar_w, 1);
       mbar_init(&s.bar_w3, 1);
       mbar_fence_init();
-      load_weight_images(a.m, w1_img, w2_img, w3_img, N3t, &s.bar_w, !kStream);
-      if (kStream) load_w3_rows(a.m, w3_img, 0, N3a, N3t, N3buf, &s.bar_w3);
+      load_weight_images<kH>(a.m, w1_img, w2_img, w3_img, N3t, &s.bar_w, !kStream);
+      if (kStream) load_w3_rows<kH>(a.m, w3_img, 0, N3a, N3t, N3buf, &s.bar_w3);
     }
     for (int i = tid; i < kH; i += kThreads) s.b2[i] = a.m.mlp2_b2[i];
     for (int i = tid; i < kMaxN3; i += kThreads) s.b3[i] = i < N3t ? a.m.mlp2_b3[i] : 0.0f;
@@ -500,14 +514,15 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
       if (kStream && warp == 0 && ev == 3) { mbar_wait(&s.bar_w3, n_w3 & 1); ++n_w3; }  // this half of W3 has landed
       if (warp == 0 && elect_one()) {
         fence_after_sync();
-        if (ev == 0) issue_gemm_ts<kSplit3>(tmem + kColD, tmem + kColA, w1_hi, w1_lo, kH, 1, kSbo16);
-        else issue_gemm_ts<kSplit3>(tmem + kColD, tmem + kColA, w3_hi, w3_lo, N3b, kH / 16, kSbo);  // (the buffer holds that half)
+        if (ev == 0) issue_gemm_ts<kSplit3, kALo>(tmem + kColD, tmem + kColA, w1_hi, w1_lo, kH, 1, kSbo16);
+        else issue_gemm_ts<kSplit3, kALo>(tmem + kColD, tmem + kColA, w3_hi, w3_lo, N3b, kH / 16, kSbo);  // (the buffer holds that half)
         mma_commit(done);
       }
       __syncwarp();
     };
     // products M2 and M3 in two K-halves (issue_gemm_ts_half).  half 0 = the K-steps fed by every thread's first 16
     // activation columns (even steps: thread columns 32 cg .. 32 cg + 15 are K-step 2 cg), half 1 = the rest and the commit(s).
+    // H = 64: one part, issued whole with its commit(s) once every thread's 16 columns are in TMEM.
     auto issue_k = [&](int ev, int half) {
       tmem_st_wait();
       fence_before_sync();
@@ -515,17 +530,17 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
       if (kStream && warp == 0 && ev >= 2 && half == 0) { mbar_wait(&s.bar_w3, n_w3 & 1); ++n_w3; }  // this half of W3 has landed
       if (warp == 0 && elect_one()) {
         fence_after_sync();
-        if (ev == 1) issue_gemm_ts_half<kSplit3>(tmem + kColD, tmem + kColA, w2_hi, w2_lo, kH, kH / 16, kSbo, half);
+        if (ev == 1) issue_gemm_ts_half<kSplit3, kALo, kChunks>(tmem + kColD, tmem + kColA, w2_hi, w2_lo, kH, kH / 16, kSbo, half);
         else if (kSplitD) {
-          issue_gemm_ts_half<kSplit3>(tmem + kColD, tmem + kColA, w3_hi, w3_lo, N3h, kH / 16, kSbo, half);
-          if (half == 1) mma_commit(done);  // first column half: the epilogue starts on it while the second half computes
-          issue_gemm_ts_half<kSplit3>(tmem + kColD + N3h, tmem + kColA, w3_hi + (uint32_t)(N3h / 8) * kSbo, w3_lo + (uint32_t)(N3h / 8) * kSbo,
-                                      N3t - N3h, kH / 16, kSbo, half);
-          if (half == 1) mma_commit(&s.done[1]);
+          issue_gemm_ts_half<kSplit3, kALo, kChunks>(tmem + kColD, tmem + kColA, w3_hi, w3_lo, N3h, kH / 16, kSbo, half);
+          if (half == kChunks - 1) mma_commit(done);  // first column half: the epilogue starts on it while the second half computes
+          issue_gemm_ts_half<kSplit3, kALo, kChunks>(tmem + kColD + N3h, tmem + kColA, w3_hi + (uint32_t)(N3h / 8) * kSbo,
+                                                     w3_lo + (uint32_t)(N3h / 8) * kSbo, N3t - N3h, kH / 16, kSbo, half);
+          if (half == kChunks - 1) mma_commit(&s.done[1]);
         } else {
-          issue_gemm_ts_half<kSplit3>(tmem + kColD, tmem + kColA, w3_hi, w3_lo, N3a, kH / 16, kSbo, half);
+          issue_gemm_ts_half<kSplit3, kALo, kChunks>(tmem + kColD, tmem + kColA, w3_hi, w3_lo, N3a, kH / 16, kSbo, half);
         }
-        if (half == 1 && !(ev == 2 && kSplitD)) mma_commit(done);
+        if (half == kChunks - 1 && !(ev == 2 && kSplitD)) mma_commit(done);
       }
       __syncwarp();
     };
@@ -537,14 +552,14 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
     // the next product may overwrite the accumulator; bias_kind: 0 none, 1 b2, 2 per-sample first-layer bias
     auto hidden_split = [&](int ev_next, int bias_kind, int kk) {
       f2_t va[8], vb[8];
-      const int n0 = 32 * cg;
+      const int n0 = 16 * kChunks * cg;
       if (active_w) {
         ldtm16p(tD + n0, va);
-        ldtm16p(tD + n0 + 16, vb);
+        if constexpr (kChunks == 2) ldtm16p(tD + n0 + 16, vb);
         tmem_ld_wait();
       }
 #pragma unroll
-      for (int c16 = 0; c16 < 2; ++c16) {
+      for (int c16 = 0; c16 < kChunks; ++c16) {
         if (active_w) {
           f2_t (&v)[8] = c16 == 0 ? va : vb;
           const int nn = n0 + 16 * c16;
@@ -569,7 +584,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
           uint32_t ph[8], pl[8];
           pack16<kSplit3>(v, ph, pl);
           tmem_st8(tA + nn / 2, ph);
-          if (kSplit3) tmem_st8(tA + 64 + nn / 2, pl);
+          if (kSplit3) tmem_st8(tA + kALo + nn / 2, pl);
         }
         issue_k(ev_next, c16);
       }
@@ -618,7 +633,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
           uint32_t ph[8], pl[8];
           pack16<kSplit3>(v, ph, pl);
           tmem_st8(tA, ph);
-          if (kSplit3) tmem_st8(tA + 64, pl);
+          if (kSplit3) tmem_st8(tA + kALo, pl);
         }
         mark(0);
         issue(0);
@@ -648,7 +663,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
         wait_mma();
         mark(5);
         // the first half's product has read the W3 buffer: the second half streams in under this epilogue
-        if (kStream && warp == 0 && elect_one()) load_w3_rows(a.m, w3_img, N3a, N3b, N3t, N3buf, &s.bar_w3);
+        if (kStream && warp == 0 && elect_one()) load_w3_rows<kH>(a.m, w3_img, N3a, N3b, N3t, N3buf, &s.bar_w3);
         const uint32_t tDcg = tD + 8 * cg;
         const float *b3cg = s.b3 + 8 * cg, *phcg = s.phase + cg, *wtcg = s.weight + cg;
         if constexpr (kSplitD) {
@@ -666,7 +681,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
           wait_mma();
           mark(7);
           // ... and the first half again for the next step (or the next tile), under this epilogue and the next step's E1 / E2
-          if (warp == 0 && elect_one()) load_w3_rows(a.m, w3_img, 0, N3a, N3t, N3buf, &s.bar_w3);
+          if (warp == 0 && elect_one()) load_w3_rows<kH>(a.m, w3_img, 0, N3a, N3t, N3buf, &s.bar_w3);
           // the second half's units, now in column 0.. of the D region
           if (active) L3GU<NX, S, kUnitsA, kUnits, kUnitsA, kSplit3, kRcp % 10, kPerRow>::run(tDcg, b3cg, phcg, wtcg, cg, delta, rd, rs);
         }
@@ -731,7 +746,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_tc2_kernel(Args a) {
 template <int NX>
 struct SmemTailPP {
   alignas(8) uint64_t bar_w;
-  alignas(16) float b2[kH];
+  alignas(16) float b2[kMaxH];
   alignas(16) float b3[256];
   float phase[kMaxS], weight[kMaxS];
   float smean[kMaxNx], sinv[kMaxNx];
@@ -743,10 +758,12 @@ struct SmemTailPP {
 };
 constexpr int kThreadsPP = kThreads + 128;    // 16 epilogue warps + the MMA warp's group (setmaxnreg works on groups of 4 warps)
 
-template <int NX, int S, bool kSplit3, int kRcp>
+template <int H, int NX, int S, bool kSplit3, int kRcp>
 __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int Lp = NX + 2;
+  constexpr int kH = H, kChunks = H / 64;  // 16-column chunks of hidden units per thread
+  constexpr uint32_t kSbo = kSboH<H>, kALo = H / 2, kColD = H;
   // the (theta, phi) columns in the group-uniform order (l3_units_gu): units of 32 columns, the first four in the first half
   constexpr int kUnits = PPShape<NX, S>::kUnits, N3t = PPShape<NX, S>::N3u;
   constexpr int kUnitsA = kUnits < 4 ? kUnits : 4;
@@ -766,7 +783,7 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
     if (warp == 0 && elect_one()) {  // weight images by TMA bulk copies; only the MMA warp waits for them (see rollout_tc2_kernel)
       mbar_init(&s.bar_w, 1);
       mbar_fence_init();
-      load_weight_images(a.m, w1_img, w2_img, w3_img, N3t, &s.bar_w);
+      load_weight_images<kH>(a.m, w1_img, w2_img, w3_img, N3t, &s.bar_w);
     }
     for (int i = tid; i < kH; i += kThreadsPP) s.b2[i] = a.m.mlp2_b2[i];
     for (int i = tid; i < 256; i += kThreadsPP) s.b3[i] = i < N3t ? a.m.mlp2_b3[i] : 0.0f;
@@ -823,11 +840,11 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
         __syncwarp();
         const uint32_t tg = tmem + kGroupCols * x;
         uint64_t* done = &s.done[x];
-        if (ev == 0) issue_gemm_ts_fn<1, kSplit3>(tg + kColD, tg + kColA, smem_desc(w1_hi, kLbo, kSbo16), smem_desc(w1_lo, kLbo, kSbo16), idesc_f16_f32(kRows, kH), done);
-        else if (ev == 1) issue_gemm_ts_fn<kH / 16, kSplit3>(tg + kColD, tg + kColA, smem_desc(w2_hi, kLbo, kSbo), smem_desc(w2_lo, kLbo, kSbo), idesc_f16_f32(kRows, kH), done);
-        else if (ev == 2) issue_gemm_ts_fn<kH / 16, kSplit3>(tg + kColD, tg + kColA, smem_desc(w3_hi, kLbo, kSbo), smem_desc(w3_lo, kLbo, kSbo), idesc_f16_f32(kRows, N3a), done);
-        else issue_gemm_ts_fn<kH / 16, kSplit3>(tg + kColD, tg + kColA, smem_desc(w3_hi + w3b_off, kLbo, kSbo), smem_desc(w3_lo + w3b_off, kLbo, kSbo),
-                                                idesc_f16_f32(kRows, N3b > 0 ? N3b : 16), done);
+        if (ev == 0) issue_gemm_ts_fn<1, kSplit3, kALo>(tg + kColD, tg + kColA, smem_desc(w1_hi, kLbo, kSbo16), smem_desc(w1_lo, kLbo, kSbo16), idesc_f16_f32(kRows, kH), done);
+        else if (ev == 1) issue_gemm_ts_fn<kH / 16, kSplit3, kALo>(tg + kColD, tg + kColA, smem_desc(w2_hi, kLbo, kSbo), smem_desc(w2_lo, kLbo, kSbo), idesc_f16_f32(kRows, kH), done);
+        else if (ev == 2) issue_gemm_ts_fn<kH / 16, kSplit3, kALo>(tg + kColD, tg + kColA, smem_desc(w3_hi, kLbo, kSbo), smem_desc(w3_lo, kLbo, kSbo), idesc_f16_f32(kRows, N3a), done);
+        else issue_gemm_ts_fn<kH / 16, kSplit3, kALo>(tg + kColD, tg + kColA, smem_desc(w3_hi + w3b_off, kLbo, kSbo), smem_desc(w3_lo + w3b_off, kLbo, kSbo),
+                                                      idesc_f16_f32(kRows, N3b > 0 ? N3b : 16), done);
         if (lane == 0 && a.trace && blockIdx.x == 0 && mstep < 51 && mprod < 8) a.trace[52 * 256 + mstep * 256 + 2 * mprod + 1] = clock64();
         ++mprod;
       };
@@ -918,20 +935,20 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
         pack16<kSplit3>(v, ph, pl);
         const uint32_t tA = tlane + kGroupCols * x + kColA;
         tmem_st8(tA, ph);
-        if (kSplit3) tmem_st8(tA + 64, pl);
+        if (kSplit3) tmem_st8(tA + kALo, pl);
       }
     };
     // hidden layer epilogue: (+ bias,) tanh, re-written as the fp16 hi/lo A operand of the next layer
     auto hidden = [&](int x, bool with_bias) {
       const uint32_t tA = tlane + kGroupCols * x + kColA, tD = tlane + kGroupCols * x + kColD;
       if ((amask >> x) & 1) {
-        f2_t vv[2][8];
-        ldtm16p(tD + 32 * cg, vv[0]);
-        ldtm16p(tD + 32 * cg + 16, vv[1]);
+        f2_t vv[kChunks][8];
+        ldtm16p(tD + 16 * kChunks * cg, vv[0]);
+        if constexpr (kChunks == 2) ldtm16p(tD + 32 * cg + 16, vv[kChunks - 1]);
         tmem_ld_wait();
 #pragma unroll
-        for (int c16 = 0; c16 < 2; ++c16) {
-          const int n0 = 32 * cg + 16 * c16;
+        for (int c16 = 0; c16 < kChunks; ++c16) {
+          const int n0 = 16 * kChunks * cg + 16 * c16;
           f2_t (&v)[8] = vv[c16];
           if (with_bias) {
 #pragma unroll
@@ -945,7 +962,7 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
           uint32_t ph[8], pl[8];
           pack16<kSplit3>(v, ph, pl);
           tmem_st8(tA + n0 / 2, ph);
-          if (kSplit3) tmem_st8(tA + 64 + n0 / 2, pl);
+          if (kSplit3) tmem_st8(tA + kALo + n0 / 2, pl);
         }
       }
     };
@@ -1110,12 +1127,12 @@ __global__ void __launch_bounds__(kThreadsPP, 1) rollout_pp_kernel(Args a) {
   if (warp == 0) tmem_dealloc(tmem, kTmemCols);
 }
 
-template <int NX, int S, bool kSplit3, int kRcp>
+template <int kH, int NX, int S, bool kSplit3, int kRcp>
 static int launch_pp(const Args& a, cudaStream_t stream) {
   constexpr int N3t = PPShape<NX, S>::N3u;
   const size_t smem = 2 * (size_t)kH * 16 * 2 + 2 * (size_t)kH * kH * 2 + 2 * (size_t)N3t * kH * 2 + sizeof(SmemTailPP<NX>) + 128;
   NLC_REQUIRE(smem <= 227 * 1024, NLC_ERR_SHAPE, "tcgen05 rollout: %zu bytes of shared memory needed", smem);
-  auto kern = rollout_pp_kernel<NX, S, kSplit3, kRcp>;
+  auto kern = rollout_pp_kernel<kH, NX, S, kSplit3, kRcp>;
   NLC_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int grid = (a.K + 63) / 64;   // at least one warp of samples per tile slot, at most one CTA per SM
   if (grid > 148) grid = 148;
@@ -1126,13 +1143,13 @@ static int launch_pp(const Args& a, cudaStream_t stream) {
   return NLC_OK;
 }
 
-template <int NX, int S, bool kSplit3, int kRcp, bool kPerRow = false>
+template <int kH, int NX, int S, bool kSplit3, int kRcp, bool kPerRow = false>
 static int launch_one_t(const Args& a, cudaStream_t stream) {
   constexpr int kUnits = PPShape<NX, S>::kUnits, N3t = PPShape<NX, S>::N3u;
-  constexpr int N3buf = N3t > 256 ? 32 * ((kUnits + 1) / 2) : N3t;  // streamed W3: one half resident
+  constexpr int N3buf = kH == 128 && N3t > 256 ? 32 * ((kUnits + 1) / 2) : N3t;  // streamed W3: one half resident
   const size_t smem = 2 * (size_t)kH * 16 * 2 + 2 * (size_t)kH * kH * 2 + 2 * (size_t)N3buf * kH * 2 + sizeof(SmemTail) + 128;
   NLC_REQUIRE(smem <= 227 * 1024, NLC_ERR_SHAPE, "tcgen05 rollout: %zu bytes of shared memory needed", smem);
-  auto kern = rollout_tc2_kernel<NX, S, kSplit3, kRcp, kPerRow>;
+  auto kern = rollout_tc2_kernel<kH, NX, S, kSplit3, kRcp, kPerRow>;
   NLC_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   // one tile per 32..128 samples: enough CTAs to give every tile at least one warp of samples, at most one per SM
   int grid = (a.K + 31) / 32;
@@ -1145,25 +1162,26 @@ static int launch_one_t(const Args& a, cudaStream_t stream) {
 }
 
 // tiles == 3: the ping-pong form (plans of more than one wave of 128-sample tiles), else one tile on all 16 warps
-template <int NX, int S, bool kSplit3, int kRcp>
+template <int kH, int NX, int S, bool kSplit3, int kRcp>
 static int launch_one(const Args& a, int tiles, cudaStream_t stream) {
   if (a.row_b1) {  // per-sample prediction times: the one-tile form's kPerRow instantiation (fp32-class arithmetic only)
-    if constexpr (kSplit3) return launch_one_t<NX, S, true, kRcp, true>(a, stream);
+    if constexpr (kSplit3) return launch_one_t<kH, NX, S, true, kRcp, true>(a, stream);
     else return NLC_ERR_UNSUPPORTED;
   }
   if constexpr (2 * NX * S > 256) {
-    // more (theta, phi) columns than the ping-pong form's accumulators hold: the one-tile form with W3 streamed, whatever
-    // the plan size
-    return launch_one_t<NX, S, kSplit3, kRcp>(a, stream);
+    // more (theta, phi) columns than the ping-pong form's accumulators hold: the one-tile form (with W3 streamed at H = 128),
+    // whatever the plan size
+    return launch_one_t<kH, NX, S, kSplit3, kRcp>(a, stream);
   } else {
-    return tiles == 3 ? launch_pp<NX, S, kSplit3, kRcp>(a, stream) : launch_one_t<NX, S, kSplit3, kRcp>(a, stream);
+    return tiles == 3 ? launch_pp<kH, NX, S, kSplit3, kRcp>(a, stream) : launch_one_t<kH, NX, S, kSplit3, kRcp>(a, stream);
   }
 }
 
 }  // namespace rt2
 
+// both MLP widths the model accepts (128 and 64) have every (nx, S) pair below
 bool rollout_has_tensor_core_form(const nlc_model_s* m) {
-  return m->Hm == 128 && (m->S == 17 || m->S == 33) && (m->nx == 3 || m->nx == 5 || m->nx == 6);
+  return (m->S == 17 || m->S == 33) && (m->nx == 3 || m->nx == 5 || m->nx == 6);
 }
 
 // returns NLC_ERR_UNSUPPORTED when the (nx, S) pair has no tensor-core instantiation (caller falls back)
@@ -1189,10 +1207,14 @@ int launch_rollout_tc2(nlc_model_s* m, const nlc_rollout_opts* o, const float* s
   // reciprocal flavour of the fp32-class epilogues: Newton on the FMA pipe for both the MLP tanh and the L3 pair ("33").
   // Ping-pong form at config 4: 1.412 ms; MUFU for the L3 pair ("30") 1.447, for the tanh ("03") 1.427, for both ("00") 1.466
   // (round 2; round 1 measured 1.71 vs 1.85 ms with the ping-pong form's two-group predecessor, profiles/r1_rollout_sweep.md)
-#define NLC_RT2_CASE(NX_, S_)                                                                \
-  if (m->nx == NX_ && m->S == S_) {                                                          \
-    if (!split3) return rt2::launch_one<NX_, S_, false, 0>(a, tiles_per_cta, stream);        \
-    return rt2::launch_one<NX_, S_, true, 33>(a, tiles_per_cta, stream);                     \
+#define NLC_RT2_CASE(NX_, S_)                                                                   \
+  if (m->nx == NX_ && m->S == S_) {                                                             \
+    if (m->Hm == 64) {                                                                          \
+      if (!split3) return rt2::launch_one<64, NX_, S_, false, 0>(a, tiles_per_cta, stream);     \
+      return rt2::launch_one<64, NX_, S_, true, 33>(a, tiles_per_cta, stream);                  \
+    }                                                                                           \
+    if (!split3) return rt2::launch_one<128, NX_, S_, false, 0>(a, tiles_per_cta, stream);      \
+    return rt2::launch_one<128, NX_, S_, true, 33>(a, tiles_per_cta, stream);                   \
   }
   NLC_RT2_CASE(3, 17)
   NLC_RT2_CASE(5, 17)
