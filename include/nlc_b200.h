@@ -423,6 +423,19 @@ typedef struct nlc_batch_planner_s* nlc_batch_planner_t;
  * reproduces nlc_planner_create(desc with seed = seeds[i]).                                         */
 int nlc_batch_planner_create(nlc_batch_planner_t* out, nlc_model_t model, const nlc_planner_desc* desc, int n_instances,
                              const uint64_t* seeds_host, int device);
+/* The same with a model and a delay of its own per instance (the reference's env x delay x model x seed grid, one checkpoint
+ * per task, run_exp_multi.py:135-165): instance i reproduces nlc_planner_create(model_of_instance[i], desc with
+ * rollout.delay = delay_of_instance[i] and seed = seeds[i]).  model_of_instance [I]: every entry a model for Neural Laplace
+ * dynamics, every entry NULL (or the array NULL) for the analytic dynamics - the two are not mixed.  delay_of_instance [I]
+ * (NULL: desc->rollout.delay for all), each in [0, B); the Neural Laplace rollout does not read it.  Models may differ in
+ * hidden_units, s_terms, encode_obs_time and normalisation; each must match desc->nx / desc->mppi.nu, live on `device` and
+ * not have been destroyed.  The handle takes one reference on each distinct model.
+ * The instances are planned in RUNS, maximal ranges of consecutive instances with the same (model, delay): one encoder and
+ * one rollout launch per run over its samples, on that model's kernels.  Several runs go side by side on a small pool of
+ * streams the handle owns, forked from the caller's stream after stage 1 and joined back before stage 4; one run (e.g.
+ * nlc_batch_planner_create) launches on the caller's stream only.  Order the instances so that runs are long.              */
+int nlc_batch_planner_create_multi(nlc_batch_planner_t* out, const nlc_model_t* model_of_instance, const int32_t* delay_of_instance,
+                                   const nlc_planner_desc* desc, int n_instances, const uint64_t* seeds_host, int device);
 int nlc_batch_planner_destroy(nlc_batch_planner_t p);
 /* U_host fp64 [n_instances][T][nu]                                                                  */
 int nlc_batch_planner_set_U(nlc_batch_planner_t p, const double* U_host);
@@ -430,7 +443,8 @@ int nlc_batch_planner_set_U(nlc_batch_planner_t p, const double* U_host);
 int nlc_batch_planner_buffer(nlc_batch_planner_t p, int which, void** dev_ptr, int64_t* n_floats);
 /* MPPIDelay.command for every instance: state_dev [I][nx], action_buffer_dev [I][B][nu],
  * noise_in_dev [I][K][T][nu] or NULL (on-device sampler), action_dev [I][nu] (env units).
- * Stage 1 and 4 run per instance, the encoder and the rollout once over all I*K samples.            */
+ * Stage 1 and 4 run per instance, the encoder and the rollout once per run over its samples.  Every model is checked to
+ * be folded for desc->rollout.dt, as nlc_planner_step does.                                        */
 int nlc_batch_planner_command(nlc_batch_planner_t p, const float* state_dev, const float* action_buffer_dev,
                               const float* noise_in_dev, float* action_dev, void* stream);
 
@@ -447,6 +461,15 @@ int nlc_env_step(const nlc_rollout_opts* o, float* state_dev, float* action_buff
  * [0, B), B in [1, 8], nu that of env; reward_dev [I] may be NULL.  The argument checks run before any CUDA call.       */
 int nlc_env_step_f64(int env, int delay, double dt, double* state_dev, double* action_buffer_dev, const double* action_dev,
                      int I, int B, int nu, double* reward_dev, void* stream);
+/* nlc_env_step / nlc_env_step_f64 with one delay per instance: delay_dev [I] int32 on the device (o->delay is not read).
+ * The host-side argument checks run before any CUDA call.  The delays are checked on the device: an entry outside [0, B)
+ * sets *status_dev = 1 (a device word the caller zeroes and reads; the call does not synchronise) and leaves that
+ * instance's state, buffer and reward untouched.                                                     */
+int nlc_env_step_delays(const nlc_rollout_opts* o, const int32_t* delay_dev, float* state_dev, float* action_buffer_dev,
+                        const float* action_dev, int I, int B, int nu, float* reward_dev, unsigned int* status_dev, void* stream);
+int nlc_env_step_f64_delays(int env, const int32_t* delay_dev, double dt, double* state_dev, double* action_buffer_dev,
+                            const double* action_dev, int I, int B, int nu, double* reward_dev, unsigned int* status_dev,
+                            void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Generic Fourier-series inverse Laplace transform (torchlaplace's Fourier ILT as called from

@@ -129,12 +129,16 @@ SIGNATURES = {
     "nlc_planner_f64_command_host": (C.c_int, [C.c_void_p, _dp, _dp, _dp, C.c_void_p]),
     "nlc_batch_planner_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.POINTER(PlannerDesc), C.c_int,
                                            C.POINTER(C.c_uint64), C.c_int]),
+    "nlc_batch_planner_create_multi": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int32),
+                                                 C.POINTER(PlannerDesc), C.c_int, C.POINTER(C.c_uint64), C.c_int]),
     "nlc_batch_planner_destroy": (C.c_int, [C.c_void_p]),
     "nlc_batch_planner_set_U": (C.c_int, [C.c_void_p, _dp]),
     "nlc_batch_planner_buffer": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),
     "nlc_batch_planner_command": (C.c_int, [C.c_void_p, _fp, _fp, _fp, _fp, C.c_void_p]),
     "nlc_env_step": (C.c_int, [C.POINTER(RolloutOpts), _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_void_p]),
     "nlc_env_step_f64": (C.c_int, [C.c_int, C.c_int, C.c_double, _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_void_p]),
+    "nlc_env_step_delays": (C.c_int, [C.POINTER(RolloutOpts), _fp, _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, _fp, C.c_void_p]),
+    "nlc_env_step_f64_delays": (C.c_int, [C.c_int, _fp, C.c_double, _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, _fp, C.c_void_p]),
     "nlc_ilt_fourier": (C.c_int, [_fp, _fp, C.c_int, C.c_int64, C.c_int, C.c_int, _fp, C.c_void_p]),
     "nlc_selftest_umma_gemm_ts": (C.c_int, [_fp, _fp, C.c_int, C.c_int, C.c_int, C.c_int, _fp, C.c_void_p]),
     "nlc_selftest_umma_gemm": (C.c_int, [_fp, _fp, C.c_int, C.c_int, C.c_int, C.c_int, _fp, C.c_void_p]),

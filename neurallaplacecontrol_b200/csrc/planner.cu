@@ -652,16 +652,29 @@ extern "C" int nlc_planner_command_host(nlc_planner_t p, const double* state_hos
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// Instance-batched planner (BASELINE config 5: many env x seed instances planning in the same control step).
-// I independent MPPIDelay objects of one environment / model share ONE wide encoder launch and ONE rollout launch over
-// the concatenated I*K samples (both kernels are row-independent; the rollout reads each instance's state through the
-// rows-per-state form of `state_per_sample`); stage 1 and stage 4 run per instance on the instance's contiguous slices
-// with the same kernels - and hence the same arithmetic - as the single planner, so instance i of a batch reproduces a
-// stand-alone planner with the same seed.
+// Instance-batched planner (BASELINE config 5: many env x delay x seed instances planning in the same control step).
+// I independent MPPIDelay objects of one environment; stage 1 and stage 4 run per instance on the instance's contiguous
+// slices with the same kernels - and hence the same arithmetic - as the single planner.  Between them the instances are
+// planned in RUNS: maximal ranges of consecutive instances with the same model and delay.  A run is ONE encoder launch and
+// ONE rollout launch over its n*K samples (both kernels are row-independent; the rollout reads each instance's state through
+// the rows-per-state form of `state_per_sample`), on its own model's kernels.  So instance i of a batch reproduces a
+// stand-alone planner with the same model, delay and seed.
+// With one run (one model for every instance: nlc_batch_planner_create) the launches go to the caller's stream.  With more,
+// the runs are spread round-robin over a small pool of the handle's own streams, forked from the caller's stream after stage 1
+// and joined back before stage 4, so the runs' kernels fill the GPU side by side.  Runs write disjoint slices of the handle's
+// buffers, and nlc_encode_history / nlc_rollout_cost write nothing owned by the model handle (its arena holds weights and
+// folded constants, read only; every output and scratch pointer is an argument), so two runs of one model may be in flight
+// at once.
 // ------------------------------------------------------------------------------------------------------------------
+// Streams of the fan-out pool (tools/bench_fanout.py, DESIGN.md "Many models in one batch"); NLC_FANOUT_STREAMS overrides it
+// for that measurement.
+constexpr int kFanoutStreams = 4;
+
 struct nlc_batch_planner_s {
+  struct Run { int i0, n; nlc_model_t model; int delay; };
   int device, I;
-  nlc_model_t model;
+  std::vector<Run> runs;
+  std::vector<nlc_model_t> models;  // the distinct models of the runs, one reference each
   nlc_planner_desc d;          // per instance (mppi.K = samples per instance)
   std::vector<uint64_t> seeds;
   uint64_t calls;
@@ -669,14 +682,25 @@ struct nlc_batch_planner_s {
   float *U, *U_rolled, *noise, *perturbed, *hist, *actions, *pert_cost, *p, *cost_total, *weights, *states, *triple, *stats;
   char* softmax_ws;
   size_t ws_stride;
+  std::vector<cudaStream_t> pool;   // empty with one run
+  cudaEvent_t ev_fork;
+  std::vector<cudaEvent_t> ev_join; // one per pool stream
 };
 
-extern "C" int nlc_batch_planner_create(nlc_batch_planner_t* out, nlc_model_t model, const nlc_planner_desc* d, int n_instances,
-                                        const uint64_t* seeds, int device) {
+static void batch_planner_free(nlc_batch_planner_s* p) {
+  for (cudaStream_t st : p->pool) if (st) cudaStreamDestroy(st);
+  for (cudaEvent_t e : p->ev_join) if (e) cudaEventDestroy(e);
+  if (p->ev_fork) cudaEventDestroy(p->ev_fork);
+  if (p->arena) cudaFree(p->arena);
+  cudaGetLastError();
+  delete p;
+}
+
+extern "C" int nlc_batch_planner_create_multi(nlc_batch_planner_t* out, const nlc_model_t* model_of_instance,
+                                              const int32_t* delay_of_instance, const nlc_planner_desc* d, int n_instances,
+                                              const uint64_t* seeds, int device) {
   NLC_REQUIRE(out && d && seeds, NLC_ERR_ARG, "nlc_batch_planner_create: null argument");
   *out = nullptr;
-  int rc = check_device_arch(device);
-  if (rc != NLC_OK) return rc;
   const nlc_mppi_params& mp = d->mppi;
   NLC_REQUIRE(n_instances >= 1 && n_instances <= 4096, NLC_ERR_ARG, "batch planner: 1..4096 instances");
   NLC_REQUIRE(mp.K >= 1 && mp.T >= 1 && mp.B >= 1 && mp.B <= 8, NLC_ERR_SHAPE, "batch planner: K, T >= 1 and 1 <= B <= 8 required");
@@ -685,16 +709,43 @@ extern "C" int nlc_batch_planner_create(nlc_batch_planner_t* out, nlc_model_t mo
   NLC_REQUIRE(d->n_shards == 1 && d->shard_index == 0, NLC_ERR_UNSUPPORTED, "batch planner: instances are not K-sharded (shard by instance)");
   NLC_REQUIRE(mp.lambda_ > 0.0f, NLC_ERR_ARG, "batch planner: lambda must be positive");
   NLC_REQUIRE((long long)n_instances * mp.K <= 0x7fffffffLL / (mp.T * 4), NLC_ERR_SHAPE, "batch planner: I*K*T too large");
-  if (d->rollout.dynamics == NLC_DYN_NEURAL_LAPLACE) {
-    NLC_REQUIRE(model != nullptr, NLC_ERR_ARG, "batch planner: Neural Laplace dynamics need a model handle");
-    NLC_REQUIRE(model->device == device, NLC_ERR_ARG, "batch planner: model lives on device %d, planner on %d", model->device, device);
-    NLC_REQUIRE(model->nx == d->nx && model->nu == mp.nu, NLC_ERR_SHAPE, "batch planner: model dims do not match");
-  }
   // stage 4 reads each instance's cost slice 16 bytes wide (nlc_softmax_partial): instance i starts at cost_total + i*K
   NLC_REQUIRE(n_instances == 1 || mp.K % 4 == 0, NLC_ERR_SHAPE, "batch planner: samples per instance (%d) must be a multiple of 4", mp.K);
-  NLC_REQUIRE(model == nullptr || !model->destroy_requested, NLC_ERR_ARG, "batch planner: the model handle has been destroyed");
+  const bool nl = d->rollout.dynamics == NLC_DYN_NEURAL_LAPLACE;
+  NLC_REQUIRE(nl || d->rollout.dynamics == NLC_DYN_ANALYTIC_DELAY, NLC_ERR_ARG, "batch planner: unknown dynamics kind %d", d->rollout.dynamics);
+  // host-side checks first (they run without a device): delays, and which instances carry a model
+  for (int i = 0; i < n_instances; ++i) {
+    const int delay = delay_of_instance ? delay_of_instance[i] : d->rollout.delay;
+    NLC_REQUIRE(delay >= 0 && delay < mp.B, NLC_ERR_ARG, "batch planner: instance %d has delay %d outside the %d-entry action buffer",
+                i, delay, mp.B);
+    const bool has_model = model_of_instance && model_of_instance[i];
+    NLC_REQUIRE(has_model == nl, NLC_ERR_ARG, nl ? "batch planner: Neural Laplace dynamics need a model handle for every instance "
+                                                  "(instance %d has none; analytic and Neural Laplace instances are not mixed)"
+                                                : "batch planner: analytic dynamics take no model handle (instance %d has one; analytic "
+                                                  "and Neural Laplace instances are not mixed)", i);
+  }
+  int rc = check_device_arch(device);
+  if (rc != NLC_OK) return rc;
+  std::vector<nlc_batch_planner_s::Run> runs;
+  std::vector<nlc_model_t> models;
+  for (int i = 0; i < n_instances; ++i) {
+    const nlc_model_t m = nl ? model_of_instance[i] : nullptr;
+    const int delay = delay_of_instance ? delay_of_instance[i] : d->rollout.delay;
+    if (m) {
+      NLC_REQUIRE(!m->destroy_requested, NLC_ERR_ARG, "batch planner: the model handle of instance %d has been destroyed", i);
+      NLC_REQUIRE(m->device == device, NLC_ERR_ARG, "batch planner: instance %d's model lives on device %d, planner on %d", i, m->device, device);
+      NLC_REQUIRE(m->nx == d->nx && m->nu == mp.nu, NLC_ERR_SHAPE, "batch planner: instance %d's model dims (%d, %d) do not match (%d, %d)",
+                  i, m->nx, m->nu, d->nx, mp.nu);
+      bool seen = false;
+      for (nlc_model_t x : models) seen = seen || x == m;
+      if (!seen) models.push_back(m);
+    }
+    if (!runs.empty() && runs.back().model == m && runs.back().delay == delay) runs.back().n++;
+    else runs.push_back({i, 1, m, delay});
+  }
   nlc_batch_planner_s* p = new nlc_batch_planner_s();
-  p->device = device; p->I = n_instances; p->model = model; p->d = *d; p->calls = 0; p->arena = nullptr;
+  p->device = device; p->I = n_instances; p->d = *d; p->calls = 0; p->arena = nullptr; p->ev_fork = nullptr;
+  p->runs = runs; p->models = models;
   p->seeds.assign(seeds, seeds + n_instances);
   const size_t I = n_instances, K = mp.K, T = mp.T, nu = mp.nu, B = mp.B, nx = d->nx, L = B - 1 + T, TN = T * nu, IK = I * K;
   p->ws_stride = ((size_t)nlc_softmax_workspace_bytes((int)K, (int)TN) + 255) / 256 * 256;
@@ -703,7 +754,7 @@ extern "C" int nlc_batch_planner_create(nlc_batch_planner_t* out, nlc_model_t mo
   std::vector<size_t> offs;
   size_t total = 0;
   for (size_t s : sizes) { offs.push_back(total); total += (s + 63) / 64 * 64; }
-  auto fail = [&](int code) { if (p->arena) cudaFree(p->arena); delete p; return code; };
+  auto fail = [&](int code) { batch_planner_free(p); return code; };
   if (cudaSetDevice(device) != cudaSuccess) { set_error("cudaSetDevice failed"); return fail(NLC_ERR_CUDA); }
   if (cudaMalloc(&p->arena, total * sizeof(float)) != cudaSuccess) { cudaGetLastError(); p->arena = nullptr; set_error("batch planner: cudaMalloc(%zu) failed", total * sizeof(float)); return fail(NLC_ERR_NOMEM); }
   if (cudaMemset(p->arena, 0, total * sizeof(float)) != cudaSuccess) { set_error("batch planner: memset failed"); return fail(NLC_ERR_CUDA); }
@@ -713,18 +764,38 @@ extern "C" int nlc_batch_planner_create(nlc_batch_planner_t* out, nlc_model_t mo
   for (size_t i = 0; i < sizeof(slots) / sizeof(slots[0]); ++i) *slots[i] = base + offs[i];
   if (!d->keep_states) p->states = nullptr;
   p->softmax_ws = reinterpret_cast<char*>(base + offs[13]);
-  if (model) model->refs++;
+  if (runs.size() > 1) {
+    int n_streams = kFanoutStreams;
+    if (const char* e = getenv("NLC_FANOUT_STREAMS")) if (atoi(e) >= 1) n_streams = atoi(e);
+    if ((size_t)n_streams > runs.size()) n_streams = (int)runs.size();
+    p->pool.assign(n_streams, nullptr);
+    p->ev_join.assign(n_streams, nullptr);
+    bool ok = cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming) == cudaSuccess;
+    for (int j = 0; ok && j < n_streams; ++j)
+      ok = cudaStreamCreateWithFlags(&p->pool[j], cudaStreamNonBlocking) == cudaSuccess &&
+           cudaEventCreateWithFlags(&p->ev_join[j], cudaEventDisableTiming) == cudaSuccess;
+    if (!ok) { cudaGetLastError(); set_error("batch planner: fan-out streams could not be created"); return fail(NLC_ERR_NOMEM); }
+  }
+  for (nlc_model_t m : models) m->refs++;
   *out = p;
   return NLC_OK;
+}
+
+extern "C" int nlc_batch_planner_create(nlc_batch_planner_t* out, nlc_model_t model, const nlc_planner_desc* d, int n_instances,
+                                        const uint64_t* seeds, int device) {
+  NLC_REQUIRE(out && d && seeds, NLC_ERR_ARG, "nlc_batch_planner_create: null argument");
+  NLC_REQUIRE(n_instances >= 1 && n_instances <= 4096, NLC_ERR_ARG, "batch planner: 1..4096 instances");
+  // one model (none for the analytic dynamics) and the desc's delay for every instance: a single run
+  const std::vector<nlc_model_t> models(n_instances, d->rollout.dynamics == NLC_DYN_NEURAL_LAPLACE ? model : nullptr);
+  return nlc_batch_planner_create_multi(out, models.data(), nullptr, d, n_instances, seeds, device);
 }
 
 extern "C" int nlc_batch_planner_destroy(nlc_batch_planner_t p) {
   if (!p) return NLC_OK;
   cudaSetDevice(p->device);
   cudaDeviceSynchronize();
-  model_release(p->model);
-  if (p->arena) cudaFree(p->arena);
-  delete p;
+  for (nlc_model_t m : p->models) model_release(m);
+  batch_planner_free(p);
   return NLC_OK;
 }
 
@@ -751,6 +822,22 @@ extern "C" int nlc_batch_planner_buffer(nlc_batch_planner_t p, int which, void**
   return NLC_OK;
 }
 
+// stages 2a + 2b/3 of one run: the encoder and the rollout over the run's contiguous n*K samples, on its own model
+static int batch_run_stages(nlc_batch_planner_t p, const nlc_batch_planner_s::Run& r, const float* state_dev, cudaStream_t s) {
+  const nlc_mppi_params& mp = p->d.mppi;
+  const size_t K = mp.K, T = mp.T, nu = mp.nu, B = mp.B, L = B - 1 + T, nx = p->d.nx, o = (size_t)r.i0 * K;
+  const int n = (int)(r.n * K);
+  nlc_rollout_opts ro = p->d.rollout;
+  ro.delay = r.delay;
+  if (ro.dynamics == NLC_DYN_NEURAL_LAPLACE) {
+    int rc = nlc_encode_history(r.model, p->hist + o * L * nu, n, (int)T, (int)B, p->p + o * T * 2, p->d.math_mode, s);
+    if (rc != NLC_OK) return rc;
+  }
+  // sample k of the run reads the state of instance i0 + k / K
+  return nlc_rollout_cost(r.model, &ro, state_dev + (size_t)r.i0 * nx, (int)K, p->p + o * T * 2, p->hist + o * L * nu, p->pert_cost + o,
+                          n, (int)T, (int)B, (int)nu, p->cost_total + o, p->states ? p->states + o * T * nx : nullptr, p->d.math_mode, s);
+}
+
 extern "C" int nlc_batch_planner_command(nlc_batch_planner_t p, const float* state_dev, const float* action_buffer_dev,
                                          const float* noise_in_dev, float* action_dev, void* stream) {
   NLC_REQUIRE(p && state_dev && action_buffer_dev && action_dev, NLC_ERR_ARG, "nlc_batch_planner_command: null argument");
@@ -760,11 +847,10 @@ extern "C" int nlc_batch_planner_command(nlc_batch_planner_t p, const float* sta
   NLC_CUDA_OK(cudaSetDevice(p->device));
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   int rc;
-  if (p->d.rollout.dynamics == NLC_DYN_NEURAL_LAPLACE) {
-    const double want = (double)p->d.rollout.dt;
-    NLC_REQUIRE(!p->model->destroy_requested && fabs(p->model->ts_pred - want) <= 1e-6 * fabs(want), NLC_ERR_ARG,
-                "batch planner: the model is folded for prediction time %.9g, not dt = %.9g", p->model->ts_pred, want);
-  }
+  const double want = (double)p->d.rollout.dt;
+  for (nlc_model_t m : p->models)  // every run rolls out on constants folded for dt
+    NLC_REQUIRE(!m->destroy_requested && fabs(m->ts_pred - want) <= 1e-6 * fabs(want), NLC_ERR_ARG,
+                "batch planner: the model is folded for prediction time %.9g, not dt = %.9g", m->ts_pred, want);
   for (int i = 0; i < I; ++i) {  // stage 1 per instance (its own U, action buffer and RNG stream)
     const size_t o = (size_t)i * K;
     rc = nlc_perturb(&mp, p->U + i * TN, p->U_rolled + i * TN, 1, noise_in_dev ? noise_in_dev + o * TN : nullptr, p->seeds[i], p->calls,
@@ -773,15 +859,22 @@ extern "C" int nlc_batch_planner_command(nlc_batch_planner_t p, const float* sta
     if (rc != NLC_OK) return rc;
   }
   p->calls++;
-  const int IK = (int)(I * K);
-  if (p->d.rollout.dynamics == NLC_DYN_NEURAL_LAPLACE) {  // stage 2a: every window of every instance in one pass
-    rc = nlc_encode_history(p->model, p->hist, IK, (int)T, (int)B, p->p, p->d.math_mode, stream);
+  if (p->pool.empty()) {  // one run: every window of every instance in one encoder pass, one rollout launch
+    rc = batch_run_stages(p, p->runs[0], state_dev, s);
+    if (rc != NLC_OK) return rc;
+  } else {
+    const int P = (int)p->pool.size();
+    NLC_CUDA_OK(cudaEventRecord(p->ev_fork, s));
+    for (int j = 0; j < P; ++j) NLC_CUDA_OK(cudaStreamWaitEvent(p->pool[j], p->ev_fork, 0));
+    rc = NLC_OK;
+    for (size_t r = 0; r < p->runs.size() && rc == NLC_OK; ++r) rc = batch_run_stages(p, p->runs[r], state_dev, p->pool[r % P]);
+    // joined even after a failed launch: the caller's stream never runs ahead of work issued on the pool
+    for (int j = 0; j < P; ++j) {
+      NLC_CUDA_OK(cudaEventRecord(p->ev_join[j], p->pool[j]));
+      NLC_CUDA_OK(cudaStreamWaitEvent(s, p->ev_join[j], 0));
+    }
     if (rc != NLC_OK) return rc;
   }
-  // stages 2b+3: one launch; sample k reads the state of instance k / K
-  rc = nlc_rollout_cost(p->model, &p->d.rollout, state_dev, (int)K, p->p, p->hist, p->pert_cost, IK, (int)T, (int)B, (int)nu,
-                        p->cost_total, p->states, p->d.math_mode, stream);
-  if (rc != NLC_OK) return rc;
   NLC_CUDA_OK(cudaMemcpyAsync(p->U, p->U_rolled, sizeof(float) * I * TN, cudaMemcpyDeviceToDevice, s));
   for (int i = 0; i < I; ++i) {  // stage 4 per instance
     const size_t o = (size_t)i * K;

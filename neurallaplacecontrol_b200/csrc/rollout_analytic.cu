@@ -48,16 +48,21 @@ int launch_rollout_analytic(const nlc_rollout_opts* o, int nx, const float* stat
 // buffer and pick the delayed action (get_action, :25-28), advance the state by one explicit-Euler step of the true
 // dynamics (base_env.py:136-173 integrate_system(2, ...) as stated analytically by oracle.py:11-224, observation form),
 // reward of the new state with the applied action (base_env.py diff_reward = -running_cost).
+// delays (optional, [I]): instance i's own delay instead of o.delay.  An entry outside [0, B) sets *status = 1 and leaves
+// that instance's state, buffer and reward untouched.
 template <int NX>
-__global__ void env_step_kernel(nlc_rollout_opts o, float* __restrict__ state, float* __restrict__ abuf,
-                                const float* __restrict__ action, int I, int B, int nu, float* __restrict__ reward) {
+__global__ void env_step_kernel(nlc_rollout_opts o, const int32_t* __restrict__ delays, float* __restrict__ state,
+                                float* __restrict__ abuf, const float* __restrict__ action, int I, int B, int nu,
+                                float* __restrict__ reward, unsigned int* __restrict__ status) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= I) return;
+  const int delay = delays ? delays[i] : o.delay;
+  if (delay < 0 || delay >= B) { if (status) *status = 1u; return; }
   float* b = abuf + (size_t)i * B * nu;
   for (int j = 0; j + 1 < B; ++j)
     for (int u = 0; u < nu; ++u) b[j * nu + u] = b[(j + 1) * nu + u];
   for (int u = 0; u < nu; ++u) b[(B - 1) * nu + u] = action[(size_t)i * nu + u];
-  const float* at = b + (size_t)(B - 1 - o.delay) * nu;
+  const float* at = b + (size_t)(B - 1 - delay) * nu;
   float s[NX];
 #pragma unroll
   for (int c = 0; c < NX; ++c) s[c] = state[(size_t)i * NX + c];
@@ -70,10 +75,13 @@ __global__ void env_step_kernel(nlc_rollout_opts o, float* __restrict__ state, f
 // env_step_kernel in fp64 (the closed loop around the fp64 planner): the same buffer roll and delayed action, the fp64 Euler
 // step and running cost of env_cost.cuh that the fp64 planner's analytic rollout uses, dt in fp64.
 template <int NX>
-__global__ void env_step_f64_kernel(int env, int delay, double dt, double* __restrict__ state, double* __restrict__ abuf,
-                                    const double* __restrict__ action, int I, int B, int nu, double* __restrict__ reward) {
+__global__ void env_step_f64_kernel(int env, int delay0, const int32_t* __restrict__ delays, double dt, double* __restrict__ state,
+                                    double* __restrict__ abuf, const double* __restrict__ action, int I, int B, int nu,
+                                    double* __restrict__ reward, unsigned int* __restrict__ status) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= I) return;
+  const int delay = delays ? delays[i] : delay0;
+  if (delay < 0 || delay >= B) { if (status) *status = 1u; return; }
   double* b = abuf + (size_t)i * B * nu;
   for (int j = 0; j + 1 < B; ++j)
     for (int u = 0; u < nu; ++u) b[j * nu + u] = b[(j + 1) * nu + u];
@@ -88,48 +96,71 @@ __global__ void env_step_f64_kernel(int env, int delay, double dt, double* __res
   if (reward) reward[i] = -env_running_cost(env, 0, 0.0, s, at, nu);
 }
 
-}  // namespace nlc
-
-extern "C" int nlc_env_step(const nlc_rollout_opts* o, float* state_dev, float* action_buffer_dev, const float* action_dev,
-                            int I, int B, int nu, float* reward_dev, void* stream) {
-  using namespace nlc;
-  NLC_REQUIRE(o && state_dev && action_buffer_dev && action_dev, NLC_ERR_ARG, "nlc_env_step: null pointer");
-  NLC_REQUIRE(I >= 1 && B >= 1 && B <= 8, NLC_ERR_ARG, "nlc_env_step: I >= 1 and 1 <= B <= 8 required");
-  NLC_REQUIRE(o->env >= NLC_ENV_PENDULUM && o->env <= NLC_ENV_ACROBOT, NLC_ERR_ARG, "unknown env id %d", o->env);
-  NLC_REQUIRE(o->delay >= 0 && o->delay < B, NLC_ERR_ARG, "nlc_env_step: delay %d outside the %d-entry action buffer", o->delay, B);
-  const int env_nu[3] = {1, 1, 2};
-  NLC_REQUIRE(nu == env_nu[o->env], NLC_ERR_SHAPE, "env %d takes nu=%d actions, got %d", o->env, env_nu[o->env], nu);
-  int dev = 0;
-  NLC_CUDA_OK(cudaGetDevice(&dev));
-  int rc = check_device_arch(dev);
-  if (rc != NLC_OK) return rc;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const int grid = (I + 127) / 128;
-  if (o->env == NLC_ENV_PENDULUM) env_step_kernel<3><<<grid, 128, 0, s>>>(*o, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
-  else if (o->env == NLC_ENV_CARTPOLE) env_step_kernel<5><<<grid, 128, 0, s>>>(*o, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
-  else env_step_kernel<6><<<grid, 128, 0, s>>>(*o, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
-  NLC_LAUNCH_OK("env_step_kernel");
-  return NLC_OK;
-}
-
-extern "C" int nlc_env_step_f64(int env, int delay, double dt, double* state_dev, double* action_buffer_dev, const double* action_dev,
-                                int I, int B, int nu, double* reward_dev, void* stream) {
-  using namespace nlc;
-  NLC_REQUIRE(state_dev && action_buffer_dev && action_dev, NLC_ERR_ARG, "nlc_env_step_f64: null pointer");
-  NLC_REQUIRE(I >= 1 && B >= 1 && B <= 8, NLC_ERR_ARG, "nlc_env_step_f64: I >= 1 and 1 <= B <= 8 required");
+// The argument checks of both precisions, before any CUDA call.  delay_dev == nullptr: the scalar delay, checked here;
+// otherwise the per-instance delays, checked on the device (status_dev required).
+static int env_step_check(const char* name, int env, int delay, const int32_t* delay_dev, unsigned int* status_dev, const void* state_dev,
+                          const void* action_buffer_dev, const void* action_dev, int I, int B, int nu) {
+  NLC_REQUIRE(state_dev && action_buffer_dev && action_dev, NLC_ERR_ARG, "%s: null pointer", name);
+  NLC_REQUIRE(!delay_dev || status_dev, NLC_ERR_ARG, "%s: per-instance delays need a status word", name);
+  NLC_REQUIRE(I >= 1 && B >= 1 && B <= 8, NLC_ERR_ARG, "%s: I >= 1 and 1 <= B <= 8 required", name);
   NLC_REQUIRE(env >= NLC_ENV_PENDULUM && env <= NLC_ENV_ACROBOT, NLC_ERR_ARG, "unknown env id %d", env);
-  NLC_REQUIRE(delay >= 0 && delay < B, NLC_ERR_ARG, "nlc_env_step_f64: delay %d outside the %d-entry action buffer", delay, B);
+  NLC_REQUIRE(delay_dev || (delay >= 0 && delay < B), NLC_ERR_ARG, "%s: delay %d outside the %d-entry action buffer", name, delay, B);
   const int env_nu[3] = {1, 1, 2};
   NLC_REQUIRE(nu == env_nu[env], NLC_ERR_SHAPE, "env %d takes nu=%d actions, got %d", env, env_nu[env], nu);
   int dev = 0;
   NLC_CUDA_OK(cudaGetDevice(&dev));
-  int rc = check_device_arch(dev);
+  return check_device_arch(dev);
+}
+
+static int env_step_launch(const nlc_rollout_opts* o, const int32_t* delay_dev, float* state_dev, float* action_buffer_dev,
+                           const float* action_dev, int I, int B, int nu, float* reward_dev, unsigned int* status_dev, void* stream) {
+  NLC_REQUIRE(o, NLC_ERR_ARG, "nlc_env_step: null pointer");
+  int rc = env_step_check("nlc_env_step", o->env, o->delay, delay_dev, status_dev, state_dev, action_buffer_dev, action_dev, I, B, nu);
   if (rc != NLC_OK) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const int grid = (I + 127) / 128;
-  if (env == NLC_ENV_PENDULUM) env_step_f64_kernel<3><<<grid, 128, 0, s>>>(env, delay, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
-  else if (env == NLC_ENV_CARTPOLE) env_step_f64_kernel<5><<<grid, 128, 0, s>>>(env, delay, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
-  else env_step_f64_kernel<6><<<grid, 128, 0, s>>>(env, delay, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev);
+  if (o->env == NLC_ENV_PENDULUM) env_step_kernel<3><<<grid, 128, 0, s>>>(*o, delay_dev, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev, status_dev);
+  else if (o->env == NLC_ENV_CARTPOLE) env_step_kernel<5><<<grid, 128, 0, s>>>(*o, delay_dev, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev, status_dev);
+  else env_step_kernel<6><<<grid, 128, 0, s>>>(*o, delay_dev, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev, status_dev);
+  NLC_LAUNCH_OK("env_step_kernel");
+  return NLC_OK;
+}
+
+static int env_step_f64_launch(int env, int delay, const int32_t* delay_dev, double dt, double* state_dev, double* action_buffer_dev,
+                               const double* action_dev, int I, int B, int nu, double* reward_dev, unsigned int* status_dev, void* stream) {
+  int rc = env_step_check("nlc_env_step_f64", env, delay, delay_dev, status_dev, state_dev, action_buffer_dev, action_dev, I, B, nu);
+  if (rc != NLC_OK) return rc;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int grid = (I + 127) / 128;
+  if (env == NLC_ENV_PENDULUM) env_step_f64_kernel<3><<<grid, 128, 0, s>>>(env, delay, delay_dev, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev, status_dev);
+  else if (env == NLC_ENV_CARTPOLE) env_step_f64_kernel<5><<<grid, 128, 0, s>>>(env, delay, delay_dev, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev, status_dev);
+  else env_step_f64_kernel<6><<<grid, 128, 0, s>>>(env, delay, delay_dev, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev, status_dev);
   NLC_LAUNCH_OK("env_step_f64_kernel");
   return NLC_OK;
+}
+
+}  // namespace nlc
+
+extern "C" int nlc_env_step(const nlc_rollout_opts* o, float* state_dev, float* action_buffer_dev, const float* action_dev,
+                            int I, int B, int nu, float* reward_dev, void* stream) {
+  return nlc::env_step_launch(o, nullptr, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev, nullptr, stream);
+}
+
+extern "C" int nlc_env_step_delays(const nlc_rollout_opts* o, const int32_t* delay_dev, float* state_dev, float* action_buffer_dev,
+                                   const float* action_dev, int I, int B, int nu, float* reward_dev, unsigned int* status_dev,
+                                   void* stream) {
+  NLC_REQUIRE(delay_dev, NLC_ERR_ARG, "nlc_env_step_delays: null delays");
+  return nlc::env_step_launch(o, delay_dev, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev, status_dev, stream);
+}
+
+extern "C" int nlc_env_step_f64(int env, int delay, double dt, double* state_dev, double* action_buffer_dev, const double* action_dev,
+                                int I, int B, int nu, double* reward_dev, void* stream) {
+  return nlc::env_step_f64_launch(env, delay, nullptr, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev, nullptr, stream);
+}
+
+extern "C" int nlc_env_step_f64_delays(int env, const int32_t* delay_dev, double dt, double* state_dev, double* action_buffer_dev,
+                                       const double* action_dev, int I, int B, int nu, double* reward_dev, unsigned int* status_dev,
+                                       void* stream) {
+  NLC_REQUIRE(delay_dev, NLC_ERR_ARG, "nlc_env_step_f64_delays: null delays");
+  return nlc::env_step_f64_launch(env, 0, delay_dev, dt, state_dev, action_buffer_dev, action_dev, I, B, nu, reward_dev, status_dev, stream);
 }

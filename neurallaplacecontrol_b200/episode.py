@@ -5,11 +5,13 @@ The reference evaluates one (env, delay, model, seed) instance per process: ``lo
 one Euler step of the true dynamics, reward) and a host round trip per control step (``:254,267``).  Here ``I`` instances
 of one environment share every kernel launch and nothing leaves the device inside the loop:
 
-* :class:`BatchedMPPIDelay` - ``I`` independent ``MPPIDelay`` objects (own control sequence, action buffer, sampler seed):
-  stage 1 and stage 4 per instance, ONE encoder launch and ONE rollout launch over all ``I*K`` samples
-  (``nlc_batch_planner_*``).  Instance ``i`` reproduces a stand-alone ``MPPIDelay(..., seed=seeds[i])``.
+* :class:`BatchedMPPIDelay` - ``I`` independent ``MPPIDelay`` objects (own control sequence, action buffer, sampler seed,
+  and optionally own model or analytic delay): stage 1 and stage 4 per instance, ONE encoder launch and ONE rollout launch
+  per run of consecutive instances sharing a model (``nlc_batch_planner_*``), the runs side by side on the GPU.  Instance
+  ``i`` reproduces a stand-alone ``MPPIDelay(dynamics_i, ..., seed=seeds[i])``.
 * :func:`env_step` - ``step_env`` for ``I`` instances on the device (``nlc_env_step``, or ``nlc_env_step_f64`` on fp64
-  tensors; dynamics as stated by the reference's ``oracle.py:11-224``, golden-pinned in ``tests/golden/env_step_*.npz``).
+  tensors, ``*_delays`` with one action delay per instance; dynamics as stated by the reference's ``oracle.py:11-224``,
+  golden-pinned in ``tests/golden/env_step_*.npz``).
 * :func:`run_closed_loop` - ``loop()`` for ``I`` instances of a ``BatchedMPPIDelay``, or in fp64 over one
   ``MPPIDelay(math_mode="fp64")`` per instance; returns the reference's result keys per instance.
 
@@ -23,15 +25,22 @@ import time
 import torch
 
 from . import _lib
+from .closures import AnalyticDelayDynamics, NLDynamics
 from .planners.mppi_delay import MPPIDelay, _MPPIDelayF64, _buffer_view
 
 
 class BatchedMPPIDelay:
-    """``n_instances`` planners of one environment / model behind one set of kernel launches.
+    """``n_instances`` planners of one environment behind one set of kernel launches.
 
     Constructor arguments are ``MPPIDelay``'s (``planners/mppi_delay.py:64-90``) plus ``n_instances``, ``seeds``
     (one sampler seed per instance, default ``range(n_instances)``) and ``U_init`` of shape ``(T, nu)`` (shared) or
-    ``(I, T, nu)``.  ``process_group`` is not accepted: a batch is sharded by instance, never by sample (SURVEY 8e)."""
+    ``(I, T, nu)``.  ``process_group`` is not accepted: a batch is sharded by instance, never by sample (SURVEY 8e).
+
+    ``dynamics`` is one handle for every instance, or a sequence of ``n_instances`` handles - all ``NLDynamics`` (each
+    instance plans with its own model; instances holding the same model object share its device handle) or all
+    ``AnalyticDelayDynamics`` (each with its own delay), with one ``dt``.  The reference's grid of one checkpoint per
+    (delay, seed) then plans as one batch: consecutive instances with the same model (or analytic delay) form a run, one
+    encoder and one rollout launch per run, the runs side by side on the GPU.  Keep instances of one model adjacent."""
     _c_buffer, _typestr = "nlc_batch_planner_buffer", "<f4"
 
     def __init__(self, dynamics, running_cost, nx, noise_sigma, n_instances, seeds=None, U_init=None, **kw):
@@ -44,9 +53,10 @@ class BatchedMPPIDelay:
         self.seeds = list(range(self.I)) if seeds is None else [int(s) for s in seeds]
         if len(self.seeds) != self.I:
             raise ValueError("seeds must have one entry per instance")
+        self._dyns = self._check_dynamics(dynamics, nx, running_cost, kw.get("action_buffer_size", 4))
         kw.setdefault("keep_states", False)
         T = kw.get("horizon", 15)
-        self._tpl = MPPIDelay(dynamics, running_cost, nx, noise_sigma, U_init=torch.zeros(T, 1 if torch.as_tensor(noise_sigma).dim() == 0
+        self._tpl = MPPIDelay(self._dyns[0], running_cost, nx, noise_sigma, U_init=torch.zeros(T, 1 if torch.as_tensor(noise_sigma).dim() == 0
                                                                                          else torch.as_tensor(noise_sigma).shape[0]), **kw)
         t = self._tpl
         self.K, self.T, self.nx, self.nu, self.B, self.d, self.dtype = t.K, t.T, t.nx, t.nu, t.B, t.d, t.dtype
@@ -61,19 +71,57 @@ class BatchedMPPIDelay:
         self._lib = _lib.load()
         self._handle, self._handle_B, self._handle_model, self._views, self._calls = None, None, None, {}, 0
 
+    def _check_dynamics(self, dynamics, nx, running_cost, B):
+        """One dynamics handle per instance, checked before anything reaches the device."""
+        if not isinstance(dynamics, (list, tuple)):
+            return [dynamics] * self.I
+        dyns = list(dynamics)
+        if len(dyns) != self.I:
+            raise ValueError(f"dynamics must be one handle or one per instance ({self.I}), got {len(dyns)}")
+        if not (all(isinstance(d, NLDynamics) for d in dyns) or all(isinstance(d, AnalyticDelayDynamics) for d in dyns)):
+            raise TypeError("the dynamics of one batch must be all NLDynamics or all AnalyticDelayDynamics handles")
+        if len({d.dt for d in dyns}) != 1:
+            raise ValueError("the dynamics of one batch must share dt")
+        nu = _lib.ENV_DIMS[running_cost.env_name][1]
+        for i, d in enumerate(dyns):
+            if isinstance(d, NLDynamics) and (d.model.output_dim, d.model.action_dim) != (nx, nu):
+                raise ValueError(f"instance {i}: the model's (state_dim, action_dim) = {(d.model.output_dim, d.model.action_dim)}, "
+                                 f"the batch plans ({nx}, {nu})")
+            if isinstance(d, AnalyticDelayDynamics):
+                if d.env_name != running_cost.env_name:
+                    raise ValueError(f"instance {i}: analytic dynamics of {d.env_name} in a batch of {running_cost.env_name}")
+                if not 0 <= d.delay < int(B):
+                    raise ValueError(f"instance {i}: delay {d.delay} outside the {int(B)}-entry action buffer")
+        return dyns
+
+    def _model_handles(self):
+        """The device handle of every instance's model (None for the analytic dynamics).  Each distinct model is re-fetched
+        on every call (see MPPIDelay._ensure): a rebuilt or re-folded model handle must never be planned on silently."""
+        if not isinstance(self._dyns[0], NLDynamics):
+            return None
+        by_model = {}
+        for d in self._dyns:
+            if id(d.model) not in by_model:
+                if d.model._cuda_device is None:
+                    d.model._cuda_device = self.d
+                by_model[id(d.model)] = self._tpl._fetch_handle(d.model)
+        return [by_model[id(d.model)] for d in self._dyns]
+
     def _ensure(self, B):
-        # the packed model is re-fetched on every call (see MPPIDelay._ensure): a rebuilt or re-folded model handle
-        # must never be planned on silently
-        model_h = self._tpl._model_handle()
-        key = None if model_h is None else model_h.value
+        handles = self._model_handles()
+        delays = [int(d.delay) for d in self._dyns]
+        key = (None if handles is None else tuple(h.value for h in handles), tuple(delays))
         if self._handle is not None and self._handle_B == B and self._handle_model == key:
             return self._handle
         self._destroy()
         self._handle_model = key
         d = self._tpl._desc(B, self.K, 0, self.K, 1, 0)
         seeds = (C.c_uint64 * self.I)(*self.seeds)
+        models = None if handles is None else (C.c_void_p * self.I)(*key[0])
+        dl = (C.c_int32 * self.I)(*delays)
         h = C.c_void_p()
-        _lib.check(self._lib.nlc_batch_planner_create(C.byref(h), model_h, C.byref(d), self.I, seeds, self.d.index), "nlc_batch_planner_create")
+        _lib.check(self._lib.nlc_batch_planner_create_multi(C.byref(h), models, dl, C.byref(d), self.I, seeds, self.d.index),
+                   "nlc_batch_planner_create_multi")
         ptr, keep = _lib.as_double_array(self._U_host.numpy())
         _lib.check(self._lib.nlc_batch_planner_set_U(h, ptr), "nlc_batch_planner_set_U")
         self._handle, self._handle_B, self._views = h, B, {}
@@ -144,10 +192,53 @@ class BatchedMPPIDelay:
         return out.to(self.dtype)
 
 
+def _delays(action_delay, I, B, device):
+    """``action_delay`` as the env step takes it: an int (returned as is), or one delay per instance (a sequence or an integer
+    tensor of ``I`` entries, each in ``[0, B)``, checked here on the host) returned as an int32 CUDA tensor."""
+    d = torch.as_tensor(action_delay).detach().cpu()
+    if d.dim() == 0:
+        return int(action_delay)
+    if d.is_floating_point() or d.is_complex() or d.dtype == torch.bool:
+        raise TypeError("per-instance delays must be integers")
+    d = d.reshape(-1)
+    if d.numel() != I:
+        raise ValueError(f"action_delay must be an int or hold one delay per instance ({I}), got {d.numel()}")
+    if bool(((d < 0) | (d >= B)).any()):
+        raise ValueError(f"action delays {d.tolist()} must lie in [0, {B}) (the action buffer has {B} entries)")
+    return d.to(device=device, dtype=torch.int32)
+
+
+def _env_step(env_name, states, action_buffers, actions, delay, dt, rewards, status):
+    """The launch of :func:`env_step` on checked arguments: ``delay`` an int or the int32 CUDA tensor of ``_delays``,
+    ``status`` an int32 CUDA word (per-instance delays only; set to 1 by the kernel for an entry out of range)."""
+    I, B, nu = action_buffers.shape
+    lib, env, stream = _lib.load(), _lib.ENV_IDS[env_name], _lib.current_stream_ptr()
+    per_instance = torch.is_tensor(delay)
+    if states.dtype == torch.float64:
+        if per_instance:
+            _lib.check(lib.nlc_env_step_f64_delays(env, delay.data_ptr(), float(dt), states.data_ptr(), action_buffers.data_ptr(),
+                                                   actions.data_ptr(), I, B, nu, _lib.ptr(rewards), status.data_ptr(), stream),
+                       "nlc_env_step_f64_delays")
+        else:
+            _lib.check(lib.nlc_env_step_f64(env, delay, float(dt), states.data_ptr(), action_buffers.data_ptr(), actions.data_ptr(),
+                                            I, B, nu, _lib.ptr(rewards), stream), "nlc_env_step_f64")
+        return
+    ro = _lib.RolloutOpts()
+    ro.env, ro.state_constraint, ro.goal_x, ro.dynamics, ro.delay, ro.dt = env, 0, 0.0, _lib.DYN_ANALYTIC_DELAY, 0 if per_instance else delay, float(dt)
+    if per_instance:
+        _lib.check(lib.nlc_env_step_delays(C.byref(ro), delay.data_ptr(), states.data_ptr(), action_buffers.data_ptr(), actions.data_ptr(),
+                                           I, B, nu, _lib.ptr(rewards), status.data_ptr(), stream), "nlc_env_step_delays")
+    else:
+        _lib.check(lib.nlc_env_step(C.byref(ro), states.data_ptr(), action_buffers.data_ptr(), actions.data_ptr(), I, B, nu,
+                                    _lib.ptr(rewards), stream), "nlc_env_step")
+
+
 def env_step(env_name, states, action_buffers, actions, action_delay, dt=0.05, rewards=None):
     """``step_env`` (``mppi_with_model.py:193-216``) for I instances, in place on CUDA tensors: ``action_buffers``
     (I, B, nu) is rolled and receives ``actions`` (I, nu) (``get_action``, ``:25-28``), ``states`` (I, nx) advances by
     one Euler step of the true dynamics driven by the delayed action, ``rewards`` (I) receives the step reward.
+    ``action_delay`` is one int for every instance, or one delay per instance (a sequence or an integer tensor of I entries,
+    each in ``[0, B)``; checked on the host before the launch) - the reference's delay grid in one call.
 
     All tensors (``rewards`` if given) are contiguous and either all fp32 (``nlc_env_step``) or all fp64
     (``nlc_env_step_f64``: the reference's own precision and evaluation order, ``dt`` kept in fp64); anything else raises
@@ -159,15 +250,9 @@ def env_step(env_name, states, action_buffers, actions, action_delay, dt=0.05, r
         raise TypeError("env_step works in place on contiguous CUDA tensors, all fp32 or all fp64 (no CPU fallback)")
     I, B, nu = action_buffers.shape
     with torch.cuda.device(states.device):
-        if dtype == torch.float64:
-            _lib.check(_lib.load().nlc_env_step_f64(_lib.ENV_IDS[env_name], int(action_delay), float(dt), states.data_ptr(),
-                                                    action_buffers.data_ptr(), actions.data_ptr(), I, B, nu, _lib.ptr(rewards),
-                                                    _lib.current_stream_ptr()), "nlc_env_step_f64")
-            return
-        ro = _lib.RolloutOpts()
-        ro.env, ro.state_constraint, ro.goal_x, ro.dynamics, ro.delay, ro.dt = _lib.ENV_IDS[env_name], 0, 0.0, _lib.DYN_ANALYTIC_DELAY, int(action_delay), float(dt)
-        _lib.check(_lib.load().nlc_env_step(C.byref(ro), states.data_ptr(), action_buffers.data_ptr(), actions.data_ptr(), I, B, nu,
-                                            _lib.ptr(rewards), _lib.current_stream_ptr()), "nlc_env_step")
+        delay = _delays(action_delay, I, B, states.device)
+        status = torch.zeros(1, dtype=torch.int32, device=states.device) if torch.is_tensor(delay) else None
+        _env_step(env_name, states, action_buffers, actions, delay, dt, rewards, status)
 
 
 class _F64Instances:
@@ -218,7 +303,9 @@ def run_closed_loop(planner, env_name, states0, action_delay, n_steps, dt=0.05, 
     ``MPPIDelay(math_mode="fp64")`` objects, one per instance (``I = len(planner)``; they share ``nx``, ``nu``, the action
     buffer size and the device, and take ``u_per_command == 1``): then the state, the buffers and the rewards are fp64 like
     the reference's loop, each instance plans on its own planner and one fp64 ``env_step`` advances them all.
-    ``roll_outs`` / ``time_steps`` of the result are those of the first planner.
+    ``roll_outs`` / ``time_steps`` of the result are those of the first planner.  ``action_delay`` is one int or one delay per
+    instance (as :func:`env_step` takes it, checked before the first control step); the result's ``"delay"`` is then an
+    array of the I delays.
 
     NOT the reference environment's integrator: ``env_step`` takes ONE EXPLICIT EULER step of the dynamics as the
     reference's ``oracle.py`` states them (what its "oracle" planner model uses), whereas the reference's gym envs
@@ -230,6 +317,9 @@ def run_closed_loop(planner, env_name, states0, action_delay, n_steps, dt=0.05, 
     else:
         dtype = torch.float32
     I, B, nu, dev = planner.I, planner.B, planner.nu, planner.d
+    with torch.cuda.device(dev):
+        delay = _delays(action_delay, I, B, dev)  # checked once, before the first launch
+        status = torch.zeros(1, dtype=torch.int32, device=dev) if torch.is_tensor(delay) else None
     states = torch.as_tensor(states0).to(device=dev, dtype=dtype).reshape(I, planner.nx).clone()
     bufs = torch.zeros(I, B, nu, dtype=dtype, device=dev)
     total = torch.zeros(I, dtype=dtype, device=dev)
@@ -240,11 +330,13 @@ def run_closed_loop(planner, env_name, states0, action_delay, n_steps, dt=0.05, 
         actions = planner.command(states, bufs, None if noise_fn is None else noise_fn(it))
         torch.cuda.synchronize(dev)
         elapsed += time.perf_counter() - t0  # the reference's bracket (:255-264) around command()
-        env_step(env_name, states, bufs, actions.to(dtype).contiguous(), action_delay, dt, reward)
+        with torch.cuda.device(dev):
+            _env_step(env_name, states, bufs, actions.to(dtype).contiguous(), delay, dt, reward, status)
         total += reward
     torch.cuda.synchronize(dev)
     tot = total.double().cpu().numpy()
     return {"env_name": env_name, "roll_outs": planner.K, "time_steps": planner.T, "episode_elapsed_time": elapsed,
-            "episode_elapsed_time_per_it": elapsed / max(int(n_steps), 1), "dt": dt, "delay": action_delay, "planner": "mpc",
+            "episode_elapsed_time_per_it": elapsed / max(int(n_steps), 1), "dt": dt,
+            "delay": delay.cpu().numpy() if torch.is_tensor(delay) else action_delay, "planner": "mpc",
             "total_reward_raw": tot, "total_reward": tot * (200.0 / max(int(n_steps), 1)), "final_states": states.double().cpu().numpy(),
             "n_instances": I}
