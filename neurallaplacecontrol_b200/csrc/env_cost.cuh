@@ -78,6 +78,10 @@ __device__ __forceinline__ float env_running_cost_fast(const nlc_rollout_opts& o
   return -reward;
 }
 
+// torch.clamp of the reference's dynamics (oracle.py): a NaN action stays NaN, where fminf(fmaxf(u, lo), hi) would return lo.
+__device__ __forceinline__ float clamp_nan(float u, float lo, float hi) { return u != u ? u : fminf(fmaxf(u, lo), hi); }
+__device__ __forceinline__ double clamp_nan(double u, double lo, double hi) { return u != u ? u : fmin(fmax(u, lo), hi); }
+
 // One explicit-Euler step with the action delayed by `delay` entries (oracle.py:11-224, friction=False,
 // trigonometric observation form).  `u` points at window[-(delay+1)].
 __device__ __forceinline__ void env_analytic_step(const nlc_rollout_opts& o, float* s, const float* u) {
@@ -85,7 +89,7 @@ __device__ __forceinline__ void env_analytic_step(const nlc_rollout_opts& o, flo
   if (o.env == NLC_ENV_PENDULUM) {
     const float th = trig2angle(s[0], s[1]);
     const float thdot = s[2];
-    const float uu = fminf(fmaxf(u[0], -2.0f), 2.0f);
+    const float uu = clamp_nan(u[0], -2.0f, 2.0f);
     const float newth = th + thdot * ts;
     float sn, cs;
     sincosf(newth, &sn, &cs);
@@ -97,7 +101,7 @@ __device__ __forceinline__ void env_analytic_step(const nlc_rollout_opts& o, flo
     const float costheta = s[2] / C, sintheta = s[3] / C;
     const float theta = atan2f(sintheta / C, costheta / C);
     const float gravity = 9.8f, force_mag = 3.0f, masspole = 0.1f, total_mass = 1.1f, polemass_length = 0.1f;
-    const float uu = fminf(fmaxf(u[0], -3.0f), 3.0f);
+    const float uu = clamp_nan(u[0], -3.0f, 3.0f);
     const float force = uu * force_mag;
     const float temp = (force + polemass_length * theta_dot * theta_dot * sintheta) / total_mass;
     const float thetaacc = (gravity * sintheta - costheta * temp) / (1.0f * (4.0f / 3.0f - masspole * costheta * costheta / total_mass));
@@ -111,7 +115,7 @@ __device__ __forceinline__ void env_analytic_step(const nlc_rollout_opts& o, flo
     const float theta2 = trig2angle(s[2], s[3]);
     const float dtheta1 = s[4], dtheta2 = s[5];
     const float g = 9.8f, half_pi = 1.57079632679489662f;
-    const float u0 = fminf(fmaxf(u[0], -5.0f), 5.0f), u1 = fminf(fmaxf(u[1], -5.0f), 5.0f);
+    const float u0 = clamp_nan(u[0], -5.0f, 5.0f), u1 = clamp_nan(u[1], -5.0f, 5.0f);
     const float c2 = cosf(theta2), s2 = sinf(theta2);
     // m1=m2=1, l1=1, lc1=lc2=0.5, I1=I2=1
     const float d1 = 0.25f + (1.0f + 0.25f + c2) + 1.0f + 1.0f;
@@ -174,7 +178,7 @@ __device__ __forceinline__ void env_analytic_step(int env, double ts, double* s,
   if (env == NLC_ENV_PENDULUM) {
     const double th = trig2angle(s[0], s[1]);
     const double thdot = s[2];
-    const double uu = fmin(fmax(u[0], -2.0), 2.0);
+    const double uu = clamp_nan(u[0], -2.0, 2.0);
     const double newth = th + thdot * ts;
     const double newthdot = thdot + (-15.0 * sin(th + 3.141592653589793) + 3.0 * uu) * ts;
     double sn, cs;
@@ -185,7 +189,7 @@ __device__ __forceinline__ void env_analytic_step(int env, double ts, double* s,
     const double C = s[2] * s[2] + s[3] * s[3];
     const double costheta = s[2] / C, sintheta = s[3] / C;
     const double theta = atan2(sintheta / C, costheta / C);
-    const double force = fmin(fmax(u[0], -3.0), 3.0) * 3.0;
+    const double force = clamp_nan(u[0], -3.0, 3.0) * 3.0;
     const double total_mass = 0.1 + 1.0, pml = 0.1 * 1.0;
     const double temp = (force + pml * theta_dot * theta_dot * sintheta) / total_mass;
     const double thetaacc = (9.8 * sintheta - costheta * temp) / (1.0 * (4.0 / 3.0 - 0.1 * costheta * costheta / total_mass));
@@ -198,7 +202,7 @@ __device__ __forceinline__ void env_analytic_step(int env, double ts, double* s,
     const double th1 = trig2angle(s[0], s[1]);
     const double th2 = trig2angle(s[2], s[3]);
     const double d1_ = s[4], d2_ = s[5];
-    const double a0 = fmin(fmax(u[0], -5.0), 5.0), a1 = fmin(fmax(u[1], -5.0), 5.0);
+    const double a0 = clamp_nan(u[0], -5.0, 5.0), a1 = clamp_nan(u[1], -5.0, 5.0);
     const double c2 = cos(th2), s2 = sin(th2);
     // m1 = m2 = l1 = I1 = I2 = 1, lc1 = lc2 = 0.5, g = 9.8 (oracle/dynamics.py)
     const double d1 = 0.25 + (1.0 + 0.25 + 1.0 * c2) + 1.0 + 1.0;

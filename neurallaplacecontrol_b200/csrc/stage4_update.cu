@@ -22,6 +22,15 @@ __device__ __forceinline__ float ord2f(unsigned u) {
   return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
 }
 
+// Weight exp(-inv_lambda (c - beta)) of cost c against the minimum beta, as torch.exp gives it (mppi_delay.py:210-211): 0 for
+// a +inf cost - also when beta is +inf, i.e. every cost of a shard overflowed - and for an argument below the fp32 range of
+// exp (exp_acc's rounding-error FMA is NaN once x * log2(e) overflows, x < -2.4e38); a NaN cost stays NaN.  Every other
+// argument goes through exp_acc, which is 0 anyway below -104: the result is exp_acc's wherever that is finite.
+__device__ __forceinline__ float exp_weight(float c, float beta, float inv_lambda) {
+  const float x = -inv_lambda * (c - beta);
+  return (c == INFINITY || x < -104.0f) ? 0.0f : exp_acc(x);
+}
+
 struct SoftWs {           // workspace header (device)
   unsigned min_ord;       // ordered-uint encoding of the running min
   unsigned ticket;        // blocks finished in pass 2
@@ -75,7 +84,7 @@ __global__ void __launch_bounds__(256) softmax_sum_kernel(const float* __restric
     const int k = k0 + lane;
     float w = 0.0f;
     if (k < ke) {
-      w = exp_acc(-inv_lambda * (__ldg(cost + k) - beta));  // _ensure_non_zero, mppi_delay.py:12-13
+      w = exp_weight(__ldg(cost + k), beta, inv_lambda);  // _ensure_non_zero, mppi_delay.py:12-13
       if (weights) weights[k] = w;
     }
     eta += w;
@@ -188,10 +197,10 @@ __global__ void softmax_combine_kernel(const float* __restrict__ triples, int G,
   float beta = INFINITY;
   for (int g = 0; g < G; ++g) beta = fminf(beta, triples[g * stride]);
   float eta = 0.0f;
-  for (int g = 0; g < G; ++g) eta = fmaf(triples[g * stride + 1], exp_acc(-inv_lambda * (triples[g * stride] - beta)), eta);
+  for (int g = 0; g < G; ++g) eta = fmaf(triples[g * stride + 1], exp_weight(triples[g * stride], beta, inv_lambda), eta);
   for (int c = threadIdx.x; c < TN; c += blockDim.x) {
     float W = 0.0f;
-    for (int g = 0; g < G; ++g) W = fmaf(triples[g * stride + 2 + c], exp_acc(-inv_lambda * (triples[g * stride] - beta)), W);
+    for (int g = 0; g < G; ++g) W = fmaf(triples[g * stride + 2 + c], exp_weight(triples[g * stride], beta, inv_lambda), W);
     const float u = (tl.U_src ? tl.U_src[c] : U[c]) + W / eta;  // mppi_delay.py:214-216
     U[c] = u;
     if (c < nu && action) action[c] = u * u_scale;  // :217-224
@@ -231,10 +240,10 @@ __global__ void __launch_bounds__(128) softmax_combine_exchange_kernel(float* ma
   float beta = INFINITY;
   for (int g = 0; g < G; ++g) beta = fminf(beta, triples[g * stride]);
   float eta = 0.0f;
-  for (int g = 0; g < G; ++g) eta = fmaf(triples[g * stride + 1], exp_acc(-inv_lambda * (triples[g * stride] - beta)), eta);
+  for (int g = 0; g < G; ++g) eta = fmaf(triples[g * stride + 1], exp_weight(triples[g * stride], beta, inv_lambda), eta);
   for (int c = threadIdx.x; c < TN; c += blockDim.x) {
     float W = 0.0f;
-    for (int g = 0; g < G; ++g) W = fmaf(triples[g * stride + 2 + c], exp_acc(-inv_lambda * (triples[g * stride] - beta)), W);
+    for (int g = 0; g < G; ++g) W = fmaf(triples[g * stride + 2 + c], exp_weight(triples[g * stride], beta, inv_lambda), W);
     const float u = (tl.U_src ? tl.U_src[c] : U[c]) + W / eta;  // mppi_delay.py:214-216
     U[c] = u;
     if (c < nu && action) action[c] = u * u_scale;  // :217-224

@@ -100,9 +100,11 @@ def command(U, state, action_buffer, noise, dynamics, running_cost, *, noise_sig
 
 
 def shard_triple(cost_total, noise, lambda_):
-    """Per-shard partial of stage 4: (beta_g, eta_g, W_g[T,nu])."""
+    """Per-shard partial of stage 4: (beta_g, eta_g, W_g[T,nu]).  A +inf cost weighs 0 as in ``softmax_update``, also when
+    every cost of the shard is +inf (beta_g = +inf, where exp(-(inf - inf)) would be NaN): such a shard adds nothing."""
     beta = torch.min(cost_total)
     w = torch.exp(-(1.0 / lambda_) * (cost_total - beta))
+    w = torch.where(cost_total == float("inf"), torch.zeros_like(w), w)
     return beta, torch.sum(w), torch.einsum("k,ktu->tu", w, noise)
 
 

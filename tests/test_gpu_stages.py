@@ -93,7 +93,7 @@ def _softmax(cost, noise, lam, G):
     return triples, weights_out
 
 
-@pytest.mark.parametrize("K,T,nu", [(1, 1, 1), (7, 3, 2), (1000, 20, 1), (8192, 30, 1), (65536, 50, 2)])
+@pytest.mark.parametrize("K,T,nu", [(1, 1, 1), (7, 3, 2), (1000, 20, 1), (8192, 30, 1), (65536, 50, 2), (513, 256, 1), (300, 128, 2)])
 def test_softmax_update_and_shard_combine(K, T, nu):
     from oracle import mppi
 

@@ -95,6 +95,25 @@ def test_shard_combine_equals_unsharded():
         assert relerr(U_ref, U_sh) < 1e-13
 
 
+def test_shard_combine_with_an_all_infinite_shard():
+    """A shard whose every cost is +inf (beta_g = +inf) adds nothing to the combine: the same U as the unsharded update, in
+    which those samples weigh exp(-inf) = 0."""
+    g = torch.Generator().manual_seed(1)
+    K, T, nu = 96, 5, 2
+    cost = torch.rand(K, generator=g, dtype=torch.float64) * 30
+    noise = torch.randn(K, T, nu, generator=g, dtype=torch.float64)
+    U = torch.randn(T, nu, generator=g, dtype=torch.float64)
+    for G in (2, 3, 8):
+        idx = torch.tensor_split(torch.arange(K), G)
+        c = cost.clone()
+        c[idx[1]] = float("inf")
+        U_ref, _, _ = mppi.softmax_update(U, c, noise, 0.7)
+        assert torch.isfinite(U_ref).all()
+        U_sh, beta, _ = mppi.combine_shards(U, [mppi.shard_triple(c[i], noise[i], 0.7) for i in idx], 0.7)
+        assert float(beta) == float(c.min())
+        assert relerr(U_ref, U_sh) < 1e-13, G
+
+
 @pytest.mark.skipif(not ref_harness.available(), reason="reference tree not present")
 @pytest.mark.parametrize("env", ENVS)
 def test_live_reference_plan(env):
